@@ -8,6 +8,7 @@ no data-path collective => weak scaling).
 
     python bench.py [--gpus N] [--steps K] [--warmup W]          # this framework
     python bench.py --impl reference [...]                       # the reference's own CPU path
+    python bench.py [...] --dump-outputs DIR                     # + the last timed step's output as .npy
 
 For N > 1 launch one rank per GPU with torchrun (RANK/LOCAL_RANK/WORLD_SIZE/MASTER_* from env).
 Rank 0 prints ONE JSON line.
@@ -31,6 +32,8 @@ SIGMAS = (70.0, 50.0, 20.0)
 FLOP_PER_PIXEL = 33 * (2 * RADIUS + 1) ** 2 + 4
 BYTES_PER_PIXEL = 11  # depth f32 in + BGR u8x3 in + filtered f32 out
 FP32_NOMINAL_TFLOPS = 74.4  # 148 SM x 128 FMA/clk x 2 x 1.965 GHz
+# --dump-outputs: a fixed, seeded sample of the output frames; 48 x 640x480 f32 = 59 MB, under 64 MB in all
+DUMP_FRAMES, DUMP_SEED = 48, 2024
 
 
 def parse():
@@ -50,7 +53,15 @@ def parse():
     ap.add_argument("--config1", action="store_true",
                     help="configs[0] instead of the headline line: the bundled 640x480 frame, reference defaults "
                          "(window 5, 70/50/20), timed on the host cores and on the GPU, with parity figures")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the filtered depth the last timed step returned to "
+                         f"DIR/filtered.npy (float32 [n,H,W]: a fixed seeded sample of at most {DUMP_FRAMES} frames, "
+                         "rank 0's shard; with --config1 its one GPU frame) and their stream frame numbers to "
+                         "DIR/filtered_frame_index.npy (float64)")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    return args
 
 
 # ------------------------------------------------------------------ helpers
@@ -159,6 +170,18 @@ def profiled_pipes():
     return out
 
 
+def dump_outputs(dirname: str, filtered, first_frame: int = 0):
+    """--dump-outputs: `filtered` [N,H,W] (torch or numpy) is what the timed path returned in its last step.  The
+    inputs are seeded, so two builds run with the same arguments can be compared file for file."""
+    import numpy as np
+    n = filtered.shape[0]
+    idx = np.sort(np.random.default_rng(DUMP_SEED).choice(n, size=min(n, DUMP_FRAMES), replace=False))
+    sample = filtered[idx] if isinstance(filtered, np.ndarray) else filtered[idx.tolist()].cpu().numpy()
+    os.makedirs(dirname, exist_ok=True)
+    np.save(os.path.join(dirname, "filtered.npy"), np.ascontiguousarray(sample, dtype=np.float32))
+    np.save(os.path.join(dirname, "filtered_frame_index.npy"), (first_frame + idx).astype(np.float64))
+
+
 def cpu_baseline(budget_s: float, frames_np=None):
     """The reference's own kernel text on the host cores (oracle/_ref), else the C restatement (port)."""
     import numpy as np
@@ -203,7 +226,7 @@ def run_reference(args):
 
     def one_frame():
         g = oracle.presmooth(c)
-        oracle.jbf(d, g, 2 * RADIUS + 1, *SIGMAS, precision="f32", impl=impl, threads=cores)
+        return oracle.jbf(d, g, 2 * RADIUS + 1, *SIGMAS, precision="f32", impl=impl, threads=cores)
 
     t0 = time.perf_counter(); one_frame(); t1 = time.perf_counter() - t0
     total_steps = args.steps + args.warmup
@@ -214,8 +237,10 @@ def run_reference(args):
     t0 = time.perf_counter()
     for _ in range(args.steps):
         for _ in range(per_step):
-            one_frame()
+            last = one_frame()
     dt = time.perf_counter() - t0
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, last[None])   # every frame of this arm is frame 0 of the stream
     v = args.steps * per_step * W * H / dt / 1e6
     sample = f"{per_step} frame(s) per step of the 640x480 r=7 stream, {kind}, {cores} threads"
     print(json.dumps({
@@ -265,6 +290,8 @@ def run_config1(args):
     torch.cuda.synchronize()
     gpu_ms = e0.elapsed_time(e1) / 200
     out = f.getFiltered_Device().cpu().numpy()
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, out[None])
     o64 = oracle.jbf(depth, guide, 5, 70.0, 50.0, 20.0, precision="f64")
     err = np.abs(out.astype(np.float64) - o64)
     e32 = np.abs(cpu_out.astype(np.float64) - o64)
@@ -349,18 +376,17 @@ def e2e_leg(jbf, depth, bgr, out, ne, steps, world, dev, dist, u16: bool):
         dist.barrier()
     torch.cuda.synchronize()
     t0 = time.perf_counter()
-    e_steps = max(2, steps)
-    for _ in range(e_steps):
+    for _ in range(steps):
         jbf.process_host(dh, ch, oh)   # synchronous: returns when oh is complete
     torch.cuda.synchronize()
     dt = time.perf_counter() - t0
     te = torch.tensor([dt], device=dev, dtype=torch.float64)
     if world > 1:
         dist.all_reduce(te, op=dist.ReduceOp.MAX)
-    res = {"value": world * ne * W * H * e_steps / float(te.item()) / 1e6, "unit": "Mpixel/s",
+    res = {"value": world * ne * W * H * steps / float(te.item()) / 1e6, "unit": "Mpixel/s",
            "h2d_bytes_per_step": ne * W * H * (5 if u16 else 7), "d2h_bytes_per_step": ne * W * H * 4,
-           "frames_per_step": ne, "steps": e_steps,
-           "host_gbs_total": world * ne * W * H * (9 if u16 else 11) * e_steps / float(te.item()) / 1e9,
+           "frames_per_step": ne, "steps": steps,
+           "host_gbs_total": world * ne * W * H * (9 if u16 else 11) * steps / float(te.item()) / 1e9,
            "how": ("jbf_process_host_u16: pinned host depth (uint16 mm, the sensor's format) + BGR" if u16 else
                    "jbf_process_host: pinned host depth (f32) + BGR") +
                   " -> H2D -> pre-smooth + filter -> D2H, three-slot chunked pipeline on three streams, "
@@ -423,6 +449,8 @@ def main():
     e1.record()
     barrier()
     ms = e0.elapsed_time(e1)
+    if args.dump_outputs and rank == 0:   # before the kernel-only timing below overwrites `out`
+        dump_outputs(args.dump_outputs, out, first)
     refined_per_step = jbf.refine_stats()[0] / max(1, args.steps)
     # dominant kernel alone: the two-pass filter (+ its fp64 refinement launch) on the already smoothed guide,
     # same data, same stream
@@ -431,7 +459,7 @@ def main():
     k0, k1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     n_k = 0
     k0.record()
-    for _ in range(max(1, args.steps)):
+    for _ in range(args.steps):
         for f0 in range(0, n_frames - args.chunk + 1, args.chunk):
             jbf.filter_guide4(depth[f0:f0 + args.chunk], guide4, out[f0:f0 + args.chunk])
             n_k += 1

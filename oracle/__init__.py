@@ -31,7 +31,7 @@ MRF_WINDOW, MRF_SIGMA_C, MRF_SMOOTH = 5, 50.0, 150.0
 
 
 def build(force: bool = False) -> None:
-    """Compile the C restatement (and oracle/_ref when /root/reference is present)."""
+    """Compile the C restatement (and oracle/_ref where oracle/build_ref.py finds a reference checkout)."""
     src = os.path.join(_HERE, "kdme_oracle.c")
     if force or not os.path.isfile(_LIB_PATH) or os.path.getmtime(_LIB_PATH) < os.path.getmtime(src):
         subprocess.run(
@@ -96,7 +96,7 @@ def ref():
     global _ref
     if _ref is None:
         if not ref_available():
-            raise FileNotFoundError(_REF_PATH + " (run oracle/build_ref.py where /root/reference exists)")
+            raise FileNotFoundError(_REF_PATH + " (run oracle/build_ref.py with a reference checkout)")
         R = C.CDLL(_REF_PATH)
         R.ref_jbf.argtypes = [C.c_int, C.c_int, _f32p, _u8p, _f32p, _f32p, C.c_int, C.c_float, C.c_float,
                               C.c_int]

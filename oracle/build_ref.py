@@ -6,10 +6,13 @@ TEST INFRASTRUCTURE ONLY (see oracle/kdme_oracle.c header).
 The reference's hot-path kernels use nothing from OpenCV/OpenNI except
 ``GpuMat::data``, so their text compiles for the host behind a small shim
 (SURVEY.md 8(c)).  This script reads the cited line ranges from the sources
-WHERE THEY LIE under /root/reference, concatenates shim + text + drivers in
-memory and pipes the translation unit to ``g++ -x c++ -``.  The only output is
-``oracle/_ref/libkdme_ref.so`` (git-ignored, shipped to the GPU box by gpurun).
-No reference source is written into this repository.
+WHERE THEY LIE in a checkout of the reference -- $KDME_REFERENCE_ROOT, else a
+directory named ``reference`` beside this repository's checkout -- concatenates
+shim + text + drivers in memory and pipes the translation unit to
+``g++ -x c++ -``.  The only output is ``oracle/_ref/libkdme_ref.so``
+(git-ignored).  No reference source is written into this repository; where no
+reference checkout is found nothing is built and the committed golden vectors
+(tests/golden/ref_golden.npz) stand in for the reference.
 
 The reference's own build system (two MSVC .props files) is not run.
 """
@@ -19,7 +22,7 @@ import subprocess
 import sys
 
 HERE = os.path.dirname(os.path.abspath(__file__))
-REF = os.environ.get("KDME_REFERENCE_ROOT", "/root/reference")
+REF = os.environ.get("KDME_REFERENCE_ROOT") or os.path.join(os.path.dirname(os.path.dirname(HERE)), "reference")
 OUT_DIR = os.path.join(HERE, "_ref")
 OUT = os.path.join(OUT_DIR, "libkdme_ref.so")
 
@@ -49,10 +52,10 @@ def available() -> bool:
 
 
 def build(verbose: bool = True) -> str | None:
-    """Returns the path of the built library, or None when /root/reference is absent."""
+    """Returns the path of the built library, or None when the reference checkout is absent."""
     if not available():
         if verbose:
-            print(f"[build_ref] {REF} not present; keeping any prebuilt {OUT}")
+            print(f"[build_ref] reference checkout {REF} not present; keeping any prebuilt {OUT}")
         return OUT if os.path.isfile(OUT) else None
     parts = [open(os.path.join(HERE, "ref_shim_pre.h"), encoding="utf-8").read()]
     for rel, lo, hi, sha in RANGES:

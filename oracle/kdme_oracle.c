@@ -25,10 +25,10 @@
  * Parity pinning: the reference holds NO golden vectors, tests or fixtures for
  * this path (SURVEY.md section 4).  The restatement is pinned instead against
  * the reference's own kernel text compiled for the host (oracle/_ref, built by
- * oracle/build_ref.py from the sources where they lie under /root/reference):
- * tests/test_oracle.py asserts bit-for-bit equality in fp32 whenever
- * oracle/_ref is populated.  The third-party guide pre-smooth
- * (cv::gpu::bilateralFilter, OpenCV 2.4.3, not under /root/reference) is
+ * oracle/build_ref.py from the sources where they lie in a reference checkout):
+ * tests/test_oracle.py asserts bit-for-bit equality in fp32 against the
+ * committed golden vectors always, and live whenever oracle/_ref is populated.  The third-party guide pre-smooth
+ * (cv::gpu::bilateralFilter, OpenCV 2.4.3, not in the reference) is
  * "parity unpinned": restated from its published algorithm and cross-checked
  * against cv2.bilateralFilter (OpenCV 4.13 CPU) in tests/.
  *

@@ -4,7 +4,7 @@
  * TEST INFRASTRUCTURE ONLY (see oracle/kdme_oracle.c header).
  *
  * oracle/build_ref.py streams this file, then line ranges of the reference's
- * .cu sources read in place from /root/reference, then ref_shim_post.h, into
+ * .cu sources read in place from the reference checkout, then ref_shim_post.h, into
  * `g++ -x c++ -` and writes only oracle/_ref/libkdme_ref.so.  No reference
  * source text is copied into this repository.
  *

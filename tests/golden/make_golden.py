@@ -1,13 +1,13 @@
 #!/usr/bin/env python3
 """Generates tests/golden/*.npz from the REFERENCE'S OWN kernel text.
 
-Run in the build container, where /root/reference exists:
-    python tests/golden/make_golden.py
+Run with a checkout of the reference:
+    python tests/golden/make_golden.py     # checkout found as oracle/build_ref.py describes
 It builds oracle/_ref (the reference kernels compiled for the host, read in place from
-/root/reference by oracle/build_ref.py) and records their outputs on small seeded inputs.
+that checkout by oracle/build_ref.py) and records their outputs on small seeded inputs.
 The reference itself ships no golden vectors (SURVEY.md section 4); these fixtures pin the
-committed C restatement (oracle/kdme_oracle.c) to the reference on machines where
-/root/reference is absent (the GPU box).
+committed C restatement (oracle/kdme_oracle.c) to the reference wherever the reference
+checkout is absent.
 
 guide_frame_640x480.png holds the decoded pixels (cv2.imread(..., 1); pixel sha256 67e5a97a...1614c) of
 the reference's bundled sample frame input/color.jpg, written losslessly by this script; the matching
@@ -29,7 +29,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 
 
 def main():
-    assert build_ref.available(), "needs /root/reference"
+    assert build_ref.available(), "needs a reference checkout (see oracle/build_ref.py)"
     oracle.build(force=True)
     W, H = 96, 64
     d, c = synth.rgbd_frame(W, H, seed=77, frame=3)

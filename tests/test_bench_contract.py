@@ -5,9 +5,10 @@ import os
 import subprocess
 import sys
 
+import numpy as np
 import pytest
 
-from conftest import ROOT
+from conftest import ROOT, synth_np
 
 REQUIRED = ["metric", "value", "unit", "n_gpus", "steps", "warmup", "ms_per_step", "higher_is_better", "scaling",
             "vs_baseline", "dtype", "data", "config", "e2e", "gpu_launches"]
@@ -22,14 +23,35 @@ def _run(args, timeout=600):
     return json.loads(lines[0])
 
 
-def test_reference_arm_line():
-    line = _run(["--impl", "reference", "--steps", "1", "--warmup", "0"])
+def _dumped(dirname):
+    out = np.load(os.path.join(dirname, "filtered.npy"))
+    idx = np.load(os.path.join(dirname, "filtered_frame_index.npy"))
+    assert out.dtype == np.float32 and idx.dtype == np.float64
+    assert out.ndim == 3 and out.shape[1:] == (480, 640) and idx.shape == (out.shape[0],)
+    assert out.nbytes + idx.nbytes <= 64 * 10 ** 6
+    return out, idx.astype(np.int64)
+
+
+def test_reference_arm_line(tmp_path):
+    line = _run(["--impl", "reference", "--steps", "1", "--warmup", "0", "--dump-outputs", str(tmp_path)])
     for k in REQUIRED + ["impl", "cpu_baseline"]:
         assert k in line, k
     assert line["impl"] == "reference" and line["unit"] == "Mpixel/s" and line["higher_is_better"] is True
     assert line["value"] > 0 and line["cpu_baseline"]["kind"] in ("reference", "port")
     assert line["cpu_baseline"]["cores"] >= 1 and line["e2e"]["h2d_bytes_per_step"] == 0
     assert "workload" in line["config"] and "model" not in line["config"]
+    # the dump holds what the timed path computed: frame 0 of the seeded stream through pre-smooth + filter
+    import oracle
+    out, idx = _dumped(tmp_path)
+    d, c = synth_np(640, 480, seed=1234, frame=0)
+    assert idx.tolist() == [0]
+    assert np.array_equal(out[0], oracle.jbf_process(d, c, 15))
+
+
+def test_steps_must_be_positive():
+    res = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--impl", "reference", "--steps", "0"],
+                         capture_output=True, text=True, timeout=120, cwd=ROOT)
+    assert res.returncode != 0 and "--steps" in res.stderr and res.stdout == ""
 
 
 def test_reference_arm_non_zero_rank_is_silent():
@@ -58,11 +80,27 @@ def test_static_roofline_fields_parse_from_committed_profiles():
 
 
 @pytest.mark.gpu
-def test_gpu_arm_line():
+def test_gpu_arm_line(tmp_path):
     line = _run(["--frames", "256", "--steps", "2", "--warmup", "3", "--e2e-frames", "128", "--cpu-seconds", "3",
-                 "--band-size", "2048"], timeout=900)
+                 "--band-size", "2048", "--dump-outputs", str(tmp_path)], timeout=900)
     for k in REQUIRED + ["roofline", "cpu_baseline", "clocks", "parity", "extra", "e2e_u16"]:
         assert k in line, k
+    assert line["steps"] == 2 and line["e2e"]["steps"] == 2 and line["e2e_u16"]["steps"] == 2
+    # the dump: a seeded sample of the 256 frames the timed path returned, equal to filtering each frame alone
+    # (the stream tiles 64 distinct frames) and, independently of the kernels, within the north_star tolerance
+    # of the fp64 oracle
+    import oracle
+    from kinectdepthmapenhancement_b200 import JointBilateralFilter, synth
+    out, idx = _dumped(tmp_path)
+    assert len(set(idx.tolist())) == out.shape[0] == 48 and 0 <= idx.min() and idx.max() < 256
+    f = JointBilateralFilter(640, 480, window_radius=7)
+    for k in (0, out.shape[0] - 1):
+        d, c = synth.rgbd_frame(640, 480, seed=1234, frame=int(idx[k]) % 64, device="cuda")
+        f.Process(d, c)
+        assert np.array_equal(f.getFiltered_Device().cpu().numpy().view(np.uint32), out[k].view(np.uint32))
+    d, c = synth_np(640, 480, seed=1234, frame=int(idx[0]) % 64)
+    par = oracle.parity_block(out[0], d, oracle.presmooth(c), 15)
+    assert par["mask_mismatches"] == 0 and par["nan"] == 0 and par["max_abs_regular_mm"] <= 1e-3, par
     rf = line["roofline"]
     for k in ("bound", "achieved", "peak", "unit", "frac", "traffic"):
         assert k in rf, k
@@ -84,3 +122,18 @@ def test_gpu_arm_line():
     assert ex["bands_nccl"]["oracle_seam_check"]["max_abs_regular_mm"] <= 1e-3
     assert ex["single_frame"]["r7_us"] > 0 and ex["upsample"]["ms"] > 0 and len(ex["sweep"]["rows"]) == 13
     assert ex["strong"]["scaling"] == "strong"
+
+
+@pytest.mark.gpu
+def test_config1_dump(tmp_path):
+    """--config1 dumps its one GPU frame: the bundled colour frame + seeded surrogate depth, reference defaults."""
+    import cv2
+    import oracle
+    line = _run(["--config1", "--cpu-seconds", "0.5", "--dump-outputs", str(tmp_path)])
+    assert line["parity"]["mask_bit_exact"] is True
+    out, idx = _dumped(tmp_path)
+    assert idx.tolist() == [0] and out.shape[0] == 1
+    img = cv2.imread(os.path.join(ROOT, "tests", "golden", "guide_frame_640x480.png"), 1)
+    d, _ = synth_np(640, 480, seed=2013, frame=0)
+    par = oracle.parity_block(out[0], d, oracle.presmooth(img), 5)
+    assert par["mask_mismatches"] == 0 and par["nan"] == 0 and par["max_abs_regular_mm"] <= 1e-3, par

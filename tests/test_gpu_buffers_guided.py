@@ -101,7 +101,7 @@ def test_guided_fill_golden(golden_dir):
 
 def test_jbf_golden(golden_dir):
     """GPU vs the reference kernel text's own fp32 outputs (tests/golden/ref_golden.npz, generated from
-    /root/reference by make_golden.py), including the exotic-sigma cases where fp32 products underflow and
+    the reference checkout by make_golden.py), including the exotic-sigma cases where fp32 products underflow and
     flip `weight > 0` (colour guard at sigma_c = 20 -> generic kernel; spatial LUT underflowing to 0 at
     sigma_s = 0.5): the valid/hole mask must equal the reference's bit for bit, and every value must be as
     close to the reference's as the reference itself is to the exact (fp64) formula, + 1e-3 mm."""

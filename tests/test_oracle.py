@@ -62,7 +62,8 @@ def test_buffer2d_matches_reference_golden(gold):
 
 
 # ---------------------------------------------------------------- live check against oracle/_ref
-needs_ref = pytest.mark.skipif(not oracle.ref_available(), reason="oracle/_ref not built (no /root/reference)")
+needs_ref = pytest.mark.skipif(not oracle.ref_available(),
+                               reason="oracle/_ref not built (no reference checkout found)")
 
 
 @needs_ref

@@ -170,7 +170,7 @@ def _two_rank_worker(rank, world, port, size, q):
 
 
 @pytest.mark.gpu
-@pytest.mark.skipif(torch.cuda.device_count() < 2, reason="needs two GPUs on one NVLink box (gpurun --gpus 2)")
+@pytest.mark.skipif(torch.cuda.device_count() < 2, reason="needs two GPUs on one NVLink box")
 def test_real_two_rank_bands_nccl_and_peer_memory():
     """The real thing on two GPUs: NCCL send/recv halos and in-kernel peer-memory halos.  Every rank re-filters
     the rows on both sides of the seam without band logic (bit for bit), rank 0 checks the two seam rows against
