@@ -17,6 +17,7 @@ KDME_OK = 0
 KDME_EINVAL = -100001
 KDME_ENOTSUP = -100002
 KDME_MAX_RADIUS = 15
+KDME_GUIDE_GRAY, KDME_GUIDE_BGR, KDME_GUIDE_BGRX = 1, 3, 4
 
 
 class KdmeError(RuntimeError):
@@ -45,6 +46,7 @@ SIGNATURES = {
     "jbf_create": (_i, [C.POINTER(_vp), _i, _i, _f, _f, _f, _i, _i, _i, _vp]),
     "jbf_destroy": (None, [_vp]),
     "jbf_set_presmooth": (_i, [_vp, _i, _f, _f]),
+    "jbf_set_guide_channels": (_i, [_vp, _i]),
     "jbf_process": (_i, [_vp, _vp, _vp, _sz]),
     "jbf_process_xyz": (_i, [_vp, _vp, _vp, _sz, _vp, _f, _f, _i, _i]),
     "jbf_refine_stats": (_i, [_vp, C.POINTER(C.c_ulonglong), C.POINTER(C.c_ulonglong)]),
@@ -71,6 +73,8 @@ SIGNATURES = {
     "kdme_mean_3d_error": (_i, [_vp, _vp, C.c_longlong, C.POINTER(C.c_double), C.POINTER(C.c_longlong), _vp]),
     "kdme_guided_upsample": (_i, [_vp, _i, _i, _vp, _vp, _sz, _vp, _i, _i, _i, _f, _f, _f, _vp]),
     "kdme_guided_fill": (_i, [_vp, _vp, _vp, _sz, _vp, _i, _i, _i, _f, _f, _f, _vp]),
+    "kdme_guided_upsample_ex": (_i, [_vp, _i, _i, _vp, _vp, _sz, _i, _vp, _i, _i, _i, _f, _f, _f, _vp]),
+    "kdme_guided_fill_ex": (_i, [_vp, _vp, _vp, _sz, _i, _vp, _i, _i, _i, _f, _f, _f, _vp]),
     "buf2d_create": (_i, [C.POINTER(_vp), _i, _i, _i, _vp]),
     "buf2d_destroy": (None, [_vp]),
     "buf2d_init": (_i, [_vp]),

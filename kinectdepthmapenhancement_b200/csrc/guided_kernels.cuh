@@ -14,6 +14,10 @@
 // shared memory once.  Weights are evaluated as one ex2 of summed log2-domain terms
 // with the reference's skip-if-zero guards made explicit.
 //
+// The guide has C = 1 (GRAY), 3 (BGR) or 4 (BGRX) bytes per pixel; a GRAY pixel g is staged as
+// the word {g,0,0,0} and a BGRX pixel as {b,g,r,0}, so the colour distance is that of the BGR
+// image (g,0,0) or (b,g,r), bit for bit.
+//
 // mrf_kernel follows MarkovRandomField/MarkovRandomField.cu:4-40 (next row f1).
 #pragma once
 #include "common.cuh"
@@ -24,7 +28,7 @@ struct GuidedParams {
     int width, height, radius;
     const float* depth;
     const int32_t* labels;  // nullable
-    const uint8_t* bgr;     // RAW guide, packed BGR
+    const uint8_t* bgr;     // RAW guide, packed C-channel pixels (kernel template parameter C = 1, 3 or 4)
     long long bgr_step;
     float* out;
     float sigma_c, sigma_d;
@@ -43,7 +47,7 @@ __device__ __forceinline__ int guided_upsample_site(int x, int W, int wl) {
     return ((int)(((2LL * xl + 1) * W) / (2LL * wl)) == x) ? xl : -1;
 }
 
-template <int TW, int TH>
+template <int TW, int TH, int C>
 __global__ void __launch_bounds__(TW * TH) guided_fill_kernel(const __grid_constant__ GuidedParams p) {
     constexpr int NT = TW * TH;
     const int R = p.radius, WS = 2 * R + 1, SP = TW + 2 * R, SH = TH + 2 * R;
@@ -69,8 +73,9 @@ __global__ void __launch_bounds__(TW * TH) guided_fill_kernel(const __grid_const
             } else {
                 d = __ldg(p.depth + k);
             }
-            const uint8_t* q = p.bgr + (long long)gy * p.bgr_step + 3 * gx;
-            g = (uint32_t)__ldg(q) | ((uint32_t)__ldg(q + 1) << 8) | ((uint32_t)__ldg(q + 2) << 16);
+            const uint8_t* q = p.bgr + (long long)gy * p.bgr_step + C * gx;
+            if constexpr (C == 1) g = (uint32_t)__ldg(q);
+            else g = (uint32_t)__ldg(q) | ((uint32_t)__ldg(q + 1) << 8) | ((uint32_t)__ldg(q + 2) << 16);
             if (p.labels) l = __ldg(p.labels + k);
         }
         sD[idx] = (d > kValidDepth) ? d : 0.f;  // 0 marks "not a sample" (also out of bounds)
@@ -196,7 +201,7 @@ struct GuidedFastParams {
     float ltab[(2 * R + 1) * (2 * R + 1)];   // log2(S_ij) + kWeightBias, or kWeightBias where S_ij == 0
 };
 
-template <int R, int TW, int TH>
+template <int R, int TW, int TH, int C>
 __global__ void __launch_bounds__(TW * TH) guided_fill_fast_kernel(const __grid_constant__ GuidedFastParams<R> p) {
     constexpr int NT = TW * TH, WS = 2 * R + 1, SP = TW + 2 * R, SH = TH + 2 * R;
     static_assert(WS * WS <= 64, "the same-label mask is one 64-bit word");
@@ -220,8 +225,9 @@ __global__ void __launch_bounds__(TW * TH) guided_fill_fast_kernel(const __grid_
             } else {
                 d = __ldg(p.depth + k);
             }
-            const uint8_t* q = p.bgr + (long long)gy * p.bgr_step + 3 * gx;
-            g = (uint32_t)__ldg(q) | ((uint32_t)__ldg(q + 1) << 8) | ((uint32_t)__ldg(q + 2) << 16);
+            const uint8_t* q = p.bgr + (long long)gy * p.bgr_step + C * gx;
+            if constexpr (C == 1) g = (uint32_t)__ldg(q);
+            else g = (uint32_t)__ldg(q) | ((uint32_t)__ldg(q + 1) << 8) | ((uint32_t)__ldg(q + 2) << 16);
             if (p.labels) l = __ldg(p.labels + k);
         }
         sD[idx] = (d > kValidDepth) ? d : 0.f;

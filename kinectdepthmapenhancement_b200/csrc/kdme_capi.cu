@@ -122,7 +122,9 @@ struct jbf_handle {
     float* filtered_host = nullptr;  // Filtered_Host (pinned, lazy)
     uint32_t* guide4 = nullptr;      // smooth_Device in the internal u8x4 layout, max_batch frames
     int guide_pitch = 0;             // words
-    uint8_t* smooth_bgr = nullptr;   // packed copy for getSmoothImage_Device (lazy)
+    uint8_t* smooth_bgr = nullptr;   // copy in the guide's format for getSmoothImage_Device (lazy)
+    size_t smooth_bytes = 0;         // its size
+    int guide_channels = 3;          // bytes per pixel of every raw guide the handle reads (1, 3 or 4)
     float* ltab_dev = nullptr;       // fast layout [WS][LP]
     float* ltab_pairs_dev = nullptr; // packed-math layout [WS][LPP][2] = {L[i][j], L[i][j-1]}, j = 1..WS-1 (pass 2, bias 32)
     float* ltab_pairs1_dev = nullptr;// same layout for pass 1, bias `bias1`
@@ -470,19 +472,67 @@ extern "C" int jbf_set_presmooth(jbf_handle* h, int ksize, float sigma_color, fl
     return build_presmooth_luts(h);
 }
 
+extern "C" int jbf_set_guide_channels(jbf_handle* h, int channels) {
+    if (!h) return fail(KDME_EINVAL, "jbf_set_guide_channels: NULL handle");
+    if (channels != KDME_GUIDE_GRAY && channels != KDME_GUIDE_BGR && channels != KDME_GUIDE_BGRX)
+        return fail(KDME_EINVAL, "jbf_set_guide_channels: channels must be 1 (GRAY), 3 (BGR) or 4 (BGRX)");
+    h->guide_channels = channels;
+    return KDME_OK;
+}
+
+// Default (0) and minimum row step of a raw guide of the handle's format.
+static int guide_step(const jbf_handle* h, size_t* step, const char* who) {
+    const size_t row = (size_t)h->guide_channels * h->width;
+    if (*step == 0) *step = row;
+    if (*step < row)
+        return fail(KDME_EINVAL, std::string(who) + ": guide step smaller than " + std::to_string(h->guide_channels) +
+                                 "*width");
+    return KDME_OK;
+}
+
 // ------------------------------------------------------------------ launches
+template <int C>
+static void launch_guide4_convert(jbf_handle* h, const uint8_t* bgr, size_t bgr_step, long long bgr_frame_stride,
+                                  uint32_t* guide4, int guide_pitch, long long guide_frame_stride, int rows, int n) {
+    dim3 blk(128), grd((h->width + 127) / 128, rows, n);
+    bgr_to_guide4_kernel<C><<<grd, blk, 0, h->stream>>>(bgr, (long long)bgr_step, bgr_frame_stride, guide4, guide_pitch,
+                                                        guide_frame_stride, h->width, rows);
+}
+
+template <int C>
+static void launch_presmooth_c(jbf_handle* h, const PresmoothParams& p, int rows, int n) {
+    if (h->ps_ksize == 5) {
+        // 64x16 tiles, 128 threads, 4x2 pixels per thread; a launch too small to fill the GPU with them (one
+        // Kinect frame is 300) uses 64x8 tiles of 128 threads with 4x1 pixels: four times the warps
+        constexpr int TW = 64;
+        const long long ctas16 = (long long)((h->width + TW - 1) / TW) * ((rows + 15) / 16) * n;
+        if (ctas16 >= 148LL * 6) {
+            dim3 grd((h->width + TW - 1) / TW, (rows + 15) / 16, n);
+            presmooth5_kernel<TW, 16, 2, C><<<grd, (TW / 4) * 8, 0, h->stream>>>(p);
+        } else {
+            dim3 grd((h->width + TW - 1) / TW, (rows + 7) / 8, n);
+            presmooth5_kernel<TW, 8, 1, C><<<grd, (TW / 4) * 8, 0, h->stream>>>(p);
+        }
+    } else {
+        constexpr int TW = 32, TH = 8;
+        dim3 grd((h->width + TW - 1) / TW, (rows + TH - 1) / TH, n);
+        presmooth_kernel<TW, TH, C><<<grd, TW * TH, 0, h->stream>>>(p);
+    }
+}
+
 static int launch_presmooth(jbf_handle* h, const uint8_t* bgr, size_t bgr_step, uint32_t* guide4, int guide_pitch,
                             int n, int rows = -1, const uint8_t* bgr_up = nullptr, const uint8_t* bgr_dn = nullptr,
                             int band0 = 0, int band1 = 0) {
     if (rows < 0) rows = h->height;
-    if (bgr_step == 0) bgr_step = (size_t)3 * h->width;
-    if (bgr_step < (size_t)3 * h->width) return fail(KDME_EINVAL, "bgr step smaller than 3*width");
+    { int rc = guide_step(h, &bgr_step, "pre-smooth"); if (rc != KDME_OK) return rc; }
     if (h->ps_ksize == 0) {
         if (bgr_up || bgr_dn) return fail(KDME_ENOTSUP, "peer-memory halos need the guide pre-smooth enabled");
-        dim3 blk(128), grd((h->width + 127) / 128, rows, n);
-        bgr_to_guide4_kernel<<<grd, blk, 0, h->stream>>>(bgr, (long long)bgr_step, (long long)bgr_step * rows,
-                                                         guide4, guide_pitch, (long long)guide_pitch * rows,
-                                                         h->width, rows);
+        const long long bfs = (long long)bgr_step * rows, gfs = (long long)guide_pitch * rows;
+        switch (h->guide_channels) {
+            case 1: launch_guide4_convert<1>(h, bgr, bgr_step, bfs, guide4, guide_pitch, gfs, rows, n); break;
+            case 4: launch_guide4_convert<4>(h, bgr, bgr_step, bfs, guide4, guide_pitch, gfs, rows, n); break;
+            default: launch_guide4_convert<3>(h, bgr, bgr_step, bfs, guide4, guide_pitch, gfs, rows, n); break;
+        }
     } else {
         PresmoothParams p;
         p.width = h->width; p.height = rows; p.n_frames = n;
@@ -490,22 +540,10 @@ static int launch_presmooth(jbf_handle* h, const uint8_t* bgr, size_t bgr_step, 
         p.guide4 = guide4; p.guide_pitch = guide_pitch; p.guide_frame_stride = (long long)guide_pitch * rows;
         p.ksize = h->ps_ksize; p.space_lut = h->ps_space_dev; p.color_lut = h->ps_color_dev;
         p.bgr_up = bgr_up; p.bgr_dn = bgr_dn; p.band0 = band0; p.band1 = band1;
-        if (h->ps_ksize == 5) {
-            // 64x16 tiles, 128 threads, 4x2 pixels per thread; a launch too small to fill the GPU with them (one
-            // Kinect frame is 300) uses 64x8 tiles of 128 threads with 4x1 pixels: four times the warps
-            constexpr int TW = 64;
-            const long long ctas16 = (long long)((h->width + TW - 1) / TW) * ((rows + 15) / 16) * n;
-            if (ctas16 >= 148LL * 6) {
-                dim3 grd((h->width + TW - 1) / TW, (rows + 15) / 16, n);
-                presmooth5_kernel<TW, 16, 2><<<grd, (TW / 4) * 8, 0, h->stream>>>(p);
-            } else {
-                dim3 grd((h->width + TW - 1) / TW, (rows + 7) / 8, n);
-                presmooth5_kernel<TW, 8, 1><<<grd, (TW / 4) * 8, 0, h->stream>>>(p);
-            }
-        } else {
-            constexpr int TW = 32, TH = 8;
-            dim3 grd((h->width + TW - 1) / TW, (rows + TH - 1) / TH, n);
-            presmooth_kernel<TW, TH><<<grd, TW * TH, 0, h->stream>>>(p);
+        switch (h->guide_channels) {
+            case 1: launch_presmooth_c<1>(h, p, rows, n); break;
+            case 4: launch_presmooth_c<4>(h, p, rows, n); break;
+            default: launch_presmooth_c<3>(h, p, rows, n); break;
         }
     }
     CK(cudaGetLastError());
@@ -891,7 +929,7 @@ extern "C" int jbf_process_batch(jbf_handle* h, const float* depth_dev, const ui
                                  float* out_dev, int n_frames) {
     if (!h || !depth_dev || !bgr_dev || !out_dev) return fail(KDME_EINVAL, "jbf_process_batch: NULL argument");
     if (n_frames < 1) return fail(KDME_EINVAL, "jbf_process_batch: n_frames must be >= 1");
-    if (bgr_step == 0) bgr_step = (size_t)3 * h->width;
+    { int rc = guide_step(h, &bgr_step, "jbf_process_batch"); if (rc != KDME_OK) return rc; }
     DeviceGuard g(h->device);
     const size_t plane = (size_t)h->width * h->height;
     // more than one chunk: alternate the chunks between the caller's stream and the internal lane
@@ -999,10 +1037,9 @@ static int ensure_pipe(jbf_handle* h, size_t bgr_step) {
 
 static int process_host_impl(jbf_handle* h, const float* depth_host, const uint16_t* depth16_host,
                              const uint8_t* bgr_host, size_t bgr_step, float* out_host, int n_frames) {
-    if (bgr_step == 0) bgr_step = (size_t)3 * h->width;
-    if (bgr_step < (size_t)3 * h->width) return fail(KDME_EINVAL, "bgr step smaller than 3*width");
+    { int rc = guide_step(h, &bgr_step, "jbf_process_host"); if (rc != KDME_OK) return rc; }
     DeviceGuard g(h->device);
-    int rc = ensure_pipe(h, bgr_step);
+    int rc = ensure_pipe(h, bgr_step);   // re-sizes the guide slots when the guide's row bytes change
     if (rc != KDME_OK) return rc;
     const size_t plane = (size_t)h->width * h->height;
     const size_t bgr_frame = bgr_step * h->height;
@@ -1109,13 +1146,28 @@ extern "C" const uint8_t* jbf_guide4_device(jbf_handle* h, size_t* step) {
 extern "C" const uint8_t* jbf_smooth_device(jbf_handle* h, size_t* step) {
     if (!h) return nullptr;
     DeviceGuard g(h->device);
-    if (!h->smooth_bgr && cudaMalloc(&h->smooth_bgr, (size_t)h->width * h->height * 3) != cudaSuccess) {
-        fail(KDME_EINVAL, "jbf_smooth_device: cudaMalloc failed");
-        return nullptr;
+    const int C = h->guide_channels;
+    const size_t bytes = (size_t)h->width * h->height * C;
+    if (h->smooth_bytes != bytes) {
+        if (h->smooth_bgr && cudaStreamSynchronize(h->stream) != cudaSuccess) {
+            fail(KDME_EINVAL, "jbf_smooth_device: stream synchronisation failed");
+            return nullptr;
+        }
+        cudaFree(h->smooth_bgr);
+        h->smooth_bgr = nullptr; h->smooth_bytes = 0;
+        if (cudaMalloc(&h->smooth_bgr, bytes) != cudaSuccess) {
+            fail(KDME_EINVAL, "jbf_smooth_device: cudaMalloc failed");
+            return nullptr;
+        }
+        h->smooth_bytes = bytes;
     }
     dim3 blk(128), grd((h->width + 127) / 128, h->height);
-    guide4_to_bgr_kernel<<<grd, blk, 0, h->stream>>>(h->guide4, h->guide_pitch, h->smooth_bgr, h->width, h->height);
-    if (step) *step = (size_t)h->width * 3;
+    switch (C) {
+        case 1: guide4_to_image_kernel<1><<<grd, blk, 0, h->stream>>>(h->guide4, h->guide_pitch, h->smooth_bgr, h->width, h->height); break;
+        case 4: guide4_to_image_kernel<4><<<grd, blk, 0, h->stream>>>(h->guide4, h->guide_pitch, h->smooth_bgr, h->width, h->height); break;
+        default: guide4_to_image_kernel<3><<<grd, blk, 0, h->stream>>>(h->guide4, h->guide_pitch, h->smooth_bgr, h->width, h->height); break;
+    }
+    if (step) *step = (size_t)h->width * C;
     return h->smooth_bgr;
 }
 
@@ -1127,12 +1179,13 @@ extern "C" int jbf_mrf(jbf_handle* h, const float* depth_dev, const uint8_t* bgr
     if (!h || !depth_dev || !bgr_dev || !out_dev) return fail(KDME_EINVAL, "jbf_mrf: NULL argument");
     if (window_radius < 0 || window_radius > KDME_MAX_RADIUS) return fail(KDME_EINVAL, "jbf_mrf: bad radius");
     if (depth_dev == out_dev) return fail(KDME_EINVAL, "jbf_mrf: in-place operation is not supported");
-    if (bgr_step == 0) bgr_step = (size_t)3 * h->width;
-    if (bgr_step < (size_t)3 * h->width) return fail(KDME_EINVAL, "jbf_mrf: bgr step smaller than 3*width");
+    { int rc = guide_step(h, &bgr_step, "jbf_mrf"); if (rc != KDME_OK) return rc; }
     DeviceGuard g(h->device);
-    dim3 blk(128), grd((h->width + 127) / 128, h->height, 1);
-    bgr_to_guide4_kernel<<<grd, blk, 0, h->stream>>>(bgr_dev, (long long)bgr_step, 0, h->guide4, h->guide_pitch, 0,
-                                                     h->width, h->height);
+    switch (h->guide_channels) {
+        case 1: launch_guide4_convert<1>(h, bgr_dev, bgr_step, 0, h->guide4, h->guide_pitch, 0, h->height, 1); break;
+        case 4: launch_guide4_convert<4>(h, bgr_dev, bgr_step, 0, h->guide4, h->guide_pitch, 0, h->height, 1); break;
+        default: launch_guide4_convert<3>(h, bgr_dev, bgr_step, 0, h->guide4, h->guide_pitch, 0, h->height, 1); break;
+    }
     CK(cudaGetLastError());
     constexpr int TW = 32, TH = 8;
     const int SP = TW + 2 * window_radius, SH = TH + 2 * window_radius;
@@ -1223,7 +1276,7 @@ extern "C" int kdme_mean_3d_error(const float* points_dev, const float* truth_de
 }
 
 // ------------------------------------------------------------------ guided fill
-template <int R>
+template <int R, int C>
 static int guided_launch_fast(const float* depth_dev, const float* depth_lo_dev, int wl, int hl, const int32_t* labels_dev,
                               const uint8_t* bgr_dev, size_t bgr_step, float* out_dev, int width, int height,
                               const std::vector<float>& lut, float sigma_color, float sigma_depth, cudaStream_t stream) {
@@ -1239,16 +1292,15 @@ static int guided_launch_fast(const float* depth_dev, const float* depth_lo_dev,
     p.depth_lo = depth_lo_dev; p.wl = wl; p.hl = hl;
     constexpr int TW = 32, TH = 8;
     dim3 grd((width + TW - 1) / TW, (height + TH - 1) / TH);
-    guided_fill_fast_kernel<R, TW, TH><<<grd, TW * TH, 0, stream>>>(p);
+    guided_fill_fast_kernel<R, TW, TH, C><<<grd, TW * TH, 0, stream>>>(p);
     CK(cudaGetLastError());
     return KDME_OK;
 }
 
-static int guided_launch(const float* depth_dev, const float* depth_lo_dev, int wl, int hl, const int32_t* labels_dev,
-                         const uint8_t* bgr_dev, size_t bgr_step, float* out_dev, int width, int height,
-                         int window_radius, float sigma_spatial, float sigma_color, float sigma_depth, void* stream) {
-    if (bgr_step == 0) bgr_step = (size_t)3 * width;
-    if (bgr_step < (size_t)3 * width) return fail(KDME_EINVAL, "bgr step smaller than 3*width");
+template <int C>
+static int guided_launch_c(const float* depth_dev, const float* depth_lo_dev, int wl, int hl, const int32_t* labels_dev,
+                           const uint8_t* bgr_dev, size_t bgr_step, float* out_dev, int width, int height,
+                           int window_radius, float sigma_spatial, float sigma_color, float sigma_depth, void* stream) {
     const int ws = 2 * window_radius + 1;
     std::vector<float> lut;
     host_spatial_lut(lut, ws, sigma_spatial);
@@ -1257,9 +1309,9 @@ static int guided_launch(const float* depth_dev, const float* depth_lo_dev, int 
                          expf(-(float)(3 * 255 * 255) / (2 * (sigma_color * sigma_color))) != 0.0f;
     if (fast_ok) {
         switch (window_radius) {
-            case 1: return guided_launch_fast<1>(depth_dev, depth_lo_dev, wl, hl, labels_dev, bgr_dev, bgr_step, out_dev, width, height, lut, sigma_color, sigma_depth, (cudaStream_t)stream);
-            case 2: return guided_launch_fast<2>(depth_dev, depth_lo_dev, wl, hl, labels_dev, bgr_dev, bgr_step, out_dev, width, height, lut, sigma_color, sigma_depth, (cudaStream_t)stream);
-            case 3: return guided_launch_fast<3>(depth_dev, depth_lo_dev, wl, hl, labels_dev, bgr_dev, bgr_step, out_dev, width, height, lut, sigma_color, sigma_depth, (cudaStream_t)stream);
+            case 1: return guided_launch_fast<1, C>(depth_dev, depth_lo_dev, wl, hl, labels_dev, bgr_dev, bgr_step, out_dev, width, height, lut, sigma_color, sigma_depth, (cudaStream_t)stream);
+            case 2: return guided_launch_fast<2, C>(depth_dev, depth_lo_dev, wl, hl, labels_dev, bgr_dev, bgr_step, out_dev, width, height, lut, sigma_color, sigma_depth, (cudaStream_t)stream);
+            case 3: return guided_launch_fast<3, C>(depth_dev, depth_lo_dev, wl, hl, labels_dev, bgr_dev, bgr_step, out_dev, width, height, lut, sigma_color, sigma_depth, (cudaStream_t)stream);
             default: break;
         }
     }
@@ -1273,34 +1325,68 @@ static int guided_launch(const float* depth_dev, const float* depth_lo_dev, int 
     constexpr int TW = 32, TH = 8;
     const int SP = TW + 2 * window_radius, SH = TH + 2 * window_radius;
     dim3 grd((width + TW - 1) / TW, (height + TH - 1) / TH);
-    guided_fill_kernel<TW, TH><<<grd, TW * TH, (size_t)SP * SH * 12, (cudaStream_t)stream>>>(p);
+    guided_fill_kernel<TW, TH, C><<<grd, TW * TH, (size_t)SP * SH * 12, (cudaStream_t)stream>>>(p);
     CK(cudaGetLastError());
     return KDME_OK;
 }
 
-extern "C" int kdme_guided_fill(const float* depth_dev, const int32_t* labels_dev, const uint8_t* bgr_dev,
-                                size_t bgr_step, float* out_dev, int width, int height, int window_radius,
-                                float sigma_spatial, float sigma_color, float sigma_depth, void* stream) {
+static int guided_launch(const float* depth_dev, const float* depth_lo_dev, int wl, int hl, const int32_t* labels_dev,
+                         const uint8_t* bgr_dev, size_t bgr_step, int channels, float* out_dev, int width, int height,
+                         int window_radius, float sigma_spatial, float sigma_color, float sigma_depth, void* stream) {
+    if (channels != KDME_GUIDE_GRAY && channels != KDME_GUIDE_BGR && channels != KDME_GUIDE_BGRX)
+        return fail(KDME_EINVAL, "guided fill: guide_channels must be 1 (GRAY), 3 (BGR) or 4 (BGRX)");
+    if (bgr_step == 0) bgr_step = (size_t)channels * width;
+    if (bgr_step < (size_t)channels * width)
+        return fail(KDME_EINVAL, "guided fill: guide step smaller than " + std::to_string(channels) + "*width");
+#define KDME_GUIDED(C) guided_launch_c<C>(depth_dev, depth_lo_dev, wl, hl, labels_dev, bgr_dev, bgr_step, out_dev, width, \
+                                          height, window_radius, sigma_spatial, sigma_color, sigma_depth, stream)
+    switch (channels) {
+        case 1: return KDME_GUIDED(1);
+        case 4: return KDME_GUIDED(4);
+        default: return KDME_GUIDED(3);
+    }
+#undef KDME_GUIDED
+}
+
+extern "C" int kdme_guided_fill_ex(const float* depth_dev, const int32_t* labels_dev, const uint8_t* bgr_dev,
+                                   size_t bgr_step, int guide_channels, float* out_dev, int width, int height,
+                                   int window_radius, float sigma_spatial, float sigma_color, float sigma_depth,
+                                   void* stream) {
     if (!depth_dev || !bgr_dev || !out_dev) return fail(KDME_EINVAL, "kdme_guided_fill: NULL argument");
     if (width <= 0 || height <= 0) return fail(KDME_EINVAL, "kdme_guided_fill: bad size");
     if (window_radius < 0 || window_radius > KDME_MAX_RADIUS) return fail(KDME_EINVAL, "kdme_guided_fill: bad radius");
     if (depth_dev == out_dev) return fail(KDME_EINVAL, "kdme_guided_fill: in-place operation is not supported");
     { int rcd = check_pointer_device(depth_dev, "kdme_guided_fill"); if (rcd != KDME_OK) return rcd; }
-    return guided_launch(depth_dev, nullptr, 0, 0, labels_dev, bgr_dev, bgr_step, out_dev, width, height, window_radius,
-                         sigma_spatial, sigma_color, sigma_depth, stream);
+    return guided_launch(depth_dev, nullptr, 0, 0, labels_dev, bgr_dev, bgr_step, guide_channels, out_dev, width, height,
+                         window_radius, sigma_spatial, sigma_color, sigma_depth, stream);
+}
+
+extern "C" int kdme_guided_fill(const float* depth_dev, const int32_t* labels_dev, const uint8_t* bgr_dev,
+                                size_t bgr_step, float* out_dev, int width, int height, int window_radius,
+                                float sigma_spatial, float sigma_color, float sigma_depth, void* stream) {
+    return kdme_guided_fill_ex(depth_dev, labels_dev, bgr_dev, bgr_step, KDME_GUIDE_BGR, out_dev, width, height,
+                               window_radius, sigma_spatial, sigma_color, sigma_depth, stream);
+}
+
+extern "C" int kdme_guided_upsample_ex(const float* depth_lo_dev, int wl, int hl, const int32_t* labels_hi_dev,
+                                       const uint8_t* bgr_hi_dev, size_t bgr_step, int guide_channels, float* out_hi_dev,
+                                       int width, int height, int window_radius, float sigma_spatial, float sigma_color,
+                                       float sigma_depth, void* stream) {
+    if (!depth_lo_dev || !bgr_hi_dev || !out_hi_dev) return fail(KDME_EINVAL, "kdme_guided_upsample: NULL argument");
+    if (width <= 0 || height <= 0 || wl <= 0 || hl <= 0 || wl > width || hl > height)
+        return fail(KDME_EINVAL, "kdme_guided_upsample: low-res size must be positive and <= the high-res size");
+    if (window_radius < 0 || window_radius > KDME_MAX_RADIUS) return fail(KDME_EINVAL, "kdme_guided_upsample: bad radius");
+    { int rcd = check_pointer_device(depth_lo_dev, "kdme_guided_upsample"); if (rcd != KDME_OK) return rcd; }
+    return guided_launch(nullptr, depth_lo_dev, wl, hl, labels_hi_dev, bgr_hi_dev, bgr_step, guide_channels, out_hi_dev,
+                         width, height, window_radius, sigma_spatial, sigma_color, sigma_depth, stream);
 }
 
 extern "C" int kdme_guided_upsample(const float* depth_lo_dev, int wl, int hl, const int32_t* labels_hi_dev,
                                     const uint8_t* bgr_hi_dev, size_t bgr_step, float* out_hi_dev, int width,
                                     int height, int window_radius, float sigma_spatial, float sigma_color,
                                     float sigma_depth, void* stream) {
-    if (!depth_lo_dev || !bgr_hi_dev || !out_hi_dev) return fail(KDME_EINVAL, "kdme_guided_upsample: NULL argument");
-    if (width <= 0 || height <= 0 || wl <= 0 || hl <= 0 || wl > width || hl > height)
-        return fail(KDME_EINVAL, "kdme_guided_upsample: low-res size must be positive and <= the high-res size");
-    if (window_radius < 0 || window_radius > KDME_MAX_RADIUS) return fail(KDME_EINVAL, "kdme_guided_upsample: bad radius");
-    { int rcd = check_pointer_device(depth_lo_dev, "kdme_guided_upsample"); if (rcd != KDME_OK) return rcd; }
-    return guided_launch(nullptr, depth_lo_dev, wl, hl, labels_hi_dev, bgr_hi_dev, bgr_step, out_hi_dev, width, height,
-                         window_radius, sigma_spatial, sigma_color, sigma_depth, stream);
+    return kdme_guided_upsample_ex(depth_lo_dev, wl, hl, labels_hi_dev, bgr_hi_dev, bgr_step, KDME_GUIDE_BGR, out_hi_dev,
+                                   width, height, window_radius, sigma_spatial, sigma_color, sigma_depth, stream);
 }
 
 // ------------------------------------------------------------------ Buffer2D
