@@ -16,7 +16,7 @@
  * Guide formats: Process, ProcessXYZ and Upsampling take the guide's format from
  * color_image.channels(): CV_8UC3 BGR (the reference's), CV_8UC4 BGRX/BGRA (Kinect v2, Azure
  * Kinect colour frames; the 4th byte is ignored) or CV_8UC1 GRAY/IR (filters as the BGR image
- * (g,0,0)).  The pointer-based ProcessBatch / ProcessHost read the format set by setGuideChannels
+ * (g,0,0)).  The pointer-based ProcessBatch / ProcessHost / UpsamplingBatch read the format set by setGuideChannels
  * (default 3).  getSmoothImage_Device returns the smoothed guide in the format of the last call.
  */
 #ifndef KDME_JOINT_BILATERALFILTER_H
@@ -78,6 +78,17 @@ public:
                       int n_frames) {
         check(jbf_process_batch(h_, depth_device, bgr_device, bgr_step, out_device, n_frames));
     }
+    /* n_frames Upsampling calls: low-res frames back to back (float or uint16 millimetres, the ToF sensor's
+     * format), guides height*bgr_step bytes apart, n_frames high-res planes out. */
+    void UpsamplingBatch(const float* depthlow_device, int low_width, int low_height, const unsigned char* bgr_device,
+                         size_t bgr_step, float* out_device, int n_frames) {
+        check(jbf_upsample_batch(h_, depthlow_device, low_width, low_height, bgr_device, bgr_step, out_device, n_frames));
+    }
+    void UpsamplingBatch(const unsigned short* depthlow_device, int low_width, int low_height,
+                         const unsigned char* bgr_device, size_t bgr_step, float* out_device, int n_frames) {
+        check(jbf_upsample_batch_u16(h_, depthlow_device, low_width, low_height, bgr_device, bgr_step, out_device,
+                                     n_frames));
+    }
     /* Process + DimensionConvertor::projectiveToReal fused (main.cpp:179 + :182): xyz_device = float3[W*H]. */
     void ProcessXYZ(float* depth_device, cv::gpu::GpuMat color_image, float* xyz_device, float fx, float fy, int cx, int cy) {
         useGuide(color_image);
@@ -90,7 +101,7 @@ public:
     void ProcessHost(const unsigned short* depth_host, const unsigned char* bgr_host, size_t bgr_step, float* out_host, int n_frames) {
         check(jbf_process_host_u16(h_, depth_host, bgr_host, bgr_step, out_host, n_frames));
     }
-    /* Guide format (1 GRAY, 3 BGR, 4 BGRX) of the pointer-based calls ProcessBatch / ProcessHost. */
+    /* Guide format (1 GRAY, 3 BGR, 4 BGRX) of the pointer-based calls ProcessBatch / ProcessHost / UpsamplingBatch. */
     void setGuideChannels(int channels) {
         if (channels != Channels) { check(jbf_set_guide_channels(h_, channels)); Channels = channels; }
     }

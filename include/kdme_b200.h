@@ -64,7 +64,8 @@ typedef struct jbf_handle jbf_handle;
  *   WindowSize/SpatialSigma/ColorSigma/DepthSigma (.cpp:3-6) become arguments
  *   (reference values: radius 2, 70, 50, 20).  Builds the spatial LUT
  *   (calcSpatialFilter, .cpp:31-40) and owns Filtered_Device / smooth_Device.
- *   max_batch >= 1 sizes the internal smoothed-guide buffer for jbf_process_batch. */
+ *   max_batch >= 1 sizes the internal smoothed-guide buffer for jbf_process_batch, and with it the
+ *   chunks of jbf_upsample_batch / jbf_upsample_batch_u16. */
 int jbf_create(jbf_handle **out, int width, int height, float sigma_spatial, float sigma_color,
                float sigma_depth, int window_radius, int max_batch, int device, void *stream);
 
@@ -76,7 +77,8 @@ void jbf_destroy(jbf_handle *h);
 int jbf_set_presmooth(jbf_handle *h, int ksize, float sigma_color, float sigma_spatial);
 
 /* Format of the raw guide every later call on this handle reads (jbf_process, _batch, _xyz, _host,
- * _host_u16, jbf_presmooth, _presmooth_rows, _presmooth_rows_p2p, jbf_upsample, jbf_mrf):
+ * _host_u16, jbf_presmooth, _presmooth_rows, _presmooth_rows_p2p, jbf_upsample, _upsample_batch,
+ * _upsample_batch_u16, jbf_mrf):
  * KDME_GUIDE_GRAY, KDME_GUIDE_BGR (the default) or KDME_GUIDE_BGRX; any other value is KDME_EINVAL.
  * Handle state only: no synchronisation, no allocation (the host pipeline's guide slots and the
  * jbf_smooth_device buffer are re-sized when next used). */
@@ -192,6 +194,20 @@ const uint8_t *jbf_guide4_device(jbf_handle *h, size_t *step);
  * an input: the scatter happens while staging tiles. */
 int jbf_upsample(jbf_handle *h, const float *depth_lo_dev, int wl, int hl, const uint8_t *bgr_hi_dev,
                  size_t bgr_step, float *out_hi_dev);
+
+/* n_frames independent Upsampling calls (a recorded ToF sequence in one call).  Frame strides: wl*hl depth
+ * samples, height*bgr_step guide bytes, width*height output floats.  Chunks of max_batch frames; with more
+ * than one chunk the chunks alternate between the handle's stream and the internal lane, with
+ * jbf_process_batch's stream semantics.  Frame k of the result equals jbf_upsample of frame k alone, bit for
+ * bit.  KDME_EINVAL: n_frames < 1, a NULL pointer, wl / hl outside [1, width] / [1, height], a guide step
+ * below C*width. */
+int jbf_upsample_batch(jbf_handle *h, const float *depth_lo_dev, int wl, int hl, const uint8_t *bgr_hi_dev,
+                       size_t bgr_step, float *out_hi_dev, int n_frames);
+/* The same with sensor depth: uint16 millimetres (Kinect v2, Azure Kinect), read directly by the kernels
+ * (no conversion pass); a sample s filters exactly as the float (float)s, so values <= 50 are holes as
+ * before. */
+int jbf_upsample_batch_u16(jbf_handle *h, const uint16_t *depth_lo_dev, int wl, int hl, const uint8_t *bgr_hi_dev,
+                           size_t bgr_step, float *out_hi_dev, int n_frames);
 
 /* Which kernel the handle selected: 0 = register-tiled fast path, 1 = generic path
  * (exotic sigmas / radius); bit 8 (0x100) set when the last launch staged tiles by TMA,

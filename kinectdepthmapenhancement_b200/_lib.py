@@ -66,6 +66,8 @@ SIGNATURES = {
     "jbf_smooth_device": (_vp, [_vp, C.POINTER(_sz)]),
     "jbf_guide4_device": (_vp, [_vp, C.POINTER(_sz)]),
     "jbf_upsample": (_i, [_vp, _vp, _i, _i, _vp, _sz, _vp]),
+    "jbf_upsample_batch": (_i, [_vp, _vp, _i, _i, _vp, _sz, _vp, _i]),
+    "jbf_upsample_batch_u16": (_i, [_vp, _vp, _i, _i, _vp, _sz, _vp, _i]),
     "jbf_kernel_variant": (_i, [_vp]),
     "jbf_mrf": (_i, [_vp, _vp, _vp, _sz, _vp, _i, _f, _f]),
     "kdme_projective_to_real": (_i, [_vp, _vp, _i, _i, _f, _f, _i, _i, _vp]),

@@ -62,7 +62,9 @@ struct JbfParams {
     float flag_scale;            // a pixel is refined in fp64 when den < wsum * flag_scale (ill-conditioned)
     double kc, kd;               // 1/(2 sigma_c^2), 1/(2 sigma_d^2) (fp64 refinement path)
     int mode;                    // StageMode
-    const float* depth_lo;       // upsample: low-res depth [hl][wl]
+    const float* depth_lo;       // upsample: low-res depth [n][hl][wl] ...
+    const uint16_t* depth_lo16;  // ... or, when non-null, the same as uint16 millimetres (read through upsample_sample)
+    long long lo_frame_stride;   // samples per low-res frame (wl * hl)
     int wl, hl;
     const int* ups_inv_x;        // upsample, optional: low-res column landing on high-res column x, or -1 ([width]); null = compute
     const int* ups_inv_y;        // same for rows ([height])
@@ -123,6 +125,13 @@ __device__ __forceinline__ int upsample_site(int x, int W, int wl) {
     int xl = (num <= 0) ? 0 : (int)((num + 2LL * W - 1) / (2LL * W));
     if (xl >= wl) return -1;
     return ((int)(((2LL * xl + 1) * W) / (2LL * wl)) == x) ? xl : -1;
+}
+
+// low-res sample (xl, yl) of `frame`: every upsampling kernel reads the low-res depth through here.  A uint16
+// sample s reads as the float (float)s, exactly (s <= 50 is a hole, as for the float input).
+__device__ __forceinline__ float upsample_sample(const JbfParams& p, int frame, int xl, int yl) {
+    const long long i = (long long)frame * p.lo_frame_stride + (long long)yl * p.wl + xl;
+    return p.depth_lo16 ? (float)__ldg(p.depth_lo16 + i) : __ldg(p.depth_lo + i);
 }
 
 // pass-1 row sums are first added plainly in groups of this many window rows, the group sums are then
@@ -233,7 +242,7 @@ __device__ __forceinline__ void jbf_fast_body(const CUtensorMap& tm_depth, const
                     d = __ldg(row + gx);
                 } else {  // scatter the low-res sample onto its high-res site
                     const int xl = colmap[sx], yl = rowmap[sy];
-                    if ((xl >= 0) & (yl >= 0)) d = __ldg(p.depth_lo + (long long)yl * p.wl + xl);
+                    if ((xl >= 0) & (yl >= 0)) d = upsample_sample(p, frame, xl, yl);
                 }
             }
             sD[idx] = d;
@@ -645,7 +654,8 @@ jbf_fast_kernel(const __grid_constant__ CUtensorMap tm_depth, const __grid_const
 // sweeps site rows x site columns.  The arithmetic per pixel is the dense kernel's, tap for tap and in the
 // same order (taps that are not sites have weight exactly 0 there and add nothing), so the result equals
 // jbf_fast_kernel on the materialised sparse image BIT FOR BIT -- including the accumulation origin rule,
-// the 2Sum row partials and the fp64 refinement queue.
+// the 2Sum row partials and the fp64 refinement queue.  Frames of a batch are blockIdx.z; every frame shares the
+// lattice tables, and its low-res depth is read through upsample_sample (float or uint16).
 // padding of a pair-table row of the gather kernel: entries for window columns -2 .. WS+4 (WS + 7 is even, so a
 // table is a whole number of 16-byte words)
 constexpr int kUpsPad = 7;
@@ -740,7 +750,9 @@ jbf_upsample_gather_kernel(const JbfParams p, const UpsampleGeom g) {
     int* sYs = sXs + g.ncol_max;                                         // [nrow_max] site y
 
     const int tid = threadIdx.x;
-    const int x0 = blockIdx.x * TW, y0 = blockIdx.y * TH;
+    const int x0 = blockIdx.x * TW, y0 = blockIdx.y * TH, frame = blockIdx.z;
+    const uint32_t* gsrc = p.guide4 + (long long)frame * p.guide_frame_stride;
+    const long long fpix = (long long)frame * p.width * p.out_rows;   // first output pixel of the frame
     for (int idx = tid; idx < WS * LPW / 2; idx += NT) {
         reinterpret_cast<float4*>(sL1)[idx] = __ldg(reinterpret_cast<const float4*>(g.ltab1) + idx);
         reinterpret_cast<float4*>(sL2)[idx] = __ldg(reinterpret_cast<const float4*>(g.ltab2) + idx);
@@ -758,9 +770,9 @@ jbf_upsample_gather_kernel(const JbfParams p, const UpsampleGeom g) {
     __syncthreads();
     for (int idx = tid; idx < ncol * nrow; idx += NT) {
         const int sr = idx / ncol, sc = idx - sr * ncol;
-        const float d = __ldg(p.depth_lo + (long long)(yl0 + sr) * p.wl + (xl0 + sc));
+        const float d = upsample_sample(p, frame, xl0 + sc, yl0 + sr);
         sSd[sr * g.ncol_max + sc] = (d > kValidDepth) ? d : 0.f;
-        sSg[sr * g.ncol_max + sc] = __ldg(p.guide4 + (long long)sYs[sr] * p.guide_pitch + sXs[sc]);
+        sSg[sr * g.ncol_max + sc] = __ldg(gsrc + (long long)sYs[sr] * p.guide_pitch + sXs[sc]);
     }
     __syncthreads();
 
@@ -770,7 +782,7 @@ jbf_upsample_gather_kernel(const JbfParams p, const UpsampleGeom g) {
     if (gy < p.height) {
 #pragma unroll
         for (int k = 0; k < 4; ++k)
-            if (gx + k < p.width) gp[k] = __ldg(p.guide4 + (long long)gy * p.guide_pitch + gx + k);
+            if (gx + k < p.width) gp[k] = __ldg(gsrc + (long long)gy * p.guide_pitch + gx + k);
     }
     // this thread's site rows [r_lo, r_hi) and site columns [c_lo, c_hi) (union over its 4 pixels)
     // (the lattice is near-uniform: start from the proportional guess and correct by a step or two instead of
@@ -934,11 +946,11 @@ jbf_upsample_gather_kernel(const JbfParams p, const UpsampleGeom g) {
             if ((m[k] >> lane) & 1u) {
                 const unsigned slot = base + (unsigned)before;
                 ++before;
-                if (slot < p.q_capacity) p.q_items[slot] = (unsigned)((long long)gy * p.width + gx + k);
+                if (slot < p.q_capacity) p.q_items[slot] = (unsigned)(fpix + (long long)gy * p.width + gx + k);
             }
     }
     if (gy < p.height && gx < p.width) {
-        float* dst = p.out + (long long)gy * p.width + gx;
+        float* dst = p.out + fpix + (long long)gy * p.width + gx;
         if (gx + 3 < p.width && ((reinterpret_cast<uintptr_t>(dst) & 15) == 0)) {
             stg_stream_f4(reinterpret_cast<float4*>(dst), make_float4(o[0], o[1], o[2], o[3]));
         } else {
@@ -978,7 +990,7 @@ __device__ __forceinline__ float jbf_sample_depth(const JbfParams& p, int frame,
     if (p.mode == kStageUpsample) {
         const int xl = p.ups_inv_x ? __ldg(p.ups_inv_x + gx) : upsample_site(gx, p.width, p.wl);
         const int yl = p.ups_inv_y ? __ldg(p.ups_inv_y + gy) : upsample_site(gy, p.height, p.hl);
-        return ((xl >= 0) & (yl >= 0)) ? __ldg(p.depth_lo + (long long)yl * p.wl + xl) : 0.f;
+        return ((xl >= 0) & (yl >= 0)) ? upsample_sample(p, frame, xl, yl) : 0.f;
     }
     const float* row = p.depth + (long long)frame * p.depth_frame_stride + (long long)gy * p.width;
     if (p.depth_up != nullptr && gy < p.band0) row = p.depth_up + (long long)gy * p.width;
@@ -1161,7 +1173,7 @@ jbf_generic_kernel(const JbfGenericParams gp_) {
             if (p.mode == kStageUpsample) {
                 int xl = upsample_site(gx, p.width, p.wl);
                 int yl = upsample_site(gy, p.height, p.hl);
-                if ((xl >= 0) & (yl >= 0)) d = __ldg(p.depth_lo + (long long)yl * p.wl + xl);
+                if ((xl >= 0) & (yl >= 0)) d = upsample_sample(p, frame, xl, yl);
             } else {
                 d = __ldg(dsrc + (long long)gy * p.width + gx);
             }

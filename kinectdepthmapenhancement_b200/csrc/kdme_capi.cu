@@ -654,10 +654,60 @@ static bool fast_radius_available(int r) {
     }
 }
 
+// Upsampling runs in gather form (jbf_upsample_gather_kernel, tiles kUpsTW x kUpsTH) on the fast path unless the
+// dense form is asked for (KDME_UPSAMPLE_DENSE), the back-projection epilogue is on, or the staged sites of a tile
+// would not fit in shared memory.  Fills the launch geometry except the lattice pointers.
+constexpr int kUpsTW = 64, kUpsTH = 16;
+static bool ups_gather_form(const jbf_handle* h, int wl, int hl, int rows, bool xyz, UpsampleGeom* g, size_t* smem) {
+    if (!h->fast || xyz || getenv("KDME_UPSAMPLE_DENSE")) return false;
+    g->radius = h->radius;
+    g->ncol_max = (int)(((long long)(kUpsTW + 2 * h->radius) * wl + h->width - 1) / h->width) + 2;
+    g->nrow_max = (int)(((long long)(kUpsTH + 2 * h->radius) * hl + rows - 1) / rows) + 2;
+    g->ltab1 = h->ltab_ups1_dev;
+    g->ltab2 = h->ltab_ups2_dev;
+    const int ws = 2 * h->radius + 1;
+    *smem = (size_t)g->ncol_max * g->nrow_max * 8 + (size_t)(g->ncol_max + g->nrow_max + 1) * 4 +
+            (size_t)ws * (ws + kUpsPad) * 16 + 16;
+    return *smem <= 200 * 1024;
+}
+
+// The site lattice of (wl, hl) in frames of `rows` rows for the gather form, tabulated once (no 64-bit division is
+// left in the kernel): site_x[wl], site_y[hl], tile_xl[tiles_x][2], tile_yl[tiles_y][2], then the inverse maps of
+// the fp64 refinement.  Shared by both chunk lanes: a rebuild synchronises the handle's stream before it frees the
+// old table, so it runs on the caller's stream before any chunk is forked to the internal lane.
+static int ensure_ups_table(jbf_handle* h, int wl, int hl, int rows) {
+    if (h->ups_tab_dev && h->ups_wl == wl && h->ups_hl == hl && h->ups_rows == rows) return KDME_OK;
+    const int W = h->width, ntx = (W + kUpsTW - 1) / kUpsTW, nty = (rows + kUpsTH - 1) / kUpsTH;
+    std::vector<int> tab((size_t)wl + hl + 2 * (size_t)(ntx + nty) + (size_t)W + rows, -1);
+    for (int x = 0; x < wl; ++x) tab[x] = (int)(((2LL * x + 1) * W) / (2LL * wl));
+    for (int y = 0; y < hl; ++y) tab[(size_t)wl + y] = (int)(((2LL * y + 1) * rows) / (2LL * hl));
+    int* tx = tab.data() + wl + hl;
+    int* ty = tx + 2 * ntx;
+    for (int b = 0; b < ntx; ++b) {
+        tx[2 * b] = upsample_first_site_at_or_after(b * kUpsTW - h->radius, W, wl);
+        tx[2 * b + 1] = upsample_first_site_at_or_after(b * kUpsTW + kUpsTW + h->radius, W, wl);
+    }
+    for (int b = 0; b < nty; ++b) {
+        ty[2 * b] = upsample_first_site_at_or_after(b * kUpsTH - h->radius, rows, hl);
+        ty[2 * b + 1] = upsample_first_site_at_or_after(b * kUpsTH + kUpsTH + h->radius, rows, hl);
+    }
+    int* ix = ty + 2 * nty;      // inverse maps (fp64 refinement of upsampled pixels): column -> xl or -1
+    int* iy = ix + W;
+    for (int x = 0; x < wl; ++x) ix[tab[x]] = x;
+    for (int y = 0; y < hl; ++y) iy[tab[(size_t)wl + y]] = y;
+    CK(cudaStreamSynchronize(h->stream));
+    cudaFree(h->ups_tab_dev);
+    h->ups_tab_dev = nullptr;
+    CK(cudaMalloc(&h->ups_tab_dev, tab.size() * sizeof(int)));
+    CK(cudaMemcpy(h->ups_tab_dev, tab.data(), tab.size() * sizeof(int), cudaMemcpyHostToDevice));
+    h->ups_wl = wl; h->ups_hl = hl; h->ups_rows = rows;
+    return KDME_OK;
+}
+
 static int launch_filter(jbf_handle* h, const float* depth, const uint32_t* guide4, int guide_pitch, float* out,
                          int n, int mode, const float* depth_lo, int wl, int hl, int rows = -1, int y_off = 0,
                          int out_rows = -1, const float* depth_up = nullptr, const float* depth_dn = nullptr,
-                         int band0 = 0, int band1 = 0, bool pdl = false) {
+                         int band0 = 0, int band1 = 0, bool pdl = false, const uint16_t* depth_lo16 = nullptr) {
     JbfParams p;
     if (rows < 0) rows = h->height;
     if (out_rows < 0) out_rows = rows;
@@ -674,7 +724,8 @@ static int launch_filter(jbf_handle* h, const float* depth, const uint32_t* guid
     p.flag_scale = h->flag_scale; p.kc = h->kc; p.kd = h->kd; p.slut = h->slut_dev; p.stats = h->stats_dev;
     p.q_count = h->q_count_dev + h->q_cur; p.q_count_prev = h->q_count_dev + (h->q_cur ^ 1);
     p.q_items = h->q_items_dev; p.q_capacity = (unsigned)h->q_capacity;
-    p.mode = mode; p.depth_lo = depth_lo; p.wl = wl; p.hl = hl; p.ups_inv_x = nullptr; p.ups_inv_y = nullptr;
+    p.mode = mode; p.depth_lo = depth_lo; p.depth_lo16 = depth_lo16; p.lo_frame_stride = (long long)wl * hl;
+    p.wl = wl; p.hl = hl; p.ups_inv_x = nullptr; p.ups_inv_y = nullptr;
     p.xyz = h->xyz_out; p.fx = h->xyz_fx; p.fy = h->xyz_fy; p.cx = h->xyz_cx; p.cy = h->xyz_cy; p.y_img0 = h->xyz_yimg0;
     if (p.xyz && !h->fast) return fail(KDME_ENOTSUP, "the fused back-projection needs the fast kernel (default sigmas, r = 1..15)");
     if (h->fast) {
@@ -715,76 +766,44 @@ static int launch_filter(jbf_handle* h, const float* depth, const uint32_t* guid
         }
         p.q_items = h->q_items_dev; p.q_capacity = (unsigned)h->q_capacity;
         int rc = KDME_ENOTSUP;
-        if (p.mode == kStageUpsample && !getenv("KDME_UPSAMPLE_DENSE") && !p.xyz) {
+        UpsampleGeom g;
+        size_t smem = 0;
+        if (p.mode == kStageUpsample && ups_gather_form(h, wl, hl, rows, p.xyz != nullptr, &g, &smem)) {
             // gather form: only the sites of the low-res lattice are visited (bit-identical to the dense form)
-            constexpr int TW = 64, TH = 16;
-            UpsampleGeom g;
-            g.radius = h->radius;
-            g.ncol_max = (int)(((long long)(TW + 2 * h->radius) * wl + h->width - 1) / h->width) + 2;
-            g.nrow_max = (int)(((long long)(TH + 2 * h->radius) * hl + rows - 1) / rows) + 2;
-            g.ltab1 = h->ltab_ups1_dev;
-            g.ltab2 = h->ltab_ups2_dev;
-            const int ws_ = 2 * h->radius + 1;
-            const size_t smem = (size_t)g.ncol_max * g.nrow_max * 8 + (size_t)(g.ncol_max + g.nrow_max + 1) * 4 +
-                                (size_t)ws_ * (ws_ + kUpsPad) * 16 + 16;
-            if (smem <= 200 * 1024) {
-                const int ntx = (p.width + TW - 1) / TW, nty = (rows + TH - 1) / TH;
-                if (!h->ups_tab_dev || h->ups_wl != wl || h->ups_hl != hl || h->ups_rows != rows) {
-                    // the lattice of (wl, hl) in this frame size, once: no 64-bit division is left in the kernel
-                    std::vector<int> tab((size_t)wl + hl + 2 * (size_t)(ntx + nty) + (size_t)p.width + rows, -1);
-                    for (int x = 0; x < wl; ++x) tab[x] = (int)(((2LL * x + 1) * p.width) / (2LL * wl));
-                    for (int y = 0; y < hl; ++y) tab[(size_t)wl + y] = (int)(((2LL * y + 1) * rows) / (2LL * hl));
-                    int* tx = tab.data() + wl + hl;
-                    int* ty = tx + 2 * ntx;
-                    for (int b = 0; b < ntx; ++b) {
-                        tx[2 * b] = upsample_first_site_at_or_after(b * TW - h->radius, p.width, wl);
-                        tx[2 * b + 1] = upsample_first_site_at_or_after(b * TW + TW + h->radius, p.width, wl);
-                    }
-                    for (int b = 0; b < nty; ++b) {
-                        ty[2 * b] = upsample_first_site_at_or_after(b * TH - h->radius, rows, hl);
-                        ty[2 * b + 1] = upsample_first_site_at_or_after(b * TH + TH + h->radius, rows, hl);
-                    }
-                    int* ix = ty + 2 * nty;      // inverse maps (fp64 refinement of upsampled pixels): column -> xl or -1
-                    int* iy = ix + p.width;
-                    for (int x = 0; x < wl; ++x) ix[tab[x]] = x;
-                    for (int y = 0; y < hl; ++y) iy[tab[(size_t)wl + y]] = y;
-                    CK(cudaStreamSynchronize(h->stream));
-                    cudaFree(h->ups_tab_dev);
-                    h->ups_tab_dev = nullptr;
-                    CK(cudaMalloc(&h->ups_tab_dev, tab.size() * sizeof(int)));
-                    CK(cudaMemcpy(h->ups_tab_dev, tab.data(), tab.size() * sizeof(int), cudaMemcpyHostToDevice));
-                    h->ups_wl = wl; h->ups_hl = hl; h->ups_rows = rows;
-                }
-                g.site_x = h->ups_tab_dev; g.site_y = h->ups_tab_dev + wl;
-                g.tile_xl = h->ups_tab_dev + wl + hl; g.tile_yl = g.tile_xl + 2 * ntx;
-                p.ups_inv_x = g.tile_yl + 2 * nty; p.ups_inv_y = p.ups_inv_x + p.width;
-                // site columns any thread can see: lattice points in 2r + 4 consecutive pixels
-                const int maxc = (int)(((long long)(2 * h->radius + 4) * wl + h->width - 1) / h->width);
-                auto kern = maxc <= 5 ? jbf_upsample_gather_kernel<TW, TH, 5>
-                          : maxc <= 8 ? jbf_upsample_gather_kernel<TW, TH, 8> : jbf_upsample_gather_kernel<TW, TH, 0>;
-                if (getenv("KDME_GATHER_GENERIC")) kern = jbf_upsample_gather_kernel<TW, TH, 0>;
-                static std::atomic<unsigned long long> attr_done{0};
-                const unsigned long long bit = 1ull << (h->device & 63);
-                if (!(attr_done.load(std::memory_order_acquire) & bit)) {
-                    CK(cudaFuncSetAttribute(jbf_upsample_gather_kernel<TW, TH, 5>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
-                    CK(cudaFuncSetAttribute(jbf_upsample_gather_kernel<TW, TH, 8>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
-                    CK(cudaFuncSetAttribute(jbf_upsample_gather_kernel<TW, TH, 0>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
-                    attr_done.fetch_or(bit, std::memory_order_release);
-                }
-                cudaLaunchConfig_t cfg = {};
-                cfg.gridDim = dim3((p.width + TW - 1) / TW, (rows + TH - 1) / TH, 1);
-                cfg.blockDim = dim3((TW / 4) * TH);
-                cfg.dynamicSmemBytes = smem;
-                cfg.stream = h->stream;
-                cudaLaunchAttribute attr[1];
-                attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-                attr[0].val.programmaticStreamSerializationAllowed = 1;
-                cfg.attrs = attr;
-                cfg.numAttrs = (pdl && !h->no_pdl) ? 1 : 0;
-                CK(cudaLaunchKernelEx(&cfg, kern, p, g));
-                h->last_variant = 0x1000 | 0x400;
-                rc = KDME_OK;
+            constexpr int TW = kUpsTW, TH = kUpsTH;
+            const int ntx = (p.width + TW - 1) / TW, nty = (rows + TH - 1) / TH;
+            // built by the caller, on its own stream, before any chunk went to the internal lane
+            if (!h->ups_tab_dev || h->ups_wl != wl || h->ups_hl != hl || h->ups_rows != rows)
+                return fail(KDME_EINVAL, "upsampling: the site lattice was not built for this size");
+            g.site_x = h->ups_tab_dev; g.site_y = h->ups_tab_dev + wl;
+            g.tile_xl = h->ups_tab_dev + wl + hl; g.tile_yl = g.tile_xl + 2 * ntx;
+            p.ups_inv_x = g.tile_yl + 2 * nty; p.ups_inv_y = p.ups_inv_x + p.width;
+            // site columns any thread can see: lattice points in 2r + 4 consecutive pixels
+            const int maxc = (int)(((long long)(2 * h->radius + 4) * wl + h->width - 1) / h->width);
+            auto kern = maxc <= 5 ? jbf_upsample_gather_kernel<TW, TH, 5>
+                      : maxc <= 8 ? jbf_upsample_gather_kernel<TW, TH, 8> : jbf_upsample_gather_kernel<TW, TH, 0>;
+            if (getenv("KDME_GATHER_GENERIC")) kern = jbf_upsample_gather_kernel<TW, TH, 0>;
+            static std::atomic<unsigned long long> attr_done{0};
+            const unsigned long long bit = 1ull << (h->device & 63);
+            if (!(attr_done.load(std::memory_order_acquire) & bit)) {
+                CK(cudaFuncSetAttribute(jbf_upsample_gather_kernel<TW, TH, 5>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
+                CK(cudaFuncSetAttribute(jbf_upsample_gather_kernel<TW, TH, 8>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
+                CK(cudaFuncSetAttribute(jbf_upsample_gather_kernel<TW, TH, 0>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
+                attr_done.fetch_or(bit, std::memory_order_release);
             }
+            cudaLaunchConfig_t cfg = {};
+            cfg.gridDim = dim3((p.width + TW - 1) / TW, (rows + TH - 1) / TH, n);
+            cfg.blockDim = dim3((TW / 4) * TH);
+            cfg.dynamicSmemBytes = smem;
+            cfg.stream = h->stream;
+            cudaLaunchAttribute attr[1];
+            attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
+            attr[0].val.programmaticStreamSerializationAllowed = 1;
+            cfg.attrs = attr;
+            cfg.numAttrs = (pdl && !h->no_pdl) ? 1 : 0;
+            CK(cudaLaunchKernelEx(&cfg, kern, p, g));
+            h->last_variant = 0x1000 | 0x400;
+            rc = KDME_OK;
         }
         if (rc != KDME_OK)
         switch (h->radius) {
@@ -925,13 +944,11 @@ extern "C" int jbf_filter_rows_p2p(jbf_handle* h, const float* depth_dev, const 
                          kStagePlain, nullptr, 0, 0, rows, y_off, out_rows, depth_up, depth_dn, band0, band1);
 }
 
-extern "C" int jbf_process_batch(jbf_handle* h, const float* depth_dev, const uint8_t* bgr_dev, size_t bgr_step,
-                                 float* out_dev, int n_frames) {
-    if (!h || !depth_dev || !bgr_dev || !out_dev) return fail(KDME_EINVAL, "jbf_process_batch: NULL argument");
-    if (n_frames < 1) return fail(KDME_EINVAL, "jbf_process_batch: n_frames must be >= 1");
-    { int rc = guide_step(h, &bgr_step, "jbf_process_batch"); if (rc != KDME_OK) return rc; }
-    DeviceGuard g(h->device);
-    const size_t plane = (size_t)h->width * h->height;
+// The chunk loop of the batched device calls (jbf_process_batch, jbf_upsample_batch): chunks of max_batch frames,
+// each a pre-smooth of its guides (bgr_step already resolved) into the lane's guide buffer followed by
+// filter(f0, n), which filters frames [f0, f0 + n) from that buffer.
+template <class Filter>
+static int run_chunks(jbf_handle* h, const uint8_t* bgr_dev, size_t bgr_step, int n_frames, Filter&& filter) {
     // more than one chunk: alternate the chunks between the caller's stream and the internal lane
     const bool two = n_frames > h->max_batch && !h->one_lane && h->fast;
     if (two) {
@@ -946,8 +963,7 @@ extern "C" int jbf_process_batch(jbf_handle* h, const float* depth_dev, const ui
         LaneScope lane(h, two && (chunk & 1));
         int rc = launch_presmooth(h, bgr_dev + (size_t)f0 * bgr_step * h->height, bgr_step, h->guide4, h->guide_pitch, n);
         if (rc != KDME_OK) return rc;
-        rc = launch_filter(h, depth_dev + (size_t)f0 * plane, h->guide4, h->guide_pitch, out_dev + (size_t)f0 * plane, n,
-                           kStagePlain, nullptr, 0, 0, -1, 0, -1, nullptr, nullptr, 0, 0, /*pdl=*/true);
+        rc = filter(f0, n);
         if (rc != KDME_OK) return rc;
     }
     if (two) {   // the caller's stream continues when both lanes are done
@@ -955,6 +971,19 @@ extern "C" int jbf_process_batch(jbf_handle* h, const float* depth_dev, const ui
         CK(cudaStreamWaitEvent(h->stream, h->ev_join, 0));
     }
     return KDME_OK;
+}
+
+extern "C" int jbf_process_batch(jbf_handle* h, const float* depth_dev, const uint8_t* bgr_dev, size_t bgr_step,
+                                 float* out_dev, int n_frames) {
+    if (!h || !depth_dev || !bgr_dev || !out_dev) return fail(KDME_EINVAL, "jbf_process_batch: NULL argument");
+    if (n_frames < 1) return fail(KDME_EINVAL, "jbf_process_batch: n_frames must be >= 1");
+    { int rc = guide_step(h, &bgr_step, "jbf_process_batch"); if (rc != KDME_OK) return rc; }
+    DeviceGuard g(h->device);
+    const size_t plane = (size_t)h->width * h->height;
+    return run_chunks(h, bgr_dev, bgr_step, n_frames, [&](int f0, int n) {
+        return launch_filter(h, depth_dev + (size_t)f0 * plane, h->guide4, h->guide_pitch, out_dev + (size_t)f0 * plane, n,
+                             kStagePlain, nullptr, 0, 0, -1, 0, -1, nullptr, nullptr, 0, 0, /*pdl=*/true);
+    });
 }
 
 extern "C" int jbf_process(jbf_handle* h, const float* depth_dev, const uint8_t* bgr_dev, size_t bgr_step) {
@@ -994,16 +1023,44 @@ extern "C" int jbf_refine_stats(jbf_handle* h, unsigned long long* refined, unsi
     return KDME_OK;
 }
 
+// n_frames Upsampling calls; the low-res depth is float (depth_lo) or uint16 (depth_lo16), the other one is NULL
+static int upsample_batch(jbf_handle* h, const float* depth_lo, const uint16_t* depth_lo16, int wl, int hl,
+                          const uint8_t* bgr_dev, size_t bgr_step, float* out_dev, int n_frames, const char* who) {
+    if (!h || !(depth_lo || depth_lo16) || !bgr_dev || !out_dev) return fail(KDME_EINVAL, std::string(who) + ": NULL argument");
+    if (n_frames < 1) return fail(KDME_EINVAL, std::string(who) + ": n_frames must be >= 1");
+    if (wl <= 0 || hl <= 0 || wl > h->width || hl > h->height)
+        return fail(KDME_EINVAL, std::string(who) + ": low-res size must be positive and <= the handle's size");
+    { int rc = guide_step(h, &bgr_step, who); if (rc != KDME_OK) return rc; }
+    DeviceGuard g(h->device);
+    UpsampleGeom geom;
+    size_t smem = 0;
+    if (ups_gather_form(h, wl, hl, h->height, h->xyz_out != nullptr, &geom, &smem)) {
+        int rc = ensure_ups_table(h, wl, hl, h->height);
+        if (rc != KDME_OK) return rc;
+    }
+    const size_t plane = (size_t)h->width * h->height, lo_plane = (size_t)wl * hl;
+    return run_chunks(h, bgr_dev, bgr_step, n_frames, [&](int f0, int n) {
+        return launch_filter(h, nullptr, h->guide4, h->guide_pitch, out_dev + (size_t)f0 * plane, n, kStageUpsample,
+                             depth_lo ? depth_lo + (size_t)f0 * lo_plane : nullptr, wl, hl, -1, 0, -1, nullptr, nullptr,
+                             0, 0, /*pdl=*/true, depth_lo16 ? depth_lo16 + (size_t)f0 * lo_plane : nullptr);
+    });
+}
+
+extern "C" int jbf_upsample_batch(jbf_handle* h, const float* depth_lo_dev, int wl, int hl, const uint8_t* bgr_hi_dev,
+                                  size_t bgr_step, float* out_hi_dev, int n_frames) {
+    return upsample_batch(h, depth_lo_dev, nullptr, wl, hl, bgr_hi_dev, bgr_step, out_hi_dev, n_frames,
+                          "jbf_upsample_batch");
+}
+
+extern "C" int jbf_upsample_batch_u16(jbf_handle* h, const uint16_t* depth_lo_dev, int wl, int hl,
+                                      const uint8_t* bgr_hi_dev, size_t bgr_step, float* out_hi_dev, int n_frames) {
+    return upsample_batch(h, nullptr, depth_lo_dev, wl, hl, bgr_hi_dev, bgr_step, out_hi_dev, n_frames,
+                          "jbf_upsample_batch_u16");
+}
+
 extern "C" int jbf_upsample(jbf_handle* h, const float* depth_lo_dev, int wl, int hl, const uint8_t* bgr_hi_dev,
                             size_t bgr_step, float* out_hi_dev) {
-    if (!h || !depth_lo_dev || !bgr_hi_dev || !out_hi_dev) return fail(KDME_EINVAL, "jbf_upsample: NULL argument");
-    if (wl <= 0 || hl <= 0 || wl > h->width || hl > h->height)
-        return fail(KDME_EINVAL, "jbf_upsample: low-res size must be positive and <= the handle's size");
-    DeviceGuard g(h->device);
-    int rc = launch_presmooth(h, bgr_hi_dev, bgr_step, h->guide4, h->guide_pitch, 1);
-    if (rc != KDME_OK) return rc;
-    return launch_filter(h, nullptr, h->guide4, h->guide_pitch, out_hi_dev, 1, kStageUpsample, depth_lo_dev, wl, hl, -1, 0, -1,
-                         nullptr, nullptr, 0, 0, /*pdl=*/true);
+    return jbf_upsample_batch(h, depth_lo_dev, wl, hl, bgr_hi_dev, bgr_step, out_hi_dev, 1);
 }
 
 // Host pipeline: kPipeDepth device slots of pipe_chunk frames each; H2D, compute and D2H run on three

@@ -182,6 +182,31 @@ class JointBilateralFilter:
                                            step, _ptr(out)))
         return out
 
+    def upsample_batch(self, depth_lo: torch.Tensor, color_hi: torch.Tensor,
+                       out: torch.Tensor | None = None) -> torch.Tensor:
+        """N independent Upsampling calls: depth_lo [N, hl, wl] float32 millimetres or uint16 millimetres (the ToF
+        sensor's format, read directly; torch.uint16 or a torch.int16 view of the same bits), color_hi
+        [N, H, W, 3] u8 (or [N, H, W] / [N, H, W, 1] GRAY, [N, H, W, 4] BGRX) -> out [N, H, W] float32.  Frame k
+        equals Upsampling of frame k alone, bit for bit."""
+        if not isinstance(depth_lo, torch.Tensor) or depth_lo.dtype not in (torch.float32, torch.uint16, torch.int16):
+            raise TypeError("depth_lo must be a float32 or uint16 tensor")
+        _check_cuda(depth_lo, depth_lo.dtype, "depth_lo", self.device)
+        _check_cuda(color_hi, torch.uint8, "color_hi", self.device)
+        if depth_lo.dim() != 3 or depth_lo.shape[0] < 1:
+            raise ValueError(f"depth_lo must be [N, hl, wl] with N >= 1, got {list(depth_lo.shape)}")
+        n, hl, wl = (int(v) for v in depth_lo.shape)
+        if not (1 <= wl <= self.width and 1 <= hl <= self.height):
+            raise ValueError(f"low-res size {wl}x{hl} must be positive and at most {self.width}x{self.height}")
+        step = self._use_guide(color_hi, (n, self.height, self.width), "color_hi")
+        if out is None:
+            out = torch.empty((n, self.height, self.width), dtype=torch.float32, device=self.device)
+        _check_cuda(out, torch.float32, "out", self.device)
+        if tuple(out.shape) != (n, self.height, self.width):
+            raise ValueError(f"out must be [{n}, {self.height}, {self.width}]")
+        fn = _lib.lib().jbf_upsample_batch if depth_lo.dtype == torch.float32 else _lib.lib().jbf_upsample_batch_u16
+        _lib.check(fn(self._h, _ptr(depth_lo), wl, hl, _ptr(color_hi), step, _ptr(out), n))
+        return out
+
     # -- batched / staged forms (B200-native additions) ----------------------
     def process_batch(self, depth: torch.Tensor, color: torch.Tensor, out: torch.Tensor | None = None):
         """N independent frames: depth [N,H,W] f32, color [N,H,W,3] u8 (or [N,H,W] / [N,H,W,1] GRAY,
