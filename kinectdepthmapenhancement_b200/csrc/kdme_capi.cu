@@ -112,7 +112,6 @@ constexpr int kPipeDepth = 3;  // device slots of the host pipeline (jbf_process
 struct jbf_handle {
     int width = 0, height = 0, radius = 0, max_batch = 1, device = 0;
     float sigma_s = 0, sigma_c = 0, sigma_d = 0;
-    cudaStream_t stream = nullptr;
     // pre-smooth (JointBilateralFilter.cu:285)
     int ps_ksize = 5;
     float ps_sigma_c = 30.f, ps_sigma_s = 30.f;
@@ -120,8 +119,7 @@ struct jbf_handle {
     // owned buffers
     float* filtered_dev = nullptr;   // Filtered_Device
     float* filtered_host = nullptr;  // Filtered_Host (pinned, lazy)
-    uint32_t* guide4 = nullptr;      // smooth_Device in the internal u8x4 layout, max_batch frames
-    int guide_pitch = 0;             // words
+    int guide_pitch = 0;             // words per row of a lane's guide4
     uint8_t* smooth_bgr = nullptr;   // copy in the guide's format for getSmoothImage_Device (lazy)
     size_t smooth_bytes = 0;         // its size
     int guide_channels = 3;          // bytes per pixel of every raw guide the handle reads (1, 3 or 4)
@@ -130,10 +128,6 @@ struct jbf_handle {
     float* ltab_pairs1_dev = nullptr;// same layout for pass 1, bias `bias1`
     float* slut_dev = nullptr;       // the raw fp32 LUT of calcSpatialFilter [WS][WS] (fp64 refinement path)
     unsigned long long* stats_dev = nullptr;  // [0] pixels refined in fp64, [1] dropped (queue full), since the last jbf_refine_stats
-    unsigned int* q_count_dev = nullptr;      // refinement queue (see JbfParams): two alternating counters
-    int q_cur = 0;
-    unsigned int* q_items_dev = nullptr;
-    size_t q_capacity = 0;
     float bias1 = 0.f, flag_scale = 0.f;
     double kc = 0, kd = 0;
     float* ltab_generic_dev = nullptr;  // [WS][WS], bias kWeightBias
@@ -146,30 +140,28 @@ struct jbf_handle {
     bool force_no_tma = false, force_big_tiles = false, no_refine = false, no_split_tiles = false, no_pdl = false;
     int force_tile_h = 0, res_limit = 0;
     int last_variant = 0;
-    // TMA descriptors of the last fast launch, reused while (pointers, rows, frames, box) are unchanged
-    struct MapKey { const void* depth = nullptr; const void* guide = nullptr; int rows = 0, n = 0, gp = 0, bx = 0, by = 0; } map_key;
-    CUtensorMap map_depth, map_guide;
-    // Second lane of the chunk loops (jbf_process_batch, jbf_process_host*): odd chunks run on an internal
-    // stream with their own guide buffer, refinement queue and TMA descriptors, so that a chunk's pre-smooth
-    // fills the tail of the previous chunk's filter and the fp64 refinement launch hides behind the next
-    // filter.  The lane's state is swapped into the fields above around each odd chunk (lane_swap).
+    // What a stream of launches owns; every launch is given the lane it runs on.  lanes[0] is the caller's stream
+    // with the buffers jbf_create allocates.  lanes[1] is the internal lane of the chunk loops (run_chunks),
+    // allocated on first use: odd chunks run there with their own guide buffer, refinement queue and TMA
+    // descriptors, so that a chunk's pre-smooth fills the tail of the previous chunk's filter and the fp64
+    // refinement launch hides behind the next filter.
+    struct MapKey { const void* depth = nullptr; const void* guide = nullptr; int rows = 0, n = 0, gp = 0, bx = 0, by = 0; };
     struct Lane {
         cudaStream_t stream = nullptr;
-        uint32_t* guide4 = nullptr;
-        unsigned int* q_count_dev = nullptr;
+        uint32_t* guide4 = nullptr;            // smooth_Device in the internal u8x4 layout, max_batch frames
+        unsigned int* q_count_dev = nullptr;   // refinement queue (see JbfParams): two alternating counters
         int q_cur = 0;
         unsigned int* q_items_dev = nullptr;
         size_t q_capacity = 0;
+        // TMA descriptors of the lane's last fast launch, reused while (pointers, rows, frames, box) are unchanged
         MapKey map_key;
         CUtensorMap map_depth, map_guide;
-    } alt;
+    } lanes[2];
     cudaEvent_t ev_fork = nullptr, ev_join = nullptr;
     // gather-form upsampling: the site lattice tabulated for (ups_wl, ups_hl, ups_rows): site_x[wl], site_y[hl],
     // tile_xl[tiles_x][2], tile_yl[tiles_y][2]
     int* ups_tab_dev = nullptr; int ups_wl = 0, ups_hl = 0, ups_rows = 0;
     bool one_lane = false, no_half_units = false;
-    // fused back-projection (jbf_process_xyz): set for one launch
-    float* xyz_out = nullptr; float xyz_fx = 0, xyz_fy = 0; int xyz_cx = 0, xyz_cy = 0, xyz_yimg0 = 0;
     // host pipeline (jbf_process_host)
     cudaStream_t s_h2d = nullptr, s_d2h = nullptr;
     cudaEvent_t ev_in[kPipeDepth] = {}, ev_done[kPipeDepth] = {}, ev_free[kPipeDepth] = {};
@@ -181,45 +173,31 @@ struct jbf_handle {
     int pipe_chunk = 1;
 };
 
+using Lane = jbf_handle::Lane;
+
 static bool fast_radius_available(int r);
 static int buf_blocks(long long n);
 
-// calcSpatialFilter -- JointBilateralFilter.cpp:31-40, fp32 on the host as the reference does.
-static void lane_swap(jbf_handle* h) {
-    jbf_handle::Lane& a = h->alt;
-    std::swap(h->stream, a.stream);
-    std::swap(h->guide4, a.guide4);
-    std::swap(h->q_count_dev, a.q_count_dev);
-    std::swap(h->q_cur, a.q_cur);
-    std::swap(h->q_items_dev, a.q_items_dev);
-    std::swap(h->q_capacity, a.q_capacity);
-    std::swap(h->map_key, a.map_key);
-    std::swap(h->map_depth, a.map_depth);
-    std::swap(h->map_guide, a.map_guide);
-}
-struct LaneScope {   // runs the enclosed launches on the alternate lane when `on`
-    jbf_handle* h; bool on;
-    LaneScope(jbf_handle* h_, bool on_) : h(h_), on(on_) { if (on) lane_swap(h); }
-    ~LaneScope() { if (on) lane_swap(h); }
-};
 static int ensure_alt_lane(jbf_handle* h) {
-    if (h->alt.stream) return KDME_OK;
+    Lane& a = h->lanes[1];
+    if (a.stream) return KDME_OK;
     cudaStream_t s = nullptr;
     CK(cudaStreamCreateWithFlags(&s, cudaStreamNonBlocking));
-    cudaError_t e = cudaMalloc(&h->alt.guide4, (size_t)h->max_batch * h->height * h->guide_pitch * sizeof(uint32_t));
-    if (e == cudaSuccess) e = cudaMalloc(&h->alt.q_count_dev, 2 * sizeof(unsigned int));
-    if (e == cudaSuccess) e = cudaMemset(h->alt.q_count_dev, 0, 2 * sizeof(unsigned int));
+    cudaError_t e = cudaMalloc(&a.guide4, (size_t)h->max_batch * h->height * h->guide_pitch * sizeof(uint32_t));
+    if (e == cudaSuccess) e = cudaMalloc(&a.q_count_dev, 2 * sizeof(unsigned int));
+    if (e == cudaSuccess) e = cudaMemset(a.q_count_dev, 0, 2 * sizeof(unsigned int));
     if (e == cudaSuccess) e = cudaEventCreateWithFlags(&h->ev_fork, cudaEventDisableTiming);
     if (e == cudaSuccess) e = cudaEventCreateWithFlags(&h->ev_join, cudaEventDisableTiming);
     if (e != cudaSuccess) {
-        cudaFree(h->alt.guide4); cudaFree(h->alt.q_count_dev); cudaStreamDestroy(s);
-        h->alt.guide4 = nullptr; h->alt.q_count_dev = nullptr;
+        cudaFree(a.guide4); cudaFree(a.q_count_dev); cudaStreamDestroy(s);
+        a.guide4 = nullptr; a.q_count_dev = nullptr;
         return fail(-(int)e, std::string("second chunk lane: ") + cudaGetErrorString(e));
     }
-    h->alt.stream = s;
+    a.stream = s;
     return KDME_OK;
 }
 
+// calcSpatialFilter -- JointBilateralFilter.cpp:31-40, fp32 on the host as the reference does.
 static void host_spatial_lut(std::vector<float>& lut, int ws, float sigma_s) {
     lut.resize((size_t)ws * ws);
     for (int i = 0; i < ws; i++)
@@ -231,6 +209,7 @@ static void host_spatial_lut(std::vector<float>& lut, int ws, float sigma_s) {
 }
 
 static int build_tables(jbf_handle* h) {
+    cudaStream_t st = h->lanes[0].stream;
     const int ws = 2 * h->radius + 1, lp = (ws + 3) & ~3;
     std::vector<float> lut;
     host_spatial_lut(lut, ws, h->sigma_s);
@@ -268,10 +247,10 @@ static int build_tables(jbf_handle* h) {
         }
     CK(cudaMalloc(&h->ltab_pairs_dev, lpairs.size() * sizeof(float)));
     CK(cudaMemcpyAsync(h->ltab_pairs_dev, lpairs.data(), lpairs.size() * sizeof(float), cudaMemcpyHostToDevice,
-                       h->stream));
+                       st));
     CK(cudaMalloc(&h->ltab_pairs1_dev, lpairs1.size() * sizeof(float)));
     CK(cudaMemcpyAsync(h->ltab_pairs1_dev, lpairs1.data(), lpairs1.size() * sizeof(float), cudaMemcpyHostToDevice,
-                       h->stream));
+                       st));
     {
         std::vector<float> lg1(lg.size());
         for (size_t i = 0; i < lg.size(); i++) {
@@ -304,17 +283,17 @@ static int build_tables(jbf_handle* h) {
         CK(cudaMemcpy(h->ltab_ups2_dev, t2.data(), t2.size() * sizeof(float), cudaMemcpyHostToDevice));
     }
     CK(cudaMalloc(&h->slut_dev, lut.size() * sizeof(float)));
-    CK(cudaMemcpyAsync(h->slut_dev, lut.data(), lut.size() * sizeof(float), cudaMemcpyHostToDevice, h->stream));
+    CK(cudaMemcpyAsync(h->slut_dev, lut.data(), lut.size() * sizeof(float), cudaMemcpyHostToDevice, st));
     CK(cudaMalloc(&h->stats_dev, 2 * sizeof(unsigned long long)));
-    CK(cudaMemsetAsync(h->stats_dev, 0, 2 * sizeof(unsigned long long), h->stream));
-    CK(cudaMalloc(&h->q_count_dev, 2 * sizeof(unsigned int)));
-    CK(cudaMemsetAsync(h->q_count_dev, 0, 2 * sizeof(unsigned int), h->stream));
+    CK(cudaMemsetAsync(h->stats_dev, 0, 2 * sizeof(unsigned long long), st));
+    CK(cudaMalloc(&h->lanes[0].q_count_dev, 2 * sizeof(unsigned int)));
+    CK(cudaMemsetAsync(h->lanes[0].q_count_dev, 0, 2 * sizeof(unsigned int), st));
     CK(cudaMalloc(&h->ltab_dev, lf.size() * sizeof(float)));
     CK(cudaMalloc(&h->ltab_generic_dev, lg.size() * sizeof(float)));
-    CK(cudaMemcpyAsync(h->ltab_dev, lf.data(), lf.size() * sizeof(float), cudaMemcpyHostToDevice, h->stream));
+    CK(cudaMemcpyAsync(h->ltab_dev, lf.data(), lf.size() * sizeof(float), cudaMemcpyHostToDevice, st));
     CK(cudaMemcpyAsync(h->ltab_generic_dev, lg.data(), lg.size() * sizeof(float), cudaMemcpyHostToDevice,
-                       h->stream));
-    CK(cudaStreamSynchronize(h->stream));
+                       st));
+    CK(cudaStreamSynchronize(st));
 
     // colour factor: exp(-cd/(2 sc^2)); cd is an integer in [0, 3*255^2]
     h->use_color = (h->sigma_c != 0.0f);
@@ -366,6 +345,7 @@ static int build_tables(jbf_handle* h) {
 
 static int build_presmooth_luts(jbf_handle* h) {
     if (h->ps_ksize == 0) return KDME_OK;
+    cudaStream_t st = h->lanes[0].stream;
     const int k = h->ps_ksize, r = k / 2;
     std::vector<float> sp((size_t)k * k), col(766);
     const float ss = -0.5f / (h->ps_sigma_s * h->ps_sigma_s);
@@ -378,9 +358,9 @@ static int build_presmooth_luts(jbf_handle* h) {
     for (int n = 0; n <= 765; n++) col[n] = expf((float)(n * n) * sc);
     if (!h->ps_space_dev) CK(cudaMalloc(&h->ps_space_dev, kPsMaxK * kPsMaxK * sizeof(float)));
     if (!h->ps_color_dev) CK(cudaMalloc(&h->ps_color_dev, 768 * sizeof(float)));
-    CK(cudaMemcpyAsync(h->ps_space_dev, sp.data(), sp.size() * sizeof(float), cudaMemcpyHostToDevice, h->stream));
-    CK(cudaMemcpyAsync(h->ps_color_dev, col.data(), col.size() * sizeof(float), cudaMemcpyHostToDevice, h->stream));
-    CK(cudaStreamSynchronize(h->stream));
+    CK(cudaMemcpyAsync(h->ps_space_dev, sp.data(), sp.size() * sizeof(float), cudaMemcpyHostToDevice, st));
+    CK(cudaMemcpyAsync(h->ps_color_dev, col.data(), col.size() * sizeof(float), cudaMemcpyHostToDevice, st));
+    CK(cudaStreamSynchronize(st));
     return KDME_OK;
 }
 
@@ -407,7 +387,7 @@ extern "C" int jbf_create(jbf_handle** out, int width, int height, float sigma_s
         return fail(KDME_ENOTSUP, "jbf_create: this library is built for sm_100a (B200) only");
     jbf_handle* h = new jbf_handle();
     h->width = width; h->height = height; h->radius = window_radius; h->max_batch = max_batch;
-    h->device = device; h->stream = (cudaStream_t)stream;
+    h->device = device; h->lanes[0].stream = (cudaStream_t)stream;
     h->sigma_s = sigma_spatial; h->sigma_c = sigma_color; h->sigma_d = sigma_depth;
     h->guide_pitch = (width + 3) & ~3;
     int rc = KDME_OK;
@@ -415,7 +395,7 @@ extern "C" int jbf_create(jbf_handle** out, int width, int height, float sigma_s
     cudaError_t e;
     if ((e = cudaMalloc(&h->filtered_dev, (size_t)width * height * sizeof(float))) != cudaSuccess)
         return cleanup(fail(-(int)e, "jbf_create: cudaMalloc(Filtered_Device) failed"));
-    if ((e = cudaMalloc(&h->guide4, (size_t)max_batch * height * h->guide_pitch * sizeof(uint32_t))) != cudaSuccess)
+    if ((e = cudaMalloc(&h->lanes[0].guide4, (size_t)max_batch * height * h->guide_pitch * sizeof(uint32_t))) != cudaSuccess)
         return cleanup(fail(-(int)e, "jbf_create: cudaMalloc(smooth_Device) failed"));
     if ((rc = build_tables(h)) != KDME_OK) return cleanup(rc);
     if ((rc = build_presmooth_luts(h)) != KDME_OK) return cleanup(rc);
@@ -428,22 +408,21 @@ extern "C" void jbf_destroy(jbf_handle* h) {
     DeviceGuard g(h->device);
     cudaFree(h->filtered_dev);
     if (h->filtered_host) cudaFreeHost(h->filtered_host);
-    cudaFree(h->guide4);
     cudaFree(h->smooth_bgr);
     cudaFree(h->ltab_dev);
     cudaFree(h->ltab_pairs_dev);
     cudaFree(h->ltab_pairs1_dev);
     cudaFree(h->slut_dev);
     cudaFree(h->stats_dev);
-    cudaFree(h->q_count_dev);
-    cudaFree(h->q_items_dev);
     cudaFree(h->ups_tab_dev);
     cudaFree(h->ltab_ups1_dev);
     cudaFree(h->ltab_ups2_dev);
-    cudaFree(h->alt.guide4);
-    cudaFree(h->alt.q_count_dev);
-    cudaFree(h->alt.q_items_dev);
-    if (h->alt.stream) cudaStreamDestroy(h->alt.stream);
+    for (Lane& l : h->lanes) {
+        cudaFree(l.guide4);
+        cudaFree(l.q_count_dev);
+        cudaFree(l.q_items_dev);
+    }
+    if (h->lanes[1].stream) cudaStreamDestroy(h->lanes[1].stream);   // lanes[0] runs on the caller's stream
     if (h->ev_fork) cudaEventDestroy(h->ev_fork);
     if (h->ev_join) cudaEventDestroy(h->ev_join);
     cudaFree(h->ltab_generic_dev);
@@ -490,17 +469,41 @@ static int guide_step(const jbf_handle* h, size_t* step, const char* who) {
     return KDME_OK;
 }
 
+// Default (0) and checks of the row step of a caller's internal u8x4 guide; *pitch_words is the step in words.
+static int guide4_step(const jbf_handle* h, size_t* step, int* pitch_words, const char* who) {
+    if (*step == 0) *step = (size_t)h->guide_pitch * 4;
+    if (*step % 4 != 0 || *step < (size_t)h->width * 4)
+        return fail(KDME_EINVAL, std::string(who) + ": guide_step must be a multiple of 4 and >= 4*width");
+    *pitch_words = (int)(*step / 4);
+    return KDME_OK;
+}
+
 // ------------------------------------------------------------------ launches
 template <int C>
-static void launch_guide4_convert(jbf_handle* h, const uint8_t* bgr, size_t bgr_step, long long bgr_frame_stride,
-                                  uint32_t* guide4, int guide_pitch, long long guide_frame_stride, int rows, int n) {
+static void launch_guide4_convert_c(jbf_handle* h, Lane& lane, const uint8_t* bgr, size_t bgr_step,
+                                    long long bgr_frame_stride, uint32_t* guide4, int guide_pitch,
+                                    long long guide_frame_stride, int rows, int n) {
     dim3 blk(128), grd((h->width + 127) / 128, rows, n);
-    bgr_to_guide4_kernel<C><<<grd, blk, 0, h->stream>>>(bgr, (long long)bgr_step, bgr_frame_stride, guide4, guide_pitch,
-                                                        guide_frame_stride, h->width, rows);
+    bgr_to_guide4_kernel<C><<<grd, blk, 0, lane.stream>>>(bgr, (long long)bgr_step, bgr_frame_stride, guide4,
+                                                          guide_pitch, guide_frame_stride, h->width, rows);
+}
+
+// The raw guide in the handle's format -> the internal u8x4 guide, without smoothing.
+static void launch_guide4_convert(jbf_handle* h, Lane& lane, const uint8_t* bgr, size_t bgr_step,
+                                  long long bgr_frame_stride, uint32_t* guide4, int guide_pitch,
+                                  long long guide_frame_stride, int rows, int n) {
+#define KDME_CONVERT(C) launch_guide4_convert_c<C>(h, lane, bgr, bgr_step, bgr_frame_stride, guide4, guide_pitch, \
+                                                   guide_frame_stride, rows, n)
+    switch (h->guide_channels) {
+        case 1: KDME_CONVERT(1); break;
+        case 4: KDME_CONVERT(4); break;
+        default: KDME_CONVERT(3); break;
+    }
+#undef KDME_CONVERT
 }
 
 template <int C>
-static void launch_presmooth_c(jbf_handle* h, const PresmoothParams& p, int rows, int n) {
+static void launch_presmooth_c(jbf_handle* h, Lane& lane, const PresmoothParams& p, int rows, int n) {
     if (h->ps_ksize == 5) {
         // 64x16 tiles, 128 threads, 4x2 pixels per thread; a launch too small to fill the GPU with them (one
         // Kinect frame is 300) uses 64x8 tiles of 128 threads with 4x1 pixels: four times the warps
@@ -508,31 +511,27 @@ static void launch_presmooth_c(jbf_handle* h, const PresmoothParams& p, int rows
         const long long ctas16 = (long long)((h->width + TW - 1) / TW) * ((rows + 15) / 16) * n;
         if (ctas16 >= 148LL * 6) {
             dim3 grd((h->width + TW - 1) / TW, (rows + 15) / 16, n);
-            presmooth5_kernel<TW, 16, 2, C><<<grd, (TW / 4) * 8, 0, h->stream>>>(p);
+            presmooth5_kernel<TW, 16, 2, C><<<grd, (TW / 4) * 8, 0, lane.stream>>>(p);
         } else {
             dim3 grd((h->width + TW - 1) / TW, (rows + 7) / 8, n);
-            presmooth5_kernel<TW, 8, 1, C><<<grd, (TW / 4) * 8, 0, h->stream>>>(p);
+            presmooth5_kernel<TW, 8, 1, C><<<grd, (TW / 4) * 8, 0, lane.stream>>>(p);
         }
     } else {
         constexpr int TW = 32, TH = 8;
         dim3 grd((h->width + TW - 1) / TW, (rows + TH - 1) / TH, n);
-        presmooth_kernel<TW, TH, C><<<grd, TW * TH, 0, h->stream>>>(p);
+        presmooth_kernel<TW, TH, C><<<grd, TW * TH, 0, lane.stream>>>(p);
     }
 }
 
-static int launch_presmooth(jbf_handle* h, const uint8_t* bgr, size_t bgr_step, uint32_t* guide4, int guide_pitch,
-                            int n, int rows = -1, const uint8_t* bgr_up = nullptr, const uint8_t* bgr_dn = nullptr,
-                            int band0 = 0, int band1 = 0) {
+static int launch_presmooth(jbf_handle* h, Lane& lane, const uint8_t* bgr, size_t bgr_step, uint32_t* guide4,
+                            int guide_pitch, int n, int rows = -1, const uint8_t* bgr_up = nullptr,
+                            const uint8_t* bgr_dn = nullptr, int band0 = 0, int band1 = 0) {
     if (rows < 0) rows = h->height;
     { int rc = guide_step(h, &bgr_step, "pre-smooth"); if (rc != KDME_OK) return rc; }
     if (h->ps_ksize == 0) {
         if (bgr_up || bgr_dn) return fail(KDME_ENOTSUP, "peer-memory halos need the guide pre-smooth enabled");
-        const long long bfs = (long long)bgr_step * rows, gfs = (long long)guide_pitch * rows;
-        switch (h->guide_channels) {
-            case 1: launch_guide4_convert<1>(h, bgr, bgr_step, bfs, guide4, guide_pitch, gfs, rows, n); break;
-            case 4: launch_guide4_convert<4>(h, bgr, bgr_step, bfs, guide4, guide_pitch, gfs, rows, n); break;
-            default: launch_guide4_convert<3>(h, bgr, bgr_step, bfs, guide4, guide_pitch, gfs, rows, n); break;
-        }
+        launch_guide4_convert(h, lane, bgr, bgr_step, (long long)bgr_step * rows, guide4, guide_pitch,
+                              (long long)guide_pitch * rows, rows, n);
     } else {
         PresmoothParams p;
         p.width = h->width; p.height = rows; p.n_frames = n;
@@ -541,9 +540,9 @@ static int launch_presmooth(jbf_handle* h, const uint8_t* bgr, size_t bgr_step, 
         p.ksize = h->ps_ksize; p.space_lut = h->ps_space_dev; p.color_lut = h->ps_color_dev;
         p.bgr_up = bgr_up; p.bgr_dn = bgr_dn; p.band0 = band0; p.band1 = band1;
         switch (h->guide_channels) {
-            case 1: launch_presmooth_c<1>(h, p, rows, n); break;
-            case 4: launch_presmooth_c<4>(h, p, rows, n); break;
-            default: launch_presmooth_c<3>(h, p, rows, n); break;
+            case 1: launch_presmooth_c<1>(h, lane, p, rows, n); break;
+            case 4: launch_presmooth_c<4>(h, lane, p, rows, n); break;
+            default: launch_presmooth_c<3>(h, lane, p, rows, n); break;
         }
     }
     CK(cudaGetLastError());
@@ -552,8 +551,9 @@ static int launch_presmooth(jbf_handle* h, const uint8_t* bgr, size_t bgr_step, 
 
 // One (radius, tile height) instantiation: encode (or reuse) the TMA maps for its box and launch.
 template <int R, int TH>
-static int launch_fast_rt(jbf_handle* h, JbfParams p, bool want_tma, int rows, bool pdl) {
+static int launch_fast_rt(jbf_handle* h, Lane& lane, JbfParams p, bool want_tma, bool pdl) {
     constexpr int TW = 64;
+    const int rows = p.height;
     using T = JbfTile<R, TW, TH>;
     // resident CTAs per SM: by registers (<= 80 for r <= 9, <= 128 above: the row segment alone is
     // 3 x (2r + 8) registers) and by shared memory
@@ -571,12 +571,12 @@ static int launch_fast_rt(jbf_handle* h, JbfParams p, bool want_tma, int rows, b
         attr_done.fetch_or(bit, std::memory_order_release);
     }
     if (want_tma) {
-        jbf_handle::MapKey& k = h->map_key;
+        jbf_handle::MapKey& k = lane.map_key;
         if (k.depth != p.depth || k.guide != p.guide4 || k.rows != rows || k.n != p.n_frames || k.gp != p.guide_pitch ||
             k.bx != T::SP || k.by != T::SH) {
-            bool ok = encode_map(&h->map_depth, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, p.depth, p.width, rows, p.n_frames,
+            bool ok = encode_map(&lane.map_depth, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, p.depth, p.width, rows, p.n_frames,
                                  (long long)p.width * 4, (long long)p.width * rows * 4, T::SP, T::SH) &&
-                      encode_map(&h->map_guide, CU_TENSOR_MAP_DATA_TYPE_UINT32, p.guide4, p.width, rows, p.n_frames,
+                      encode_map(&lane.map_guide, CU_TENSOR_MAP_DATA_TYPE_UINT32, p.guide4, p.width, rows, p.n_frames,
                                  (long long)p.guide_pitch * 4, (long long)p.guide_pitch * rows * 4, T::SP, T::SH);
             if (ok) {
                 k.depth = p.depth; k.guide = p.guide4; k.rows = rows; k.n = p.n_frames; k.gp = p.guide_pitch;
@@ -632,13 +632,13 @@ static int launch_fast_rt(jbf_handle* h, JbfParams p, bool want_tma, int rows, b
     cfg.gridDim = dim3(tx, tile_rows, p.n_frames);
     cfg.blockDim = dim3(T::NT);
     cfg.dynamicSmemBytes = smem_bytes;
-    cfg.stream = h->stream;
+    cfg.stream = lane.stream;
     cudaLaunchAttribute attr[1];
     attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
     attr[0].val.programmaticStreamSerializationAllowed = 1;
     cfg.attrs = attr;
     cfg.numAttrs = (pdl && !h->no_pdl) ? 1 : 0;
-    CK(cudaLaunchKernelEx(&cfg, kern, h->map_depth, h->map_guide, p));
+    CK(cudaLaunchKernelEx(&cfg, kern, lane.map_depth, lane.map_guide, p));
     return KDME_OK;
 }
 
@@ -655,11 +655,11 @@ static bool fast_radius_available(int r) {
 }
 
 // Upsampling runs in gather form (jbf_upsample_gather_kernel, tiles kUpsTW x kUpsTH) on the fast path unless the
-// dense form is asked for (KDME_UPSAMPLE_DENSE), the back-projection epilogue is on, or the staged sites of a tile
-// would not fit in shared memory.  Fills the launch geometry except the lattice pointers.
+// dense form is asked for (KDME_UPSAMPLE_DENSE) or the staged sites of a tile would not fit in shared memory.
+// Fills the launch geometry except the lattice pointers.
 constexpr int kUpsTW = 64, kUpsTH = 16;
-static bool ups_gather_form(const jbf_handle* h, int wl, int hl, int rows, bool xyz, UpsampleGeom* g, size_t* smem) {
-    if (!h->fast || xyz || getenv("KDME_UPSAMPLE_DENSE")) return false;
+static bool ups_gather_form(const jbf_handle* h, int wl, int hl, int rows, UpsampleGeom* g, size_t* smem) {
+    if (!h->fast || getenv("KDME_UPSAMPLE_DENSE")) return false;
     g->radius = h->radius;
     g->ncol_max = (int)(((long long)(kUpsTW + 2 * h->radius) * wl + h->width - 1) / h->width) + 2;
     g->nrow_max = (int)(((long long)(kUpsTH + 2 * h->radius) * hl + rows - 1) / rows) + 2;
@@ -673,8 +673,8 @@ static bool ups_gather_form(const jbf_handle* h, int wl, int hl, int rows, bool 
 
 // The site lattice of (wl, hl) in frames of `rows` rows for the gather form, tabulated once (no 64-bit division is
 // left in the kernel): site_x[wl], site_y[hl], tile_xl[tiles_x][2], tile_yl[tiles_y][2], then the inverse maps of
-// the fp64 refinement.  Shared by both chunk lanes: a rebuild synchronises the handle's stream before it frees the
-// old table, so it runs on the caller's stream before any chunk is forked to the internal lane.
+// the fp64 refinement.  Shared by both chunk lanes: a rebuild synchronises the caller's stream (lanes[0]) before it
+// frees the old table, so it runs before any chunk is forked to the internal lane.
 static int ensure_ups_table(jbf_handle* h, int wl, int hl, int rows) {
     if (h->ups_tab_dev && h->ups_wl == wl && h->ups_hl == hl && h->ups_rows == rows) return KDME_OK;
     const int W = h->width, ntx = (W + kUpsTW - 1) / kUpsTW, nty = (rows + kUpsTH - 1) / kUpsTH;
@@ -695,7 +695,7 @@ static int ensure_ups_table(jbf_handle* h, int wl, int hl, int rows) {
     int* iy = ix + W;
     for (int x = 0; x < wl; ++x) ix[tab[x]] = x;
     for (int y = 0; y < hl; ++y) iy[tab[(size_t)wl + y]] = y;
-    CK(cudaStreamSynchronize(h->stream));
+    CK(cudaStreamSynchronize(h->lanes[0].stream));
     cudaFree(h->ups_tab_dev);
     h->ups_tab_dev = nullptr;
     CK(cudaMalloc(&h->ups_tab_dev, tab.size() * sizeof(int)));
@@ -704,37 +704,37 @@ static int ensure_ups_table(jbf_handle* h, int wl, int hl, int rows) {
     return KDME_OK;
 }
 
-static int launch_filter(jbf_handle* h, const float* depth, const uint32_t* guide4, int guide_pitch, float* out,
-                         int n, int mode, const float* depth_lo, int wl, int hl, int rows = -1, int y_off = 0,
-                         int out_rows = -1, const float* depth_up = nullptr, const float* depth_dn = nullptr,
-                         int band0 = 0, int band1 = 0, bool pdl = false, const uint16_t* depth_lo16 = nullptr) {
-    JbfParams p;
-    if (rows < 0) rows = h->height;
-    if (out_rows < 0) out_rows = rows;
-    p.width = h->width; p.height = rows; p.n_frames = n;
-    p.y_off = y_off; p.out_rows = out_rows;
-    p.depth_up = depth_up; p.depth_dn = depth_dn; p.band0 = band0; p.band1 = band1;
-    if ((depth_up || depth_dn) && !h->fast)
+// The request of a filter launch over n whole frames: rows = out_rows = height, no halos, no low-res input, no
+// back-projection, plain mode.  Callers set what their call differs in; launch_filter fills the rest.
+static JbfParams filter_request(const jbf_handle* h, const float* depth, const uint32_t* guide4, int guide_pitch,
+                                float* out, int n) {
+    JbfParams p = {};
+    p.width = h->width; p.height = h->height; p.out_rows = h->height; p.n_frames = n;
+    p.depth = depth; p.guide4 = guide4; p.guide_pitch = guide_pitch; p.out = out;
+    p.mode = kStagePlain;
+    return p;
+}
+
+// Launches request p on `lane`: its stream, refinement queue and TMA descriptors.
+static int launch_filter(jbf_handle* h, Lane& lane, JbfParams p, bool pdl) {
+    if ((p.depth_up || p.depth_dn) && !h->fast)
         return fail(KDME_ENOTSUP, "peer-memory halos are implemented for the fast kernel (default sigmas, r = 1..15)");
-    p.depth = depth; p.guide4 = guide4; p.out = out;
+    if (p.xyz && !h->fast) return fail(KDME_ENOTSUP, "the fused back-projection needs the fast kernel (default sigmas, r = 1..15)");
+    const int rows = p.height, n = p.n_frames, wl = p.wl, hl = p.hl;
     p.depth_frame_stride = (long long)h->width * rows;
-    p.guide_frame_stride = (long long)guide_pitch * rows;
-    p.guide_pitch = guide_pitch;
+    p.guide_frame_stride = (long long)p.guide_pitch * rows;
+    p.lo_frame_stride = (long long)wl * hl;
     p.nkc = h->nkc; p.sq = h->sq; p.inv_sq = h->inv_sq; p.e_thr = h->e_thr;
     p.flag_scale = h->flag_scale; p.kc = h->kc; p.kd = h->kd; p.slut = h->slut_dev; p.stats = h->stats_dev;
-    p.q_count = h->q_count_dev + h->q_cur; p.q_count_prev = h->q_count_dev + (h->q_cur ^ 1);
-    p.q_items = h->q_items_dev; p.q_capacity = (unsigned)h->q_capacity;
-    p.mode = mode; p.depth_lo = depth_lo; p.depth_lo16 = depth_lo16; p.lo_frame_stride = (long long)wl * hl;
-    p.wl = wl; p.hl = hl; p.ups_inv_x = nullptr; p.ups_inv_y = nullptr;
-    p.xyz = h->xyz_out; p.fx = h->xyz_fx; p.fy = h->xyz_fy; p.cx = h->xyz_cx; p.cy = h->xyz_cy; p.y_img0 = h->xyz_yimg0;
-    if (p.xyz && !h->fast) return fail(KDME_ENOTSUP, "the fused back-projection needs the fast kernel (default sigmas, r = 1..15)");
+    p.q_count = lane.q_count_dev + lane.q_cur; p.q_count_prev = lane.q_count_dev + (lane.q_cur ^ 1);
+    p.q_items = lane.q_items_dev; p.q_capacity = (unsigned)lane.q_capacity;
     if (h->fast) {
         p.ltab = h->ltab_dev;
         p.ltab_pairs = h->ltab_pairs_dev;
         p.ltab_pairs1 = h->ltab_pairs1_dev;
         const bool want_tma = p.mode == kStagePlain && !h->force_no_tma && (h->width % 4 == 0) &&
-                              (guide_pitch % 4 == 0) && ((reinterpret_cast<uintptr_t>(depth) & 15) == 0) &&
-                              ((reinterpret_cast<uintptr_t>(guide4) & 15) == 0);
+                              (p.guide_pitch % 4 == 0) && ((reinterpret_cast<uintptr_t>(p.depth) & 15) == 0) &&
+                              ((reinterpret_cast<uintptr_t>(p.guide4) & 15) == 0);
         // Tile height: the arithmetic of a pixel does not depend on the tile it falls in, so the choice is
         // purely a scheduling one.  Large launches use 64x16 tiles (least halo per pixel); a launch of only
         // a few waves (one Kinect frame is 300 such tiles on 148 SMs) is cut finer so that the most loaded
@@ -745,7 +745,7 @@ static int launch_filter(jbf_handle* h, const float* depth, const uint32_t* guid
         const int cand[3] = {16, 8, 4};
         for (int ci = 0; ci < 3; ++ci) {
             const int th = cand[ci];
-            const long long ctas = (long long)tx * ((out_rows + th - 1) / th) * n;
+            const long long ctas = (long long)tx * ((p.out_rows + th - 1) / th) * n;
             const long long per_sm = (ctas + 147) / 148;
             const double cost = (double)per_sm * (th + 0.06 * (th + 2 * h->radius) + 0.25);
             if (cost < best_cost * 0.97) { best_cost = cost; best_th = th; }
@@ -754,21 +754,21 @@ static int launch_filter(jbf_handle* h, const float* depth, const uint32_t* guid
         if (h->force_tile_h == 16 || h->force_tile_h == 8 || h->force_tile_h == 4) best_th = h->force_tile_h;
         // queue of ill-conditioned pixels: a quarter of the launch's pixels (at least 64 K entries); pixels
         // beyond it keep their fp32 value and are counted (jbf_refine_stats)
-        const unsigned long long px = (unsigned long long)h->width * out_rows * n;
+        const unsigned long long px = (unsigned long long)h->width * p.out_rows * n;
         if (px > 0xFFFFFFFFull) return fail(KDME_ENOTSUP, "more than 2^32 pixels in one launch");
         size_t want = (size_t)std::min<unsigned long long>(std::max<unsigned long long>(px / 4, 65536ull), px);
-        if (h->flag_scale > 0.f && want > h->q_capacity) {
-            CK(cudaStreamSynchronize(h->stream));
-            cudaFree(h->q_items_dev);
-            h->q_items_dev = nullptr; h->q_capacity = 0;
-            CK(cudaMalloc(&h->q_items_dev, want * sizeof(unsigned int)));
-            h->q_capacity = want;
+        if (h->flag_scale > 0.f && want > lane.q_capacity) {
+            CK(cudaStreamSynchronize(lane.stream));
+            cudaFree(lane.q_items_dev);
+            lane.q_items_dev = nullptr; lane.q_capacity = 0;
+            CK(cudaMalloc(&lane.q_items_dev, want * sizeof(unsigned int)));
+            lane.q_capacity = want;
         }
-        p.q_items = h->q_items_dev; p.q_capacity = (unsigned)h->q_capacity;
+        p.q_items = lane.q_items_dev; p.q_capacity = (unsigned)lane.q_capacity;
         int rc = KDME_ENOTSUP;
         UpsampleGeom g;
         size_t smem = 0;
-        if (p.mode == kStageUpsample && ups_gather_form(h, wl, hl, rows, p.xyz != nullptr, &g, &smem)) {
+        if (p.mode == kStageUpsample && ups_gather_form(h, wl, hl, rows, &g, &smem)) {
             // gather form: only the sites of the low-res lattice are visited (bit-identical to the dense form)
             constexpr int TW = kUpsTW, TH = kUpsTH;
             const int ntx = (p.width + TW - 1) / TW, nty = (rows + TH - 1) / TH;
@@ -795,7 +795,7 @@ static int launch_filter(jbf_handle* h, const float* depth, const uint32_t* guid
             cfg.gridDim = dim3((p.width + TW - 1) / TW, (rows + TH - 1) / TH, n);
             cfg.blockDim = dim3((TW / 4) * TH);
             cfg.dynamicSmemBytes = smem;
-            cfg.stream = h->stream;
+            cfg.stream = lane.stream;
             cudaLaunchAttribute attr[1];
             attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
             attr[0].val.programmaticStreamSerializationAllowed = 1;
@@ -807,15 +807,15 @@ static int launch_filter(jbf_handle* h, const float* depth, const uint32_t* guid
         }
         if (rc != KDME_OK)
         switch (h->radius) {
-#define X(R) case R: rc = best_th == 16 ? launch_fast_rt<R, 16>(h, p, want_tma, rows, pdl)                     \
-                        : best_th == 8 ? launch_fast_rt<R, 8>(h, p, want_tma, rows, pdl)                       \
-                                       : launch_fast_rt<R, 4>(h, p, want_tma, rows, pdl); break;
+#define X(R) case R: rc = best_th == 16 ? launch_fast_rt<R, 16>(h, lane, p, want_tma, pdl)                     \
+                        : best_th == 8 ? launch_fast_rt<R, 8>(h, lane, p, want_tma, pdl)                       \
+                                       : launch_fast_rt<R, 4>(h, lane, p, want_tma, pdl); break;
             KDME_FAST_RADII(X)
 #undef X
             default: return fail(KDME_ENOTSUP, "no fast kernel for this radius");
         }
         if (rc != KDME_OK) return rc;
-        h->q_cur ^= 1;
+        lane.q_cur ^= 1;
         if (h->flag_scale > 0.f) {
             // fp64 re-evaluation of the queued pixels; launched with programmatic stream serialisation so its
             // launch latency hides behind the filter (it waits for the filter's completion on the device)
@@ -823,7 +823,7 @@ static int launch_filter(jbf_handle* h, const float* depth, const uint32_t* guid
             cudaLaunchConfig_t cfg = {};
             cfg.gridDim = dim3(148 * 5);
             cfg.blockDim = dim3(128);
-            cfg.stream = h->stream;
+            cfg.stream = lane.stream;
             cudaLaunchAttribute attr[1];
             attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
             attr[0].val.programmaticStreamSerializationAllowed = 1;
@@ -858,7 +858,7 @@ static int launch_filter(jbf_handle* h, const float* depth, const uint32_t* guid
         attr_done.fetch_or(bit, std::memory_order_release);
     }
     dim3 grd((p.width + TW - 1) / TW, (p.out_rows + TH - 1) / TH, n);
-    jbf_generic_kernel<TW, TH><<<grd, TW * TH, smem, h->stream>>>(gp);
+    jbf_generic_kernel<TW, TH><<<grd, TW * TH, smem, lane.stream>>>(gp);
     CK(cudaGetLastError());
     h->last_variant = 1;
     return KDME_OK;
@@ -868,12 +868,10 @@ extern "C" int jbf_presmooth(jbf_handle* h, const uint8_t* bgr_dev, size_t bgr_s
                              size_t guide_step, int n_frames) {
     if (!h || !bgr_dev || !guide4_dev) return fail(KDME_EINVAL, "jbf_presmooth: NULL argument");
     if (n_frames < 1) return fail(KDME_EINVAL, "jbf_presmooth: n_frames must be >= 1");
-    if (guide_step == 0) guide_step = (size_t)h->guide_pitch * 4;
-    if (guide_step % 4 != 0 || guide_step < (size_t)h->width * 4)
-        return fail(KDME_EINVAL, "jbf_presmooth: guide_step must be a multiple of 4 and >= 4*width");
+    int pitch = 0;
+    { int rc = guide4_step(h, &guide_step, &pitch, "jbf_presmooth"); if (rc != KDME_OK) return rc; }
     DeviceGuard g(h->device);
-    return launch_presmooth(h, bgr_dev, bgr_step, reinterpret_cast<uint32_t*>(guide4_dev), (int)(guide_step / 4),
-                            n_frames);
+    return launch_presmooth(h, h->lanes[0], bgr_dev, bgr_step, reinterpret_cast<uint32_t*>(guide4_dev), pitch, n_frames);
 }
 
 extern "C" int jbf_filter_guide4(jbf_handle* h, const float* depth_dev, const uint8_t* guide4_dev, size_t guide_step,
@@ -881,23 +879,22 @@ extern "C" int jbf_filter_guide4(jbf_handle* h, const float* depth_dev, const ui
     if (!h || !depth_dev || !guide4_dev || !out_dev) return fail(KDME_EINVAL, "jbf_filter_guide4: NULL argument");
     if (n_frames < 1 || n_frames > 65535) return fail(KDME_EINVAL, "jbf_filter_guide4: n_frames must be in [1, 65535] (frames are grid.z of one launch)");
     if (depth_dev == out_dev) return fail(KDME_EINVAL, "jbf_filter_guide4: in-place operation is not supported");
-    if (guide_step == 0) guide_step = (size_t)h->guide_pitch * 4;
-    if (guide_step % 4 != 0 || guide_step < (size_t)h->width * 4)
-        return fail(KDME_EINVAL, "jbf_filter_guide4: guide_step must be a multiple of 4 and >= 4*width");
+    int pitch = 0;
+    { int rc = guide4_step(h, &guide_step, &pitch, "jbf_filter_guide4"); if (rc != KDME_OK) return rc; }
     DeviceGuard g(h->device);
-    return launch_filter(h, depth_dev, reinterpret_cast<const uint32_t*>(guide4_dev), (int)(guide_step / 4), out_dev,
-                         n_frames, kStagePlain, nullptr, 0, 0);
+    return launch_filter(h, h->lanes[0],
+                         filter_request(h, depth_dev, reinterpret_cast<const uint32_t*>(guide4_dev), pitch, out_dev, n_frames),
+                         /*pdl=*/false);
 }
 
 extern "C" int jbf_presmooth_rows(jbf_handle* h, const uint8_t* bgr_dev, size_t bgr_step, uint8_t* guide4_dev,
                                   size_t guide_step, int rows) {
     if (!h || !bgr_dev || !guide4_dev) return fail(KDME_EINVAL, "jbf_presmooth_rows: NULL argument");
     if (rows < 1) return fail(KDME_EINVAL, "jbf_presmooth_rows: rows must be >= 1");
-    if (guide_step == 0) guide_step = (size_t)h->guide_pitch * 4;
-    if (guide_step % 4 != 0 || guide_step < (size_t)h->width * 4)
-        return fail(KDME_EINVAL, "jbf_presmooth_rows: guide_step must be a multiple of 4 and >= 4*width");
+    int pitch = 0;
+    { int rc = guide4_step(h, &guide_step, &pitch, "jbf_presmooth_rows"); if (rc != KDME_OK) return rc; }
     DeviceGuard g(h->device);
-    return launch_presmooth(h, bgr_dev, bgr_step, reinterpret_cast<uint32_t*>(guide4_dev), (int)(guide_step / 4), 1, rows);
+    return launch_presmooth(h, h->lanes[0], bgr_dev, bgr_step, reinterpret_cast<uint32_t*>(guide4_dev), pitch, 1, rows);
 }
 
 extern "C" int jbf_filter_rows(jbf_handle* h, const float* depth_dev, const uint8_t* guide4_dev, size_t guide_step,
@@ -905,12 +902,12 @@ extern "C" int jbf_filter_rows(jbf_handle* h, const float* depth_dev, const uint
     if (!h || !depth_dev || !guide4_dev || !out_dev) return fail(KDME_EINVAL, "jbf_filter_rows: NULL argument");
     if (rows < 1 || y_off < 0 || out_rows < 1 || y_off + out_rows > rows)
         return fail(KDME_EINVAL, "jbf_filter_rows: need 0 <= y_off and y_off + out_rows <= rows");
-    if (guide_step == 0) guide_step = (size_t)h->guide_pitch * 4;
-    if (guide_step % 4 != 0 || guide_step < (size_t)h->width * 4)
-        return fail(KDME_EINVAL, "jbf_filter_rows: guide_step must be a multiple of 4 and >= 4*width");
+    int pitch = 0;
+    { int rc = guide4_step(h, &guide_step, &pitch, "jbf_filter_rows"); if (rc != KDME_OK) return rc; }
     DeviceGuard g(h->device);
-    return launch_filter(h, depth_dev, reinterpret_cast<const uint32_t*>(guide4_dev), (int)(guide_step / 4), out_dev, 1,
-                         kStagePlain, nullptr, 0, 0, rows, y_off, out_rows);
+    JbfParams p = filter_request(h, depth_dev, reinterpret_cast<const uint32_t*>(guide4_dev), pitch, out_dev, 1);
+    p.height = rows; p.y_off = y_off; p.out_rows = out_rows;
+    return launch_filter(h, h->lanes[0], p, /*pdl=*/false);
 }
 
 // Row bands with the halos read from the neighbour GPUs' memory inside the kernels (NVLink peer loads):
@@ -922,11 +919,10 @@ extern "C" int jbf_presmooth_rows_p2p(jbf_handle* h, const uint8_t* bgr_dev, siz
     if (!h || !bgr_dev || !guide4_dev) return fail(KDME_EINVAL, "jbf_presmooth_rows_p2p: NULL argument");
     if (rows < 1 || band0 < 0 || band1 > rows || band0 >= band1)
         return fail(KDME_EINVAL, "jbf_presmooth_rows_p2p: need 0 <= band0 < band1 <= rows");
-    if (guide_step == 0) guide_step = (size_t)h->guide_pitch * 4;
-    if (guide_step % 4 != 0 || guide_step < (size_t)h->width * 4)
-        return fail(KDME_EINVAL, "jbf_presmooth_rows_p2p: guide_step must be a multiple of 4 and >= 4*width");
+    int pitch = 0;
+    { int rc = guide4_step(h, &guide_step, &pitch, "jbf_presmooth_rows_p2p"); if (rc != KDME_OK) return rc; }
     DeviceGuard g(h->device);
-    return launch_presmooth(h, bgr_dev, bgr_step, reinterpret_cast<uint32_t*>(guide4_dev), (int)(guide_step / 4), 1, rows,
+    return launch_presmooth(h, h->lanes[0], bgr_dev, bgr_step, reinterpret_cast<uint32_t*>(guide4_dev), pitch, 1, rows,
                             bgr_up, bgr_dn, band0, band1);
 }
 
@@ -936,39 +932,36 @@ extern "C" int jbf_filter_rows_p2p(jbf_handle* h, const float* depth_dev, const 
     if (!h || !depth_dev || !guide4_dev || !out_dev) return fail(KDME_EINVAL, "jbf_filter_rows_p2p: NULL argument");
     if (rows < 1 || y_off < 0 || out_rows < 1 || y_off + out_rows > rows || band0 < 0 || band1 > rows || band0 >= band1)
         return fail(KDME_EINVAL, "jbf_filter_rows_p2p: bad row ranges");
-    if (guide_step == 0) guide_step = (size_t)h->guide_pitch * 4;
-    if (guide_step % 4 != 0 || guide_step < (size_t)h->width * 4)
-        return fail(KDME_EINVAL, "jbf_filter_rows_p2p: guide_step must be a multiple of 4 and >= 4*width");
+    int pitch = 0;
+    { int rc = guide4_step(h, &guide_step, &pitch, "jbf_filter_rows_p2p"); if (rc != KDME_OK) return rc; }
     DeviceGuard g(h->device);
-    return launch_filter(h, depth_dev, reinterpret_cast<const uint32_t*>(guide4_dev), (int)(guide_step / 4), out_dev, 1,
-                         kStagePlain, nullptr, 0, 0, rows, y_off, out_rows, depth_up, depth_dn, band0, band1);
+    JbfParams p = filter_request(h, depth_dev, reinterpret_cast<const uint32_t*>(guide4_dev), pitch, out_dev, 1);
+    p.height = rows; p.y_off = y_off; p.out_rows = out_rows;
+    p.depth_up = depth_up; p.depth_dn = depth_dn; p.band0 = band0; p.band1 = band1;
+    return launch_filter(h, h->lanes[0], p, /*pdl=*/false);
 }
 
-// The chunk loop of the batched device calls (jbf_process_batch, jbf_upsample_batch): chunks of max_batch frames,
-// each a pre-smooth of its guides (bgr_step already resolved) into the lane's guide buffer followed by
-// filter(f0, n), which filters frames [f0, f0 + n) from that buffer.
-template <class Filter>
-static int run_chunks(jbf_handle* h, const uint8_t* bgr_dev, size_t bgr_step, int n_frames, Filter&& filter) {
-    // more than one chunk: alternate the chunks between the caller's stream and the internal lane
-    const bool two = n_frames > h->max_batch && !h->one_lane && h->fast;
+// The chunk loop of the batched calls: chunks of `chunk` frames, fn(lane, c, f0, n) enqueues chunk c, frames
+// [f0, f0 + n), on `lane`.  With more than one chunk on the fast path, the chunks alternate between the caller's
+// stream (lanes[0]) and the internal lane (lanes[1]), which is forked from the caller's stream before the first
+// chunk and joined back into it after the last, so the call keeps the caller's stream semantics.
+template <class Fn>
+static int run_chunks(jbf_handle* h, int n_frames, int chunk, Fn&& fn) {
+    const bool two = n_frames > chunk && !h->one_lane && h->fast;
+    Lane &l0 = h->lanes[0], &l1 = h->lanes[1];
     if (two) {
         int rc = ensure_alt_lane(h);
         if (rc != KDME_OK) return rc;
-        CK(cudaEventRecord(h->ev_fork, h->stream));
-        CK(cudaStreamWaitEvent(h->alt.stream, h->ev_fork, 0));
+        CK(cudaEventRecord(h->ev_fork, l0.stream));
+        CK(cudaStreamWaitEvent(l1.stream, h->ev_fork, 0));
     }
-    int chunk = 0;
-    for (int f0 = 0; f0 < n_frames; f0 += h->max_batch, ++chunk) {
-        const int n = (n_frames - f0 < h->max_batch) ? (n_frames - f0) : h->max_batch;
-        LaneScope lane(h, two && (chunk & 1));
-        int rc = launch_presmooth(h, bgr_dev + (size_t)f0 * bgr_step * h->height, bgr_step, h->guide4, h->guide_pitch, n);
-        if (rc != KDME_OK) return rc;
-        rc = filter(f0, n);
+    for (int c = 0, f0 = 0; f0 < n_frames; f0 += chunk, ++c) {
+        int rc = fn(two && (c & 1) ? l1 : l0, c, f0, std::min(chunk, n_frames - f0));
         if (rc != KDME_OK) return rc;
     }
-    if (two) {   // the caller's stream continues when both lanes are done
-        CK(cudaEventRecord(h->ev_join, h->alt.stream));
-        CK(cudaStreamWaitEvent(h->stream, h->ev_join, 0));
+    if (two) {
+        CK(cudaEventRecord(h->ev_join, l1.stream));
+        CK(cudaStreamWaitEvent(l0.stream, h->ev_join, 0));
     }
     return KDME_OK;
 }
@@ -980,9 +973,12 @@ extern "C" int jbf_process_batch(jbf_handle* h, const float* depth_dev, const ui
     { int rc = guide_step(h, &bgr_step, "jbf_process_batch"); if (rc != KDME_OK) return rc; }
     DeviceGuard g(h->device);
     const size_t plane = (size_t)h->width * h->height;
-    return run_chunks(h, bgr_dev, bgr_step, n_frames, [&](int f0, int n) {
-        return launch_filter(h, depth_dev + (size_t)f0 * plane, h->guide4, h->guide_pitch, out_dev + (size_t)f0 * plane, n,
-                             kStagePlain, nullptr, 0, 0, -1, 0, -1, nullptr, nullptr, 0, 0, /*pdl=*/true);
+    return run_chunks(h, n_frames, h->max_batch, [&](Lane& lane, int, int f0, int n) {
+        int rc = launch_presmooth(h, lane, bgr_dev + (size_t)f0 * bgr_step * h->height, bgr_step, lane.guide4,
+                                  h->guide_pitch, n);
+        if (rc != KDME_OK) return rc;
+        return launch_filter(h, lane, filter_request(h, depth_dev + (size_t)f0 * plane, lane.guide4, h->guide_pitch,
+                                                     out_dev + (size_t)f0 * plane, n), /*pdl=*/true);
     });
 }
 
@@ -1001,12 +997,16 @@ extern "C" int jbf_process_xyz(jbf_handle* h, const float* depth_dev, const uint
         int rc2 = jbf_process_batch(h, depth_dev, bgr_dev, bgr_step, h->filtered_dev, 1);
         if (rc2 != KDME_OK) return rc2;
         DeviceGuard g(h->device);
-        return kdme_projective_to_real(h->filtered_dev, xyz_dev, h->width, h->height, fx, fy, cx, cy, h->stream);
+        return kdme_projective_to_real(h->filtered_dev, xyz_dev, h->width, h->height, fx, fy, cx, cy, h->lanes[0].stream);
     }
-    h->xyz_out = xyz_dev; h->xyz_fx = fx; h->xyz_fy = fy; h->xyz_cx = cx; h->xyz_cy = cy; h->xyz_yimg0 = 0;
-    const int rc = jbf_process_batch(h, depth_dev, bgr_dev, bgr_step, h->filtered_dev, 1);
-    h->xyz_out = nullptr;
-    return rc;
+    { int rc = guide_step(h, &bgr_step, "jbf_process_xyz"); if (rc != KDME_OK) return rc; }
+    DeviceGuard g(h->device);
+    Lane& lane = h->lanes[0];   // one frame: one chunk, on the caller's stream
+    int rc = launch_presmooth(h, lane, bgr_dev, bgr_step, lane.guide4, h->guide_pitch, 1);
+    if (rc != KDME_OK) return rc;
+    JbfParams p = filter_request(h, depth_dev, lane.guide4, h->guide_pitch, h->filtered_dev, 1);
+    p.xyz = xyz_dev; p.fx = fx; p.fy = fy; p.cx = cx; p.cy = cy;
+    return launch_filter(h, lane, p, /*pdl=*/true);
 }
 
 // Pixels re-evaluated in fp64 (ill-conditioned: no sample near the pass-1 mean) and pixels dropped because
@@ -1015,9 +1015,9 @@ extern "C" int jbf_refine_stats(jbf_handle* h, unsigned long long* refined, unsi
     if (!h) return fail(KDME_EINVAL, "jbf_refine_stats: NULL handle");
     DeviceGuard g(h->device);
     unsigned long long v[2] = {0, 0};
-    CK(cudaMemcpyAsync(v, h->stats_dev, sizeof(v), cudaMemcpyDeviceToHost, h->stream));
-    CK(cudaMemsetAsync(h->stats_dev, 0, sizeof(v), h->stream));
-    CK(cudaStreamSynchronize(h->stream));
+    CK(cudaMemcpyAsync(v, h->stats_dev, sizeof(v), cudaMemcpyDeviceToHost, h->lanes[0].stream));
+    CK(cudaMemsetAsync(h->stats_dev, 0, sizeof(v), h->lanes[0].stream));
+    CK(cudaStreamSynchronize(h->lanes[0].stream));
     if (refined) *refined = v[0];
     if (dropped) *dropped = v[1];
     return KDME_OK;
@@ -1034,15 +1034,20 @@ static int upsample_batch(jbf_handle* h, const float* depth_lo, const uint16_t* 
     DeviceGuard g(h->device);
     UpsampleGeom geom;
     size_t smem = 0;
-    if (ups_gather_form(h, wl, hl, h->height, h->xyz_out != nullptr, &geom, &smem)) {
+    if (ups_gather_form(h, wl, hl, h->height, &geom, &smem)) {
         int rc = ensure_ups_table(h, wl, hl, h->height);
         if (rc != KDME_OK) return rc;
     }
     const size_t plane = (size_t)h->width * h->height, lo_plane = (size_t)wl * hl;
-    return run_chunks(h, bgr_dev, bgr_step, n_frames, [&](int f0, int n) {
-        return launch_filter(h, nullptr, h->guide4, h->guide_pitch, out_dev + (size_t)f0 * plane, n, kStageUpsample,
-                             depth_lo ? depth_lo + (size_t)f0 * lo_plane : nullptr, wl, hl, -1, 0, -1, nullptr, nullptr,
-                             0, 0, /*pdl=*/true, depth_lo16 ? depth_lo16 + (size_t)f0 * lo_plane : nullptr);
+    return run_chunks(h, n_frames, h->max_batch, [&](Lane& lane, int, int f0, int n) {
+        int rc = launch_presmooth(h, lane, bgr_dev + (size_t)f0 * bgr_step * h->height, bgr_step, lane.guide4,
+                                  h->guide_pitch, n);
+        if (rc != KDME_OK) return rc;
+        JbfParams p = filter_request(h, nullptr, lane.guide4, h->guide_pitch, out_dev + (size_t)f0 * plane, n);
+        p.mode = kStageUpsample; p.wl = wl; p.hl = hl;
+        p.depth_lo = depth_lo ? depth_lo + (size_t)f0 * lo_plane : nullptr;
+        p.depth_lo16 = depth_lo16 ? depth_lo16 + (size_t)f0 * lo_plane : nullptr;
+        return launch_filter(h, lane, p, /*pdl=*/true);
     });
 }
 
@@ -1103,20 +1108,9 @@ static int process_host_impl(jbf_handle* h, const float* depth_host, const uint1
     if (depth16_host)
         for (int b = 0; b < kPipeDepth; b++)
             if (!h->pipe_depth16[b]) CK(cudaMalloc(&h->pipe_depth16[b], plane * h->pipe_chunk * sizeof(uint16_t)));
-    // compute of odd chunks runs on the internal lane (own stream, guide buffer and refinement queue)
-    const bool two = n_frames > h->pipe_chunk && !h->one_lane && h->fast;
-    if (two) {
-        rc = ensure_alt_lane(h);
-        if (rc != KDME_OK) return rc;
-        CK(cudaEventRecord(h->ev_fork, h->stream));
-        CK(cudaStreamWaitEvent(h->alt.stream, h->ev_fork, 0));
-    }
-    int chunk = 0;
-    for (int f0 = 0; f0 < n_frames; f0 += h->pipe_chunk, ++chunk) {
-        const int n = (n_frames - f0 < h->pipe_chunk) ? (n_frames - f0) : h->pipe_chunk;
-        const int b = chunk % kPipeDepth;
-        LaneScope lane(h, two && (chunk & 1));
-        if (chunk >= kPipeDepth) CK(cudaStreamWaitEvent(h->s_h2d, h->ev_done[b], 0));  // slot inputs consumed
+    rc = run_chunks(h, n_frames, h->pipe_chunk, [&](Lane& lane, int c, int f0, int n) {
+        const int b = c % kPipeDepth;
+        if (c >= kPipeDepth) CK(cudaStreamWaitEvent(h->s_h2d, h->ev_done[b], 0));  // slot inputs consumed
         if (depth16_host)
             CK(cudaMemcpyAsync(h->pipe_depth16[b], depth16_host + (size_t)f0 * plane, plane * n * sizeof(uint16_t),
                                cudaMemcpyHostToDevice, h->s_h2d));
@@ -1126,27 +1120,28 @@ static int process_host_impl(jbf_handle* h, const float* depth_host, const uint1
         CK(cudaMemcpyAsync(h->pipe_bgr[b], bgr_host + (size_t)f0 * bgr_frame, bgr_frame * n, cudaMemcpyHostToDevice,
                            h->s_h2d));
         CK(cudaEventRecord(h->ev_in[b], h->s_h2d));
-        CK(cudaStreamWaitEvent(h->stream, h->ev_in[b], 0));
-        if (chunk >= kPipeDepth) CK(cudaStreamWaitEvent(h->stream, h->ev_free[b], 0));  // slot output drained
+        CK(cudaStreamWaitEvent(lane.stream, h->ev_in[b], 0));
+        if (c >= kPipeDepth) CK(cudaStreamWaitEvent(lane.stream, h->ev_free[b], 0));  // slot output drained
         if (depth16_host) {   // sensor millimetres -> float, as Buffer2D::insertData(xn::DepthMetaData*) does (Buffer2D.cpp:18-32)
             const long long cnt = (long long)plane * n;
-            u16_to_f32_kernel<<<buf_blocks(cnt), 256, 0, h->stream>>>(h->pipe_depth16[b], h->pipe_depth[b], cnt);
+            u16_to_f32_kernel<<<buf_blocks(cnt), 256, 0, lane.stream>>>(h->pipe_depth16[b], h->pipe_depth[b], cnt);
             CK(cudaGetLastError());
         }
-        rc = launch_presmooth(h, h->pipe_bgr[b], bgr_step, h->guide4, h->guide_pitch, n);
+        int rc = launch_presmooth(h, lane, h->pipe_bgr[b], bgr_step, lane.guide4, h->guide_pitch, n);
         if (rc != KDME_OK) return rc;
-        rc = launch_filter(h, h->pipe_depth[b], h->guide4, h->guide_pitch, h->pipe_out[b], n, kStagePlain, nullptr, 0, 0, -1, 0,
-                           -1, nullptr, nullptr, 0, 0, /*pdl=*/true);
+        rc = launch_filter(h, lane, filter_request(h, h->pipe_depth[b], lane.guide4, h->guide_pitch, h->pipe_out[b], n),
+                           /*pdl=*/true);
         if (rc != KDME_OK) return rc;
-        CK(cudaEventRecord(h->ev_done[b], h->stream));
+        CK(cudaEventRecord(h->ev_done[b], lane.stream));
         CK(cudaStreamWaitEvent(h->s_d2h, h->ev_done[b], 0));
         CK(cudaMemcpyAsync(out_host + (size_t)f0 * plane, h->pipe_out[b], plane * n * sizeof(float),
                            cudaMemcpyDeviceToHost, h->s_d2h));
         CK(cudaEventRecord(h->ev_free[b], h->s_d2h));
-    }
+        return KDME_OK;
+    });
+    if (rc != KDME_OK) return rc;
     CK(cudaStreamSynchronize(h->s_d2h));
-    if (two) CK(cudaStreamSynchronize(h->alt.stream));
-    CK(cudaStreamSynchronize(h->stream));
+    CK(cudaStreamSynchronize(h->lanes[0].stream));
     return KDME_OK;
 }
 
@@ -1186,8 +1181,9 @@ extern "C" const float* jbf_filtered_host(jbf_handle* h) {
         fail(KDME_EINVAL, "jbf_filtered_host: cudaMallocHost failed");
         return nullptr;
     }
-    if (cudaMemcpyAsync(h->filtered_host, h->filtered_dev, bytes, cudaMemcpyDeviceToHost, h->stream) != cudaSuccess ||
-        cudaStreamSynchronize(h->stream) != cudaSuccess) {
+    cudaStream_t st = h->lanes[0].stream;
+    if (cudaMemcpyAsync(h->filtered_host, h->filtered_dev, bytes, cudaMemcpyDeviceToHost, st) != cudaSuccess ||
+        cudaStreamSynchronize(st) != cudaSuccess) {
         fail(KDME_EINVAL, "jbf_filtered_host: D2H copy failed");
         return nullptr;
     }
@@ -1197,16 +1193,17 @@ extern "C" const float* jbf_filtered_host(jbf_handle* h) {
 extern "C" const uint8_t* jbf_guide4_device(jbf_handle* h, size_t* step) {
     if (!h) return nullptr;
     if (step) *step = (size_t)h->guide_pitch * 4;
-    return reinterpret_cast<const uint8_t*>(h->guide4);
+    return reinterpret_cast<const uint8_t*>(h->lanes[0].guide4);
 }
 
 extern "C" const uint8_t* jbf_smooth_device(jbf_handle* h, size_t* step) {
     if (!h) return nullptr;
     DeviceGuard g(h->device);
+    const Lane& l0 = h->lanes[0];   // the guide of the last jbf_process
     const int C = h->guide_channels;
     const size_t bytes = (size_t)h->width * h->height * C;
     if (h->smooth_bytes != bytes) {
-        if (h->smooth_bgr && cudaStreamSynchronize(h->stream) != cudaSuccess) {
+        if (h->smooth_bgr && cudaStreamSynchronize(l0.stream) != cudaSuccess) {
             fail(KDME_EINVAL, "jbf_smooth_device: stream synchronisation failed");
             return nullptr;
         }
@@ -1220,9 +1217,9 @@ extern "C" const uint8_t* jbf_smooth_device(jbf_handle* h, size_t* step) {
     }
     dim3 blk(128), grd((h->width + 127) / 128, h->height);
     switch (C) {
-        case 1: guide4_to_image_kernel<1><<<grd, blk, 0, h->stream>>>(h->guide4, h->guide_pitch, h->smooth_bgr, h->width, h->height); break;
-        case 4: guide4_to_image_kernel<4><<<grd, blk, 0, h->stream>>>(h->guide4, h->guide_pitch, h->smooth_bgr, h->width, h->height); break;
-        default: guide4_to_image_kernel<3><<<grd, blk, 0, h->stream>>>(h->guide4, h->guide_pitch, h->smooth_bgr, h->width, h->height); break;
+        case 1: guide4_to_image_kernel<1><<<grd, blk, 0, l0.stream>>>(l0.guide4, h->guide_pitch, h->smooth_bgr, h->width, h->height); break;
+        case 4: guide4_to_image_kernel<4><<<grd, blk, 0, l0.stream>>>(l0.guide4, h->guide_pitch, h->smooth_bgr, h->width, h->height); break;
+        default: guide4_to_image_kernel<3><<<grd, blk, 0, l0.stream>>>(l0.guide4, h->guide_pitch, h->smooth_bgr, h->width, h->height); break;
     }
     if (step) *step = (size_t)h->width * C;
     return h->smooth_bgr;
@@ -1238,16 +1235,13 @@ extern "C" int jbf_mrf(jbf_handle* h, const float* depth_dev, const uint8_t* bgr
     if (depth_dev == out_dev) return fail(KDME_EINVAL, "jbf_mrf: in-place operation is not supported");
     { int rc = guide_step(h, &bgr_step, "jbf_mrf"); if (rc != KDME_OK) return rc; }
     DeviceGuard g(h->device);
-    switch (h->guide_channels) {
-        case 1: launch_guide4_convert<1>(h, bgr_dev, bgr_step, 0, h->guide4, h->guide_pitch, 0, h->height, 1); break;
-        case 4: launch_guide4_convert<4>(h, bgr_dev, bgr_step, 0, h->guide4, h->guide_pitch, 0, h->height, 1); break;
-        default: launch_guide4_convert<3>(h, bgr_dev, bgr_step, 0, h->guide4, h->guide_pitch, 0, h->height, 1); break;
-    }
+    Lane& l0 = h->lanes[0];
+    launch_guide4_convert(h, l0, bgr_dev, bgr_step, 0, l0.guide4, h->guide_pitch, 0, h->height, 1);
     CK(cudaGetLastError());
     constexpr int TW = 32, TH = 8;
     const int SP = TW + 2 * window_radius, SH = TH + 2 * window_radius;
     dim3 g2((h->width + TW - 1) / TW, (h->height + TH - 1) / TH);
-    mrf_kernel<TW, TH><<<g2, TW * TH, (size_t)SP * SH * 8, h->stream>>>(depth_dev, h->guide4, h->guide_pitch, out_dev,
+    mrf_kernel<TW, TH><<<g2, TW * TH, (size_t)SP * SH * 8, l0.stream>>>(depth_dev, l0.guide4, h->guide_pitch, out_dev,
                                                                         h->width, h->height, window_radius,
                                                                         color_sigma, smooth_sigma);
     CK(cudaGetLastError());

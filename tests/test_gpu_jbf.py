@@ -363,6 +363,49 @@ def test_two_lane_chunk_pipeline_bit_identical_and_repeatable(monkeypatch):
     assert torch.equal(oh.view(torch.int32), want.view(torch.int32))
 
 
+def test_two_lane_caches_follow_changing_calls(monkeypatch):
+    """Each lane keeps its own TMA descriptors and refinement queue from call to call.  A sequence whose buffers,
+    frame counts and kinds change between calls (so both lanes' cached descriptors go stale, and the host pipeline
+    and two upsampling sizes follow) gives the same bits and refinement counts as a single-lane handle."""
+    from kinectdepthmapenhancement_b200 import synth
+    w, h = 320, 240
+    depth, bgr = synth.rgbd_stream(12, w, h, seed=8)
+    a_d, a_c = depth[:7].cuda(), bgr[:7].cuda()
+    b_d, b_c = depth[7:].cuda(), bgr[7:].cuda()
+    dh, ch = depth[2:7].pin_memory(), bgr[2:7].pin_memory()
+    ups = []
+    for wl, hl in ((160, 120), (107, 80)):
+        lo = torch.stack([synth.rgbd_frame(wl, hl, seed=8, frame=k, noise_rel=0.01, hole_frac=0.1)[0]
+                          for k in range(5)])
+        ups.append((lo.cuda(), bgr[:5].cuda()))
+    JBF = _jbf_cls()
+
+    def run(f):
+        results = []
+
+        def record(out):
+            results.append((out.cpu().view(torch.int32), f.refine_stats()))
+
+        record(f.process_batch(a_d, a_c))
+        record(f.process_batch(b_d, b_c))
+        record(f.process_batch(a_d, a_c))
+        oh = torch.empty_like(dh).pin_memory()
+        f.process_host(dh, ch, oh)
+        record(oh)
+        for lo, hi in ups:
+            record(f.upsample_batch(lo, hi))
+        return results
+
+    monkeypatch.setenv("KDME_ONE_LANE", "1")
+    want = run(JBF(w, h, window_radius=7, max_batch=2))
+    monkeypatch.delenv("KDME_ONE_LANE")
+    got = run(JBF(w, h, window_radius=7, max_batch=2))
+    assert sum(stats[0] for _, stats in want) > 0     # the refinement queues are exercised
+    for k, ((g, gs), (e, es)) in enumerate(zip(got, want)):
+        assert torch.equal(g, e), k
+        assert gs == es, k
+
+
 def test_pitched_gpumat_step_is_honoured():
     """cv::gpu::GpuMat rows may be padded (step > 3*width); the reference ignores step (it indexes
     (y*W+x)*3, JointBilateralFilter.cu:22-24) and only works for continuous images.  Through the C ABI a
