@@ -98,7 +98,7 @@ def check_against_f64(out, depth, guide3, ws, ss, sc, sd, label=""):
 
 @pytest.mark.parametrize("w,h,radius", [(640, 480, 2), (640, 480, 7), (320, 240, 9), (256, 128, 15),
                                         (128, 96, 1), (192, 160, 4)])
-def test_filter_matches_f64_oracle_tma_path(w, h, radius):
+def test_filter_matches_f64_oracle_tma_path_both_tile_heights(w, h, radius):
     depth, bgr = synth_np(w, h, seed=1234, frame=radius)
     guide = oracle.presmooth(bgr)
     out, variant = gpu_filter(depth, guide, radius)
@@ -106,7 +106,7 @@ def test_filter_matches_f64_oracle_tma_path(w, h, radius):
     assert (variant & 1) == 0
     check_against_f64(out, depth, guide, 2 * radius + 1, 70.0, 50.0, 20.0, f"{w}x{h} variant=0x{variant:x}")
     # the other tile shape (64x16 instead of the 64x8 picked for small launches) must pass the same bound
-    out_big, vbig = gpu_filter(depth, guide, radius, env={"KDME_BIG_TILES": "1"})
+    out_big, vbig = gpu_filter(depth, guide, radius, env={"KDME_TILE_H": "16"})
     assert not (vbig & 0xA00)
     check_against_f64(out_big, depth, guide, 2 * radius + 1, 70.0, 50.0, 20.0, f"{w}x{h} variant=0x{vbig:x}")
 
