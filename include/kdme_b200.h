@@ -267,6 +267,37 @@ int kdme_guided_upsample_ex(const float *depth_lo_dev, int wl, int hl, const int
                             int width, int height, int window_radius, float sigma_spatial, float sigma_color,
                             float sigma_depth, void *stream);
 
+/* Streams of frames (a recorded ToF or Kinect sequence in one call): n_frames independent fills stored back to
+ * back, asynchronous on `stream`.  Frame strides: width*height depth samples, height*bgr_step guide bytes,
+ * width*height labels (labels_dev is NULL for one label, or holds n_frames label maps) and width*height output
+ * floats.  Frame k of the result equals kdme_guided_fill_ex on frame k alone, bit for bit; kdme_guided_fill(_ex)
+ * is the batch of one.  KDME_EINVAL: n_frames < 1, a NULL depth / guide / output pointer, a non-positive size, a
+ * radius outside [0, KDME_MAX_RADIUS], a guide format other than KDME_GUIDE_*, a guide step below C*width, or
+ * an output whose bytes overlap the depth input's (the fill does not run in place). */
+int kdme_guided_fill_batch(const float *depth_dev, const int32_t *labels_dev, const uint8_t *bgr_dev,
+                           size_t bgr_step, int guide_channels, float *out_dev, int width, int height, int n_frames,
+                           int window_radius, float sigma_spatial, float sigma_color, float sigma_depth,
+                           void *stream);
+/* The same with sensor depth: uint16 millimetres, read directly by the kernels (no conversion pass); a sample s
+ * filters exactly as the float (float)s, so values <= 50 are holes as before. */
+int kdme_guided_fill_batch_u16(const uint16_t *depth_dev, const int32_t *labels_dev, const uint8_t *bgr_dev,
+                               size_t bgr_step, int guide_channels, float *out_dev, int width, int height,
+                               int n_frames, int window_radius, float sigma_spatial, float sigma_color,
+                               float sigma_depth, void *stream);
+/* n_frames independent label-guided upsamplings, as kdme_guided_fill_batch: frame strides wl*hl low-res depth
+ * samples, height*bgr_step guide bytes, width*height labels (or NULL) and width*height output floats.  Frame k
+ * equals kdme_guided_upsample_ex on frame k alone, bit for bit; kdme_guided_upsample(_ex) is the batch of one.
+ * KDME_EINVAL as for the fill, with wl / hl outside [1, width] / [1, height] in place of the overlap check. */
+int kdme_guided_upsample_batch(const float *depth_lo_dev, int wl, int hl, const int32_t *labels_hi_dev,
+                               const uint8_t *bgr_hi_dev, size_t bgr_step, int guide_channels, float *out_hi_dev,
+                               int width, int height, int n_frames, int window_radius, float sigma_spatial,
+                               float sigma_color, float sigma_depth, void *stream);
+/* The same with uint16 low-res depth (Kinect v2 512x424, Azure Kinect 640x576 millimetres). */
+int kdme_guided_upsample_batch_u16(const uint16_t *depth_lo_dev, int wl, int hl, const int32_t *labels_hi_dev,
+                                   const uint8_t *bgr_hi_dev, size_t bgr_step, int guide_channels,
+                                   float *out_hi_dev, int width, int height, int n_frames, int window_radius,
+                                   float sigma_spatial, float sigma_color, float sigma_depth, void *stream);
+
 /* ========================= ArrayBuffer / Buffer2D ========================= */
 typedef struct buf2d_handle buf2d_handle;
 

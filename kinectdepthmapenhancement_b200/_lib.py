@@ -77,6 +77,10 @@ SIGNATURES = {
     "kdme_guided_fill": (_i, [_vp, _vp, _vp, _sz, _vp, _i, _i, _i, _f, _f, _f, _vp]),
     "kdme_guided_upsample_ex": (_i, [_vp, _i, _i, _vp, _vp, _sz, _i, _vp, _i, _i, _i, _f, _f, _f, _vp]),
     "kdme_guided_fill_ex": (_i, [_vp, _vp, _vp, _sz, _i, _vp, _i, _i, _i, _f, _f, _f, _vp]),
+    "kdme_guided_fill_batch": (_i, [_vp, _vp, _vp, _sz, _i, _vp, _i, _i, _i, _i, _f, _f, _f, _vp]),
+    "kdme_guided_fill_batch_u16": (_i, [_vp, _vp, _vp, _sz, _i, _vp, _i, _i, _i, _i, _f, _f, _f, _vp]),
+    "kdme_guided_upsample_batch": (_i, [_vp, _i, _i, _vp, _vp, _sz, _i, _vp, _i, _i, _i, _i, _f, _f, _f, _vp]),
+    "kdme_guided_upsample_batch_u16": (_i, [_vp, _i, _i, _vp, _vp, _sz, _i, _vp, _i, _i, _i, _i, _f, _f, _f, _vp]),
     "buf2d_create": (_i, [C.POINTER(_vp), _i, _i, _i, _vp]),
     "buf2d_destroy": (None, [_vp]),
     "buf2d_init": (_i, [_vp]),

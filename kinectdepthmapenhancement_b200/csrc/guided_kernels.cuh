@@ -18,6 +18,11 @@
 // the word {g,0,0,0} and a BGRX pixel as {b,g,r,0}, so the colour distance is that of the BGR
 // image (g,0,0) or (b,g,r), bit for bit.
 //
+// Both guided kernels filter a stream of frames: the frame is blockIdx.z, which offsets every plane by its
+// per-frame stride, so frame k of a launch equals a launch on frame k alone, bit for bit.  The depth is float32 or,
+// in the U16 instantiations, uint16 millimetres (see guided_depth); a template parameter rather than a branch keeps
+// the float32 kernels' code as it was.
+//
 // mrf_kernel follows MarkovRandomField/MarkovRandomField.cu:4-40 (next row f1).
 #pragma once
 #include "common.cuh"
@@ -27,15 +32,20 @@ namespace kdme {
 struct GuidedParams {
     int width, height, radius;
     const float* depth;
+    const uint16_t* depth16;  // the depth as uint16 millimetres, read instead of `depth` by the U16 kernels
     const int32_t* labels;  // nullable
     const uint8_t* bgr;     // RAW guide, packed C-channel pixels (kernel template parameter C = 1, 3 or 4)
     long long bgr_step;
     float* out;
     float sigma_c, sigma_d;
-    // upsampling form (SURVEY.md 8(d) config 3, label-guided variant): when depth_lo != nullptr the depth
-    // plane is the sparse scatter of a wl x hl low-res map (see upsample_site) and `depth` is ignored
+    // upsampling form (SURVEY.md 8(d) config 3, label-guided variant): when depth_lo or depth_lo16 is non-null the
+    // depth plane is the sparse scatter of a wl x hl low-res map (see upsample_site) and `depth` is ignored
     const float* depth_lo;
+    const uint16_t* depth_lo16;   // read instead of depth_lo by the U16 kernels
     int wl, hl;
+    // per-frame strides (frame = blockIdx.z): depth samples (width*height, or wl*hl for the upsampling), guide bytes
+    // (height*bgr_step), labels (width*height; 0 without labels), output floats (width*height)
+    long long depth_stride, bgr_stride, labels_stride, out_stride;
     float spatial[31 * 31];  // the reference's fp32 LUT (EdgeRefinedSuperpixel.cpp:46-55)
 };
 
@@ -47,7 +57,22 @@ __device__ __forceinline__ int guided_upsample_site(int x, int W, int wl) {
     return ((int)(((2LL * xl + 1) * W) / (2LL * wl)) == x) ? xl : -1;
 }
 
-template <int TW, int TH, int C>
+// Depth at image pixel (gx, gy) of `frame`: every depth read of both guided kernels goes through here.  The
+// upsampling reads the low-res sample landing on the pixel (0 where none does).  A uint16 sample s reads as the
+// float (float)s, exactly (s <= 50 is a hole, as for the float input).
+template <bool U16, class P>
+__device__ __forceinline__ float guided_depth(const P& p, long long frame, int gx, int gy) {
+    if (p.depth_lo || p.depth_lo16) {
+        const int xl = guided_upsample_site(gx, p.width, p.wl), yl = guided_upsample_site(gy, p.height, p.hl);
+        if ((xl < 0) | (yl < 0)) return 0.f;
+        const long long i = (long long)frame * p.depth_stride + (long long)yl * p.wl + xl;
+        if constexpr (U16) return (float)__ldg(p.depth_lo16 + i); else return __ldg(p.depth_lo + i);
+    }
+    const long long i = (long long)frame * p.depth_stride + (long long)gy * p.width + gx;
+    if constexpr (U16) return (float)__ldg(p.depth16 + i); else return __ldg(p.depth + i);
+}
+
+template <int TW, int TH, int C, bool U16>
 __global__ void __launch_bounds__(TW * TH) guided_fill_kernel(const __grid_constant__ GuidedParams p) {
     constexpr int NT = TW * TH;
     const int R = p.radius, WS = 2 * R + 1, SP = TW + 2 * R, SH = TH + 2 * R;
@@ -58,6 +83,9 @@ __global__ void __launch_bounds__(TW * TH) guided_fill_kernel(const __grid_const
     __shared__ float sL[31 * 31];
     const int tid = threadIdx.x;
     const int x0 = blockIdx.x * TW, y0 = blockIdx.y * TH;
+    const long long frame = blockIdx.z;
+    const uint8_t* bgr = p.bgr + frame * p.bgr_stride;
+    const int32_t* labels = p.labels ? p.labels + frame * p.labels_stride : nullptr;
     for (int idx = tid; idx < SP * SH; idx += NT) {
         int sy = idx / SP, sx = idx - sy * SP;
         int gx = x0 - R + sx, gy = y0 - R + sy;
@@ -66,17 +94,11 @@ __global__ void __launch_bounds__(TW * TH) guided_fill_kernel(const __grid_const
         uint32_t g = 0u;
         int32_t l = 0;
         if (in) {
-            const long long k = (long long)gy * p.width + gx;
-            if (p.depth_lo) {
-                const int xl = guided_upsample_site(gx, p.width, p.wl), yl = guided_upsample_site(gy, p.height, p.hl);
-                if ((xl >= 0) & (yl >= 0)) d = __ldg(p.depth_lo + (long long)yl * p.wl + xl);
-            } else {
-                d = __ldg(p.depth + k);
-            }
-            const uint8_t* q = p.bgr + (long long)gy * p.bgr_step + C * gx;
+            d = guided_depth<U16>(p, frame, gx, gy);
+            const uint8_t* q = bgr + (long long)gy * p.bgr_step + C * gx;
             if constexpr (C == 1) g = (uint32_t)__ldg(q);
             else g = (uint32_t)__ldg(q) | ((uint32_t)__ldg(q + 1) << 8) | ((uint32_t)__ldg(q + 2) << 16);
-            if (p.labels) l = __ldg(p.labels + k);
+            if (labels) l = __ldg(labels + (long long)gy * p.width + gx);
         }
         sD[idx] = (d > kValidDepth) ? d : 0.f;  // 0 marks "not a sample" (also out of bounds)
         sG[idx] = g;
@@ -176,7 +198,7 @@ __global__ void __launch_bounds__(TW * TH) guided_fill_kernel(const __grid_const
         if (poisoned) o = __int_as_float(0x7fc00000);
         else o = (den == 0.0f) ? 0.0f : mean + num / den;
     }
-    p.out[(long long)gy * p.width + gx] = o;
+    p.out[frame * p.out_stride + (long long)gy * p.width + gx] = o;
 }
 
 // -----------------------------------------------------------------------------
@@ -191,17 +213,20 @@ template <int R>
 struct GuidedFastParams {
     int width, height;
     const float* depth;
+    const uint16_t* depth16;
     const int32_t* labels;  // nullable
     const uint8_t* bgr;
     long long bgr_step;
     float* out;
     float sigma_c, nk0 /* -log2e/(2 sigma_c^2) */, sq /* sqrt(log2e/(2 sigma_d^2)) */;
     const float* depth_lo;
+    const uint16_t* depth_lo16;
     int wl, hl;
+    long long depth_stride, bgr_stride, labels_stride, out_stride;   // as in GuidedParams
     float ltab[(2 * R + 1) * (2 * R + 1)];   // log2(S_ij) + kWeightBias, or kWeightBias where S_ij == 0
 };
 
-template <int R, int TW, int TH, int C>
+template <int R, int TW, int TH, int C, bool U16>
 __global__ void __launch_bounds__(TW * TH) guided_fill_fast_kernel(const __grid_constant__ GuidedFastParams<R> p) {
     constexpr int NT = TW * TH, WS = 2 * R + 1, SP = TW + 2 * R, SH = TH + 2 * R;
     static_assert(WS * WS <= 64, "the same-label mask is one 64-bit word");
@@ -210,6 +235,9 @@ __global__ void __launch_bounds__(TW * TH) guided_fill_fast_kernel(const __grid_
     __shared__ int32_t sLab[SP * SH];
     const int tid = threadIdx.x;
     const int x0 = blockIdx.x * TW, y0 = blockIdx.y * TH;
+    const long long frame = blockIdx.z;
+    const uint8_t* bgr = p.bgr + frame * p.bgr_stride;
+    const int32_t* labels = p.labels ? p.labels + frame * p.labels_stride : nullptr;
     for (int idx = tid; idx < SP * SH; idx += NT) {
         int sy = idx / SP, sx = idx - sy * SP;
         int gx = x0 - R + sx, gy = y0 - R + sy;
@@ -218,17 +246,11 @@ __global__ void __launch_bounds__(TW * TH) guided_fill_fast_kernel(const __grid_
         uint32_t g = 0u;
         int32_t l = 0;
         if (in) {
-            const long long k = (long long)gy * p.width + gx;
-            if (p.depth_lo) {
-                const int xl = guided_upsample_site(gx, p.width, p.wl), yl = guided_upsample_site(gy, p.height, p.hl);
-                if ((xl >= 0) & (yl >= 0)) d = __ldg(p.depth_lo + (long long)yl * p.wl + xl);
-            } else {
-                d = __ldg(p.depth + k);
-            }
-            const uint8_t* q = p.bgr + (long long)gy * p.bgr_step + C * gx;
+            d = guided_depth<U16>(p, frame, gx, gy);
+            const uint8_t* q = bgr + (long long)gy * p.bgr_step + C * gx;
             if constexpr (C == 1) g = (uint32_t)__ldg(q);
             else g = (uint32_t)__ldg(q) | ((uint32_t)__ldg(q + 1) << 8) | ((uint32_t)__ldg(q + 2) << 16);
-            if (p.labels) l = __ldg(p.labels + k);
+            if (labels) l = __ldg(labels + (long long)gy * p.width + gx);
         }
         sD[idx] = (d > kValidDepth) ? d : 0.f;
         sG[idx] = g;
@@ -344,7 +366,7 @@ __global__ void __launch_bounds__(TW * TH) guided_fill_fast_kernel(const __grid_
         if (poisoned) o = __int_as_float(0x7fc00000);
         else o = (den == 0.0f) ? 0.0f : mean + num / den;
     }
-    p.out[(long long)gy * p.width + gx] = o;
+    p.out[frame * p.out_stride + (long long)gy * p.width + gx] = o;
 }
 
 // MarkovRandomField.cu:4-40: out = (d_p + sum f d_q) / (1 + sum f), f = smooth * expf(-sigma_c * cd)

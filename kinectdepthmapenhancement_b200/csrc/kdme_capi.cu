@@ -1291,89 +1291,173 @@ extern "C" int kdme_mean_3d_error(const float* points_dev, const float* truth_de
 }
 
 // ------------------------------------------------------------------ guided fill
+// One guided call over n_frames frames stored back to back.  The depth is exactly one of depth / depth16 (the fill:
+// width x height samples per frame) or depth_lo / depth_lo16 (the upsampling: wl x hl samples per frame).
+struct GuidedCall {
+    const float* depth; const uint16_t* depth16;
+    const float* depth_lo; const uint16_t* depth_lo16; int wl, hl;
+    const int32_t* labels; const uint8_t* bgr; size_t bgr_step;
+    float* out; int width, height, n_frames, radius;
+    float sigma_s, sigma_c, sigma_d;
+};
+
+constexpr int kGuidedTW = 32, kGuidedTH = 8;
+constexpr int kMaxGridZ = 65535;   // gridDim.z limit: frames per launch
+
+template <class T>
+static T* advance(T* ptr, long long n) { return ptr ? ptr + n : ptr; }
+
+// The fields GuidedParams and GuidedFastParams<R> share: image, pointers and per-frame strides.
+template <class P>
+static void guided_common(P& p, const GuidedCall& c) {
+    const long long plane = (long long)c.width * c.height;
+    p.width = c.width; p.height = c.height;
+    p.depth = c.depth; p.depth16 = c.depth16; p.depth_lo = c.depth_lo; p.depth_lo16 = c.depth_lo16;
+    p.wl = c.wl; p.hl = c.hl;
+    p.labels = c.labels; p.bgr = c.bgr; p.bgr_step = (long long)c.bgr_step; p.out = c.out;
+    p.depth_stride = (c.depth_lo || c.depth_lo16) ? (long long)c.wl * c.hl : plane;
+    p.bgr_stride = (long long)c.height * (long long)c.bgr_step;
+    p.labels_stride = c.labels ? plane : 0;
+    p.out_stride = plane;
+}
+
+// Launches `kernel` over the call's frames in slices of at most kMaxGridZ frames (blockIdx.z), in order on one
+// stream; each slice's pointers start at its first frame.
+template <class P>
+static int guided_slices(const P& p0, int n_frames, void (*kernel)(const P), size_t smem, cudaStream_t st) {
+    P p = p0;
+    for (int f0 = 0; f0 < n_frames; f0 += kMaxGridZ) {
+        const long long f = f0;
+        p.depth = advance(p0.depth, f * p0.depth_stride);
+        p.depth16 = advance(p0.depth16, f * p0.depth_stride);
+        p.depth_lo = advance(p0.depth_lo, f * p0.depth_stride);
+        p.depth_lo16 = advance(p0.depth_lo16, f * p0.depth_stride);
+        p.labels = advance(p0.labels, f * p0.labels_stride);
+        p.bgr = p0.bgr + f * p0.bgr_stride;
+        p.out = p0.out + f * p0.out_stride;
+        const dim3 grd((p.width + kGuidedTW - 1) / kGuidedTW, (p.height + kGuidedTH - 1) / kGuidedTH,
+                       std::min(kMaxGridZ, n_frames - f0));
+        kernel<<<grd, kGuidedTW * kGuidedTH, smem, st>>>(p);
+        CK(cudaGetLastError());
+    }
+    return KDME_OK;
+}
+
 template <int R, int C>
-static int guided_launch_fast(const float* depth_dev, const float* depth_lo_dev, int wl, int hl, const int32_t* labels_dev,
-                              const uint8_t* bgr_dev, size_t bgr_step, float* out_dev, int width, int height,
-                              const std::vector<float>& lut, float sigma_color, float sigma_depth, cudaStream_t stream) {
+static int guided_launch_fast(const GuidedCall& c, const std::vector<float>& lut, cudaStream_t stream) {
     constexpr int ws = 2 * R + 1;
     GuidedFastParams<R> p;
     for (int i = 0; i < ws * ws; i++)
         p.ltab[i] = (lut[i] != 0.0f) ? (float)(std::log2((double)lut[i]) + (double)kWeightBias) : kWeightBias;
-    p.width = width; p.height = height;
-    p.depth = depth_dev; p.labels = labels_dev; p.bgr = bgr_dev; p.bgr_step = (long long)bgr_step; p.out = out_dev;
-    p.sigma_c = sigma_color;
-    p.nk0 = (float)(-kLog2e / (2.0 * (double)sigma_color * (double)sigma_color));
-    p.sq = sqrtf((float)kLog2e / (2.0f * sigma_depth * sigma_depth));
-    p.depth_lo = depth_lo_dev; p.wl = wl; p.hl = hl;
-    constexpr int TW = 32, TH = 8;
-    dim3 grd((width + TW - 1) / TW, (height + TH - 1) / TH);
-    guided_fill_fast_kernel<R, TW, TH, C><<<grd, TW * TH, 0, stream>>>(p);
-    CK(cudaGetLastError());
-    return KDME_OK;
+    guided_common(p, c);
+    p.sigma_c = c.sigma_c;
+    p.nk0 = (float)(-kLog2e / (2.0 * (double)c.sigma_c * (double)c.sigma_c));
+    p.sq = sqrtf((float)kLog2e / (2.0f * c.sigma_d * c.sigma_d));
+    if (c.depth16 || c.depth_lo16)
+        return guided_slices(p, c.n_frames, guided_fill_fast_kernel<R, kGuidedTW, kGuidedTH, C, true>, 0, stream);
+    return guided_slices(p, c.n_frames, guided_fill_fast_kernel<R, kGuidedTW, kGuidedTH, C, false>, 0, stream);
 }
 
+// The spatial LUT and the kernel are chosen once per call, whatever the number of frames.
 template <int C>
-static int guided_launch_c(const float* depth_dev, const float* depth_lo_dev, int wl, int hl, const int32_t* labels_dev,
-                           const uint8_t* bgr_dev, size_t bgr_step, float* out_dev, int width, int height,
-                           int window_radius, float sigma_spatial, float sigma_color, float sigma_depth, void* stream) {
-    const int ws = 2 * window_radius + 1;
+static int guided_launch_c(const GuidedCall& c, cudaStream_t stream) {
+    const int ws = 2 * c.radius + 1;
     std::vector<float> lut;
-    host_spatial_lut(lut, ws, sigma_spatial);
+    host_spatial_lut(lut, ws, c.sigma_s);
     // fast form: compile-time window (3..7), sweep-1 colour guard cannot fire (expf(-3*255^2/(2 sc^2)) != 0)
-    const bool fast_ok = sigma_color != 0.0f && sigma_depth != 0.0f &&
-                         expf(-(float)(3 * 255 * 255) / (2 * (sigma_color * sigma_color))) != 0.0f;
-    auto fast = [&](auto r) {
-        return guided_launch_fast<decltype(r)::value, C>(depth_dev, depth_lo_dev, wl, hl, labels_dev, bgr_dev, bgr_step,
-                                                         out_dev, width, height, lut, sigma_color, sigma_depth,
-                                                         (cudaStream_t)stream);
-    };
+    const bool fast_ok = c.sigma_c != 0.0f && c.sigma_d != 0.0f &&
+                         expf(-(float)(3 * 255 * 255) / (2 * (c.sigma_c * c.sigma_c))) != 0.0f;
     if (fast_ok) {
-        switch (window_radius) {
-            case 1: return fast(std::integral_constant<int, 1>{});
-            case 2: return fast(std::integral_constant<int, 2>{});
-            case 3: return fast(std::integral_constant<int, 3>{});
+        switch (c.radius) {
+            case 1: return guided_launch_fast<1, C>(c, lut, stream);
+            case 2: return guided_launch_fast<2, C>(c, lut, stream);
+            case 3: return guided_launch_fast<3, C>(c, lut, stream);
             default: break;
         }
     }
     GuidedParams p;
     if (ws * ws > (int)(sizeof(p.spatial) / sizeof(float))) return fail(KDME_ENOTSUP, "guided fill: window too large");
     for (int i = 0; i < ws * ws; i++) p.spatial[i] = lut[i];
-    p.width = width; p.height = height; p.radius = window_radius;
-    p.depth = depth_dev; p.labels = labels_dev; p.bgr = bgr_dev; p.bgr_step = (long long)bgr_step; p.out = out_dev;
-    p.sigma_c = sigma_color; p.sigma_d = sigma_depth;
-    p.depth_lo = depth_lo_dev; p.wl = wl; p.hl = hl;
-    constexpr int TW = 32, TH = 8;
-    const int SP = TW + 2 * window_radius, SH = TH + 2 * window_radius;
-    dim3 grd((width + TW - 1) / TW, (height + TH - 1) / TH);
-    guided_fill_kernel<TW, TH, C><<<grd, TW * TH, (size_t)SP * SH * 12, (cudaStream_t)stream>>>(p);
-    CK(cudaGetLastError());
-    return KDME_OK;
+    guided_common(p, c);
+    p.radius = c.radius;
+    p.sigma_c = c.sigma_c; p.sigma_d = c.sigma_d;
+    const int SP = kGuidedTW + 2 * c.radius, SH = kGuidedTH + 2 * c.radius;
+    if (c.depth16 || c.depth_lo16)
+        return guided_slices(p, c.n_frames, guided_fill_kernel<kGuidedTW, kGuidedTH, C, true>, (size_t)SP * SH * 12, stream);
+    return guided_slices(p, c.n_frames, guided_fill_kernel<kGuidedTW, kGuidedTH, C, false>, (size_t)SP * SH * 12, stream);
 }
 
-static int guided_launch(const float* depth_dev, const float* depth_lo_dev, int wl, int hl, const int32_t* labels_dev,
-                         const uint8_t* bgr_dev, size_t bgr_step, int channels, float* out_dev, int width, int height,
-                         int window_radius, float sigma_spatial, float sigma_color, float sigma_depth, void* stream) {
+// The checks every guided entry point shares, then the launch.  `depth` is the call's depth input (any of the four
+// forms), on the current device.
+static int guided_run(GuidedCall c, const void* depth, int channels, void* stream, const char* who) {
+    if (c.radius < 0 || c.radius > KDME_MAX_RADIUS) return fail(KDME_EINVAL, std::string(who) + ": bad radius");
     if (channels != KDME_GUIDE_GRAY && channels != KDME_GUIDE_BGR && channels != KDME_GUIDE_BGRX)
-        return fail(KDME_EINVAL, "guided fill: guide_channels must be 1 (GRAY), 3 (BGR) or 4 (BGRX)");
-    { int rc = check_guide_step(channels, width, &bgr_step, "guided fill"); if (rc != KDME_OK) return rc; }
-    return with_channels(channels, [&](auto c) {
-        return guided_launch_c<decltype(c)::value>(depth_dev, depth_lo_dev, wl, hl, labels_dev, bgr_dev, bgr_step, out_dev,
-                                                   width, height, window_radius, sigma_spatial, sigma_color, sigma_depth,
-                                                   stream);
-    });
+        return fail(KDME_EINVAL, std::string(who) + ": guide_channels must be 1 (GRAY), 3 (BGR) or 4 (BGRX)");
+    { int rc = check_guide_step(channels, c.width, &c.bgr_step, who); if (rc != KDME_OK) return rc; }
+    { int rcd = check_pointer_device(depth, who); if (rcd != KDME_OK) return rcd; }
+    return with_channels(channels, [&](auto ch) { return guided_launch_c<decltype(ch)::value>(c, (cudaStream_t)stream); });
+}
+
+// n_frames fills; the depth is float (depth) or uint16 (depth16), the other one is NULL.
+static int guided_fill_batch(const float* depth, const uint16_t* depth16, const int32_t* labels, const uint8_t* bgr,
+                             size_t bgr_step, int channels, float* out, int width, int height, int n_frames,
+                             int window_radius, float sigma_spatial, float sigma_color, float sigma_depth, void* stream,
+                             const char* who) {
+    const void* in = depth ? (const void*)depth : (const void*)depth16;
+    if (!in || !bgr || !out) return fail(KDME_EINVAL, std::string(who) + ": NULL argument");
+    if (n_frames < 1) return fail(KDME_EINVAL, std::string(who) + ": n_frames must be >= 1");
+    if (width <= 0 || height <= 0) return fail(KDME_EINVAL, std::string(who) + ": bad size");
+    // the kernels read every frame's depth while they write the output: the two byte ranges must be disjoint
+    const unsigned long long px = (unsigned long long)width * height * n_frames;
+    const uintptr_t i0 = (uintptr_t)in, i1 = i0 + px * (depth ? sizeof(float) : sizeof(uint16_t));
+    const uintptr_t o0 = (uintptr_t)out, o1 = o0 + px * sizeof(float);
+    if (i0 < o1 && o0 < i1)
+        return fail(KDME_EINVAL, std::string(who) + ": the output overlaps the depth input (in-place operation is not supported)");
+    GuidedCall c{depth, depth16, nullptr, nullptr, 0, 0, labels, bgr, bgr_step, out, width, height, n_frames,
+                 window_radius, sigma_spatial, sigma_color, sigma_depth};
+    return guided_run(c, in, channels, stream, who);
+}
+
+// n_frames upsamplings; the low-res depth is float (depth_lo) or uint16 (depth_lo16), the other one is NULL.
+static int guided_upsample_batch(const float* depth_lo, const uint16_t* depth_lo16, int wl, int hl,
+                                 const int32_t* labels_hi, const uint8_t* bgr_hi, size_t bgr_step, int channels,
+                                 float* out_hi, int width, int height, int n_frames, int window_radius,
+                                 float sigma_spatial, float sigma_color, float sigma_depth, void* stream,
+                                 const char* who) {
+    const void* in = depth_lo ? (const void*)depth_lo : (const void*)depth_lo16;
+    if (!in || !bgr_hi || !out_hi) return fail(KDME_EINVAL, std::string(who) + ": NULL argument");
+    if (n_frames < 1) return fail(KDME_EINVAL, std::string(who) + ": n_frames must be >= 1");
+    if (width <= 0 || height <= 0 || wl <= 0 || hl <= 0 || wl > width || hl > height)
+        return fail(KDME_EINVAL, std::string(who) + ": low-res size must be positive and <= the high-res size");
+    GuidedCall c{nullptr, nullptr, depth_lo, depth_lo16, wl, hl, labels_hi, bgr_hi, bgr_step, out_hi, width, height,
+                 n_frames, window_radius, sigma_spatial, sigma_color, sigma_depth};
+    return guided_run(c, in, channels, stream, who);
+}
+
+extern "C" int kdme_guided_fill_batch(const float* depth_dev, const int32_t* labels_dev, const uint8_t* bgr_dev,
+                                      size_t bgr_step, int guide_channels, float* out_dev, int width, int height,
+                                      int n_frames, int window_radius, float sigma_spatial, float sigma_color,
+                                      float sigma_depth, void* stream) {
+    return guided_fill_batch(depth_dev, nullptr, labels_dev, bgr_dev, bgr_step, guide_channels, out_dev, width, height,
+                             n_frames, window_radius, sigma_spatial, sigma_color, sigma_depth, stream,
+                             "kdme_guided_fill_batch");
+}
+
+extern "C" int kdme_guided_fill_batch_u16(const uint16_t* depth_dev, const int32_t* labels_dev, const uint8_t* bgr_dev,
+                                          size_t bgr_step, int guide_channels, float* out_dev, int width, int height,
+                                          int n_frames, int window_radius, float sigma_spatial, float sigma_color,
+                                          float sigma_depth, void* stream) {
+    return guided_fill_batch(nullptr, depth_dev, labels_dev, bgr_dev, bgr_step, guide_channels, out_dev, width, height,
+                             n_frames, window_radius, sigma_spatial, sigma_color, sigma_depth, stream,
+                             "kdme_guided_fill_batch_u16");
 }
 
 extern "C" int kdme_guided_fill_ex(const float* depth_dev, const int32_t* labels_dev, const uint8_t* bgr_dev,
                                    size_t bgr_step, int guide_channels, float* out_dev, int width, int height,
                                    int window_radius, float sigma_spatial, float sigma_color, float sigma_depth,
                                    void* stream) {
-    if (!depth_dev || !bgr_dev || !out_dev) return fail(KDME_EINVAL, "kdme_guided_fill: NULL argument");
-    if (width <= 0 || height <= 0) return fail(KDME_EINVAL, "kdme_guided_fill: bad size");
-    if (window_radius < 0 || window_radius > KDME_MAX_RADIUS) return fail(KDME_EINVAL, "kdme_guided_fill: bad radius");
-    if (depth_dev == out_dev) return fail(KDME_EINVAL, "kdme_guided_fill: in-place operation is not supported");
-    { int rcd = check_pointer_device(depth_dev, "kdme_guided_fill"); if (rcd != KDME_OK) return rcd; }
-    return guided_launch(depth_dev, nullptr, 0, 0, labels_dev, bgr_dev, bgr_step, guide_channels, out_dev, width, height,
-                         window_radius, sigma_spatial, sigma_color, sigma_depth, stream);
+    return guided_fill_batch(depth_dev, nullptr, labels_dev, bgr_dev, bgr_step, guide_channels, out_dev, width, height,
+                             1, window_radius, sigma_spatial, sigma_color, sigma_depth, stream, "kdme_guided_fill");
 }
 
 extern "C" int kdme_guided_fill(const float* depth_dev, const int32_t* labels_dev, const uint8_t* bgr_dev,
@@ -1383,17 +1467,32 @@ extern "C" int kdme_guided_fill(const float* depth_dev, const int32_t* labels_de
                                window_radius, sigma_spatial, sigma_color, sigma_depth, stream);
 }
 
+extern "C" int kdme_guided_upsample_batch(const float* depth_lo_dev, int wl, int hl, const int32_t* labels_hi_dev,
+                                          const uint8_t* bgr_hi_dev, size_t bgr_step, int guide_channels,
+                                          float* out_hi_dev, int width, int height, int n_frames, int window_radius,
+                                          float sigma_spatial, float sigma_color, float sigma_depth, void* stream) {
+    return guided_upsample_batch(depth_lo_dev, nullptr, wl, hl, labels_hi_dev, bgr_hi_dev, bgr_step, guide_channels,
+                                 out_hi_dev, width, height, n_frames, window_radius, sigma_spatial, sigma_color,
+                                 sigma_depth, stream, "kdme_guided_upsample_batch");
+}
+
+extern "C" int kdme_guided_upsample_batch_u16(const uint16_t* depth_lo_dev, int wl, int hl,
+                                              const int32_t* labels_hi_dev, const uint8_t* bgr_hi_dev, size_t bgr_step,
+                                              int guide_channels, float* out_hi_dev, int width, int height,
+                                              int n_frames, int window_radius, float sigma_spatial, float sigma_color,
+                                              float sigma_depth, void* stream) {
+    return guided_upsample_batch(nullptr, depth_lo_dev, wl, hl, labels_hi_dev, bgr_hi_dev, bgr_step, guide_channels,
+                                 out_hi_dev, width, height, n_frames, window_radius, sigma_spatial, sigma_color,
+                                 sigma_depth, stream, "kdme_guided_upsample_batch_u16");
+}
+
 extern "C" int kdme_guided_upsample_ex(const float* depth_lo_dev, int wl, int hl, const int32_t* labels_hi_dev,
                                        const uint8_t* bgr_hi_dev, size_t bgr_step, int guide_channels, float* out_hi_dev,
                                        int width, int height, int window_radius, float sigma_spatial, float sigma_color,
                                        float sigma_depth, void* stream) {
-    if (!depth_lo_dev || !bgr_hi_dev || !out_hi_dev) return fail(KDME_EINVAL, "kdme_guided_upsample: NULL argument");
-    if (width <= 0 || height <= 0 || wl <= 0 || hl <= 0 || wl > width || hl > height)
-        return fail(KDME_EINVAL, "kdme_guided_upsample: low-res size must be positive and <= the high-res size");
-    if (window_radius < 0 || window_radius > KDME_MAX_RADIUS) return fail(KDME_EINVAL, "kdme_guided_upsample: bad radius");
-    { int rcd = check_pointer_device(depth_lo_dev, "kdme_guided_upsample"); if (rcd != KDME_OK) return rcd; }
-    return guided_launch(nullptr, depth_lo_dev, wl, hl, labels_hi_dev, bgr_hi_dev, bgr_step, guide_channels, out_hi_dev,
-                         width, height, window_radius, sigma_spatial, sigma_color, sigma_depth, stream);
+    return guided_upsample_batch(depth_lo_dev, nullptr, wl, hl, labels_hi_dev, bgr_hi_dev, bgr_step, guide_channels,
+                                 out_hi_dev, width, height, 1, window_radius, sigma_spatial, sigma_color, sigma_depth,
+                                 stream, "kdme_guided_upsample");
 }
 
 extern "C" int kdme_guided_upsample(const float* depth_lo_dev, int wl, int hl, const int32_t* labels_hi_dev,
