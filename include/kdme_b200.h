@@ -226,7 +226,8 @@ int kdme_projective_to_real(const float *depth_dev, float *xyz_dev, int width, i
 
 /* "Next" row f2: Projection_GPU::bilateralfilter (Projection_GPU.cu:213-246, launched :264-265) -- depth-only
  * bilateral on the z of a packed float3 cloud, then x,y = normalized.x,y * z.  Race-free: in != out.
- * Reference constants (Projection_GPU.cpp:3-5): radius 3, sigma_spatial 20, sigma_depth 100. */
+ * Reference constants (Projection_GPU.cpp:3-5): radius 3, sigma_spatial 20, sigma_depth 100.
+ * sigma_spatial and sigma_depth must be > 0 (KDME_EINVAL otherwise). */
 int kdme_depth_bilateral_xyz(const float *normalized_dev, const float *in_dev, float *out_dev, int width,
                              int height, int window_radius, float sigma_spatial, float sigma_depth, void *stream);
 

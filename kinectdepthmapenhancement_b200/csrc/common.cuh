@@ -10,6 +10,7 @@ namespace kdme {
 // reference's skip-if-zero guards (JointBilateralFilter.cu:30-33,63-68) fire there.
 constexpr double kExpZeroArg = 103.97207708399179;  // natural-log units
 constexpr double kLog2e = 1.4426950408889634;
+constexpr double kLn2 = 0.6931471805599453;
 // All tap weights are evaluated as 2^(arg + kWeightBias): only ratios of weights
 // matter, and the bias keeps every weight the reference can represent (down to its
 // fp32 denormals, 2^-149) inside the normal range of ex2.approx.ftz.

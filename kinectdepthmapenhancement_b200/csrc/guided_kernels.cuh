@@ -369,8 +369,17 @@ __global__ void __launch_bounds__(TW * TH) guided_fill_fast_kernel(const __grid_
     p.out[frame * p.out_stride + (long long)gy * p.width + gx] = o;
 }
 
+// m * 2^a for a tap weight whose log2 is a, as a double.  Heavy taps (a >= -100) take ex2 of a itself, so their
+// argument is rounded near 0 rather than near kWeightBias; lighter ones are lifted by 2^32 into ex2.approx.ftz's
+// normal range and scaled back exactly in double, which keeps the weights the reference holds as fp32 subnormals.
+__device__ __forceinline__ double ex2_weight(float a, float m = 1.0f) {
+    const bool light = a < -100.f;
+    return (double)(ex2_approx(light ? a + kWeightBias : a) * m) * (light ? 0x1p-32 /* 2^-kWeightBias */ : 1.0);
+}
+
 // MarkovRandomField.cu:4-40: out = (d_p + sum f d_q) / (1 + sum f), f = smooth * expf(-sigma_c * cd)
-// over valid taps; evaluated as d_p + sum f (d_q - d_p) / (1 + sum f).
+// over valid taps; f == 0 where fp32 expf() returns 0 (kExpZeroArg).  Sums in double: up to 961 taps of equal
+// weight would otherwise round to more than 1e-3 mm.
 template <int TW, int TH>
 __global__ void __launch_bounds__(TW * TH)
 mrf_kernel(const float* __restrict__ depth, const uint32_t* __restrict__ guide4, int guide_pitch,
@@ -397,34 +406,44 @@ mrf_kernel(const float* __restrict__ depth, const uint32_t* __restrict__ guide4,
     const uint32_t gpix = sG[pc];
     const float dp = sD[pc];
     const float nk = -color_sigma * (float)kLog2e;
-    float num = 0.f, den = 1.0f;
+    // sigma_c == 0 weights every tap 0 (the reference skips expf there): no argument passes a +inf cut
+    const float cut = (color_sigma != 0.0f) ? -(float)(kExpZeroArg * kLog2e) : __int_as_float(0x7f800000);
+    const double sm = smooth_sigma;
+    double num = dp, den = 1.0;
     for (int i = 0; i < WS; ++i)
         for (int j = 0; j < WS; ++j) {
             const int q = (ly + i) * SP + lx + j;
             const float d = sD[q];
-            if (!(d > kValidDepth)) continue;
             const uint32_t ad = __vabsdiffu4(gpix, sG[q]);
-            const float cd = (float)__dp4a(ad, ad, 0u);
-            const float f = (color_sigma != 0.0f) ? smooth_sigma * ex2_approx(cd * nk) : 0.f;
-            num = fmaf(f, d - dp, num);
+            const float a = (float)__dp4a(ad, ad, 0u) * nk;
+            if (!(d > kValidDepth) || !(a >= cut)) continue;
+            const double f = sm * ex2_weight(a);
+            num = fma(f, (double)d, num);
             den += f;
         }
-    out[(long long)gy * width + gx] = (den == 0.0f) ? 0.0f : dp + num / den;
+    out[(long long)gy * width + gx] = (den == 0.0) ? 0.0f : (float)(num / den);
 }
 
 // Projection_GPU::bilateralfilter -- Projection_GPU.cu:213-246 (next row f2): depth-only bilateral on the
 // z of a packed float3 cloud, centred on the pixel's own z, weights expf(-dz^2/(2 sd^2)) * S; then
-// x,y = normalized.x,y * z.  Race-free (reads `in`, writes `out`).
+// x,y = normalized.x,y * z.  Race-free (reads `in`, writes `out`).  A tap is skipped where fp32 expf() returns 0,
+// |dz| > e_cut = sqrt(2 kExpZeroArg) sd: without the cut a hole whose valid taps all lie just past it gets filled.
+// A hole whose taps all lie near the cut is a weighted mean of weights ~2^-150 S: there the log2 depth term
+// (~ -150) carries the rounding errors of both fp32 products and of the constant, recovered with FMAs, and
+// the product with S is formed in double, down to 2^-299.  Sums in double, as in mrf_kernel; the window's z and S
+// are staged in shared memory as doubles too, so a tap converts one value, not four.
 template <int TW, int TH>
 __global__ void __launch_bounds__(TW * TH)
 depth_bilateral_xyz_kernel(const float* __restrict__ normalized, const float* __restrict__ in,
-                           float* __restrict__ out, const float* __restrict__ ltab /*log2 S, [ws*ws]*/,
-                           int width, int height, int R, float nkd /* -log2e/(2 sd^2) */) {
+                           float* __restrict__ out, const float* __restrict__ stab /*S, [ws*ws]*/,
+                           int width, int height, int R, float nkd /* -log2e/(2 sd^2) */,
+                           float nkd_lo /* its rounding error */, float e_cut) {
     constexpr int NT = TW * TH;
     const int WS = 2 * R + 1, SP = TW + 2 * R, SH = TH + 2 * R;
     extern __shared__ __align__(16) uint8_t smem_dbx[];
-    float* sZ = reinterpret_cast<float*>(smem_dbx);
-    float* sL = sZ + SP * SH;
+    double* sZd = reinterpret_cast<double*>(smem_dbx);
+    double* sS = sZd + SP * SH;
+    float* sZ = reinterpret_cast<float*>(sS + WS * WS);
     const int tid = threadIdx.x;
     const int x0 = blockIdx.x * TW, y0 = blockIdx.y * TH;
     for (int idx = tid; idx < SP * SH; idx += NT) {
@@ -432,28 +451,28 @@ depth_bilateral_xyz_kernel(const float* __restrict__ normalized, const float* __
         int gx = x0 - R + sx, gy = y0 - R + sy;
         bool inb = (gx >= 0) & (gx < width) & (gy >= 0) & (gy < height);
         sZ[idx] = inb ? __ldg(in + 3 * ((long long)gy * width + gx) + 2) : 0.f;
+        sZd[idx] = sZ[idx];
     }
-    for (int idx = tid; idx < WS * WS; idx += NT) sL[idx] = __ldg(ltab + idx);
+    for (int idx = tid; idx < WS * WS; idx += NT) sS[idx] = __ldg(stab + idx);
     __syncthreads();
     const int lx = tid % TW, ly = tid / TW;
     const int gx = x0 + lx, gy = y0 + ly;
     if (gx >= width || gy >= height) return;
     const float zc = sZ[(ly + R) * SP + lx + R];
-    float num = 0.f, den = 0.f;
-    for (int i = 0; i < WS; ++i) {
-        float rn = 0.f, rd = 0.f;
+    double num = 0.0, den = 0.0;
+    for (int i = 0; i < WS; ++i)
         for (int j = 0; j < WS; ++j) {
-            const float zq = sZ[(ly + i) * SP + lx + j];
-            if (!(zq > kValidDepth)) continue;
+            const int q = (ly + i) * SP + lx + j;
+            const float zq = sZ[q];
             const float e = zq - zc;
-            const float f = ex2_approx(fmaf(e * nkd, e, sL[i * WS + j] + kWeightBias));
-            rn = fmaf(f, e, rn);
-            rd += f;
+            if (!(zq > kValidDepth) || !(fabsf(e) <= e_cut)) continue;
+            const float p = __fmul_rn(e, nkd), pe = fmaf(e, nkd, -p) + e * nkd_lo;
+            const float dt = __fmul_rn(p, e), dte = fmaf(p, e, -dt) + pe * e;   // log2 depth factor = dt + dte
+            const double f = ex2_weight(dt, fmaf(dte, (float)kLn2, 1.0f)) * sS[i * WS + j];
+            num = fma(f, sZd[q], num);
+            den += f;
         }
-        num += rn;
-        den += rd;
-    }
-    const float z = (den == 0.0f) ? 0.0f : zc + num / den;
+    const float z = (den == 0.0) ? 0.0f : (float)(num / den);
     const long long k = (long long)gy * width + gx;
     out[3 * k + 0] = __ldg(normalized + 3 * k + 0) * z;
     out[3 * k + 1] = __ldg(normalized + 3 * k + 1) * z;

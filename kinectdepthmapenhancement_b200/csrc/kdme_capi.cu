@@ -1230,16 +1230,17 @@ extern "C" int kdme_depth_bilateral_xyz(const float* normalized_dev, const float
                                         void* stream) {
     if (!normalized_dev || !in_dev || !out_dev) return fail(KDME_EINVAL, "kdme_depth_bilateral_xyz: NULL argument");
     if (in_dev == out_dev) return fail(KDME_EINVAL, "kdme_depth_bilateral_xyz: in-place operation is not supported");
-    if (width <= 0 || height <= 0 || window_radius < 0 || window_radius > KDME_MAX_RADIUS || !(sigma_depth > 0))
+    if (width <= 0 || height <= 0 || window_radius < 0 || window_radius > KDME_MAX_RADIUS || !(sigma_spatial > 0) ||
+        !(sigma_depth > 0))
         return fail(KDME_EINVAL, "kdme_depth_bilateral_xyz: bad size, radius or sigma");
     int rcd = check_pointer_device(in_dev, "kdme_depth_bilateral_xyz");
     if (rcd != KDME_OK) return rcd;
     const int ws = 2 * window_radius + 1;
     cudaStream_t st = (cudaStream_t)stream;
-    // log2-domain spatial LUT, cached per (device, window, sigma): built and uploaded once
+    // spatial LUT, cached per (device, window, sigma): built and uploaded once
     static std::mutex mu;
     static std::map<std::tuple<int, int, float>, float*> cache;
-    float* ltab = nullptr;
+    float* stab = nullptr;
     {
         int cur = 0;
         CK(cudaGetDevice(&cur));
@@ -1249,21 +1250,20 @@ extern "C" int kdme_depth_bilateral_xyz(const float* normalized_dev, const float
         if (it == cache.end()) {
             std::vector<float> lut;
             host_spatial_lut(lut, ws, sigma_spatial);
-            std::vector<float> l2(lut.size());
-            for (size_t i = 0; i < lut.size(); i++) l2[i] = (lut[i] > 0.f) ? (float)std::log2((double)lut[i]) : -1.0e30f;
-            CK(cudaMalloc(&ltab, l2.size() * sizeof(float)));
-            CK(cudaMemcpy(ltab, l2.data(), l2.size() * sizeof(float), cudaMemcpyHostToDevice));
-            cache[key] = ltab;
+            CK(cudaMalloc(&stab, lut.size() * sizeof(float)));
+            CK(cudaMemcpy(stab, lut.data(), lut.size() * sizeof(float), cudaMemcpyHostToDevice));
+            cache[key] = stab;
         } else {
-            ltab = it->second;
+            stab = it->second;
         }
     }
     constexpr int TW = 32, TH = 8;
     const int SP = TW + 2 * window_radius, SH = TH + 2 * window_radius;
     dim3 grd((width + TW - 1) / TW, (height + TH - 1) / TH);
-    depth_bilateral_xyz_kernel<TW, TH><<<grd, TW * TH, (size_t)(SP * SH + ws * ws) * 4, st>>>(
-        normalized_dev, in_dev, out_dev, ltab, width, height, window_radius,
-        (float)(-kLog2e / (2.0 * (double)sigma_depth * (double)sigma_depth)));
+    const double nkd = -kLog2e / (2.0 * (double)sigma_depth * (double)sigma_depth);
+    depth_bilateral_xyz_kernel<TW, TH><<<grd, TW * TH, (size_t)SP * SH * 12 + (size_t)ws * ws * 8, st>>>(
+        normalized_dev, in_dev, out_dev, stab, width, height, window_radius, (float)nkd, (float)(nkd - (float)nkd),
+        (float)(std::sqrt(2.0 * kExpZeroArg) * (double)sigma_depth));
     CK(cudaGetLastError());
     return KDME_OK;
 }

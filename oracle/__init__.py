@@ -77,6 +77,7 @@ def lib():
         L.orc_buf_init.argtypes = [_f32p, C.c_int, C.c_int]
         L.orc_mrf_f32.argtypes = [C.c_int, C.c_int, _f32p, _u8p, _f32p, C.c_int, C.c_float, C.c_float,
                                   C.c_int]
+        L.orc_mrf_f64.argtypes = L.orc_mrf_f32.argtypes
         L.orc_projective_to_real.argtypes = [_f32p, _f32p, C.c_int, C.c_int, C.c_float, C.c_float,
                                              C.c_int, C.c_int]
         L.orc_depth_bilateral_xyz.argtypes = [_f32p, _f32p, _f32p, _f32p, C.c_int, C.c_float, C.c_int, C.c_int, C.c_int]
@@ -273,14 +274,20 @@ def upsample(depth_lo, bgr_hi, radius=7, sigma_s=JBF_SIGMA_S, sigma_c=JBF_SIGMA_
     return jbf(sparse, guide, 2 * radius + 1, sigma_s, sigma_c, sigma_d, precision, threads)
 
 
-def mrf(depth, guide, window=MRF_WINDOW, sigma_c=MRF_SIGMA_C, smooth=MRF_SMOOTH, threads=0, impl="oracle"):
+def mrf(depth, guide, window=MRF_WINDOW, sigma_c=MRF_SIGMA_C, smooth=MRF_SMOOTH, threads=0, impl="oracle",
+        precision="f32"):
+    """MarkovRandomField.cu:4-40.  precision: "f32" (reference order) or "f64" (exact-math with the fp32
+    expf() == 0 rule); impl: "oracle" (C restatement) or "ref" (the reference's kernel text, fp32 only)."""
     depth = _f32(depth)
     guide = _bgr(guide)
     h, w = depth.shape
     out = np.empty((h, w), np.float32)
     threads = threads or n_cores()
     if impl == "ref":
+        assert precision == "f32"
         ref().ref_mrf(w, h, depth, guide, out, window, sigma_c, smooth, threads)
+    elif precision == "f64":
+        lib().orc_mrf_f64(w, h, depth, guide, out, window, sigma_c, smooth, threads)
     else:
         lib().orc_mrf_f32(w, h, depth, guide, out, window, sigma_c, smooth, threads)
     return out
@@ -318,6 +325,19 @@ def mean_3d_error(points, truth):
     cnt = C.c_int()
     m = lib().orc_mean_3d_error(points, truth, points.size // 3, C.byref(cnt))
     return float(m), cnt.value
+
+
+def mean_3d_error_f64(points, truth):
+    """f4 with an fp64 sum: every distance is the fp32 sqrtf((dz*dz + dy*dy) + dx*dx) (each operation rounded to
+    fp32, no contraction), so only the order of the sum differs from a kernel that evaluates them the same way.
+    Returns (mean, count)."""
+    p, t = _f32(points).reshape(-1, 3), _f32(truth).reshape(-1, 3)
+    z, zt = p[:, 2], t[:, 2]
+    m = (z > 50.0) & (z < 15000.0) & (zt > 50.0) & (zt < 15000.0)
+    d = p[m] - t[m]
+    dist = np.sqrt((d[:, 2] * d[:, 2] + d[:, 1] * d[:, 1]) + d[:, 0] * d[:, 0])
+    n = int(m.sum())
+    return (float(dist.astype(np.float64).sum()) / n if n else 0.0), n
 
 
 class Buffer2D:

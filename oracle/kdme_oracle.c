@@ -572,6 +572,37 @@ ORC_API void orc_mrf_f32(int width, int height, const float *depth, const uint8_
         }
 }
 
+/* fp64 evaluation of f1: same formula and tap order as orc_mrf_f32, accumulated in double; the only
+ * fp32 artefact kept is that expf() == 0 below -150 ln2. */
+ORC_API void orc_mrf_f64(int width, int height, const float *depth, const uint8_t *guide, float *out,
+                         int window_size, float color_sigma, float smooth_sigma, int n_threads)
+{
+    int half = window_size / 2;
+    (void)n_threads;
+#pragma omp parallel for schedule(dynamic, 2) num_threads(n_threads > 0 ? n_threads : 1)
+    for (int y = 0; y < height; y++)
+        for (int x = 0; x < width; x++) {
+            const uint8_t *gp = guide + 3 * ((size_t)y * width + x);
+            double num = depth[y * width + x], den = 1.0;
+            for (int i = -half; i <= half; i++)
+                for (int j = -half; j <= half; j++) {
+                    int xj = x + j, yi = y + i;
+                    if (xj >= 0 && xj < width && yi >= 0 && yi < height &&
+                        depth[yi * width + xj] > 50.0f) {
+                        const uint8_t *gq = guide + 3 * ((size_t)yi * width + xj);
+                        double cd = 0.0;
+                        for (int c = 0; c < 3; c++) cd += ((double)gp[c] - gq[c]) * ((double)gp[c] - gq[c]);
+                        double a = (double)color_sigma * cd;
+                        double f = (color_sigma != 0.0f && a <= ORC_EXP_ZERO_ARG) ? exp(-a) : 0.0;
+                        f *= (double)smooth_sigma;
+                        num += (double)depth[yi * width + xj] * f;
+                        den += f;
+                    }
+                }
+            out[y * width + x] = (den == 0.0) ? 0.0f : (float)(num / den);
+        }
+}
+
 /* f3: DimensionConvertor.h:34-75 via DimensionConvertor.cu:3-23 -- pixel
  * (u,v,z) -> camera XYZ; cx, cy are ints (DimensionConvertor.cpp:8-9).
  * Order of operations kept: subtract, divide by focal, multiply by z. */

@@ -42,6 +42,42 @@ def test_mrf_matches_reference_golden(gold):
     assert np.array_equal(out.view(np.uint32), gold["mrf_ws5"].view(np.uint32))
 
 
+def _mrf_f32_vs_f64(depth, bgr, ws, sc, sm):
+    """The fp64 MRF keeps the fp32 restatement's mask, and differs from it by no more than the fp32 restatement's
+    own worst-case rounding: sequential sums of ws*ws non-negative terms (num, den), expf and the quotient."""
+    o32 = oracle.mrf(depth, bgr, ws, sc, sm, threads=2)
+    o64 = oracle.mrf(depth, bgr, ws, sc, sm, threads=2, precision="f64")
+    assert np.array_equal(o32 > 0, o64 > 0) and np.array_equal(o32 == 0, o64 == 0)
+    gamma = (2 * ws * ws + 6) * 2.0 ** -24
+    err = np.abs(o32.astype(np.float64) - o64.astype(np.float64))
+    assert (err <= gamma * np.abs(o64.astype(np.float64)) + 1e-30).all(), err.max()
+    return err
+
+
+@pytest.mark.parametrize("ws,sc,sm", [(5, 50.0, 150.0), (3, 1e-2, 150.0), (11, 1e-3, 1.0), (1, 1e-4, 150.0),
+                                      (5, 0.0, 150.0), (5, 50.0, 0.0)])
+def test_mrf_f64_keeps_f32_mask_and_values(gold, ws, sc, sm):
+    _mrf_f32_vs_f64(gold["depth"], gold["bgr"], ws, sc, sm)
+    for seed in (3, 4):
+        d, c = synth_np(70, 50, seed=seed, frame=seed)
+        _mrf_f32_vs_f64(d, c, ws, sc, sm)
+
+
+def test_mrf_f64_subnormal_weights_fill_holes():
+    """A hole whose only valid neighbours are at colour distance 2: the fp32 reference weight 150 expf(-100) is
+    a subnormal, so the hole's output is a tiny positive number, not 0; past the expf() cut it is 0."""
+    d = np.zeros((3, 3), np.float32)
+    d[0, :] = 1000.0
+    c = np.zeros((3, 3, 3), np.uint8)
+    c[0, :, 0] = 1
+    c[0, :, 1] = 1
+    for sc, filled in ((50.0, True), (52.0, False)):
+        o32 = oracle.mrf(d, c, 3, sc, 150.0)
+        o64 = oracle.mrf(d, c, 3, sc, 150.0, precision="f64")
+        assert (o32[1, 1] > 0) == filled and (o64[1, 1] > 0) == filled
+        assert o64[1, 1] < 1e-35 and o64[2, 1] == 0
+
+
 def test_depth_bilateral_xyz_matches_reference_golden(gold):
     out = oracle.depth_bilateral_xyz(gold["f2_normalized"], gold["f2_points"], threads=2)
     assert np.array_equal(out.view(np.uint32), gold["f2_out"].view(np.uint32))
