@@ -11,8 +11,8 @@
 //      centred on the sweep-1 mean.
 // The per-tap sigma recurrence is sequential in tap order, so one thread owns one
 // pixel and walks the taps in the reference's order; the tile + halo is staged in
-// shared memory once.  Weights are evaluated as one ex2 of summed log2-domain terms
-// with the reference's skip-if-zero guards made explicit.
+// shared memory once.  Weights and sums are in double (guided_sweeps), with the
+// reference's skip-if-zero guards made explicit.
 //
 // The guide has C = 1 (GRAY), 3 (BGR) or 4 (BGRX) bytes per pixel; a GRAY pixel g is staged as
 // the word {g,0,0,0} and a BGRX pixel as {b,g,r,0}, so the colour distance is that of the BGR
@@ -37,7 +37,8 @@ struct GuidedParams {
     const uint8_t* bgr;     // RAW guide, packed C-channel pixels (kernel template parameter C = 1, 3 or 4)
     long long bgr_step;
     float* out;
-    float sigma_c, sigma_d;
+    float sigma_c;
+    double kc, kd;   // 1/(2 sigma_c^2), 1/(2 sigma_d^2) in double; 0 where that sigma is 0 (factor skipped)
     // upsampling form (SURVEY.md 8(d) config 3, label-guided variant): when depth_lo or depth_lo16 is non-null the
     // depth plane is the sparse scatter of a wl x hl low-res map (see upsample_site) and `depth` is ignored
     const float* depth_lo;
@@ -72,6 +73,97 @@ __device__ __forceinline__ float guided_depth(const P& p, long long frame, int g
     if constexpr (U16) return (float)__ldg(p.depth16 + i); else return __ldg(p.depth + i);
 }
 
+// The three sweeps of the pixel whose window starts at staged index `base`, in double (DESIGN.md section 2): the
+// mean, the deviation and both weighted sums are those of the fp64 oracle (orc_guided_fill_f64), in its tap order.
+// At a depth edge the output moves by about 2 kd Var(d) times the sweep-1 mean (over 100x for surfaces 1.5 m apart at
+// sigma_d = 70), so fp32 weights or sums cannot keep such pixels within 1e-3 mm.  What stays fp32 is what the
+// reference's formula holds in fp32 and the oracle keeps: the colour-sigma recurrence, 2 sigma^2 (its underflow to 0
+// decides the -0/0 NaN) and `adaptive` from the fp32 mean.  A skipped factor (argument past the expf() zero cut, or
+// its sigma 0) adds 0 to the exponent; sfac[t] is the spatial factor S, or 1 where the fp32 S is 0.
+// WS_CT > 0 is a compile-time window (the fast kernel, fully unrolled); 0 takes the window `ws` at run time.
+template <int WS_CT>
+__device__ __forceinline__ float guided_sweeps(const float* sD, const uint32_t* sG, const int32_t* sLab, int SP,
+                                               int ws, int base, const double* sfac, float sigma_c, double kc,
+                                               double kd) {
+    const int WS = (WS_CT > 0) ? WS_CT : ws;
+    const int pc = base + (WS / 2) * SP + WS / 2;
+    const uint32_t gpix = sG[pc];
+    const int32_t lp = sLab[pc];
+    const double cut = kExpZeroArg;
+
+    // ---- sweep 1: same-label weighted mean (:116-139), summed about the first such sample d0
+    double acc = 0.0, wsum = 0.0, d0 = 0.0;
+#pragma unroll (WS_CT > 0 ? WS_CT : 1)
+    for (int i = 0; i < WS; ++i)
+#pragma unroll (WS_CT > 0 ? WS_CT : 1)
+        for (int j = 0; j < WS; ++j) {
+            const int q = base + i * SP + j;
+            const float d = sD[q];
+            if (d == 0.f || sLab[q] != lp) continue;
+            const uint32_t ad = __vabsdiffu4(gpix, sG[q]);
+            const double qc = (double)__dp4a(ad, ad, 0u) * kc;
+            const double f = sfac[i * WS + j] * exp(-((qc <= cut) ? qc : 0.0));
+            if (wsum == 0.0) d0 = d;
+            acc = fma(f, (double)d - d0, acc);
+            wsum += f;
+        }
+    if (!(wsum > 0.0)) return 0.f;
+    const double m = d0 + acc / wsum;
+
+    // ---- sweep 2: mean absolute deviation of the same taps (:143-156)
+    double dev = 0.0;
+    int count = 0;
+#pragma unroll (WS_CT > 0 ? WS_CT : 1)
+    for (int i = 0; i < WS; ++i)
+#pragma unroll (WS_CT > 0 ? WS_CT : 1)
+        for (int j = 0; j < WS; ++j) {
+            const int q = base + i * SP + j;
+            const float d = sD[q];
+            if (d == 0.f || sLab[q] != lp) continue;
+            dev += fabs((double)d - m);
+            count++;
+        }
+    dev /= (double)count;
+    // 5.0*deviation/pow(w_average,2.0f): double expression, fp32 square (:171)
+    const float mf = (float)m;
+    const float adaptive = (float)(5.0 * dev / (double)__fmul_rn(mf, mf));
+
+    // ---- sweep 3: all samples, colour sigma MUTATED PER VALID TAP (:158-195)
+    float sigma = sigma_c;
+    double inv = 1.0 / (double)(2 * (sigma * sigma));   // 1 / (2 sigma^2), refreshed when sigma changes
+    double num = 0.0, den = 0.0;
+    bool poisoned = false;
+#pragma unroll (WS_CT > 0 ? WS_CT : 1)
+    for (int i = 0; i < WS; ++i)
+#pragma unroll (WS_CT > 0 ? WS_CT : 1)
+        for (int j = 0; j < WS; ++j) {
+            const int q = base + i * SP + j;
+            const float d = sD[q];
+            if (d == 0.f) continue;
+            double arg = 0.0;
+            if (sigma != 0.0f) {
+                const float t = sigma * 0.3f;
+                const float sn = (adaptive > t) ? adaptive : t;
+                if (sn != sigma) {
+                    sigma = sn;
+                    inv = 1.0 / (double)(2 * (sigma * sigma));   // 2 sigma^2 underflowed to 0: inv = +inf
+                }
+                const uint32_t ad = __vabsdiffu4(gpix, sG[q]);
+                const double qc = (double)__dp4a(ad, ad, 0u) * inv;
+                if (qc != qc) poisoned = true;                  // 0 * inf: expf(-0/0) = NaN != 0 -> filter *= NaN
+                else if (qc <= cut) arg = qc;
+            }
+            const double e = (double)d - m;
+            const double z = e * e * kd;
+            if (z <= cut) arg += z;
+            const double f = sfac[i * WS + j] * exp(-arg);
+            num = fma(f, (double)d, num);
+            den += f;
+        }
+    if (poisoned) return __int_as_float(0x7fc00000);
+    return (den == 0.0) ? 0.0f : (float)(num / den);
+}
+
 template <int TW, int TH, int C, bool U16>
 __global__ void __launch_bounds__(TW * TH) guided_fill_kernel(const __grid_constant__ GuidedParams p) {
     constexpr int NT = TW * TH;
@@ -80,7 +172,7 @@ __global__ void __launch_bounds__(TW * TH) guided_fill_kernel(const __grid_const
     float* sD = reinterpret_cast<float*>(smem_gf);
     uint32_t* sG = reinterpret_cast<uint32_t*>(sD + SP * SH);
     int32_t* sLab = reinterpret_cast<int32_t*>(sG + SP * SH);
-    __shared__ float sL[31 * 31];
+    __shared__ double sS[31 * 31];
     const int tid = threadIdx.x;
     const int x0 = blockIdx.x * TW, y0 = blockIdx.y * TH;
     const long long frame = blockIdx.z;
@@ -106,109 +198,20 @@ __global__ void __launch_bounds__(TW * TH) guided_fill_kernel(const __grid_const
     }
     for (int idx = tid; idx < WS * WS; idx += NT) {
         const float s = p.spatial[idx];
-        sL[idx] = (s != 0.0f) ? log2f(s) : 0.0f;  // skip-if-zero guard (:129-130, :185-186)
+        sS[idx] = (s != 0.0f) ? (double)s : 1.0;  // skip-if-zero guard (:129-130, :185-186)
     }
     __syncthreads();
 
     const int lx = tid % TW, ly = tid / TW;
     const int gx = x0 + lx, gy = y0 + ly;
     if (gx >= p.width || gy >= p.height) return;
-    const int pc = (ly + R) * SP + lx + R;
-    const uint32_t gpix = sG[pc];
-    const int32_t lp = sLab[pc];
-    const float kZero = -(float)kExpZeroArg;
-    const float l2e = (float)kLog2e;
-    const float sc0 = p.sigma_c;
-    const float den0 = 2 * (sc0 * sc0);
-    const float inv_den0 = (sc0 != 0.0f) ? 1.0f / den0 : 0.f;   // sweep 1: one reciprocal per pixel, not a division per tap
-
-    // accumulation origin: first sample in the window (keeps fp32 sums small)
-    float d0 = 0.f;
-    for (int t = 0; t < WS * WS && d0 == 0.f; ++t) {
-        const int i = t / WS, j = t - i * WS;
-        d0 = sD[(ly + i) * SP + lx + j];
-    }
-
-    // ---- sweep 1: same-label weighted mean (:116-139)
-    float acc = 0.f, wsum = 0.f;
-    for (int i = 0; i < WS; ++i)
-        for (int j = 0; j < WS; ++j) {
-            const int q = (ly + i) * SP + lx + j;
-            const float d = sD[q];
-            if (d == 0.f || sLab[q] != lp) continue;
-            const uint32_t ad = __vabsdiffu4(gpix, sG[q]);
-            const float cd = (float)__dp4a(ad, ad, 0u);
-            float lg = sL[i * WS + j] + kWeightBias;
-            if (sc0 != 0.0f) {
-                const float a = -cd * inv_den0;
-                if (a >= kZero) lg = fmaf(a, l2e, lg);
-            }
-            const float f = ex2_approx(lg);
-            acc = fmaf(f, d - d0, acc);
-            wsum += f;
-        }
-    float o = 0.f;
-    if (wsum > 0.f) {
-        const float delta = acc / wsum;   // mean = d0 + delta
-        const float mean = d0 + delta;    // the reference's fp32 w_average
-        // ---- sweep 2: mean absolute deviation of the same taps (:143-156)
-        float dev = 0.f;
-        int count = 0;
-        for (int i = 0; i < WS; ++i)
-            for (int j = 0; j < WS; ++j) {
-                const int q = (ly + i) * SP + lx + j;
-                const float d = sD[q];
-                if (d == 0.f || sLab[q] != lp) continue;
-                dev += fabsf((d - d0) - delta);
-                count++;
-            }
-        if (count != 0) dev /= (float)count;
-        // 5.0*deviation/pow(w_average,2.0f): double expression, fp32 square (:171)
-        const float adaptive = (float)(5.0 * (double)dev / (double)(mean * mean));
-        // ---- sweep 3: all samples, mutating colour sigma (:158-195)
-        const float sq = (p.sigma_d != 0.0f) ? sqrtf(l2e / (2.0f * p.sigma_d * p.sigma_d)) : 0.f;
-        const float e_thr = (float)1.2247448713915890e1;  // sqrt(150)
-        float sigma = sc0;
-        float num = 0.f, den = 0.f;
-        bool poisoned = false;
-        for (int i = 0; i < WS; ++i)
-            for (int j = 0; j < WS; ++j) {
-                const int q = (ly + i) * SP + lx + j;
-                const float d = sD[q];
-                if (d == 0.f) continue;
-                const uint32_t ad = __vabsdiffu4(gpix, sG[q]);
-                const float cd = (float)__dp4a(ad, ad, 0u);
-                float lg = sL[i * WS + j] + kWeightBias;
-                if (sigma != 0.0f) {
-                    if (adaptive > sigma * 0.3f) sigma = adaptive; else sigma *= 0.3f;
-                    const float dn = 2 * (sigma * sigma);
-                    // fast reciprocal where it is safe; the exact quotient near underflow, where -0/0 = NaN
-                    // (sigma^2 underflowed to 0 and cd == 0) and cd/denormal must behave as in IEEE arithmetic
-                    const float a = (dn > 1.0e-30f) ? -cd * __frcp_rn(dn) : -cd / dn;
-                    if (a != a) poisoned = true;       // expf(NaN) = NaN != 0 -> filter *= NaN
-                    else if (a >= kZero) lg = fmaf(a, l2e, lg);
-                }
-                const float e = (d - d0) - delta;
-                const float es = e * sq;
-                if (p.sigma_d != 0.0f && !(fabsf(es) > e_thr)) lg = fmaf(-es, es, lg);
-                const float f = ex2_approx(lg);
-                num = fmaf(f, e, num);
-                den += f;
-            }
-        if (poisoned) o = __int_as_float(0x7fc00000);
-        else o = (den == 0.0f) ? 0.0f : mean + num / den;
-    }
-    p.out[frame * p.out_stride + (long long)gy * p.width + gx] = o;
+    p.out[frame * p.out_stride + (long long)gy * p.width + gx] =
+        guided_sweeps<0>(sD, sG, sLab, SP, WS, ly * SP + lx, sS, p.sigma_c, p.kc, p.kd);
 }
 
 // -----------------------------------------------------------------------------
-// Fast form of the same three sweeps for the common case: compile-time radius (fully unrolled window, no
-// index arithmetic), branch-free taps (validity / label tests become selects), the log2-domain spatial LUT
-// read straight from the constant bank as an FFMA operand, the colour distance through the 2^23 magic
-// accumulator (no int->float conversion), one MUFU.RCP instead of an IEEE division per sweep-3 tap, and
-// the same-label predicate of sweep 1 kept as a bit mask for sweep 2.  Preconditions (host-checked): the
-// colour skip-if-zero guard cannot fire in sweep 1 (sigma_c >= 30.63) and sigma_c, sigma_d != 0.  The
-// per-valid-tap colour-sigma recurrence, its underflow to 0 and the -0/0 NaN poisoning are kept exactly.
+// Fast form of the same three sweeps for windows 3..7: a compile-time window, fully unrolled (no index
+// arithmetic), with the spatial factors read straight from the constant bank.
 template <int R>
 struct GuidedFastParams {
     int width, height;
@@ -218,18 +221,18 @@ struct GuidedFastParams {
     const uint8_t* bgr;
     long long bgr_step;
     float* out;
-    float sigma_c, nk0 /* -log2e/(2 sigma_c^2) */, sq /* sqrt(log2e/(2 sigma_d^2)) */;
+    float sigma_c;
+    double kc /* 1/(2 sigma_c^2) */, kd /* 1/(2 sigma_d^2) */;
     const float* depth_lo;
     const uint16_t* depth_lo16;
     int wl, hl;
     long long depth_stride, bgr_stride, labels_stride, out_stride;   // as in GuidedParams
-    float ltab[(2 * R + 1) * (2 * R + 1)];   // log2(S_ij) + kWeightBias, or kWeightBias where S_ij == 0
+    double sfac[(2 * R + 1) * (2 * R + 1)];   // S_ij, or 1 where the fp32 S_ij is 0
 };
 
 template <int R, int TW, int TH, int C, bool U16>
 __global__ void __launch_bounds__(TW * TH) guided_fill_fast_kernel(const __grid_constant__ GuidedFastParams<R> p) {
     constexpr int NT = TW * TH, WS = 2 * R + 1, SP = TW + 2 * R, SH = TH + 2 * R;
-    static_assert(WS * WS <= 64, "the same-label mask is one 64-bit word");
     __shared__ float sD[SP * SH];
     __shared__ uint32_t sG[SP * SH];
     __shared__ int32_t sLab[SP * SH];
@@ -260,113 +263,8 @@ __global__ void __launch_bounds__(TW * TH) guided_fill_fast_kernel(const __grid_
     const int lx = tid % TW, ly = tid / TW;
     const int gx = x0 + lx, gy = y0 + ly;
     if (gx >= p.width || gy >= p.height) return;
-    const int base = ly * SP + lx;
-    const uint32_t gpix = sG[base + R * SP + R];
-    const int32_t lp = sLab[base + R * SP + R];
-    // accumulation origin: the centre sample, else the first sample of the window (rare, divergent)
-    float d0 = sD[base + R * SP + R];
-    if (d0 == 0.f) {
-        for (int t = 0; t < WS * WS && d0 == 0.f; ++t) d0 = sD[base + (t / WS) * SP + (t % WS)];
-    }
-    const float nk0 = p.nk0;
-
-    // ---- sweep 1: same-label weighted mean (:116-139)
-    float acc = 0.f, wsum = 0.f;
-    unsigned long long same = 0ull;
-#pragma unroll
-    for (int i = 0; i < WS; ++i)
-#pragma unroll
-        for (int j = 0; j < WS; ++j) {
-            const int q = base + i * SP + j;
-            const float d = sD[q];
-            const bool pr = (d != 0.f) & (sLab[q] == lp);
-            const uint32_t ad = __vabsdiffu4(gpix, sG[q]);
-            const float cdf = __uint_as_float(__dp4a(ad, ad, kMagicValid)) - 8388608.0f;
-            const float f = ex2_approx(fmaf(cdf, nk0, p.ltab[i * WS + j]));
-            if (pr) {   // predicated accumulation (no selects)
-                acc = fmaf(f, d - d0, acc);
-                wsum += f;
-                same |= 1ull << (i * WS + j);
-            }
-        }
-    float o = 0.f;
-    if (wsum > 0.f) {
-        const float delta = acc / wsum;   // mean = d0 + delta
-        const float mean = d0 + delta;    // the reference's fp32 w_average
-        // ---- sweep 2: mean absolute deviation of the same taps (:143-156)
-        float dev = 0.f;
-#pragma unroll
-        for (int i = 0; i < WS; ++i)
-#pragma unroll
-            for (int j = 0; j < WS; ++j) {
-                const float x = fabsf((sD[base + i * SP + j] - d0) - delta);
-                if ((same >> (i * WS + j)) & 1ull) dev += x;
-            }
-        const int count = __popcll(same);
-        if (count != 0) dev /= (float)count;
-        // 5.0*deviation/pow(w_average,2.0f): double expression, fp32 square (:171)
-        const float adaptive = (float)(5.0 * (double)dev / (double)(mean * mean));
-        // ---- sweep 3: all samples, mutating colour sigma (:158-195)
-        const float kZero = -(float)kExpZeroArg;
-        const float l2e = (float)kLog2e;
-        const float sq = p.sq;
-        const float e_thr = (float)1.2247448713915890e1;  // sqrt(150)
-        float sigma = p.sigma_c;
-        float num = 0.f, den = 0.f;
-#pragma unroll
-        for (int i = 0; i < WS; ++i)
-#pragma unroll
-            for (int j = 0; j < WS; ++j) {
-                const int q = base + i * SP + j;
-                const float d = sD[q];
-                const bool v = d != 0.f;
-                const uint32_t ad = __vabsdiffu4(gpix, sG[q]);
-                const float cd = __uint_as_float(__dp4a(ad, ad, kMagicValid)) - 8388608.0f;
-                float lg = p.ltab[i * WS + j];
-                // the recurrence advances once per VALID tap while sigma != 0 (:170-176); branch-free
-                const bool adv = v & (sigma != 0.0f);
-                const float t = sigma * 0.3f;
-                const float sn = (adaptive > t) ? adaptive : t;
-                sigma = adv ? sn : sigma;
-                // a = -cd / (2 sigma^2) evaluated as (-cd * rcp(sigma^2)) with the factor 1/2 folded into the constants
-                // (a power of two: same bits)
-                const float s2 = sigma * sigma;
-                float rc;
-                asm("rcp.approx.ftz.f32 %0, %1;" : "=f"(rc) : "f"(s2));
-                const float a2 = -cd * rc;                      // 2a
-                // 2 sigma^2 <= 1e-30: cd >= 1 is beyond the fp32 expf() cut-off (factor skipped) and cd == 0 gives -0
-                // (factor 1) -- either way nothing is added; the one exception, -0/0 = NaN, is handled after the sweep
-                if (adv & (s2 > 0.5e-30f) & (a2 >= 2.0f * kZero)) lg = fmaf(a2, 0.5f * l2e, lg);
-                const float e = (d - d0) - delta;
-                const float es = e * sq;
-                if (!(fabsf(es) > e_thr)) lg = fmaf(-es, es, lg);
-                const float f = ex2_approx(lg);
-                if (v) {
-                    num = fmaf(f, e, num);
-                    den += f;
-                }
-            }
-        // NaN poisoning (:170-176 with sigma^2 underflowed to exactly 0 and cd == 0: expf(-0/0) = NaN).  sigma never
-        // increases once the sweep has started, so it can only have happened if the FINAL sigma squares to 0: rare,
-        // re-walked here with the recurrence alone
-        bool poisoned = false;
-        if (sigma != 0.0f ? (2 * (sigma * sigma) == 0.0f) : true) {
-            float sg = p.sigma_c;
-            for (int t2 = 0; t2 < WS * WS; ++t2) {
-                const int q = base + (t2 / WS) * SP + (t2 % WS);
-                if (sD[q] == 0.f || sg == 0.0f) continue;
-                const float tt = sg * 0.3f;
-                sg = (adaptive > tt) ? adaptive : tt;
-                if (2 * (sg * sg) == 0.0f) {
-                    const uint32_t ad = __vabsdiffu4(gpix, sG[q]);
-                    if (__dp4a(ad, ad, 0u) == 0u) poisoned = true;
-                }
-            }
-        }
-        if (poisoned) o = __int_as_float(0x7fc00000);
-        else o = (den == 0.0f) ? 0.0f : mean + num / den;
-    }
-    p.out[frame * p.out_stride + (long long)gy * p.width + gx] = o;
+    p.out[frame * p.out_stride + (long long)gy * p.width + gx] =
+        guided_sweeps<WS>(sD, sG, sLab, SP, WS, ly * SP + lx, p.sfac, p.sigma_c, p.kc, p.kd);
 }
 
 // m * 2^a for a tap weight whose log2 is a, as a double.  Heavy taps (a >= -100) take ex2 of a itself, so their

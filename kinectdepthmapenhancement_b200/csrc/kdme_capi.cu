@@ -1343,16 +1343,18 @@ static int guided_slices(const P& p0, int n_frames, void (*kernel)(const P), siz
     return KDME_OK;
 }
 
+// 1 / (2 sigma^2) in double, as the fp64 oracle forms it; 0 for sigma = 0, where the reference skips the factor.
+static double guided_k(float sigma) { return (sigma != 0.0f) ? 1.0 / (2.0 * (double)sigma * (double)sigma) : 0.0; }
+
 template <int R, int C>
 static int guided_launch_fast(const GuidedCall& c, const std::vector<float>& lut, cudaStream_t stream) {
     constexpr int ws = 2 * R + 1;
     GuidedFastParams<R> p;
-    for (int i = 0; i < ws * ws; i++)
-        p.ltab[i] = (lut[i] != 0.0f) ? (float)(std::log2((double)lut[i]) + (double)kWeightBias) : kWeightBias;
+    for (int i = 0; i < ws * ws; i++) p.sfac[i] = (lut[i] != 0.0f) ? (double)lut[i] : 1.0;
     guided_common(p, c);
     p.sigma_c = c.sigma_c;
-    p.nk0 = (float)(-kLog2e / (2.0 * (double)c.sigma_c * (double)c.sigma_c));
-    p.sq = sqrtf((float)kLog2e / (2.0f * c.sigma_d * c.sigma_d));
+    p.kc = guided_k(c.sigma_c);
+    p.kd = guided_k(c.sigma_d);
     if (c.depth16 || c.depth_lo16)
         return guided_slices(p, c.n_frames, guided_fill_fast_kernel<R, kGuidedTW, kGuidedTH, C, true>, 0, stream);
     return guided_slices(p, c.n_frames, guided_fill_fast_kernel<R, kGuidedTW, kGuidedTH, C, false>, 0, stream);
@@ -1364,23 +1366,20 @@ static int guided_launch_c(const GuidedCall& c, cudaStream_t stream) {
     const int ws = 2 * c.radius + 1;
     std::vector<float> lut;
     host_spatial_lut(lut, ws, c.sigma_s);
-    // fast form: compile-time window (3..7), sweep-1 colour guard cannot fire (expf(-3*255^2/(2 sc^2)) != 0)
-    const bool fast_ok = c.sigma_c != 0.0f && c.sigma_d != 0.0f &&
-                         expf(-(float)(3 * 255 * 255) / (2 * (c.sigma_c * c.sigma_c))) != 0.0f;
-    if (fast_ok) {
-        switch (c.radius) {
-            case 1: return guided_launch_fast<1, C>(c, lut, stream);
-            case 2: return guided_launch_fast<2, C>(c, lut, stream);
-            case 3: return guided_launch_fast<3, C>(c, lut, stream);
-            default: break;
-        }
+    // fast form: compile-time window 3..7, the same sweeps (guided_sweeps) at any sigmas
+    switch (c.radius) {
+        case 1: return guided_launch_fast<1, C>(c, lut, stream);
+        case 2: return guided_launch_fast<2, C>(c, lut, stream);
+        case 3: return guided_launch_fast<3, C>(c, lut, stream);
+        default: break;
     }
     GuidedParams p;
     if (ws * ws > (int)(sizeof(p.spatial) / sizeof(float))) return fail(KDME_ENOTSUP, "guided fill: window too large");
     for (int i = 0; i < ws * ws; i++) p.spatial[i] = lut[i];
     guided_common(p, c);
     p.radius = c.radius;
-    p.sigma_c = c.sigma_c; p.sigma_d = c.sigma_d;
+    p.sigma_c = c.sigma_c;
+    p.kc = guided_k(c.sigma_c); p.kd = guided_k(c.sigma_d);
     const int SP = kGuidedTW + 2 * c.radius, SH = kGuidedTH + 2 * c.radius;
     if (c.depth16 || c.depth_lo16)
         return guided_slices(p, c.n_frames, guided_fill_kernel<kGuidedTW, kGuidedTH, C, true>, (size_t)SP * SH * 12, stream);
@@ -1398,6 +1397,14 @@ static int guided_run(GuidedCall c, const void* depth, int channels, void* strea
     return with_channels(channels, [&](auto ch) { return guided_launch_c<decltype(ch)::value>(c, (cudaStream_t)stream); });
 }
 
+// The kernels read every frame's depth while they write the output: true where the depth input's `in_bytes` and the
+// `out_floats` output floats share a byte.
+static bool guided_overlap(const void* in, unsigned long long in_bytes, const float* out, unsigned long long out_floats) {
+    const uintptr_t i0 = (uintptr_t)in, i1 = i0 + in_bytes;
+    const uintptr_t o0 = (uintptr_t)out, o1 = o0 + out_floats * sizeof(float);
+    return i0 < o1 && o0 < i1;
+}
+
 // n_frames fills; the depth is float (depth) or uint16 (depth16), the other one is NULL.
 static int guided_fill_batch(const float* depth, const uint16_t* depth16, const int32_t* labels, const uint8_t* bgr,
                              size_t bgr_step, int channels, float* out, int width, int height, int n_frames,
@@ -1407,11 +1414,8 @@ static int guided_fill_batch(const float* depth, const uint16_t* depth16, const 
     if (!in || !bgr || !out) return fail(KDME_EINVAL, std::string(who) + ": NULL argument");
     if (n_frames < 1) return fail(KDME_EINVAL, std::string(who) + ": n_frames must be >= 1");
     if (width <= 0 || height <= 0) return fail(KDME_EINVAL, std::string(who) + ": bad size");
-    // the kernels read every frame's depth while they write the output: the two byte ranges must be disjoint
-    const unsigned long long px = (unsigned long long)width * height * n_frames;
-    const uintptr_t i0 = (uintptr_t)in, i1 = i0 + px * (depth ? sizeof(float) : sizeof(uint16_t));
-    const uintptr_t o0 = (uintptr_t)out, o1 = o0 + px * sizeof(float);
-    if (i0 < o1 && o0 < i1)
+    if (guided_overlap(in, (unsigned long long)width * height * n_frames * (depth ? sizeof(float) : sizeof(uint16_t)),
+                       out, (unsigned long long)width * height * n_frames))
         return fail(KDME_EINVAL, std::string(who) + ": the output overlaps the depth input (in-place operation is not supported)");
     GuidedCall c{depth, depth16, nullptr, nullptr, 0, 0, labels, bgr, bgr_step, out, width, height, n_frames,
                  window_radius, sigma_spatial, sigma_color, sigma_depth};
@@ -1429,6 +1433,9 @@ static int guided_upsample_batch(const float* depth_lo, const uint16_t* depth_lo
     if (n_frames < 1) return fail(KDME_EINVAL, std::string(who) + ": n_frames must be >= 1");
     if (width <= 0 || height <= 0 || wl <= 0 || hl <= 0 || wl > width || hl > height)
         return fail(KDME_EINVAL, std::string(who) + ": low-res size must be positive and <= the high-res size");
+    if (guided_overlap(in, (unsigned long long)wl * hl * n_frames * (depth_lo ? sizeof(float) : sizeof(uint16_t)), out_hi,
+                       (unsigned long long)width * height * n_frames))
+        return fail(KDME_EINVAL, std::string(who) + ": the output overlaps the depth input (in-place operation is not supported)");
     GuidedCall c{nullptr, nullptr, depth_lo, depth_lo16, wl, hl, labels_hi, bgr_hi, bgr_step, out_hi, width, height,
                  n_frames, window_radius, sigma_spatial, sigma_color, sigma_depth};
     return guided_run(c, in, channels, stream, who);

@@ -69,7 +69,7 @@ def lib():
         L.orc_guided_fill_f32.argtypes = [C.c_int, C.c_int, _f32p, _u8p, C.c_void_p, _f32p, _f32p,
                                           C.c_int, C.c_float, C.c_float, C.c_int]
         L.orc_guided_fill_f64.argtypes = [C.c_int, C.c_int, _f32p, _u8p, C.c_void_p, _f32p, _f32p, C.c_void_p,
-                                          C.c_int, C.c_float, C.c_float, C.c_int]
+                                          C.c_void_p, C.c_int, C.c_float, C.c_float, C.c_int]
         L.orc_scatter_lowres.argtypes = [_f32p, C.c_int, C.c_int, _f32p, C.c_int, C.c_int]
         for name in ("orc_buf_insert_f32", "orc_buf_insert_f32x2", "orc_buf_get_depth",
                      "orc_buf_get_weight", "orc_buf_update"):
@@ -229,8 +229,12 @@ def jbf_process(depth, bgr, window=JBF_WINDOW, sigma_s=JBF_SIGMA_S, sigma_c=JBF_
 
 
 def guided_fill(depth, guide, labels=None, window=ERS_WINDOW, sigma_s=ERS_SIGMA_S, sigma_c=ERS_SIGMA_C,
-                sigma_d=ERS_SIGMA_D, threads=0, impl="oracle", precision="f32", return_mean=False):
-    """depthmap_enhancement (EdgeRefinedSuperpixel.cu:104-205), race-free; raw (un-smoothed) guide."""
+                sigma_d=ERS_SIGMA_D, threads=0, impl="oracle", precision="f32", return_mean=False, return_guard=False):
+    """depthmap_enhancement (EdgeRefinedSuperpixel.cu:104-205), race-free; raw (un-smoothed) guide.
+
+    precision "f64" only: return_mean adds the double sweep-1 mean, return_guard a uint8 map of the guard-active
+    pixels (non-zero: a branch of the fp32 formula is decided within a few ulps of its threshold; the bits are
+    those of orc_guided_fill_f64).  The result is out, then the mean and the guard in that order, as asked."""
     depth = _f32(depth)
     guide = _bgr(guide)
     h, w = depth.shape
@@ -243,9 +247,12 @@ def guided_fill(depth, guide, labels=None, window=ERS_WINDOW, sigma_s=ERS_SIGMA_
     threads = threads or n_cores()
     if precision == "f64":
         mean = np.empty((h, w), np.float64) if return_mean else None
+        guard = np.empty((h, w), np.uint8) if return_guard else None
         lib().orc_guided_fill_f64(w, h, depth, guide, lab.ctypes.data if lab is not None else None, lut, out,
-                                  mean.ctypes.data if return_mean else None, window, sigma_c, sigma_d, threads)
-        return (out, mean) if return_mean else out
+                                  mean.ctypes.data if return_mean else None, guard.ctypes.data if return_guard else None,
+                                  window, sigma_c, sigma_d, threads)
+        extra = [a for a in (mean, guard) if a is not None]
+        return (out, *extra) if extra else out
     if impl == "ref":
         if lab is None:
             lab = np.zeros((h, w), np.int32)

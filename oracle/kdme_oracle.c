@@ -389,11 +389,31 @@ ORC_API void orc_guided_fill_f32(int width, int height, const float *depth, cons
  * sequence (it is a discrete state machine: sigma *= 0.3f or sigma = adaptive, :172-175) driven
  * by the fp32 rounding of 5.0*deviation/mean^2; the skip-if-zero guards are the explicit
  * arg < -150 ln2 tests; -0/0 (sigma^2 underflowed to 0 with cd == 0) poisons the pixel with NaN
- * exactly as expf(NaN) does in the reference. */
+ * exactly as expf(NaN) does in the reference.  The sweep-1 mean is summed about the first
+ * same-label sample d0, m = d0 + sum f (d - d0) / sum f (d - d0 is exact in double), so a window of
+ * one depth has that depth as its mean and a deviation of exactly 0 whatever the weights' rounding.
+ *
+ * guard_out (nullable) flags the pixels at which the fp32 formula jumps: some quantity that decides
+ * a branch lies within ORC_GUARD_ULPS fp32 ulps of its threshold, so an evaluation whose inputs
+ * differ from these by rounding alone may take the other side (DESIGN.md section 2):
+ *   1  a colour argument cd/dn (sweep 1 or sweep 3) or a sweep-3 depth argument e^2 kd at the
+ *      expf() zero cut, past which the factor is skipped and the tap gets full weight;
+ *   2  the recurrence test adaptive > sigma*0.3f, whose fp32 `adaptive` rounds 5*dev/mean^2;
+ *   4  2 sigma^2 at the fp32 underflow boundary with sigma = adaptive: it decides -0/0 = NaN.
+ * adaptive == 0 (a window of one depth, deviation exactly 0) is exact, so it flags nothing. */
+#define ORC_GUARD_ULPS 8.0
+
+static int orc_near_cut(double arg)
+{
+    const double cut = ORC_EXP_ZERO_ARG;
+    const double ulp = (double)(nextafterf((float)cut, INFINITY) - (float)cut);
+    return fabs(arg - cut) <= ORC_GUARD_ULPS * ulp;
+}
+
 ORC_API void orc_guided_fill_f64(int width, int height, const float *depth, const uint8_t *guide,
                                  const int32_t *labels, const float *spatial, float *out,
-                                 double *mean_out /*nullable*/, int window_size, float color_sigma_in,
-                                 float depth_sigma, int n_threads)
+                                 double *mean_out /*nullable*/, uint8_t *guard_out /*nullable*/,
+                                 int window_size, float color_sigma_in, float depth_sigma, int n_threads)
 {
     int half = window_size / 2;
     double kd = (depth_sigma != 0.0f) ? 1.0 / (2.0 * (double)depth_sigma * (double)depth_sigma) : 0.0;
@@ -403,7 +423,8 @@ ORC_API void orc_guided_fill_f64(int width, int height, const float *depth, cons
         for (int x = 0; x < width; x++) {
             int lp = labels ? labels[y * width + x] : 0;
             const uint8_t *gp = guide + (size_t)(y * width + x) * 3;
-            double a = 0.0, wt = 0.0;
+            double a = 0.0, wt = 0.0, d0 = 0.0;
+            int guard = 0;
             double den0 = 2.0 * (double)color_sigma_in * (double)color_sigma_in;
             for (int i = -half; i <= half; i++)
                 for (int j = -half; j <= half; j++) {
@@ -417,13 +438,18 @@ ORC_API void orc_guided_fill_f64(int width, int height, const float *depth, cons
                     double f = 1.0;
                     float s = spatial[(i + half) * window_size + (j + half)];
                     if (s != 0.0f) f *= (double)s;
-                    if (color_sigma_in != 0.0f && cd / den0 <= ORC_EXP_ZERO_ARG) f *= exp(-cd / den0);
-                    a += (double)depth[yi * width + xj] * f;
+                    if (color_sigma_in != 0.0f) {
+                        if (orc_near_cut(cd / den0)) guard |= 1;
+                        if (cd / den0 <= ORC_EXP_ZERO_ARG) f *= exp(-cd / den0);
+                    }
+                    if (wt == 0.0) d0 = (double)depth[yi * width + xj];
+                    a += ((double)depth[yi * width + xj] - d0) * f;
                     wt += f;
                 }
             if (mean_out) mean_out[y * width + x] = 0.0;
+            if (guard_out) guard_out[y * width + x] = 0;
             if (!(wt > 0.0)) { out[y * width + x] = 0.0f; continue; }
-            double m = a / wt;
+            double m = d0 + a / wt;
             if (mean_out) mean_out[y * width + x] = m;
             double dev = 0.0; int count = 0;
             for (int i = -half; i <= half; i++)
@@ -453,16 +479,27 @@ ORC_API void orc_guided_fill_f64(int width, int height, const float *depth, cons
                     float s = spatial[(i + half) * window_size + (j + half)];
                     if (s != 0.0f) f *= (double)s;
                     if (sigma != 0.0f) {
-                        if (adaptive > sigma * 0.3f) sigma = adaptive; else sigma *= 0.3f;
+                        float t = sigma * 0.3f;
+                        float hi = fmaxf(fabsf(adaptive), fabsf(t));
+                        if (adaptive != 0.0f && fabsf(adaptive - t) <= (float)ORC_GUARD_ULPS * (nextafterf(hi, INFINITY) - hi)) guard |= 2;
+                        if (adaptive > t) sigma = adaptive; else sigma = t;
                         float dn = 2 * (sigma * sigma);   /* fp32: may underflow to 0 */
+                        if (adaptive != 0.0f && sigma == adaptive && dn <= (float)ORC_GUARD_ULPS * 0x1p-149f) guard |= 4;
                         if (dn == 0.0f) { if (cd == 0.0) poisoned = 1; /* cd > 0: expf(-inf) = 0, skipped */ }
-                        else if (cd / (double)dn <= ORC_EXP_ZERO_ARG) f *= exp(-cd / (double)dn);
+                        else {
+                            if (orc_near_cut(cd / (double)dn)) guard |= 1;
+                            if (cd / (double)dn <= ORC_EXP_ZERO_ARG) f *= exp(-cd / (double)dn);
+                        }
                     }
                     double e = (double)depth[yi * width + xj] - m;
-                    if (depth_sigma != 0.0f && e * e * kd <= ORC_EXP_ZERO_ARG) f *= exp(-e * e * kd);
+                    if (depth_sigma != 0.0f) {
+                        if (orc_near_cut(e * e * kd)) guard |= 1;
+                        if (e * e * kd <= ORC_EXP_ZERO_ARG) f *= exp(-e * e * kd);
+                    }
                     num += (double)depth[yi * width + xj] * f;
                     den += f;
                 }
+            if (guard_out) guard_out[y * width + x] = (uint8_t)guard;
             if (poisoned) out[y * width + x] = NAN;
             else out[y * width + x] = (den == 0.0) ? 0.0f : (float)(num / den);
         }

@@ -6,6 +6,7 @@ import pytest
 import torch
 
 from conftest import synth_np
+from test_guided_f64 import check_guided_against_f64
 
 import oracle
 
@@ -71,22 +72,9 @@ def test_guided_fill_vs_oracle(w, h, radius, use_labels):
     from kinectdepthmapenhancement_b200 import guided_fill
     depth, bgr = synth_np(w, h, seed=17, frame=radius)
     labels = ((np.arange(h)[:, None] // 16) * 64 + (np.arange(w)[None, :] // 12)).astype(np.int32) if use_labels else None
-    ws = 2 * radius + 1
-    o32 = oracle.guided_fill(depth, bgr, labels, ws)
-    o64 = oracle.guided_fill(depth, bgr, labels, ws, precision="f64")
     got = guided_fill(torch.from_numpy(depth).cuda(), torch.from_numpy(bgr).cuda(),
                       torch.from_numpy(labels).cuda() if use_labels else None, radius).cpu().numpy()
-    assert np.array_equal(np.isnan(got), np.isnan(o64))
-    ok = ~np.isnan(o64)
-    assert np.array_equal(got[ok] > 0, o64[ok] > 0), "valid/hole mask differs"
-    err = np.abs(got[ok].astype(np.float64) - o64[ok])
-    e32 = np.abs(o32[ok].astype(np.float64) - o64[ok])
-    print(f"\nguided fill {w}x{h} r={radius}: gpu vs f64 median {np.median(err):.2e} p99 {np.quantile(err, 0.99):.2e} "
-          f"max {err.max():.2e} | reference-order fp32 vs f64 p99 {np.quantile(e32, 0.99):.2e} max {e32.max():.2e}")
-    # float tolerance: 1e-3 mm on the bulk; never worse than the reference's own fp32 arithmetic
-    assert np.median(err) <= 2.5e-4
-    assert np.quantile(err, 0.99) <= max(1e-3, np.quantile(e32, 0.99))
-    assert err.max() <= max(0.05, e32.max())
+    check_guided_against_f64(got, depth, bgr, labels, 2 * radius + 1, what="guided fill")
 
 
 def test_guided_fill_golden(golden_dir):
@@ -156,14 +144,7 @@ def test_guided_upsample_matches_oracle():
     labels = ((np.arange(hh)[:, None] // 24) * 64 + (np.arange(wh)[None, :] // 30)).astype(np.int32)
     got = guided_upsample(lo.cuda(), hi.cuda(), torch.from_numpy(labels).cuda(), r).cpu().numpy()
     sparse = oracle.scatter_lowres(lo.numpy(), wh, hh)
-    o64 = oracle.guided_fill(sparse, hi.numpy(), labels, 2 * r + 1, precision="f64")
-    o32 = oracle.guided_fill(sparse, hi.numpy(), labels, 2 * r + 1)
-    assert np.array_equal(np.isnan(got), np.isnan(o64))
-    ok = ~np.isnan(o64)
-    assert np.array_equal(got[ok] > 0, o64[ok] > 0)
-    err = np.abs(got[ok].astype(np.float64) - o64[ok])
-    e32 = np.abs(o32[ok].astype(np.float64) - o64[ok])
-    assert np.median(err) <= 2.5e-4 and np.quantile(err, 0.99) <= max(1e-3, np.quantile(e32, 0.99))
+    check_guided_against_f64(got, sparse, hi.numpy(), labels, 2 * r + 1, what="guided upsample")
     # identical to the same-resolution fill of the materialised sparse image
     dense = guided_fill(torch.from_numpy(sparse).cuda(), hi.cuda(), torch.from_numpy(labels).cuda(), r).cpu().numpy()
     assert np.array_equal(np.nan_to_num(dense, nan=-1).view(np.uint32), np.nan_to_num(got, nan=-1).view(np.uint32))

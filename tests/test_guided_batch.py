@@ -299,25 +299,15 @@ def test_python_batch_forms_reject_bad_shapes():
 # ------------------------------------------------------------------ GPU: oracle sanity
 @pytest.mark.gpu
 def test_last_batch_frame_matches_the_f64_oracle():
-    """Frame offsets against the fp64 formula, not only against the GPU itself (tolerance of
-    test_gpu_buffers_guided.py::test_guided_fill_vs_oracle)."""
-    import oracle
+    """Frame offsets against the fp64 formula, not only against the GPU itself."""
+    from test_guided_f64 import check_guided_against_f64
     n, w, h, r = 3, 160, 120, 3
     d = _depth(n, w, h, seed=17)
     g = _guides(n, w, h, 3, seed=17)
     lab = _labels(n, w, h, seed=17)
     got = _fill_batch(d, lab, g, 3, r)[n - 1].cpu().numpy()
-    args = (d[n - 1].cpu().numpy(), g[n - 1].cpu().numpy(), lab[n - 1].cpu().numpy(), 2 * r + 1)
-    o64 = oracle.guided_fill(*args, precision="f64")
-    o32 = oracle.guided_fill(*args)
-    assert np.array_equal(np.isnan(got), np.isnan(o64))
-    ok = ~np.isnan(o64)
-    assert np.array_equal(got[ok] > 0, o64[ok] > 0), "valid/hole mask differs"
-    err = np.abs(got[ok].astype(np.float64) - o64[ok])
-    e32 = np.abs(o32[ok].astype(np.float64) - o64[ok])
-    assert np.median(err) <= 2.5e-4
-    assert np.quantile(err, 0.99) <= max(1e-3, np.quantile(e32, 0.99))
-    assert err.max() <= max(0.05, e32.max())
+    check_guided_against_f64(got, d[n - 1].cpu().numpy(), g[n - 1].cpu().numpy(), lab[n - 1].cpu().numpy(), 2 * r + 1,
+                             SS, SC, SD, what="last batch frame")
 
 
 # ------------------------------------------------------------------ GPU: more frames than one launch holds
@@ -410,4 +400,15 @@ def test_bad_arguments_are_rejected():
                 args = list(ok)
                 args[i] = bad
                 assert fn(*args) == L.KDME_EINVAL, (fn.__name__, i, bad)
+    # the upsampling reads depth_lo while it writes out_hi: overlapping byte ranges are rejected the same way
+    lo_bytes, lo16_bytes, out_bytes = 4 * 7 * 5 * n, 2 * 7 * 5 * n, 4 * w * h * n
+    for fn, nb in ((lib.kdme_guided_upsample_batch, lo_bytes), (lib.kdme_guided_upsample_batch_u16, lo16_bytes)):
+        for i0, o0 in ((0, 0), (0, (nb - 1) // 4 * 4), (out_bytes - 4, 0)):
+            rc = fn(base + i0, 7, 5, None, g.data_ptr(), 0, 3, base + o0, w, h, n, 3, SS, SC, SD, s)
+            assert rc == L.KDME_EINVAL, (fn.__name__, i0, o0)
+        after = (nb + 255) // 256 * 256   # the first aligned float past the input
+        assert fn(base, 7, 5, None, g.data_ptr(), 0, 3, base + after, w, h, n, 3, SS, SC, SD, s) == L.KDME_OK
+        assert fn(base + out_bytes, 7, 5, None, g.data_ptr(), 0, 3, base, w, h, n, 3, SS, SC, SD, s) == L.KDME_OK
+    assert lib.kdme_guided_upsample_ex(base, 7, 5, None, g.data_ptr(), 0, 3, base + 4, w, h, 3, SS, SC, SD,
+                                       s) == L.KDME_EINVAL
     torch.cuda.synchronize()

@@ -37,6 +37,83 @@ def test_guided_fill_matches_reference_golden(gold):
     assert np.array_equal(out.view(np.uint32), gold["guided_ws7_nolabel"].view(np.uint32))
 
 
+# ---------------------------------------------------------------- guided fill: the fp64 guard (DESIGN.md section 2)
+def _guided_guard(d, c, lab=None, ws=7, **kw):
+    o, mean, guard = oracle.guided_fill(d, c, lab, ws, precision="f64", return_mean=True, return_guard=True,
+                                        threads=2, **kw)
+    return o, mean, guard
+
+
+def test_guided_guard_is_clear_on_a_smooth_frame():
+    w, h = 64, 48
+    yy, xx = np.mgrid[0:h, 0:w]
+    d = (1500.0 + 3.0 * xx + 2.0 * yy).astype(np.float32)
+    c = np.stack([(xx * 2) % 256, (yy * 3) % 256, np.full_like(xx, 128)], -1).astype(np.uint8)
+    for ws in (3, 7, 15):
+        o, _, guard = _guided_guard(d, c, ws=ws)
+        assert not np.isnan(o).any() and np.all(o > 0)
+        assert not guard.any(), ws
+
+
+def test_guided_guard_flags_a_depth_tap_at_the_cut():
+    """Two surfaces with labels of their own: the near one's sweep-1 mean is exactly 1000, and the far one is moved
+    so that e^2 kd of its taps lands on the expf() zero cut of sweep 3."""
+    w, h, ws, sd = 16, 9, 7, 70.0
+    c = np.full((h, w, 3), 100, np.uint8)
+    lab = (np.arange(w)[None, :] >= 8).astype(np.int32) * np.ones((h, 1), np.int32)
+    kd = 1.0 / (2.0 * sd * sd)
+    y, x = 4, 7                                              # the last column of the near surface
+    for far, flagged in ((1000.0 + np.sqrt(103.97207708399179 / kd), True), (1000.0 + 1015.0, False)):
+        d = np.where(lab == 0, 1000.0, far).astype(np.float32)
+        _, mean, guard = _guided_guard(d, c, lab, ws=ws, sigma_d=sd)
+        assert mean[y, x] == 1000.0
+        assert bool(guard[y, x] & 1) == flagged, far
+
+
+def test_guided_guard_flags_a_colour_tap_at_the_cut():
+    """Sweep 1 with sigma_c chosen so that cd / (2 sigma_c^2) of one tap is the cut exactly."""
+    w, h = 5, 5
+    d = np.full((h, w), 1000.0, np.float32)
+    c = np.full((h, w, 3), 50, np.uint8)
+    c[0, 0] = (60, 50, 50)                                   # cd = 100 for the centre pixel
+    sc = np.float32(np.sqrt(100.0 / (2.0 * 103.97207708399179)))
+    _, _, guard = _guided_guard(d, c, ws=5, sigma_c=float(sc))
+    assert guard[2, 2] & 1
+    _, _, guard = _guided_guard(d, c, ws=5, sigma_c=float(sc) * 1.01)
+    assert not guard[2, 2] & 1
+
+
+def test_guided_guard_flags_the_recurrence_test():
+    """adaptive = 5 dev / mean^2 within a few ulps of sigma * 0.3f at the first valid tap."""
+    w, h, ws = 3, 1, 3
+    c = np.full((h, w, 3), 7, np.uint8)
+    # three taps of one label, depths m - a, m, m + a: dev = 2a/3, adaptive = 10a / (3 m^2)
+    m = np.float32(64.0)
+    # sigma_c is set so that sigma_c * 0.3f is about adaptive; scan a until the rounding puts it within the margin
+    for a in np.linspace(1.0, 14.0, 2000, dtype=np.float32):
+        d = np.array([[m - a, m, m + a]], np.float32)
+        if (d > 50).all():
+            _, _, g = _guided_guard(d, c, ws=ws, sigma_c=float(np.float32(10.0) * np.float32(a) / (3 * m * m) / 0.3))
+            if g[0, 1] & 2:
+                break
+    else:
+        pytest.fail("no recurrence-test case found")
+
+
+def test_guided_guard_flags_the_underflow_of_2_sigma_squared():
+    """sigma = adaptive from the first valid tap (sigma_c * 0.3f is below it), with adaptive = 5 dev / mean^2 so small
+    that 2 sigma^2 is a few subnormal ulps or 0: the -0/0 NaN is decided there.  A spread of one fp32 ulp at 1e15-1e16
+    gives adaptive from 1.5e-22 (2 sigma^2 = 32 subnormal ulps: clear) down to 2.4e-23 (2 sigma^2 = 0: NaN)."""
+    c = np.full((1, 3, 3), 7, np.uint8)
+    flags = []
+    for base in (1e15, 3e15, 1e16):
+        b = np.float32(base)
+        d = np.array([[b, np.nextafter(b, np.float32(np.inf)), b]], np.float32)
+        o, _, guard = _guided_guard(d, c, ws=3, sigma_c=1e-23)
+        flags.append((bool(guard[0, 1] & 4), bool(np.isnan(o[0, 1]))))
+    assert flags == [(False, False), (True, False), (True, True)]
+
+
 def test_mrf_matches_reference_golden(gold):
     out = oracle.mrf(gold["depth"], gold["bgr"], threads=2)
     assert np.array_equal(out.view(np.uint32), gold["mrf_ws5"].view(np.uint32))
