@@ -1307,9 +1307,14 @@ constexpr int kMaxGridZ = 65535;   // gridDim.z limit: frames per launch
 template <class T>
 static T* advance(T* ptr, long long n) { return ptr ? ptr + n : ptr; }
 
-// The fields GuidedParams and GuidedFastParams<R> share: image, pointers and per-frame strides.
-template <class P>
-static void guided_common(P& p, const GuidedCall& c) {
+// 1 / (2 sigma^2) in double, as the fp64 oracle forms it; 0 for sigma = 0, where the reference skips the factor.
+static double guided_k(float sigma) { return (sigma != 0.0f) ? 1.0 / (2.0 * (double)sigma * (double)sigma) : 0.0; }
+
+// The kernel's parameters for the whole call: image, pointers, per-frame strides, sigmas and spatial factors.
+template <int WS_CT>
+static GuidedParams<WS_CT> guided_params(const GuidedCall& c) {
+    static_assert(2 * KDME_MAX_RADIUS + 1 <= 31, "GuidedParams<0> holds a window of at most 31 x 31 factors");
+    GuidedParams<WS_CT> p;
     const long long plane = (long long)c.width * c.height;
     p.width = c.width; p.height = c.height;
     p.depth = c.depth; p.depth16 = c.depth16; p.depth_lo = c.depth_lo; p.depth_lo16 = c.depth_lo16;
@@ -1319,6 +1324,14 @@ static void guided_common(P& p, const GuidedCall& c) {
     p.bgr_stride = (long long)c.height * (long long)c.bgr_step;
     p.labels_stride = c.labels ? plane : 0;
     p.out_stride = plane;
+    p.sigma_c = c.sigma_c;
+    p.radius = c.radius;
+    p.kc = guided_k(c.sigma_c);
+    p.kd = guided_k(c.sigma_d);
+    std::vector<float> lut;
+    host_spatial_lut(lut, 2 * c.radius + 1, c.sigma_s);
+    for (size_t i = 0; i < lut.size(); i++) p.sfac[i] = (lut[i] != 0.0f) ? lut[i] : 1.0f;
+    return p;
 }
 
 // Launches `kernel` over the call's frames in slices of at most kMaxGridZ frames (blockIdx.z), in order on one
@@ -1343,58 +1356,25 @@ static int guided_slices(const P& p0, int n_frames, void (*kernel)(const P), siz
     return KDME_OK;
 }
 
-// 1 / (2 sigma^2) in double, as the fp64 oracle forms it; 0 for sigma = 0, where the reference skips the factor.
-static double guided_k(float sigma) { return (sigma != 0.0f) ? 1.0 / (2.0 * (double)sigma * (double)sigma) : 0.0; }
-
-template <int R, int C>
-static int guided_launch_fast(const GuidedCall& c, const std::vector<float>& lut, cudaStream_t stream) {
-    constexpr int ws = 2 * R + 1;
-    GuidedFastParams<R> p;
-    for (int i = 0; i < ws * ws; i++) p.sfac[i] = (lut[i] != 0.0f) ? (double)lut[i] : 1.0;
-    guided_common(p, c);
-    p.sigma_c = c.sigma_c;
-    p.kc = guided_k(c.sigma_c);
-    p.kd = guided_k(c.sigma_d);
+// One launch path for both window forms; the depth type is chosen once per call, whatever the number of frames.
+template <int WS_CT, int C>
+static int guided_launch(const GuidedCall& c, cudaStream_t stream) {
+    const GuidedParams<WS_CT> p = guided_params<WS_CT>(c);
+    const size_t smem = (WS_CT > 0) ? 0 : (size_t)(kGuidedTW + 2 * c.radius) * (kGuidedTH + 2 * c.radius) * 12;
     if (c.depth16 || c.depth_lo16)
-        return guided_slices(p, c.n_frames, guided_fill_fast_kernel<R, kGuidedTW, kGuidedTH, C, true>, 0, stream);
-    return guided_slices(p, c.n_frames, guided_fill_fast_kernel<R, kGuidedTW, kGuidedTH, C, false>, 0, stream);
+        return guided_slices(p, c.n_frames, guided_fill_kernel<WS_CT, kGuidedTW, kGuidedTH, C, true>, smem, stream);
+    return guided_slices(p, c.n_frames, guided_fill_kernel<WS_CT, kGuidedTW, kGuidedTH, C, false>, smem, stream);
 }
 
-// The spatial LUT and the kernel are chosen once per call, whatever the number of frames.
+// Windows 3..7 run the compile-time-window form, every other window the run-time one; both at any sigmas.
 template <int C>
 static int guided_launch_c(const GuidedCall& c, cudaStream_t stream) {
-    const int ws = 2 * c.radius + 1;
-    std::vector<float> lut;
-    host_spatial_lut(lut, ws, c.sigma_s);
-    // fast form: compile-time window 3..7, the same sweeps (guided_sweeps) at any sigmas
     switch (c.radius) {
-        case 1: return guided_launch_fast<1, C>(c, lut, stream);
-        case 2: return guided_launch_fast<2, C>(c, lut, stream);
-        case 3: return guided_launch_fast<3, C>(c, lut, stream);
-        default: break;
+        case 1: return guided_launch<3, C>(c, stream);
+        case 2: return guided_launch<5, C>(c, stream);
+        case 3: return guided_launch<7, C>(c, stream);
+        default: return guided_launch<0, C>(c, stream);
     }
-    GuidedParams p;
-    if (ws * ws > (int)(sizeof(p.spatial) / sizeof(float))) return fail(KDME_ENOTSUP, "guided fill: window too large");
-    for (int i = 0; i < ws * ws; i++) p.spatial[i] = lut[i];
-    guided_common(p, c);
-    p.radius = c.radius;
-    p.sigma_c = c.sigma_c;
-    p.kc = guided_k(c.sigma_c); p.kd = guided_k(c.sigma_d);
-    const int SP = kGuidedTW + 2 * c.radius, SH = kGuidedTH + 2 * c.radius;
-    if (c.depth16 || c.depth_lo16)
-        return guided_slices(p, c.n_frames, guided_fill_kernel<kGuidedTW, kGuidedTH, C, true>, (size_t)SP * SH * 12, stream);
-    return guided_slices(p, c.n_frames, guided_fill_kernel<kGuidedTW, kGuidedTH, C, false>, (size_t)SP * SH * 12, stream);
-}
-
-// The checks every guided entry point shares, then the launch.  `depth` is the call's depth input (any of the four
-// forms), on the current device.
-static int guided_run(GuidedCall c, const void* depth, int channels, void* stream, const char* who) {
-    if (c.radius < 0 || c.radius > KDME_MAX_RADIUS) return fail(KDME_EINVAL, std::string(who) + ": bad radius");
-    if (channels != KDME_GUIDE_GRAY && channels != KDME_GUIDE_BGR && channels != KDME_GUIDE_BGRX)
-        return fail(KDME_EINVAL, std::string(who) + ": guide_channels must be 1 (GRAY), 3 (BGR) or 4 (BGRX)");
-    { int rc = check_guide_step(channels, c.width, &c.bgr_step, who); if (rc != KDME_OK) return rc; }
-    { int rcd = check_pointer_device(depth, who); if (rcd != KDME_OK) return rcd; }
-    return with_channels(channels, [&](auto ch) { return guided_launch_c<decltype(ch)::value>(c, (cudaStream_t)stream); });
 }
 
 // The kernels read every frame's depth while they write the output: true where the depth input's `in_bytes` and the
@@ -1405,66 +1385,54 @@ static bool guided_overlap(const void* in, unsigned long long in_bytes, const fl
     return i0 < o1 && o0 < i1;
 }
 
-// n_frames fills; the depth is float (depth) or uint16 (depth16), the other one is NULL.
-static int guided_fill_batch(const float* depth, const uint16_t* depth16, const int32_t* labels, const uint8_t* bgr,
-                             size_t bgr_step, int channels, float* out, int width, int height, int n_frames,
-                             int window_radius, float sigma_spatial, float sigma_color, float sigma_depth, void* stream,
-                             const char* who) {
-    const void* in = depth ? (const void*)depth : (const void*)depth16;
-    if (!in || !bgr || !out) return fail(KDME_EINVAL, std::string(who) + ": NULL argument");
-    if (n_frames < 1) return fail(KDME_EINVAL, std::string(who) + ": n_frames must be >= 1");
-    if (width <= 0 || height <= 0) return fail(KDME_EINVAL, std::string(who) + ": bad size");
-    if (guided_overlap(in, (unsigned long long)width * height * n_frames * (depth ? sizeof(float) : sizeof(uint16_t)),
-                       out, (unsigned long long)width * height * n_frames))
-        return fail(KDME_EINVAL, std::string(who) + ": the output overlaps the depth input (in-place operation is not supported)");
-    GuidedCall c{depth, depth16, nullptr, nullptr, 0, 0, labels, bgr, bgr_step, out, width, height, n_frames,
-                 window_radius, sigma_spatial, sigma_color, sigma_depth};
-    return guided_run(c, in, channels, stream, who);
-}
-
-// n_frames upsamplings; the low-res depth is float (depth_lo) or uint16 (depth_lo16), the other one is NULL.
-static int guided_upsample_batch(const float* depth_lo, const uint16_t* depth_lo16, int wl, int hl,
-                                 const int32_t* labels_hi, const uint8_t* bgr_hi, size_t bgr_step, int channels,
-                                 float* out_hi, int width, int height, int n_frames, int window_radius,
-                                 float sigma_spatial, float sigma_color, float sigma_depth, void* stream,
-                                 const char* who) {
-    const void* in = depth_lo ? (const void*)depth_lo : (const void*)depth_lo16;
-    if (!in || !bgr_hi || !out_hi) return fail(KDME_EINVAL, std::string(who) + ": NULL argument");
-    if (n_frames < 1) return fail(KDME_EINVAL, std::string(who) + ": n_frames must be >= 1");
-    if (width <= 0 || height <= 0 || wl <= 0 || hl <= 0 || wl > width || hl > height)
+// Every guided entry point: the checks in order, then the launch.  The call is a fill when its depth is depth or
+// depth16, an upsampling when it is depth_lo or depth_lo16; the other three are NULL.
+static int guided_batch(GuidedCall c, int channels, void* stream, const char* who) {
+    const void* lo = c.depth_lo ? (const void*)c.depth_lo : (const void*)c.depth_lo16;
+    const void* in = lo ? lo : c.depth ? (const void*)c.depth : (const void*)c.depth16;
+    if (!in || !c.bgr || !c.out) return fail(KDME_EINVAL, std::string(who) + ": NULL argument");
+    if (c.n_frames < 1) return fail(KDME_EINVAL, std::string(who) + ": n_frames must be >= 1");
+    if (!lo && (c.width <= 0 || c.height <= 0)) return fail(KDME_EINVAL, std::string(who) + ": bad size");
+    if (lo && (c.width <= 0 || c.height <= 0 || c.wl <= 0 || c.hl <= 0 || c.wl > c.width || c.hl > c.height))
         return fail(KDME_EINVAL, std::string(who) + ": low-res size must be positive and <= the high-res size");
-    if (guided_overlap(in, (unsigned long long)wl * hl * n_frames * (depth_lo ? sizeof(float) : sizeof(uint16_t)), out_hi,
-                       (unsigned long long)width * height * n_frames))
+    const unsigned long long plane = (unsigned long long)c.width * c.height;
+    const unsigned long long in_samples = lo ? (unsigned long long)c.wl * c.hl : plane;
+    const size_t sample_bytes = (c.depth16 || c.depth_lo16) ? sizeof(uint16_t) : sizeof(float);
+    if (guided_overlap(in, in_samples * c.n_frames * sample_bytes, c.out, plane * c.n_frames))
         return fail(KDME_EINVAL, std::string(who) + ": the output overlaps the depth input (in-place operation is not supported)");
-    GuidedCall c{nullptr, nullptr, depth_lo, depth_lo16, wl, hl, labels_hi, bgr_hi, bgr_step, out_hi, width, height,
-                 n_frames, window_radius, sigma_spatial, sigma_color, sigma_depth};
-    return guided_run(c, in, channels, stream, who);
+    if (c.radius < 0 || c.radius > KDME_MAX_RADIUS) return fail(KDME_EINVAL, std::string(who) + ": bad radius");
+    if (channels != KDME_GUIDE_GRAY && channels != KDME_GUIDE_BGR && channels != KDME_GUIDE_BGRX)
+        return fail(KDME_EINVAL, std::string(who) + ": guide_channels must be 1 (GRAY), 3 (BGR) or 4 (BGRX)");
+    { int rc = check_guide_step(channels, c.width, &c.bgr_step, who); if (rc != KDME_OK) return rc; }
+    { int rcd = check_pointer_device(in, who); if (rcd != KDME_OK) return rcd; }
+    return with_channels(channels, [&](auto ch) { return guided_launch_c<decltype(ch)::value>(c, (cudaStream_t)stream); });
 }
 
 extern "C" int kdme_guided_fill_batch(const float* depth_dev, const int32_t* labels_dev, const uint8_t* bgr_dev,
                                       size_t bgr_step, int guide_channels, float* out_dev, int width, int height,
                                       int n_frames, int window_radius, float sigma_spatial, float sigma_color,
                                       float sigma_depth, void* stream) {
-    return guided_fill_batch(depth_dev, nullptr, labels_dev, bgr_dev, bgr_step, guide_channels, out_dev, width, height,
-                             n_frames, window_radius, sigma_spatial, sigma_color, sigma_depth, stream,
-                             "kdme_guided_fill_batch");
+    return guided_batch({depth_dev, nullptr, nullptr, nullptr, 0, 0, labels_dev, bgr_dev, bgr_step, out_dev, width,
+                         height, n_frames, window_radius, sigma_spatial, sigma_color, sigma_depth},
+                        guide_channels, stream, "kdme_guided_fill_batch");
 }
 
 extern "C" int kdme_guided_fill_batch_u16(const uint16_t* depth_dev, const int32_t* labels_dev, const uint8_t* bgr_dev,
                                           size_t bgr_step, int guide_channels, float* out_dev, int width, int height,
                                           int n_frames, int window_radius, float sigma_spatial, float sigma_color,
                                           float sigma_depth, void* stream) {
-    return guided_fill_batch(nullptr, depth_dev, labels_dev, bgr_dev, bgr_step, guide_channels, out_dev, width, height,
-                             n_frames, window_radius, sigma_spatial, sigma_color, sigma_depth, stream,
-                             "kdme_guided_fill_batch_u16");
+    return guided_batch({nullptr, depth_dev, nullptr, nullptr, 0, 0, labels_dev, bgr_dev, bgr_step, out_dev, width,
+                         height, n_frames, window_radius, sigma_spatial, sigma_color, sigma_depth},
+                        guide_channels, stream, "kdme_guided_fill_batch_u16");
 }
 
 extern "C" int kdme_guided_fill_ex(const float* depth_dev, const int32_t* labels_dev, const uint8_t* bgr_dev,
                                    size_t bgr_step, int guide_channels, float* out_dev, int width, int height,
                                    int window_radius, float sigma_spatial, float sigma_color, float sigma_depth,
                                    void* stream) {
-    return guided_fill_batch(depth_dev, nullptr, labels_dev, bgr_dev, bgr_step, guide_channels, out_dev, width, height,
-                             1, window_radius, sigma_spatial, sigma_color, sigma_depth, stream, "kdme_guided_fill");
+    return guided_batch({depth_dev, nullptr, nullptr, nullptr, 0, 0, labels_dev, bgr_dev, bgr_step, out_dev, width,
+                         height, 1, window_radius, sigma_spatial, sigma_color, sigma_depth},
+                        guide_channels, stream, "kdme_guided_fill");
 }
 
 extern "C" int kdme_guided_fill(const float* depth_dev, const int32_t* labels_dev, const uint8_t* bgr_dev,
@@ -1478,9 +1446,9 @@ extern "C" int kdme_guided_upsample_batch(const float* depth_lo_dev, int wl, int
                                           const uint8_t* bgr_hi_dev, size_t bgr_step, int guide_channels,
                                           float* out_hi_dev, int width, int height, int n_frames, int window_radius,
                                           float sigma_spatial, float sigma_color, float sigma_depth, void* stream) {
-    return guided_upsample_batch(depth_lo_dev, nullptr, wl, hl, labels_hi_dev, bgr_hi_dev, bgr_step, guide_channels,
-                                 out_hi_dev, width, height, n_frames, window_radius, sigma_spatial, sigma_color,
-                                 sigma_depth, stream, "kdme_guided_upsample_batch");
+    return guided_batch({nullptr, nullptr, depth_lo_dev, nullptr, wl, hl, labels_hi_dev, bgr_hi_dev, bgr_step, out_hi_dev,
+                         width, height, n_frames, window_radius, sigma_spatial, sigma_color, sigma_depth},
+                        guide_channels, stream, "kdme_guided_upsample_batch");
 }
 
 extern "C" int kdme_guided_upsample_batch_u16(const uint16_t* depth_lo_dev, int wl, int hl,
@@ -1488,18 +1456,18 @@ extern "C" int kdme_guided_upsample_batch_u16(const uint16_t* depth_lo_dev, int 
                                               int guide_channels, float* out_hi_dev, int width, int height,
                                               int n_frames, int window_radius, float sigma_spatial, float sigma_color,
                                               float sigma_depth, void* stream) {
-    return guided_upsample_batch(nullptr, depth_lo_dev, wl, hl, labels_hi_dev, bgr_hi_dev, bgr_step, guide_channels,
-                                 out_hi_dev, width, height, n_frames, window_radius, sigma_spatial, sigma_color,
-                                 sigma_depth, stream, "kdme_guided_upsample_batch_u16");
+    return guided_batch({nullptr, nullptr, nullptr, depth_lo_dev, wl, hl, labels_hi_dev, bgr_hi_dev, bgr_step, out_hi_dev,
+                         width, height, n_frames, window_radius, sigma_spatial, sigma_color, sigma_depth},
+                        guide_channels, stream, "kdme_guided_upsample_batch_u16");
 }
 
 extern "C" int kdme_guided_upsample_ex(const float* depth_lo_dev, int wl, int hl, const int32_t* labels_hi_dev,
                                        const uint8_t* bgr_hi_dev, size_t bgr_step, int guide_channels, float* out_hi_dev,
                                        int width, int height, int window_radius, float sigma_spatial, float sigma_color,
                                        float sigma_depth, void* stream) {
-    return guided_upsample_batch(depth_lo_dev, nullptr, wl, hl, labels_hi_dev, bgr_hi_dev, bgr_step, guide_channels,
-                                 out_hi_dev, width, height, 1, window_radius, sigma_spatial, sigma_color, sigma_depth,
-                                 stream, "kdme_guided_upsample");
+    return guided_batch({nullptr, nullptr, depth_lo_dev, nullptr, wl, hl, labels_hi_dev, bgr_hi_dev, bgr_step, out_hi_dev,
+                         width, height, 1, window_radius, sigma_spatial, sigma_color, sigma_depth},
+                        guide_channels, stream, "kdme_guided_upsample");
 }
 
 extern "C" int kdme_guided_upsample(const float* depth_lo_dev, int wl, int hl, const int32_t* labels_hi_dev,

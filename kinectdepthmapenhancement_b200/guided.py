@@ -13,6 +13,11 @@ WindowSize, SpatialSigma, ColorSigma, DepthSigma = 7, 30.0, 50.0, 70.0
 _DEPTH_DTYPES = (torch.float32, torch.uint16, torch.int16)
 
 
+def _one(t):
+    """One frame as a batch of one (its [None] view); None stays None."""
+    return None if t is None else t[None]
+
+
 def _batch_depth(depth: torch.Tensor, name: str) -> tuple:
     """Checks a [N, rows, cols] float32 or uint16 depth batch (torch.uint16 or an int16 view of the same bits)."""
     if depth.dtype not in _DEPTH_DTYPES:
@@ -52,22 +57,10 @@ def guided_fill(depth: torch.Tensor, color: torch.Tensor, labels: torch.Tensor |
     depth's rank decides which form runs; frame k equals the fill of frame k alone, bit for bit."""
     if isinstance(depth, torch.Tensor) and depth.dim() == 3:
         return _guided_fill_batch(depth, color, labels, window_radius, spatial_sigma, color_sigma, depth_sigma, out)
-    dev = depth.device
-    _check_cuda(depth, torch.float32, "depth", dev)
-    _check_cuda(color, torch.uint8, "color", dev)
-    h, w = depth.shape
-    c = guide_channels(color, (h, w))
-    if labels is not None:
-        _check_cuda(labels, torch.int32, "labels", dev)
-        if tuple(labels.shape) != (h, w):
-            raise ValueError("labels must be [H,W]")
-    if out is None:
-        out = torch.empty_like(depth)
-    with torch.cuda.device(dev):
-        _lib.check(_lib.lib().kdme_guided_fill_ex(_ptr(depth), _ptr(labels) if labels is not None else None,
-                                                  _ptr(color), c * w, c, _ptr(out), w, h, window_radius, spatial_sigma,
-                                                  color_sigma, depth_sigma, torch.cuda.current_stream().cuda_stream))
-    return out
+    _check_cuda(depth, torch.float32, "depth", depth.device)
+    res = _guided_fill_batch(depth[None], _one(color), _one(labels), window_radius, spatial_sigma, color_sigma,
+                             depth_sigma, _one(out))
+    return res[0] if out is None else out
 
 
 def _guided_fill_batch(depth, color, labels, window_radius, spatial_sigma, color_sigma, depth_sigma, out):
@@ -96,27 +89,10 @@ def guided_upsample(depth_lo: torch.Tensor, color_hi: torch.Tensor, labels_hi: t
     if isinstance(depth_lo, torch.Tensor) and depth_lo.dim() == 3:
         return _guided_upsample_batch(depth_lo, color_hi, labels_hi, window_radius, spatial_sigma, color_sigma,
                                       depth_sigma, out)
-    dev = depth_lo.device
-    _check_cuda(depth_lo, torch.float32, "depth_lo", dev)
-    _check_cuda(color_hi, torch.uint8, "color_hi", dev)
-    hl, wl = depth_lo.shape
-    if color_hi.dim() not in (2, 3):
-        raise ValueError(f"color_hi must be [H,W] or [H,W,C], got {list(color_hi.shape)}")
-    h, w = color_hi.shape[:2]
-    c = guide_channels(color_hi, (h, w), "color_hi")
-    if labels_hi is not None:
-        _check_cuda(labels_hi, torch.int32, "labels_hi", dev)
-        if tuple(labels_hi.shape) != (h, w):
-            raise ValueError("labels must be [H,W] at the high-res size")
-    if out is None:
-        out = torch.empty((h, w), dtype=torch.float32, device=dev)
-    with torch.cuda.device(dev):
-        _lib.check(_lib.lib().kdme_guided_upsample_ex(_ptr(depth_lo), wl, hl,
-                                                      _ptr(labels_hi) if labels_hi is not None else None,
-                                                      _ptr(color_hi), c * w, c, _ptr(out), w, h, window_radius,
-                                                      spatial_sigma, color_sigma, depth_sigma,
-                                                      torch.cuda.current_stream().cuda_stream))
-    return out
+    _check_cuda(depth_lo, torch.float32, "depth_lo", depth_lo.device)
+    res = _guided_upsample_batch(depth_lo[None], _one(color_hi), _one(labels_hi), window_radius, spatial_sigma,
+                                 color_sigma, depth_sigma, _one(out))
+    return res[0] if out is None else out
 
 
 def _guided_upsample_batch(depth_lo, color_hi, labels_hi, window_radius, spatial_sigma, color_sigma, depth_sigma,

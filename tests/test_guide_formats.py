@@ -339,7 +339,7 @@ def test_mrf_and_guided_fill_and_upsample(c, w, h):
     labels = _cuda(((np.arange(h)[:, None] // 9) * 64 + (np.arange(w)[None, :] // 11)).astype(np.int32))
     lo = _cuda(depth[::3, ::3])
     for lab in (None, labels):
-        for r in (1, 3, 5):   # 1..3 fast kernel, 5 generic
+        for r in (1, 3, 5):   # 1..3 compile-time window, 5 run-time window
             assert np.array_equal(_bits(guided_fill(d, _cuda(img), lab, r)), _bits(guided_fill(d, _cuda(ref), lab, r)))
             assert np.array_equal(_bits(guided_upsample(lo, _cuda(img), lab, r)),
                                   _bits(guided_upsample(lo, _cuda(ref), lab, r)))

@@ -5,9 +5,9 @@ One identity defines the batch, checked bit for bit on the GPU:
 
     frame k of kdme_guided_*_batch(frames)  ==  kdme_guided_*_ex(frame k)
 
-for the fast kernel (r = 1..3) and the runtime-radius kernel, with and without per-frame labels, every guide format,
-float32 and uint16 depth, and batches longer than one launch's 65535 frames.  Every frame is distinct, so a wrong
-frame offset of any plane shows.
+for both forms of the guided kernel (compile-time window, r = 1..3; run-time window), with and without per-frame
+labels, every guide format, float32 and uint16 depth, and batches longer than one launch's 65535 frames.  Every frame
+is distinct, so a wrong frame offset of any plane shows.
 """
 import ctypes as C
 import os

@@ -5,8 +5,8 @@ check_guided_against_f64 is the one check: the NaN positions and the mask `out >
 and every other pixel is within 1e-3 mm of it, except the guard-active pixels the oracle names (a branch of the fp32
 formula decided within a few ulps of its threshold), which must stay inside the range of their window's samples.
 Nothing here is derived from the kernel's output.  The cases sweep the shapes (ragged against the 32x8 tile, 1x1 to
-1920x1080), both kernels (the compile-time-window fast kernel at r = 1..3, the runtime-window kernel at r = 0 and
-r >= 4), the sigmas, labels, the guide formats, uint16 depth and frames built to hit each branch of the formula.
+1920x1080), both forms of the guided kernel (the compile-time window at r = 1..3, the run-time window at r = 0
+and r >= 4), the sigmas, labels, the guide formats, uint16 depth and frames built to hit each branch of the formula.
 """
 import numpy as np
 import pytest

@@ -11,7 +11,7 @@ ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 LIB = os.path.join(ROOT, "kinectdepthmapenhancement_b200", "libkdme_b200.so")
 WANT = ("UTMALDG", "SYNCS", "VABSDIFF4", "IDP.4A", "MUFU.EX2", "MUFU.RCP", "FFMA2", "FADD2", "LDS.128", "DFMA", "DADD",
         "ACQBULK", "UTMAPF", "ATOMG", "RED")
-KERNELS = re.compile(r"jbf_fast_kernelILi(2|7|9|15)ELi64ELi(16|8)E|jbf_refine_kernelILi8E|jbf_upsample_gather|presmooth5|guided_fill_fast_kernelILi3E")
+KERNELS = re.compile(r"jbf_fast_kernelILi(2|7|9|15)ELi64ELi(16|8)E|jbf_refine_kernelILi8E|jbf_upsample_gather|presmooth5|guided_fill_kernelILi7E")
 
 
 def main():
