@@ -16,8 +16,8 @@
  * Guide formats: Process, ProcessXYZ and Upsampling take the guide's format from
  * color_image.channels(): CV_8UC3 BGR (the reference's), CV_8UC4 BGRX/BGRA (Kinect v2, Azure
  * Kinect colour frames; the 4th byte is ignored) or CV_8UC1 GRAY/IR (filters as the BGR image
- * (g,0,0)).  The pointer-based ProcessBatch / ProcessHost / UpsamplingBatch read the format set by setGuideChannels
- * (default 3).  getSmoothImage_Device returns the smoothed guide in the format of the last call.
+ * (g,0,0)).  The pointer-based ProcessBatch / ProcessXYZBatch / ProcessHost / UpsamplingBatch read the format set
+ * by setGuideChannels (default 3).  getSmoothImage_Device returns the smoothed guide in the format of the last call.
  */
 #ifndef KDME_JOINT_BILATERALFILTER_H
 #define KDME_JOINT_BILATERALFILTER_H
@@ -74,9 +74,26 @@ public:
         check(jbf_upsample(h_, depthlow_device, low_width, low_height, colorhigh_image.data, colorhigh_image.step,
                            out_device ? out_device : jbf_filtered_device(h_)));
     }
+    /* n_frames Process calls: depth frames back to back (float or uint16 millimetres, the sensor's format, read
+     * directly), guides height*bgr_step bytes apart, n_frames filtered planes out. */
     void ProcessBatch(const float* depth_device, const unsigned char* bgr_device, size_t bgr_step, float* out_device,
                       int n_frames) {
         check(jbf_process_batch(h_, depth_device, bgr_device, bgr_step, out_device, n_frames));
+    }
+    void ProcessBatch(const unsigned short* depth_device, const unsigned char* bgr_device, size_t bgr_step,
+                      float* out_device, int n_frames) {
+        check(jbf_process_batch_u16(h_, depth_device, bgr_device, bgr_step, out_device, n_frames));
+    }
+    /* n_frames ProcessXYZ calls: n_frames filtered planes in out_device, n_frames float3[W*H] clouds in xyz_device. */
+    void ProcessXYZBatch(const float* depth_device, const unsigned char* bgr_device, size_t bgr_step, float* out_device,
+                         float* xyz_device, int n_frames, float fx, float fy, int cx, int cy) {
+        check(jbf_process_batch_xyz(h_, depth_device, bgr_device, bgr_step, out_device, xyz_device, n_frames, fx, fy,
+                                    cx, cy));
+    }
+    void ProcessXYZBatch(const unsigned short* depth_device, const unsigned char* bgr_device, size_t bgr_step,
+                         float* out_device, float* xyz_device, int n_frames, float fx, float fy, int cx, int cy) {
+        check(jbf_process_batch_xyz_u16(h_, depth_device, bgr_device, bgr_step, out_device, xyz_device, n_frames, fx,
+                                        fy, cx, cy));
     }
     /* n_frames Upsampling calls: low-res frames back to back (float or uint16 millimetres, the ToF sensor's
      * format), guides height*bgr_step bytes apart, n_frames high-res planes out. */
@@ -101,7 +118,8 @@ public:
     void ProcessHost(const unsigned short* depth_host, const unsigned char* bgr_host, size_t bgr_step, float* out_host, int n_frames) {
         check(jbf_process_host_u16(h_, depth_host, bgr_host, bgr_step, out_host, n_frames));
     }
-    /* Guide format (1 GRAY, 3 BGR, 4 BGRX) of the pointer-based calls ProcessBatch / ProcessHost / UpsamplingBatch. */
+    /* Guide format (1 GRAY, 3 BGR, 4 BGRX) of the pointer-based calls ProcessBatch / ProcessXYZBatch / ProcessHost /
+     * UpsamplingBatch. */
     void setGuideChannels(int channels) {
         if (channels != Channels) { check(jbf_set_guide_channels(h_, channels)); Channels = channels; }
     }

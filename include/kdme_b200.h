@@ -76,7 +76,8 @@ void jbf_destroy(jbf_handle *h);
  *   JointBilateralFilter.cu:285.  ksize == 0 disables the pre-smooth (guide used raw). */
 int jbf_set_presmooth(jbf_handle *h, int ksize, float sigma_color, float sigma_spatial);
 
-/* Format of the raw guide every later call on this handle reads (jbf_process, _batch, _xyz, _host,
+/* Format of the raw guide every later call on this handle reads (jbf_process, _batch, _batch_u16, _batch_xyz,
+ * _batch_xyz_u16, _xyz, _host,
  * _host_u16, jbf_presmooth, _presmooth_rows, _presmooth_rows_p2p, jbf_upsample, _upsample_batch,
  * _upsample_batch_u16, jbf_mrf):
  * KDME_GUIDE_GRAY, KDME_GUIDE_BGR (the default) or KDME_GUIDE_BGRX; any other value is KDME_EINVAL.
@@ -113,6 +114,24 @@ int jbf_refine_stats(jbf_handle *h, unsigned long long *refined, unsigned long l
  * all of it (plain stream semantics; results do not depend on the chunking). */
 int jbf_process_batch(jbf_handle *h, const float *depth_dev, const uint8_t *bgr_dev, size_t bgr_step,
                       float *out_dev, int n_frames);
+/* The same with depth already on the device in the sensor's format: uint16 millimetres (Kinect, Azure Kinect
+ * frames from a decoder or a torch pipeline), read directly by the filter (no conversion pass, no float copy); a
+ * sample s filters exactly as the float (float)s, so values <= 50 are holes and frame k equals jbf_process of
+ * frame k as float, bit for bit.  KDME_EINVAL: n_frames < 1, a NULL pointer, a guide step below C*width, or an
+ * output whose bytes overlap the depth input's. */
+int jbf_process_batch_u16(jbf_handle *h, const uint16_t *depth_dev, const uint8_t *bgr_dev, size_t bgr_step,
+                          float *out_dev, int n_frames);
+/* jbf_process_xyz over n_frames frames: the filtered planes land in out_dev (n_frames planes), their clouds in
+ * xyz_dev (n_frames x height x width x 3 floats, v the row within the frame).  Stream semantics as
+ * jbf_process_batch; frame k of both outputs equals jbf_process_xyz on frame k alone (its depth plane and its
+ * cloud), bit for bit.  On a handle off the fast kernel (exotic sigmas, radius 0) each chunk is filtered and then
+ * back-projected by kdme_projective_to_real_batch on the same stream.  KDME_EINVAL: as jbf_process_batch_u16, plus
+ * a zero fx / fy and an xyz_dev that overlaps the depth input or out_dev. */
+int jbf_process_batch_xyz(jbf_handle *h, const float *depth_dev, const uint8_t *bgr_dev, size_t bgr_step,
+                          float *out_dev, float *xyz_dev, int n_frames, float fx, float fy, int cx, int cy);
+/* The same with uint16 millimetre depth (see jbf_process_batch_u16). */
+int jbf_process_batch_xyz_u16(jbf_handle *h, const uint16_t *depth_dev, const uint8_t *bgr_dev, size_t bgr_step,
+                              float *out_dev, float *xyz_dev, int n_frames, float fx, float fy, int cx, int cy);
 
 /* Filter only (JointBilateralFilter.cu:289-290): guide4_dev is an ALREADY smoothed
  * guide in the internal layout u8x4 {B,G,R,0}, row pitch guide_step bytes
@@ -157,8 +176,8 @@ int jbf_process_host(jbf_handle *h, const float *depth_host, const uint8_t *bgr_
 
 /* Same pipeline with the depth in the sensor's own format: uint16 millimetres, as xn::DepthMetaData holds it
  * (main.cpp:91-95; Buffer2D::insertData(xn::DepthMetaData*) converts it to float on the host before the
- * upload, Buffer2D.cpp:18-32).  Here the 2-byte samples are uploaded and converted on the device:
- * 5 instead of 7 bytes per pixel cross PCIe. */
+ * upload, Buffer2D.cpp:18-32).  Here the 2-byte samples are uploaded and the filter reads them directly
+ * (as jbf_process_batch_u16): 5 instead of 7 bytes per pixel cross PCIe. */
 int jbf_process_host_u16(jbf_handle *h, const uint16_t *depth_host, const uint8_t *bgr_host, size_t bgr_step,
                          float *out_host, int n_frames);
 
@@ -210,7 +229,8 @@ int jbf_upsample_batch_u16(jbf_handle *h, const uint16_t *depth_lo_dev, int wl, 
                            size_t bgr_step, float *out_hi_dev, int n_frames);
 
 /* Which kernel the handle selected: 0 = register-tiled fast path, 1 = generic path
- * (exotic sigmas / radius); bit 8 (0x100) set when the last launch staged tiles by TMA,
+ * (exotic sigmas / radius); bit 8 (0x100) set when the last launch staged tiles by TMA
+ * (uint16 depth too: needs width % 8 == 0 and a 16-byte aligned depth base, else plain loads),
  * bit 9 (0x200) when it used 64x8 tiles (small launches) instead of 64x16. */
 int jbf_kernel_variant(jbf_handle *h);
 
@@ -220,9 +240,15 @@ int jbf_mrf(jbf_handle *h, const float *depth_dev, const uint8_t *bgr_dev, size_
 
 /* "Next" row f3: DimensionConvertor::projectiveToReal(float*, float3*)
  * (DimensionConvertor.cu:3-23, DimensionConvertor.h:34-61); cx, cy truncated to
- * int as DimensionConvertor.cpp:8-9 does. */
+ * int as DimensionConvertor.cpp:8-9 does.  The batch of one of kdme_projective_to_real_batch, with its
+ * original checks (KDME_EINVAL for a NULL pointer or a non-positive size only). */
 int kdme_projective_to_real(const float *depth_dev, float *xyz_dev, int width, int height, float fx,
                             float fy, int cx, int cy, void *stream);
+/* n_frames depth planes stored back to back -> n_frames clouds [height][width][3]; v is the row within each
+ * frame, so frame k equals kdme_projective_to_real on frame k alone, bit for bit.  KDME_EINVAL: n_frames < 1, a
+ * NULL pointer, a non-positive size, a zero fx / fy, or an xyz_dev whose bytes overlap the depth input's. */
+int kdme_projective_to_real_batch(const float *depth_dev, float *xyz_dev, int width, int height, int n_frames,
+                                  float fx, float fy, int cx, int cy, void *stream);
 
 /* "Next" row f2: Projection_GPU::bilateralfilter (Projection_GPU.cu:213-246, launched :264-265) -- depth-only
  * bilateral on the z of a packed float3 cloud, then x,y = normalized.x,y * z.  Race-free: in != out.

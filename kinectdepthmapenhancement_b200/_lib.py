@@ -51,6 +51,9 @@ SIGNATURES = {
     "jbf_process_xyz": (_i, [_vp, _vp, _vp, _sz, _vp, _f, _f, _i, _i]),
     "jbf_refine_stats": (_i, [_vp, C.POINTER(C.c_ulonglong), C.POINTER(C.c_ulonglong)]),
     "jbf_process_batch": (_i, [_vp, _vp, _vp, _sz, _vp, _i]),
+    "jbf_process_batch_u16": (_i, [_vp, _vp, _vp, _sz, _vp, _i]),
+    "jbf_process_batch_xyz": (_i, [_vp, _vp, _vp, _sz, _vp, _vp, _i, _f, _f, _i, _i]),
+    "jbf_process_batch_xyz_u16": (_i, [_vp, _vp, _vp, _sz, _vp, _vp, _i, _f, _f, _i, _i]),
     "jbf_filter_guide4": (_i, [_vp, _vp, _vp, _sz, _vp, _i]),
     "jbf_presmooth": (_i, [_vp, _vp, _sz, _vp, _sz, _i]),
     "jbf_process_host": (_i, [_vp, _vp, _vp, _sz, _vp, _i]),
@@ -71,6 +74,7 @@ SIGNATURES = {
     "jbf_kernel_variant": (_i, [_vp]),
     "jbf_mrf": (_i, [_vp, _vp, _vp, _sz, _vp, _i, _f, _f]),
     "kdme_projective_to_real": (_i, [_vp, _vp, _i, _i, _f, _f, _i, _i, _vp]),
+    "kdme_projective_to_real_batch": (_i, [_vp, _vp, _i, _i, _i, _f, _f, _i, _i, _vp]),
     "kdme_depth_bilateral_xyz": (_i, [_vp, _vp, _vp, _i, _i, _i, _f, _f, _vp]),
     "kdme_mean_3d_error": (_i, [_vp, _vp, C.c_longlong, C.POINTER(C.c_double), C.POINTER(C.c_longlong), _vp]),
     "kdme_guided_upsample": (_i, [_vp, _i, _i, _vp, _vp, _sz, _vp, _i, _i, _i, _f, _f, _f, _vp]),

@@ -132,21 +132,6 @@ __global__ void __launch_bounds__(256) buf2d_update_batch_px1_kernel(float* __re
     }
 }
 
-// sensor millimetres (uint16, xn::DepthMetaData) -> float: 8 samples per thread (16-byte load, 2 x 16-byte store)
-__global__ void __launch_bounds__(256) u16_to_f32_kernel(const uint16_t* __restrict__ in, float* __restrict__ out, long long n) {
-    const long long stride = (long long)gridDim.x * blockDim.x;
-    const long long tid = (long long)blockIdx.x * blockDim.x + threadIdx.x;
-    const bool aligned = ((reinterpret_cast<uintptr_t>(in) | reinterpret_cast<uintptr_t>(out)) & 15) == 0;
-    const long long n8 = aligned ? (n >> 3) : 0;
-    for (long long k = tid; k < n8; k += stride) {
-        const uint4 v = __ldg(reinterpret_cast<const uint4*>(in) + k);
-        float4* o = reinterpret_cast<float4*>(out) + 2 * k;
-        o[0] = make_float4((float)(v.x & 0xffffu), (float)(v.x >> 16), (float)(v.y & 0xffffu), (float)(v.y >> 16));
-        o[1] = make_float4((float)(v.z & 0xffffu), (float)(v.z >> 16), (float)(v.w & 0xffffu), (float)(v.w >> 16));
-    }
-    for (long long k = (n8 << 3) + tid; k < n; k += stride) out[k] = (float)in[k];
-}
-
 // Buffer2D::insertData(xn::DepthMetaData*) -- Buffer2D.cpp:18-32 (host loop u16 -> float, H2D, updateData)
 // as ONE pass: the uint16 frame is read directly and folded into the accumulator (18 B/pixel).
 __global__ void __launch_bounds__(256) buf2d_update_u16_kernel(float* __restrict__ buf, const uint16_t* __restrict__ data,
@@ -174,15 +159,17 @@ __global__ void __launch_bounds__(256) buf2d_update_u16_kernel(float* __restrict
 }
 
 // DimensionConvertor::projectiveToReal(float*, float3*) -- DimensionConvertor.h:34-61
-// (next row f3).  IEEE division and un-fused ops, same order as the reference functor.
+// (next row f3).  IEEE division and un-fused ops, same order as the reference functor.  n_frames frames back to
+// back: v is the row within the frame.
 __global__ void __launch_bounds__(256) projective_to_real_kernel(const float* __restrict__ depth,
                                                                  float* __restrict__ xyz, int width, int height,
-                                                                 float fx, float fy, int cx, int cy) {
-    const long long n = (long long)width * height;
+                                                                 int n_frames, float fx, float fy, int cx, int cy) {
+    const long long n = (long long)width * height * n_frames;
     const long long stride = (long long)gridDim.x * blockDim.x;
     for (long long k = (long long)blockIdx.x * blockDim.x + threadIdx.x; k < n; k += stride) {
         const float z = depth[k];
-        const int v = (int)(k / width), u = (int)(k - (long long)v * width);
+        const long long row = k / width;
+        const int v = (int)(row % height), u = (int)(k - row * width);
         float py = __fsub_rn((float)cy, (float)v);
         float px = __fsub_rn((float)u, (float)cx);
         px = __fdiv_rn(px, fx);

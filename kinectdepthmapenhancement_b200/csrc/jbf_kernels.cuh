@@ -38,6 +38,8 @@
 // explicit |e| > sqrt(150) compare), two passes with the range term centred on
 // the pass-1 mean.
 #pragma once
+#include <type_traits>
+
 #include "common.cuh"
 
 namespace kdme {
@@ -46,7 +48,10 @@ enum StageMode : int { kStagePlain = 0, kStageTma = 1, kStageUpsample = 2 };
 
 struct JbfParams {
     int width, height, n_frames;
-    const float* depth;          // [n][H][W]                      (plain / TMA)
+    union {
+        const float* depth;      // [n][H][W]                      (plain / TMA)
+        const uint16_t* depth16; // the same as uint16 millimetres when depth_u16
+    };
     const uint32_t* guide4;      // [n][H][guide_pitch] u8x4 BGR0  (smoothed guide)
     float* out;                  // [n][H][W]
     long long depth_frame_stride;   // elements
@@ -100,8 +105,21 @@ struct JbfParams {
     unsigned int* q_count_prev;  // the previous launch's counter (two alternate): re-armed by this launch's filter kernel
     unsigned int* q_items;
     unsigned int q_capacity;
+    // 1: the plain / TMA depth is depth16, read by the DT = uint16_t instantiations (same layout and frame stride;
+    // whole frames only: no row bands, no peer halos).  Kept in q_capacity's padding: the layout of the block, and so
+    // the code of every kernel that takes it, stays as it was.
+    int depth_u16;
     unsigned long long* stats;   // [0] += pixels refined in fp64, [1] += pixels dropped (queue full)
 };
+
+// First sample of `frame` in the plain / TMA depth of a DT instantiation.  Its samples are read as (float)__ldg(..): a
+// uint16 sample s reads as the float (float)s, exactly, so a uint16 frame filters bit for bit like its float32 image
+// (s <= 50 is a hole).
+template <class DT>
+__device__ __forceinline__ const DT* jbf_depth_frame(const JbfParams& p, int frame) {
+    if constexpr (std::is_same<DT, uint16_t>::value) return p.depth16 + (long long)frame * p.depth_frame_stride;
+    else return p.depth + (long long)frame * p.depth_frame_stride;
+}
 
 template <int R, int TW, int TH>
 struct JbfTile {
@@ -116,6 +134,11 @@ struct JbfTile {
     static constexpr int LPP = (WS - 1 + 1) & ~1;  // pairs per LUT row, padded to an even count (16-byte rows)
     static constexpr int LBYTES = ((WS * LPP * 2 * 4 + 127) / 128) * 128;   // one paired table
     static constexpr int SMEM = 3 * PLANE + 2 * LBYTES + 128;
+    // uint16 TMA staging: halo columns rounded up to 8, so that every box starts on a 16-byte boundary of the row as
+    // the float32 boxes do (RP * 4 bytes); SP16 * SH half-words fit in one plane
+    static constexpr int RP16 = (R + 7) & ~7;
+    static constexpr int SP16 = TW + 2 * RP16;
+    static_assert((SP16 * 2) % 16 == 0 && SP16 * SH * 2 <= PLANE, "uint16 TMA box: 16-byte rows inside one plane");
 };
 
 // low-res sample index landing on high-res coordinate x, or -1 (SURVEY.md 8(d) config 3):
@@ -153,7 +176,9 @@ __device__ __forceinline__ void two_sum2(f32x2& a, const f32x2 b, f32x2& lo) {
 // a warp instruction costs the same pipe time however few lanes are active (tools/mufu_lanes.cu), so work can only
 // be cut finer than a warp by dropping instructions.  Same arithmetic per pixel (the accumulation origin is still
 // that of the 4-pixel group): results are bit-identical whichever way a pixel is computed.
-template <int R, int TW, int TH, int PSEL>
+// DT: the plain / TMA depth is float32 or uint16 millimetres (JbfParams::depth16); every step from stage B on is the
+// same for both.
+template <int R, int TW, int TH, int PSEL, class DT>
 __device__ __forceinline__ void jbf_fast_body(const CUtensorMap& tm_depth, const CUtensorMap& tm_guide, const JbfParams& p) {
     using T = JbfTile<R, TW, TH>;
     constexpr int WS = T::WS, RP = T::RP, SP = T::SP, SH = T::SH, NT = T::NT, NW = T::NW, C0 = T::C0;
@@ -204,13 +229,20 @@ __device__ __forceinline__ void jbf_fast_body(const CUtensorMap& tm_depth, const
     if (mode == kStageTma) {
         __syncthreads();
         if (tid == 0) {
-            mbar_expect_tx(bar, 2u * SP * SH * 4u);
-            tma_load_3d(sD, &tm_depth, bar, sx0, sy0, frame);
+            if constexpr (std::is_same<DT, uint16_t>::value) {
+                // the uint16 tile (SP16 columns from x0 - RP16) lands in sM, free until stage B, and is widened
+                // into sD below
+                mbar_expect_tx(bar, (uint32_t)(SP * SH * 4 + T::SP16 * SH * 2));
+                tma_load_3d(sM, &tm_depth, bar, x0 - T::RP16, sy0, frame);
+            } else {
+                mbar_expect_tx(bar, 2u * SP * SH * 4u);
+                tma_load_3d(sD, &tm_depth, bar, sx0, sy0, frame);
+            }
             tma_load_3d(sG, &tm_guide, bar, sx0, sy0, frame);
         }
     } else {
         const uint32_t* gsrc = p.guide4 + (long long)frame * p.guide_frame_stride;
-        const float* dsrc = p.depth + (long long)frame * p.depth_frame_stride;
+        const DT* dsrc = jbf_depth_frame<DT>(p, frame);
         // upsample: the low-res sample (if any) of every staged column and row, computed once per tile
         // (sM is free until stage B: its first SP + SH words hold the two maps)
         int* colmap = reinterpret_cast<int*>(sM);
@@ -236,10 +268,14 @@ __device__ __forceinline__ void jbf_fast_body(const CUtensorMap& tm_depth, const
             if (in) {
                 g = __ldg(gsrc + (long long)gy * p.guide_pitch + gx);
                 if (mode == kStagePlain) {
-                    const float* row = dsrc + (long long)gy * p.width;
-                    if (p.depth_up != nullptr && gy < p.band0) row = p.depth_up + (long long)gy * p.width;
-                    else if (p.depth_dn != nullptr && gy >= p.band1) row = p.depth_dn + (long long)(gy - p.band1) * p.width;
-                    d = __ldg(row + gx);
+                    if constexpr (std::is_same<DT, uint16_t>::value) {
+                        d = (float)__ldg(dsrc + (long long)gy * p.width + gx);
+                    } else {
+                        const float* row = dsrc + (long long)gy * p.width;
+                        if (p.depth_up != nullptr && gy < p.band0) row = p.depth_up + (long long)gy * p.width;
+                        else if (p.depth_dn != nullptr && gy >= p.band1) row = p.depth_dn + (long long)(gy - p.band1) * p.width;
+                        d = __ldg(row + gx);
+                    }
                 } else {  // scatter the low-res sample onto its high-res site
                     const int xl = colmap[sx], yl = rowmap[sy];
                     if ((xl >= 0) & (yl >= 0)) d = upsample_sample(p, frame, xl, yl);
@@ -251,6 +287,17 @@ __device__ __forceinline__ void jbf_fast_body(const CUtensorMap& tm_depth, const
     }
     if (mode == kStageTma) mbar_wait(bar, 0);
     __syncthreads();
+    if constexpr (std::is_same<DT, uint16_t>::value) {
+        // a pass of its own: stage B writes sM[idx] in the loop that would read the uint16 tile from it
+        if (mode == kStageTma) {
+            const uint16_t* s16 = reinterpret_cast<const uint16_t*>(sM) + (T::RP16 - RP);
+            for (int idx = tid; idx < SP * she; idx += NT) {
+                const int sy = idx / SP, sx = idx - sy * SP;
+                sD[idx] = (float)s16[sy * T::SP16 + sx];
+            }
+            __syncthreads();
+        }
+    }
 
     // ---------------- stage B: validity word per staged sample; holes (and NaN) read as depth 0.  The range of the
     // valid staged depths decides (CTA-uniformly) whether pass 2 needs the skip-if-zero compare at all.
@@ -630,18 +677,18 @@ __device__ __forceinline__ void jbf_fast_body(const CUtensorMap& tm_depth, const
     }
 }
 
-template <int R, int TW, int TH, int MINB>
+template <int R, int TW, int TH, int MINB, class DT>
 __global__ void __launch_bounds__((TW / 4) * TH, MINB)
 jbf_fast_kernel(const __grid_constant__ CUtensorMap tm_depth, const __grid_constant__ CUtensorMap tm_guide,
                 const JbfParams p) {
     // CTA-uniform dispatch: whole tiles and whole small tiles run the full body, half units one pair each.  The 64x16
     // instantiations (large launches) carry the full body only: the hot kernel's code is exactly the single-body one.
     if constexpr (TH >= 16) {
-        jbf_fast_body<R, TW, TH, 0>(tm_depth, tm_guide, p);
+        jbf_fast_body<R, TW, TH, 0, DT>(tm_depth, tm_guide, p);
     } else {
-        if (!p.half_units || (int)blockIdx.y < p.nbig_rows) jbf_fast_body<R, TW, TH, 0>(tm_depth, tm_guide, p);
-        else if ((((int)blockIdx.y - p.nbig_rows) & 1) == 0) jbf_fast_body<R, TW, TH, 1>(tm_depth, tm_guide, p);
-        else jbf_fast_body<R, TW, TH, 2>(tm_depth, tm_guide, p);
+        if (!p.half_units || (int)blockIdx.y < p.nbig_rows) jbf_fast_body<R, TW, TH, 0, DT>(tm_depth, tm_guide, p);
+        else if ((((int)blockIdx.y - p.nbig_rows) & 1) == 0) jbf_fast_body<R, TW, TH, 1, DT>(tm_depth, tm_guide, p);
+        else jbf_fast_body<R, TW, TH, 2, DT>(tm_depth, tm_guide, p);
     }
 }
 
@@ -1027,8 +1074,9 @@ __device__ __forceinline__ double exp_neg_f64(double x) {
 }
 
 // KMAX = taps per lane the instantiation can hold: (2r+1)^2 <= 32 * KMAX
-// PLAIN = whole-frame / local-band depth plane (no upsampling lattice, no peer-memory halos): direct loads
-template <int KMAX, bool PLAIN>
+// PLAIN = whole-frame / local-band depth plane (no upsampling lattice, no peer-memory halos): direct loads, of
+// float32 or (DT = uint16_t, PLAIN only) uint16 depth
+template <int KMAX, bool PLAIN, class DT>
 __global__ void __launch_bounds__(128) jbf_refine_kernel(const JbfParams p, const int radius) {
     const int lane = threadIdx.x & 31;
     const int ws = 2 * radius + 1, ntap = ws * ws;
@@ -1068,7 +1116,7 @@ __global__ void __launch_bounds__(128) jbf_refine_kernel(const JbfParams p, cons
         const int oy = (int)(rem / (unsigned)p.width), x = (int)(rem - (unsigned)oy * (unsigned)p.width);
         const int y = oy + p.y_off;
         const uint32_t* gsrc = p.guide4 + (long long)frame * p.guide_frame_stride;
-        const float* dsrc = p.depth + (long long)frame * p.depth_frame_stride;
+        const DT* dsrc = jbf_depth_frame<DT>(p, frame);
         // all of the lane's loads are issued before the first use (the taps are independent: one round trip
         // to L2 per pixel instead of two per tap); out-of-window taps read the centre and are masked
         float dfl[KMAX];
@@ -1079,7 +1127,7 @@ __global__ void __launch_bounds__(128) jbf_refine_kernel(const JbfParams p, cons
             const int ty = y + tdy[u], tx = x + tdx[u];
             const bool in = tx >= 0 && tx < p.width && ty >= 0 && ty < p.height;
             const int cy_ = in ? ty : y, cx_ = in ? tx : x;
-            const float df = PLAIN ? __ldg(dsrc + (long long)cy_ * p.width + cx_) : jbf_sample_depth(p, frame, cx_, cy_);
+            const float df = PLAIN ? (float)__ldg(dsrc + (long long)cy_ * p.width + cx_) : jbf_sample_depth(p, frame, cx_, cy_);
             gql[u] = __ldg(gsrc + (long long)cy_ * p.guide_pitch + cx_);
             dfl[u] = in ? df : 0.f;
         }
@@ -1146,7 +1194,7 @@ struct JbfGenericParams {
     int use_depth;    // 0 when sigma_d == 0 (depth_filter uninitialised in the reference -> skipped)
 };
 
-template <int TW, int TH>
+template <int TW, int TH, class DT>
 __global__ void __launch_bounds__(TW * TH)
 jbf_generic_kernel(const JbfGenericParams gp_) {
     const JbfParams& p = gp_.base;
@@ -1161,7 +1209,7 @@ jbf_generic_kernel(const JbfGenericParams gp_) {
     const int tid = threadIdx.x;
     const int x0 = blockIdx.x * TW, y0 = p.y_off + blockIdx.y * TH, frame = blockIdx.z;
     const uint32_t* gsrc = p.guide4 + (long long)frame * p.guide_frame_stride;
-    const float* dsrc = p.depth + (long long)frame * p.depth_frame_stride;
+    const DT* dsrc = jbf_depth_frame<DT>(p, frame);
     for (int idx = tid; idx < SP * SH; idx += NT) {
         int sy = idx / SP, sx = idx - sy * SP;
         int gx = x0 - R + sx, gy = y0 - R + sy;
@@ -1175,7 +1223,7 @@ jbf_generic_kernel(const JbfGenericParams gp_) {
                 int yl = upsample_site(gy, p.height, p.hl);
                 if ((xl >= 0) & (yl >= 0)) d = upsample_sample(p, frame, xl, yl);
             } else {
-                d = __ldg(dsrc + (long long)gy * p.width + gx);
+                d = (float)__ldg(dsrc + (long long)gy * p.width + gx);
             }
         }
         sD[idx] = d;

@@ -42,6 +42,14 @@ static int fail(int code, const std::string& msg) {
 extern "C" const char* kdme_last_error(void) { return g_err.c_str(); }
 extern "C" const char* kdme_version(void) { return "kdme_b200 0.1.0 sm_100a"; }
 
+// The kernels read every frame's input while they write the output: true where the input's `in_bytes` and the
+// `out_floats` output floats share a byte.
+static bool ranges_overlap(const void* in, unsigned long long in_bytes, const float* out, unsigned long long out_floats) {
+    const uintptr_t i0 = (uintptr_t)in, i1 = i0 + in_bytes;
+    const uintptr_t o0 = (uintptr_t)out, o1 = o0 + out_floats * sizeof(float);
+    return i0 < o1 && o0 < i1;
+}
+
 struct DeviceGuard {
     int prev = -1;
     bool ok = true;
@@ -93,7 +101,7 @@ static int check_pointer_device(const void* ptr, const char* who) {
     return KDME_OK;
 }
 
-// 3-D map over [n][rows][pitch_elems] 4-byte elements, box {bx, by, 1}, zero OOB fill.
+// 3-D map over [n][rows][pitch_elems] elements of type dt, box {bx, by, 1}, zero OOB fill.
 static bool encode_map(CUtensorMap* map, CUtensorMapDataType dt, const void* base, int width, int height, int n,
                        long long row_pitch_bytes, long long frame_pitch_bytes, int bx, int by) {
     EncodeTiledFn fn = get_encode_fn();
@@ -144,7 +152,8 @@ struct jbf_handle {
     // allocated on first use: odd chunks run there with their own guide buffer, refinement queue and TMA
     // descriptors, so that a chunk's pre-smooth fills the tail of the previous chunk's filter and the fp64
     // refinement launch hides behind the next filter.
-    struct MapKey { const void* depth = nullptr; const void* guide = nullptr; int rows = 0, n = 0, gp = 0, bx = 0, by = 0; };
+    // dt: the depth map's element type -- a float map must not be reused for a uint16 buffer at the same address
+    struct MapKey { const void* depth = nullptr; const void* guide = nullptr; int rows = 0, n = 0, gp = 0, bx = 0, by = 0, dt = 0; };
     struct Lane {
         cudaStream_t stream = nullptr;
         uint32_t* guide4 = nullptr;            // smooth_Device in the internal u8x4 layout, max_batch frames
@@ -175,7 +184,6 @@ struct jbf_handle {
 using Lane = jbf_handle::Lane;
 
 static bool fast_radius_available(int r);
-static int buf_blocks(long long n);
 
 static int ensure_alt_lane(jbf_handle* h) {
     Lane& a = h->lanes[1];
@@ -556,8 +564,8 @@ static int launch_presmooth(jbf_handle* h, Lane& lane, const uint8_t* bgr, size_
     return KDME_OK;
 }
 
-// One (radius, tile height) instantiation: encode (or reuse) the TMA maps for its box and launch.
-template <int R, int TH>
+// One (radius, tile height, depth type) instantiation: encode (or reuse) the TMA maps for its box and launch.
+template <int R, int TH, class DT>
 static int launch_fast_rt(jbf_handle* h, Lane& lane, JbfParams p, bool want_tma, bool pdl) {
     constexpr int TW = 64;
     const int rows = p.height;
@@ -569,18 +577,22 @@ static int launch_fast_rt(jbf_handle* h, Lane& lane, JbfParams p, bool want_tma,
     constexpr int kBySmem = (227 * 1024) / (T::SMEM + 1024);
     constexpr int MINB = (kByRegs < kBySmem ? kByRegs : kBySmem) < 1 ? 1 : (kByRegs < kBySmem ? kByRegs : kBySmem);
     constexpr int kSmemCap = 226 * 1024;
-    { int rc = allow_dyn_smem<jbf_fast_kernel<R, TW, TH, MINB>>(h->device, kSmemCap); if (rc != KDME_OK) return rc; }
+    { int rc = allow_dyn_smem<jbf_fast_kernel<R, TW, TH, MINB, DT>>(h->device, kSmemCap); if (rc != KDME_OK) return rc; }
     if (want_tma) {
+        constexpr bool u16 = std::is_same<DT, uint16_t>::value;
+        constexpr CUtensorMapDataType dt = u16 ? CU_TENSOR_MAP_DATA_TYPE_UINT16 : CU_TENSOR_MAP_DATA_TYPE_FLOAT32;
+        constexpr int bx = u16 ? T::SP16 : T::SP;   // depth box columns (see JbfTile::RP16)
+        const void* depth = p.depth;                 // depth16 shares the slot
         jbf_handle::MapKey& k = lane.map_key;
-        if (k.depth != p.depth || k.guide != p.guide4 || k.rows != rows || k.n != p.n_frames || k.gp != p.guide_pitch ||
-            k.bx != T::SP || k.by != T::SH) {
-            bool ok = encode_map(&lane.map_depth, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, p.depth, p.width, rows, p.n_frames,
-                                 (long long)p.width * 4, (long long)p.width * rows * 4, T::SP, T::SH) &&
+        if (k.depth != depth || k.guide != p.guide4 || k.rows != rows || k.n != p.n_frames || k.gp != p.guide_pitch ||
+            k.bx != bx || k.by != T::SH || k.dt != (int)dt) {
+            bool ok = encode_map(&lane.map_depth, dt, depth, p.width, rows, p.n_frames, (long long)p.width * sizeof(DT),
+                                 (long long)p.width * rows * sizeof(DT), bx, T::SH) &&
                       encode_map(&lane.map_guide, CU_TENSOR_MAP_DATA_TYPE_UINT32, p.guide4, p.width, rows, p.n_frames,
                                  (long long)p.guide_pitch * 4, (long long)p.guide_pitch * rows * 4, T::SP, T::SH);
             if (ok) {
-                k.depth = p.depth; k.guide = p.guide4; k.rows = rows; k.n = p.n_frames; k.gp = p.guide_pitch;
-                k.bx = T::SP; k.by = T::SH;
+                k.depth = depth; k.guide = p.guide4; k.rows = rows; k.n = p.n_frames; k.gp = p.guide_pitch;
+                k.bx = bx; k.by = T::SH; k.dt = (int)dt;
             } else {
                 k = jbf_handle::MapKey();
                 want_tma = false;
@@ -625,7 +637,7 @@ static int launch_fast_rt(jbf_handle* h, Lane& lane, JbfParams p, bool want_tma,
             if (padded > smem_bytes) smem_bytes = padded > (size_t)kSmemCap ? (size_t)kSmemCap : padded;
         }
     }
-    return launch_ex(jbf_fast_kernel<R, TW, TH, MINB>, dim3(tx, tile_rows, p.n_frames), dim3(T::NT), smem_bytes,
+    return launch_ex(jbf_fast_kernel<R, TW, TH, MINB, DT>, dim3(tx, tile_rows, p.n_frames), dim3(T::NT), smem_bytes,
                      lane.stream, pdl, lane.map_depth, lane.map_guide, p);
 }
 
@@ -703,7 +715,8 @@ static JbfParams filter_request(const jbf_handle* h, const float* depth, const u
 }
 
 // The generic kernel: runtime radius, one pixel per thread (exotic sigmas, radius 0).
-static int launch_generic(jbf_handle* h, Lane& lane, const JbfParams& p) {
+template <class DT>
+static int launch_generic_dt(jbf_handle* h, Lane& lane, const JbfParams& p) {
     JbfGenericParams gp;
     gp.base = p;
     gp.base.ltab = h->ltab_generic_dev;
@@ -711,17 +724,29 @@ static int launch_generic(jbf_handle* h, Lane& lane, const JbfParams& p) {
     constexpr int TW = 32, TH = 8;
     const int SP = TW + 2 * h->radius, SH = TH + 2 * h->radius, ws = 2 * h->radius + 1;
     size_t smem = (size_t)SP * SH * 8 + (size_t)ws * ws * 4;
-    { int rc = allow_dyn_smem<jbf_generic_kernel<TW, TH>>(h->device, 64 * 1024); if (rc != KDME_OK) return rc; }
+    { int rc = allow_dyn_smem<jbf_generic_kernel<TW, TH, DT>>(h->device, 64 * 1024); if (rc != KDME_OK) return rc; }
     dim3 grd((p.width + TW - 1) / TW, (p.out_rows + TH - 1) / TH, p.n_frames);
-    jbf_generic_kernel<TW, TH><<<grd, TW * TH, smem, lane.stream>>>(gp);
+    jbf_generic_kernel<TW, TH, DT><<<grd, TW * TH, smem, lane.stream>>>(gp);
     CK(cudaGetLastError());
     h->last_variant = 1;
     return KDME_OK;
 }
 
-// The fast kernel of the handle's radius, staged by TMA where the buffers allow it.
+static int launch_generic(jbf_handle* h, Lane& lane, const JbfParams& p) {
+    return p.depth_u16 ? launch_generic_dt<uint16_t>(h, lane, p) : launch_generic_dt<float>(h, lane, p);
+}
+
+template <int R, class DT>
+static int launch_fast_th(jbf_handle* h, Lane& lane, const JbfParams& p, int th, bool want_tma, bool pdl) {
+    return th == 16 ? launch_fast_rt<R, 16, DT>(h, lane, p, want_tma, pdl)
+         : th == 8 ? launch_fast_rt<R, 8, DT>(h, lane, p, want_tma, pdl)
+                   : launch_fast_rt<R, 4, DT>(h, lane, p, want_tma, pdl);
+}
+
+// The fast kernel of the handle's radius, staged by TMA where the buffers allow it: rows of 16-byte multiples and
+// 16-byte aligned frames (width % 4 for float32 depth, width % 8 for uint16).
 static int launch_fast(jbf_handle* h, Lane& lane, const JbfParams& p, bool pdl) {
-    const bool want_tma = p.mode == kStagePlain && !h->force_no_tma && (h->width % 4 == 0) &&
+    const bool want_tma = p.mode == kStagePlain && !h->force_no_tma && (h->width % (p.depth_u16 ? 8 : 4) == 0) &&
                           (p.guide_pitch % 4 == 0) && ((reinterpret_cast<uintptr_t>(p.depth) & 15) == 0) &&
                           ((reinterpret_cast<uintptr_t>(p.guide4) & 15) == 0);
     // Tile height: the arithmetic of a pixel does not depend on the tile it falls in, so the choice is
@@ -741,9 +766,8 @@ static int launch_fast(jbf_handle* h, Lane& lane, const JbfParams& p, bool pdl) 
     }
     if (h->force_tile_h == 16 || h->force_tile_h == 8 || h->force_tile_h == 4) best_th = h->force_tile_h;
     switch (h->radius) {
-#define X(R) case R: return best_th == 16 ? launch_fast_rt<R, 16>(h, lane, p, want_tma, pdl)                  \
-                          : best_th == 8 ? launch_fast_rt<R, 8>(h, lane, p, want_tma, pdl)                    \
-                                         : launch_fast_rt<R, 4>(h, lane, p, want_tma, pdl);
+#define X(R) case R: return p.depth_u16 ? launch_fast_th<R, uint16_t>(h, lane, p, best_th, want_tma, pdl)          \
+                                      : launch_fast_th<R, float>(h, lane, p, best_th, want_tma, pdl);
         KDME_FAST_RADII(X)
 #undef X
         default: return fail(KDME_ENOTSUP, "no fast kernel for this radius");
@@ -783,12 +807,18 @@ static int launch_gather(jbf_handle* h, Lane& lane, JbfParams& p, UpsampleGeom g
 
 // fp64 re-evaluation of the queued pixels; launched with programmatic stream serialisation so its launch latency
 // hides behind the filter (it waits for the filter's completion on the device).
+// uint16 depth is always plain (whole frames).
 static int launch_refine(const jbf_handle* h, Lane& lane, const JbfParams& p) {
     const bool plain = p.mode != kStageUpsample && !p.depth_up && !p.depth_dn;
     auto launch = [&](auto kern) { return launch_ex(kern, dim3(148 * 5), dim3(128), 0, lane.stream, true, p, h->radius); };
-    if (h->radius <= 7) return plain ? launch(jbf_refine_kernel<8, true>) : launch(jbf_refine_kernel<8, false>);
-    if (h->radius <= 10) return plain ? launch(jbf_refine_kernel<16, true>) : launch(jbf_refine_kernel<16, false>);
-    return plain ? launch(jbf_refine_kernel<31, true>) : launch(jbf_refine_kernel<31, false>);
+    if (h->radius <= 7)
+        return p.depth_u16 ? launch(jbf_refine_kernel<8, true, uint16_t>)
+             : plain ? launch(jbf_refine_kernel<8, true, float>) : launch(jbf_refine_kernel<8, false, float>);
+    if (h->radius <= 10)
+        return p.depth_u16 ? launch(jbf_refine_kernel<16, true, uint16_t>)
+             : plain ? launch(jbf_refine_kernel<16, true, float>) : launch(jbf_refine_kernel<16, false, float>);
+    return p.depth_u16 ? launch(jbf_refine_kernel<31, true, uint16_t>)
+         : plain ? launch(jbf_refine_kernel<31, true, float>) : launch(jbf_refine_kernel<31, false, float>);
 }
 
 // Launches request p on `lane`: its stream, refinement queue and TMA descriptors.
@@ -931,20 +961,76 @@ static int run_chunks(jbf_handle* h, int n_frames, int chunk, Fn&& fn) {
     return KDME_OK;
 }
 
-extern "C" int jbf_process_batch(jbf_handle* h, const float* depth_dev, const uint8_t* bgr_dev, size_t bgr_step,
-                                 float* out_dev, int n_frames) {
-    if (!h || !depth_dev || !bgr_dev || !out_dev) return fail(KDME_EINVAL, "jbf_process_batch: NULL argument");
-    if (n_frames < 1) return fail(KDME_EINVAL, "jbf_process_batch: n_frames must be >= 1");
-    { int rc = guide_step(h, &bgr_step, "jbf_process_batch"); if (rc != KDME_OK) return rc; }
-    DeviceGuard g(h->device);
+// DimensionConvertor::projectiveToReal over n_frames planes back to back, on `stream`.
+static int launch_projective(const float* depth, float* xyz, int width, int height, int n_frames, float fx, float fy,
+                             int cx, int cy, cudaStream_t stream) {
+    const long long n = (long long)width * height * n_frames;
+    const int blocks = (int)std::min<long long>((n + 255) / 256, 148 * 16);
+    projective_to_real_kernel<<<blocks, 256, 0, stream>>>(depth, xyz, width, height, n_frames, fx, fy, cx, cy);
+    CK(cudaGetLastError());
+    return KDME_OK;
+}
+
+// Every jbf_process_batch* entry point: n_frames frames of float32 (depth) or uint16 (depth16) depth filtered into out
+// and, for the xyz forms (want_xyz), back-projected into xyz.  jbf_process_batch (float32, no cloud) keeps the checks
+// it always had; the newer forms also reject zero focal lengths and outputs that overlap the input or each other.
+static int process_batch(jbf_handle* h, const float* depth, const uint16_t* depth16, const uint8_t* bgr, size_t bgr_step,
+                         float* out, bool want_xyz, float* xyz, int n_frames, float fx, float fy, int cx, int cy,
+                         const char* who) {
+    const void* in = depth ? (const void*)depth : (const void*)depth16;
+    if (!h || !in || !bgr || !out || (want_xyz && !xyz)) return fail(KDME_EINVAL, std::string(who) + ": NULL argument");
+    if (n_frames < 1) return fail(KDME_EINVAL, std::string(who) + ": n_frames must be >= 1");
+    if (want_xyz && (!(fx != 0.f) || !(fy != 0.f)))
+        return fail(KDME_EINVAL, std::string(who) + ": focal lengths must be non-zero");
     const size_t plane = (size_t)h->width * h->height;
+    if (depth16 || want_xyz) {
+        const unsigned long long px = (unsigned long long)plane * n_frames, in_bytes = px * (depth16 ? 2 : 4);
+        if (ranges_overlap(in, in_bytes, out, px) ||
+            (want_xyz && (ranges_overlap(in, in_bytes, xyz, 3 * px) || ranges_overlap(out, 4 * px, xyz, 3 * px))))
+            return fail(KDME_EINVAL, std::string(who) + ": an output overlaps the depth input or the other output "
+                                                        "(in-place operation is not supported)");
+    }
+    { int rc = guide_step(h, &bgr_step, who); if (rc != KDME_OK) return rc; }
+    DeviceGuard g(h->device);
     return run_chunks(h, n_frames, h->max_batch, [&](Lane& lane, int, int f0, int n) {
-        int rc = launch_presmooth(h, lane, bgr_dev + (size_t)f0 * bgr_step * h->height, bgr_step, lane.guide4,
+        int rc = launch_presmooth(h, lane, bgr + (size_t)f0 * bgr_step * h->height, bgr_step, lane.guide4,
                                   h->guide_pitch, n);
         if (rc != KDME_OK) return rc;
-        return launch_filter(h, lane, filter_request(h, depth_dev + (size_t)f0 * plane, lane.guide4, h->guide_pitch,
-                                                     out_dev + (size_t)f0 * plane, n), /*pdl=*/true);
+        float* o = out + (size_t)f0 * plane;
+        JbfParams p = filter_request(h, depth ? depth + (size_t)f0 * plane : nullptr, lane.guide4, h->guide_pitch, o, n);
+        if (depth16) { p.depth16 = depth16 + (size_t)f0 * plane; p.depth_u16 = 1; }
+        float* x = want_xyz ? xyz + 3 * (size_t)f0 * plane : nullptr;
+        if (x && h->fast) { p.xyz = x; p.fx = fx; p.fy = fy; p.cx = cx; p.cy = cy; }   // the fused epilogue
+        rc = launch_filter(h, lane, p, /*pdl=*/true);
+        if (rc != KDME_OK || !x || h->fast) return rc;
+        // off the fast kernel: the two calls the reference makes, back to back on the chunk's lane
+        return launch_projective(o, x, h->width, h->height, n, fx, fy, cx, cy, lane.stream);
     });
+}
+
+extern "C" int jbf_process_batch(jbf_handle* h, const float* depth_dev, const uint8_t* bgr_dev, size_t bgr_step,
+                                 float* out_dev, int n_frames) {
+    return process_batch(h, depth_dev, nullptr, bgr_dev, bgr_step, out_dev, false, nullptr, n_frames, 0.f, 0.f, 0, 0,
+                         "jbf_process_batch");
+}
+
+extern "C" int jbf_process_batch_u16(jbf_handle* h, const uint16_t* depth_dev, const uint8_t* bgr_dev, size_t bgr_step,
+                                     float* out_dev, int n_frames) {
+    return process_batch(h, nullptr, depth_dev, bgr_dev, bgr_step, out_dev, false, nullptr, n_frames, 0.f, 0.f, 0, 0,
+                         "jbf_process_batch_u16");
+}
+
+extern "C" int jbf_process_batch_xyz(jbf_handle* h, const float* depth_dev, const uint8_t* bgr_dev, size_t bgr_step,
+                                     float* out_dev, float* xyz_dev, int n_frames, float fx, float fy, int cx, int cy) {
+    return process_batch(h, depth_dev, nullptr, bgr_dev, bgr_step, out_dev, true, xyz_dev, n_frames, fx, fy, cx, cy,
+                         "jbf_process_batch_xyz");
+}
+
+extern "C" int jbf_process_batch_xyz_u16(jbf_handle* h, const uint16_t* depth_dev, const uint8_t* bgr_dev,
+                                         size_t bgr_step, float* out_dev, float* xyz_dev, int n_frames, float fx,
+                                         float fy, int cx, int cy) {
+    return process_batch(h, nullptr, depth_dev, bgr_dev, bgr_step, out_dev, true, xyz_dev, n_frames, fx, fy, cx, cy,
+                         "jbf_process_batch_xyz_u16");
 }
 
 extern "C" int jbf_process(jbf_handle* h, const float* depth_dev, const uint8_t* bgr_dev, size_t bgr_step) {
@@ -1087,15 +1173,12 @@ static int process_host_impl(jbf_handle* h, const float* depth_host, const uint1
         CK(cudaEventRecord(h->ev_in[b], h->s_h2d));
         CK(cudaStreamWaitEvent(lane.stream, h->ev_in[b], 0));
         if (c >= kPipeDepth) CK(cudaStreamWaitEvent(lane.stream, h->ev_free[b], 0));  // slot output drained
-        if (depth16_host) {   // sensor millimetres -> float, as Buffer2D::insertData(xn::DepthMetaData*) does (Buffer2D.cpp:18-32)
-            const long long cnt = (long long)plane * n;
-            u16_to_f32_kernel<<<buf_blocks(cnt), 256, 0, lane.stream>>>(h->pipe_depth16[b], h->pipe_depth[b], cnt);
-            CK(cudaGetLastError());
-        }
         int rc = launch_presmooth(h, lane, h->pipe_bgr[b], bgr_step, lane.guide4, h->guide_pitch, n);
         if (rc != KDME_OK) return rc;
-        rc = launch_filter(h, lane, filter_request(h, h->pipe_depth[b], lane.guide4, h->guide_pitch, h->pipe_out[b], n),
-                           /*pdl=*/true);
+        // the filter reads the sensor's uint16 millimetres straight from the slot
+        JbfParams p = filter_request(h, h->pipe_depth[b], lane.guide4, h->guide_pitch, h->pipe_out[b], n);
+        if (depth16_host) { p.depth16 = h->pipe_depth16[b]; p.depth_u16 = 1; }
+        rc = launch_filter(h, lane, p, /*pdl=*/true);
         if (rc != KDME_OK) return rc;
         CK(cudaEventRecord(h->ev_done[b], lane.stream));
         CK(cudaStreamWaitEvent(h->s_d2h, h->ev_done[b], 0));
@@ -1212,16 +1295,26 @@ extern "C" int jbf_mrf(jbf_handle* h, const float* depth_dev, const uint8_t* bgr
     return KDME_OK;
 }
 
+extern "C" int kdme_projective_to_real_batch(const float* depth_dev, float* xyz_dev, int width, int height,
+                                             int n_frames, float fx, float fy, int cx, int cy, void* stream) {
+    const char* who = "kdme_projective_to_real_batch";
+    if (!depth_dev || !xyz_dev) return fail(KDME_EINVAL, std::string(who) + ": NULL argument");
+    if (width <= 0 || height <= 0) return fail(KDME_EINVAL, std::string(who) + ": bad size");
+    if (n_frames < 1) return fail(KDME_EINVAL, std::string(who) + ": n_frames must be >= 1");
+    if (!(fx != 0.f) || !(fy != 0.f)) return fail(KDME_EINVAL, std::string(who) + ": focal lengths must be non-zero");
+    const unsigned long long px = (unsigned long long)width * height * n_frames;
+    if (ranges_overlap(depth_dev, 4 * px, xyz_dev, 3 * px))
+        return fail(KDME_EINVAL, std::string(who) + ": the output overlaps the depth input (in-place operation is not supported)");
+    { int rcd = check_pointer_device(depth_dev, who); if (rcd != KDME_OK) return rcd; }
+    return launch_projective(depth_dev, xyz_dev, width, height, n_frames, fx, fy, cx, cy, (cudaStream_t)stream);
+}
+
+// The batch of one, with the argument checks it always had.
 extern "C" int kdme_projective_to_real(const float* depth_dev, float* xyz_dev, int width, int height, float fx,
                                        float fy, int cx, int cy, void* stream) {
     if (!depth_dev || !xyz_dev || width <= 0 || height <= 0) return fail(KDME_EINVAL, "projective_to_real: bad argument");
     { int rcd = check_pointer_device(depth_dev, "kdme_projective_to_real"); if (rcd != KDME_OK) return rcd; }
-    const long long n = (long long)width * height;
-    int blocks = (int)((n + 255) / 256);
-    if (blocks > 148 * 16) blocks = 148 * 16;
-    projective_to_real_kernel<<<blocks, 256, 0, (cudaStream_t)stream>>>(depth_dev, xyz_dev, width, height, fx, fy, cx, cy);
-    CK(cudaGetLastError());
-    return KDME_OK;
+    return launch_projective(depth_dev, xyz_dev, width, height, 1, fx, fy, cx, cy, (cudaStream_t)stream);
 }
 
 // ------------------------------------------------------------------ next rows f2, f4
@@ -1377,14 +1470,6 @@ static int guided_launch_c(const GuidedCall& c, cudaStream_t stream) {
     }
 }
 
-// The kernels read every frame's depth while they write the output: true where the depth input's `in_bytes` and the
-// `out_floats` output floats share a byte.
-static bool guided_overlap(const void* in, unsigned long long in_bytes, const float* out, unsigned long long out_floats) {
-    const uintptr_t i0 = (uintptr_t)in, i1 = i0 + in_bytes;
-    const uintptr_t o0 = (uintptr_t)out, o1 = o0 + out_floats * sizeof(float);
-    return i0 < o1 && o0 < i1;
-}
-
 // Every guided entry point: the checks in order, then the launch.  The call is a fill when its depth is depth or
 // depth16, an upsampling when it is depth_lo or depth_lo16; the other three are NULL.
 static int guided_batch(GuidedCall c, int channels, void* stream, const char* who) {
@@ -1398,7 +1483,7 @@ static int guided_batch(GuidedCall c, int channels, void* stream, const char* wh
     const unsigned long long plane = (unsigned long long)c.width * c.height;
     const unsigned long long in_samples = lo ? (unsigned long long)c.wl * c.hl : plane;
     const size_t sample_bytes = (c.depth16 || c.depth_lo16) ? sizeof(uint16_t) : sizeof(float);
-    if (guided_overlap(in, in_samples * c.n_frames * sample_bytes, c.out, plane * c.n_frames))
+    if (ranges_overlap(in, in_samples * c.n_frames * sample_bytes, c.out, plane * c.n_frames))
         return fail(KDME_EINVAL, std::string(who) + ": the output overlaps the depth input (in-place operation is not supported)");
     if (c.radius < 0 || c.radius > KDME_MAX_RADIUS) return fail(KDME_EINVAL, std::string(who) + ": bad radius");
     if (channels != KDME_GUIDE_GRAY && channels != KDME_GUIDE_BGR && channels != KDME_GUIDE_BGRX)

@@ -208,20 +208,48 @@ class JointBilateralFilter:
         return out
 
     # -- batched / staged forms (B200-native additions) ----------------------
-    def process_batch(self, depth: torch.Tensor, color: torch.Tensor, out: torch.Tensor | None = None):
-        """N independent frames: depth [N,H,W] f32, color [N,H,W,3] u8 (or [N,H,W] / [N,H,W,1] GRAY,
-        [N,H,W,4] BGRX) -> out [N,H,W] f32."""
-        _check_cuda(depth, torch.float32, "depth", self.device)
+    def _batch_args(self, depth: torch.Tensor, color: torch.Tensor, out: torch.Tensor | None):
+        """Checks of the process_batch forms: (N, guide step, u16?, out)."""
+        if not isinstance(depth, torch.Tensor) or depth.dtype not in (torch.float32, torch.uint16, torch.int16):
+            raise TypeError("depth must be a float32 or uint16 tensor")
+        _check_cuda(depth, depth.dtype, "depth", self.device)
         _check_cuda(color, torch.uint8, "color", self.device)
-        n = depth.shape[0]
-        if tuple(depth.shape[1:]) != (self.height, self.width):
+        if depth.dim() != 3 or tuple(depth.shape[1:]) != (self.height, self.width):
             raise ValueError("depth must be [N,H,W] at the filter's size")
+        n = depth.shape[0]
         step = self._use_guide(color, (n, self.height, self.width), "color")
         if out is None:
-            out = torch.empty_like(depth)
+            out = torch.empty(tuple(depth.shape), dtype=torch.float32, device=self.device)
         _check_cuda(out, torch.float32, "out", self.device)
-        _lib.check(_lib.lib().jbf_process_batch(self._h, _ptr(depth), _ptr(color), step, _ptr(out), n))
+        if tuple(out.shape) != tuple(depth.shape):
+            raise ValueError(f"out must be [{n}, {self.height}, {self.width}]")
+        return n, step, depth.dtype != torch.float32, out
+
+    def process_batch(self, depth: torch.Tensor, color: torch.Tensor, out: torch.Tensor | None = None):
+        """N independent frames: depth [N,H,W] float32 millimetres or uint16 millimetres (the sensor's format, read
+        directly; torch.uint16 or a torch.int16 view of the same bits), color [N,H,W,3] u8 (or [N,H,W] / [N,H,W,1]
+        GRAY, [N,H,W,4] BGRX) -> out [N,H,W] f32.  A uint16 frame filters bit for bit like its float32 image."""
+        n, step, u16, out = self._batch_args(depth, color, out)
+        fn = _lib.lib().jbf_process_batch_u16 if u16 else _lib.lib().jbf_process_batch
+        _lib.check(fn(self._h, _ptr(depth), _ptr(color), step, _ptr(out), n))
         return out
+
+    def process_batch_xyz(self, depth: torch.Tensor, color: torch.Tensor, fx: float, fy: float, cx: int, cy: int,
+                          out: torch.Tensor | None = None, xyz: torch.Tensor | None = None):
+        """process_batch + DimensionConvertor::projectiveToReal of every frame (main.cpp:179 + :182 over a stream):
+        depth [N,H,W] float32 or uint16 millimetres -> (out [N,H,W] f32, xyz [N,H,W,3] f32).  Frame k of both equals
+        process_xyz on frame k alone (the depth plane and the cloud), bit for bit."""
+        n, step, u16, out = self._batch_args(depth, color, out)
+        if xyz is None:
+            xyz = torch.empty((n, self.height, self.width, 3), dtype=torch.float32, device=self.device)
+        _check_cuda(xyz, torch.float32, "xyz", self.device)
+        if tuple(xyz.shape) != (n, self.height, self.width, 3):
+            raise ValueError(f"xyz must be [{n}, {self.height}, {self.width}, 3]")
+        self._keep = (depth, color)
+        fn = _lib.lib().jbf_process_batch_xyz_u16 if u16 else _lib.lib().jbf_process_batch_xyz
+        _lib.check(fn(self._h, _ptr(depth), _ptr(color), step, _ptr(out), _ptr(xyz), n, float(fx), float(fy), int(cx),
+                      int(cy)))
+        return out, xyz
 
     def presmooth(self, color: torch.Tensor, out: torch.Tensor | None = None) -> torch.Tensor:
         """Guide pre-smooth only: [N,H,W,3] u8 (or [N,H,W] / [N,H,W,1] GRAY, [N,H,W,4] BGRX) -> internal guide
@@ -349,12 +377,20 @@ def _tensor_view(ptr: int, shape, dtype, device, owner):
 
 
 def projective_to_real(depth: torch.Tensor, fx: float, fy: float, cx: int, cy: int) -> torch.Tensor:
-    """DimensionConvertor::projectiveToReal(float*, float3*) -- DimensionConvertor.cu:3-23 (next row f3)."""
+    """DimensionConvertor::projectiveToReal(float*, float3*) -- DimensionConvertor.cu:3-23 (next row f3).
+    depth [H, W] -> [H, W, 3], or a stream of frames [N, H, W] -> [N, H, W, 3] in one launch (v is the row within
+    each frame: frame k equals the call on depth[k])."""
     if not depth.is_cuda or depth.dtype != torch.float32 or not depth.is_contiguous():
         raise TypeError("depth must be a contiguous float32 CUDA tensor")
-    h, w = depth.shape
-    out = torch.empty((h, w, 3), dtype=torch.float32, device=depth.device)
+    if depth.dim() not in (2, 3):
+        raise ValueError(f"depth must be [H, W] or [N, H, W], got {list(depth.shape)}")
+    h, w = depth.shape[-2:]
+    out = torch.empty((*depth.shape, 3), dtype=torch.float32, device=depth.device)
     with torch.cuda.device(depth.device):
-        _lib.check(_lib.lib().kdme_projective_to_real(_ptr(depth), _ptr(out), w, h, fx, fy, int(cx), int(cy),
-                                                      torch.cuda.current_stream().cuda_stream))
+        stream = torch.cuda.current_stream().cuda_stream
+        if depth.dim() == 2:
+            _lib.check(_lib.lib().kdme_projective_to_real(_ptr(depth), _ptr(out), w, h, fx, fy, int(cx), int(cy), stream))
+        else:
+            _lib.check(_lib.lib().kdme_projective_to_real_batch(_ptr(depth), _ptr(out), w, h, depth.shape[0], fx, fy,
+                                                                int(cx), int(cy), stream))
     return out
