@@ -79,7 +79,7 @@ int jbf_set_presmooth(jbf_handle *h, int ksize, float sigma_color, float sigma_s
 /* Format of the raw guide every later call on this handle reads (jbf_process, _batch, _batch_u16, _batch_xyz,
  * _batch_xyz_u16, _xyz, _host,
  * _host_u16, jbf_presmooth, _presmooth_rows, _presmooth_rows_p2p, jbf_upsample, _upsample_batch,
- * _upsample_batch_u16, jbf_mrf):
+ * _upsample_batch_u16, jbf_mrf, _mrf_batch, _mrf_batch_u16):
  * KDME_GUIDE_GRAY, KDME_GUIDE_BGR (the default) or KDME_GUIDE_BGRX; any other value is KDME_EINVAL.
  * Handle state only: no synchronisation, no allocation (the host pipeline's guide slots and the
  * jbf_smooth_device buffer are re-sized when next used). */
@@ -234,9 +234,23 @@ int jbf_upsample_batch_u16(jbf_handle *h, const uint16_t *depth_lo_dev, int wl, 
  * bit 9 (0x200) when it used 64x8 tiles (small launches) instead of 64x16. */
 int jbf_kernel_variant(jbf_handle *h);
 
-/* "Next" row f1: MarkovRandomField::Process (MarkovRandomField.cu:4-49), raw guide. */
+/* "Next" row f1: MarkovRandomField::Process (MarkovRandomField.cu:4-49), raw guide.  Reference constants
+ * (MarkovRandomField.cpp:3-6): radius 2, color_sigma 50, smooth_sigma 150.  The handle provides the size, the guide
+ * format, the device and the stream; the call leaves the handle's buffers (jbf_filtered_device, jbf_guide4_device,
+ * jbf_smooth_device) as they were.  The batch of one of jbf_mrf_batch. */
 int jbf_mrf(jbf_handle *h, const float *depth_dev, const uint8_t *bgr_dev, size_t bgr_step,
             float *out_dev, int window_radius, float color_sigma, float smooth_sigma);
+/* n_frames independent MarkovRandomField::Process calls in one call (a recorded Kinect sequence).  Frame strides:
+ * width*height depth samples, height*bgr_step guide bytes, width*height output floats.  Frame k of the result
+ * equals jbf_mrf on frame k alone, bit for bit.  Nothing is staged in HBM, so there is no max_batch chunking.
+ * KDME_EINVAL: n_frames < 1, a NULL pointer, a radius outside [0, KDME_MAX_RADIUS], a guide step below C*width, or
+ * an output whose bytes overlap the depth input's. */
+int jbf_mrf_batch(jbf_handle *h, const float *depth_dev, const uint8_t *bgr_dev, size_t bgr_step, float *out_dev,
+                  int n_frames, int window_radius, float color_sigma, float smooth_sigma);
+/* The same with sensor depth: uint16 millimetres, read directly by the kernel (no conversion pass); a sample s
+ * filters exactly as the float (float)s. */
+int jbf_mrf_batch_u16(jbf_handle *h, const uint16_t *depth_dev, const uint8_t *bgr_dev, size_t bgr_step,
+                      float *out_dev, int n_frames, int window_radius, float color_sigma, float smooth_sigma);
 
 /* "Next" row f3: DimensionConvertor::projectiveToReal(float*, float3*)
  * (DimensionConvertor.cu:3-23, DimensionConvertor.h:34-61); cx, cy truncated to

@@ -73,6 +73,8 @@ SIGNATURES = {
     "jbf_upsample_batch_u16": (_i, [_vp, _vp, _i, _i, _vp, _sz, _vp, _i]),
     "jbf_kernel_variant": (_i, [_vp]),
     "jbf_mrf": (_i, [_vp, _vp, _vp, _sz, _vp, _i, _f, _f]),
+    "jbf_mrf_batch": (_i, [_vp, _vp, _vp, _sz, _vp, _i, _i, _f, _f]),
+    "jbf_mrf_batch_u16": (_i, [_vp, _vp, _vp, _sz, _vp, _i, _i, _f, _f]),
     "kdme_projective_to_real": (_i, [_vp, _vp, _i, _i, _f, _f, _i, _i, _vp]),
     "kdme_projective_to_real_batch": (_i, [_vp, _vp, _i, _i, _i, _f, _f, _i, _i, _vp]),
     "kdme_depth_bilateral_xyz": (_i, [_vp, _vp, _vp, _i, _i, _i, _f, _f, _vp]),

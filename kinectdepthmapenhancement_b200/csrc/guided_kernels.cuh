@@ -23,7 +23,8 @@
 // in the U16 instantiations, uint16 millimetres (see guided_depth); a template parameter rather than a branch keeps
 // the float32 kernels' code as it was.
 //
-// mrf_kernel follows MarkovRandomField/MarkovRandomField.cu:4-40 (next row f1).
+// mrf_kernel follows MarkovRandomField/MarkovRandomField.cu:4-40 (next row f1).  It filters a stream of frames the
+// same way (frame = blockIdx.z) and reads the raw guide and float32 or uint16 depth while it stages its tile.
 #pragma once
 #include <type_traits>
 #include "common.cuh"
@@ -63,6 +64,15 @@ __device__ __forceinline__ int guided_upsample_site(int x, int W, int wl) {
     int xl = (num <= 0) ? 0 : (int)((num + 2LL * W - 1) / (2LL * W));
     if (xl >= wl) return -1;
     return ((int)(((2LL * xl + 1) * W) / (2LL * wl)) == x) ? xl : -1;
+}
+
+// Pixel gx of a raw guide row of C = 1, 3 or 4 bytes per pixel as the word the colour distance reads: GRAY g is
+// {g,0,0,0}, BGR and BGRX (b,g,r,x) are {b,g,r,0}.
+template <int C>
+__device__ __forceinline__ uint32_t guide_word(const uint8_t* row, int gx) {
+    const uint8_t* q = row + C * gx;
+    if constexpr (C == 1) return (uint32_t)__ldg(q);
+    else return (uint32_t)__ldg(q) | ((uint32_t)__ldg(q + 1) << 8) | ((uint32_t)__ldg(q + 2) << 16);
 }
 
 // Depth at image pixel (gx, gy) of `frame`: every depth read of both guided kernels goes through here.  The
@@ -213,9 +223,7 @@ __global__ void __launch_bounds__(TW * TH) guided_fill_kernel(const __grid_const
         int32_t l = 0;
         if (in) {
             d = guided_depth<U16>(p, frame, gx, gy);
-            const uint8_t* q = bgr + (long long)gy * p.bgr_step + C * gx;
-            if constexpr (C == 1) g = (uint32_t)__ldg(q);
-            else g = (uint32_t)__ldg(q) | ((uint32_t)__ldg(q + 1) << 8) | ((uint32_t)__ldg(q + 2) << 16);
+            g = guide_word<C>(bgr + (long long)gy * p.bgr_step, gx);
             if (labels) l = __ldg(labels + (long long)gy * p.width + gx);
         }
         sD[idx] = (d > kValidDepth) ? d : 0.f;  // 0 marks "not a sample" (also out of bounds)
@@ -239,51 +247,81 @@ __device__ __forceinline__ double ex2_weight(float a, float m = 1.0f) {
     return (double)(ex2_approx(light ? a + kWeightBias : a) * m) * (light ? 0x1p-32 /* 2^-kWeightBias */ : 1.0);
 }
 
+// The parameters of mrf_kernel: n frames stored back to back, the raw guide in the kernel's format C.
+struct MrfParams {
+    int width, height, radius;
+    const float* depth;       // float32 millimetres, or
+    const uint16_t* depth16;  // uint16 millimetres (the U16 kernels)
+    const uint8_t* bgr;       // RAW guide, C bytes per pixel
+    long long bgr_step;
+    float* out;
+    long long plane, bgr_stride;   // per-frame strides: depth samples and output floats (width*height), guide bytes
+    float color_sigma, smooth_sigma;
+};
+
 // MarkovRandomField.cu:4-40: out = (d_p + sum f d_q) / (1 + sum f), f = smooth * expf(-sigma_c * cd)
 // over valid taps; f == 0 where fp32 expf() returns 0 (kExpZeroArg).  Sums in double: up to 961 taps of equal
-// weight would otherwise round to more than 1e-3 mm.
-template <int TW, int TH>
-__global__ void __launch_bounds__(TW * TH)
-mrf_kernel(const float* __restrict__ depth, const uint32_t* __restrict__ guide4, int guide_pitch,
-           float* __restrict__ out, int width, int height, int R, float color_sigma, float smooth_sigma) {
+// weight would otherwise round to more than 1e-3 mm.  The frame is blockIdx.z.  The tile stages the raw depth (the
+// centre seeds num even when it is a hole; out of bounds is 0) and the raw guide as guide_word, so the colour
+// distances are those of the internal u8x4 guide and no conversion pass is needed.
+// R_CT >= 0 is a compile-time radius (the window fully unrolled); -1 takes the radius at run time.
+template <int R_CT, int TW, int TH, int C, bool U16>
+__global__ void __launch_bounds__(TW * TH) mrf_kernel(const __grid_constant__ MrfParams p) {
     constexpr int NT = TW * TH;
-    const int WS = 2 * R + 1, SP = TW + 2 * R, SH = TH + 2 * R;
+    const int R = (R_CT >= 0) ? R_CT : p.radius, WS = 2 * R + 1, SP = TW + 2 * R, SH = TH + 2 * R;
     extern __shared__ __align__(16) uint8_t smem_mrf[];
     float* sD = reinterpret_cast<float*>(smem_mrf);
     uint32_t* sG = reinterpret_cast<uint32_t*>(sD + SP * SH);
     const int tid = threadIdx.x;
     const int x0 = blockIdx.x * TW, y0 = blockIdx.y * TH;
+    const long long frame = blockIdx.z, f0 = frame * p.plane;
+    const uint8_t* bgr = p.bgr + frame * p.bgr_stride;
     for (int idx = tid; idx < SP * SH; idx += NT) {
         int sy = idx / SP, sx = idx - sy * SP;
         int gx = x0 - R + sx, gy = y0 - R + sy;
-        bool in = (gx >= 0) & (gx < width) & (gy >= 0) & (gy < height);
-        sD[idx] = in ? __ldg(depth + (long long)gy * width + gx) : 0.f;
-        sG[idx] = in ? __ldg(guide4 + (long long)gy * guide_pitch + gx) : 0u;
+        bool in = (gx >= 0) & (gx < p.width) & (gy >= 0) & (gy < p.height);
+        float d = 0.f;
+        uint32_t g = 0u;
+        if (in) {
+            const long long i = f0 + (long long)gy * p.width + gx;
+            if constexpr (U16) d = (float)__ldg(p.depth16 + i); else d = __ldg(p.depth + i);
+            g = guide_word<C>(bgr + (long long)gy * p.bgr_step, gx);
+        }
+        sD[idx] = d;
+        sG[idx] = g;
     }
     __syncthreads();
     const int lx = tid % TW, ly = tid / TW;
     const int gx = x0 + lx, gy = y0 + ly;
-    if (gx >= width || gy >= height) return;
+    if (gx >= p.width || gy >= p.height) return;
     const int pc = (ly + R) * SP + lx + R;
     const uint32_t gpix = sG[pc];
     const float dp = sD[pc];
-    const float nk = -color_sigma * (float)kLog2e;
+    const float nk = -p.color_sigma * (float)kLog2e;
     // sigma_c == 0 weights every tap 0 (the reference skips expf there): no argument passes a +inf cut
-    const float cut = (color_sigma != 0.0f) ? -(float)(kExpZeroArg * kLog2e) : __int_as_float(0x7f800000);
-    const double sm = smooth_sigma;
+    const float cut = (p.color_sigma != 0.0f) ? -(float)(kExpZeroArg * kLog2e) : __int_as_float(0x7f800000);
+    const double sm = p.smooth_sigma;
     double num = dp, den = 1.0;
-    for (int i = 0; i < WS; ++i)
-        for (int j = 0; j < WS; ++j) {
-            const int q = (ly + i) * SP + lx + j;
-            const float d = sD[q];
-            const uint32_t ad = __vabsdiffu4(gpix, sG[q]);
-            const float a = (float)__dp4a(ad, ad, 0u) * nk;
-            if (!(d > kValidDepth) || !(a >= cut)) continue;
-            const double f = sm * ex2_weight(a);
-            num = fma(f, (double)d, num);
-            den += f;
-        }
-    out[(long long)gy * width + gx] = (den == 0.0) ? 0.0f : (float)(num / den);
+    auto tap = [&](int i, int j) {
+        const int q = (ly + i) * SP + lx + j;
+        const float d = sD[q];
+        const uint32_t ad = __vabsdiffu4(gpix, sG[q]);
+        const float a = (float)__dp4a(ad, ad, 0u) * nk;
+        if (!(d > kValidDepth) || !(a >= cut)) return;
+        const double f = sm * ex2_weight(a);
+        num = fma(f, (double)d, num);
+        den += f;
+    };
+    if constexpr (R_CT >= 0) {
+#pragma unroll
+        for (int i = 0; i < 2 * R_CT + 1; ++i)
+#pragma unroll
+            for (int j = 0; j < 2 * R_CT + 1; ++j) tap(i, j);
+    } else {   // the compiler's own unrolling: a forced factor of 1 measured 17 % slower at r = 5
+        for (int i = 0; i < WS; ++i)
+            for (int j = 0; j < WS; ++j) tap(i, j);
+    }
+    p.out[f0 + (long long)gy * p.width + gx] = (den == 0.0) ? 0.0f : (float)(num / den);
 }
 
 // Projection_GPU::bilateralfilter -- Projection_GPU.cu:213-246 (next row f2): depth-only bilateral on the

@@ -310,16 +310,23 @@ class JointBilateralFilter:
         _lib.check(fn(self._h, _ptr(depth_host), _ptr(color_host), step, _ptr(out_host), n))
         return out_host
 
-    def mrf(self, depth: torch.Tensor, color: torch.Tensor, window_radius=2, color_sigma=50.0, smooth_sigma=150.0):
-        """MarkovRandomField::Process -- MarkovRandomField.cu:4-49 (next row f1)."""
-        _check_cuda(depth, torch.float32, "depth", self.device)
-        _check_cuda(color, torch.uint8, "color", self.device)
-        if tuple(depth.shape) != (self.height, self.width):
-            raise ValueError(f"depth must be [{self.height}, {self.width}]")
-        step = self._use_guide(color, (self.height, self.width), "color")
-        out = torch.empty_like(depth)
-        _lib.check(_lib.lib().jbf_mrf(self._h, _ptr(depth), _ptr(color), step, _ptr(out),
-                                      window_radius, color_sigma, smooth_sigma))
+    def mrf(self, depth: torch.Tensor, color: torch.Tensor, window_radius=2, color_sigma=50.0, smooth_sigma=150.0,
+            out: torch.Tensor | None = None) -> torch.Tensor:
+        """MarkovRandomField::Process -- MarkovRandomField.cu:4-49 (next row f1).  depth [H, W] float32, or a stream
+        [N, H, W] of float32 or uint16 millimetres (torch.uint16 or a torch.int16 view of the same bits); color
+        [(N,) H, W(, C)] uint8 in any guide format -> out of depth's shape, float32.  Frame k of a stream equals the
+        call on frame k alone, bit for bit.  The handle's filtered plane and smoothed guide are left as they were."""
+        if isinstance(depth, torch.Tensor) and depth.dim() == 2:
+            _check_cuda(depth, torch.float32, "depth", self.device)
+            if out is not None and out.dim() == 2:
+                out = out[None]
+            _, step, _, out = self._batch_args(depth[None], color[None], out)
+            _lib.check(_lib.lib().jbf_mrf(self._h, _ptr(depth), _ptr(color), step, _ptr(out), window_radius,
+                                          color_sigma, smooth_sigma))
+            return out[0]
+        n, step, u16, out = self._batch_args(depth, color, out)
+        fn = _lib.lib().jbf_mrf_batch_u16 if u16 else _lib.lib().jbf_mrf_batch
+        _lib.check(fn(self._h, _ptr(depth), _ptr(color), step, _ptr(out), n, window_radius, color_sigma, smooth_sigma))
         return out
 
     @property
