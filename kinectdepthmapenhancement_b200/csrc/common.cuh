@@ -120,6 +120,23 @@ __device__ __forceinline__ f32x2 add2(f32x2 a, f32x2 b) {
     return r;
 }
 
+// Depth sample i of a plane of DT (float, or uint16_t millimetres) as a float: every depth read of every kernel goes
+// through here.  A uint16 sample s reads as the float (float)s, exactly, so a uint16 frame filters bit for bit like its
+// float32 image (s <= 50 is a hole).
+template <class DT>
+__device__ __forceinline__ float load_depth(const void* base, long long i) {
+    return (float)__ldg(static_cast<const DT*>(base) + i);
+}
+
+// low-res sample index landing on high-res coordinate x, or -1 (SURVEY.md 8(d) config 3):
+// x_hi(xl) = floor((2 xl + 1) * W / (2 wl)); at most one xl per x when W >= wl.
+__device__ __forceinline__ int upsample_site(int x, int W, int wl) {
+    long long num = 2LL * wl * x - W;
+    int xl = (num <= 0) ? 0 : (int)((num + 2LL * W - 1) / (2LL * W));
+    if (xl >= wl) return -1;
+    return ((int)(((2LL * xl + 1) * W) / (2LL * wl)) == x) ? xl : -1;
+}
+
 // 16-byte streaming global accesses (read-once inputs / write-once outputs).
 __device__ __forceinline__ float4 ldg_stream_f4(const float4* p) {
     float4 v;

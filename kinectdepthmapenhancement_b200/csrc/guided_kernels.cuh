@@ -19,12 +19,12 @@
 // image (g,0,0) or (b,g,r), bit for bit.
 //
 // The guided kernel filters a stream of frames: the frame is blockIdx.z, which offsets every plane by its
-// per-frame stride, so frame k of a launch equals a launch on frame k alone, bit for bit.  The depth is float32 or,
-// in the U16 instantiations, uint16 millimetres (see guided_depth); a template parameter rather than a branch keeps
-// the float32 kernels' code as it was.
+// per-frame stride, so frame k of a launch equals a launch on frame k alone, bit for bit.  The depth is float32 or
+// uint16 millimetres, the kernel's template parameter DT (read through load_depth); a template parameter rather than a
+// branch keeps the float32 kernels' code as it was.
 //
 // mrf_kernel follows MarkovRandomField/MarkovRandomField.cu:4-40 (next row f1).  It filters a stream of frames the
-// same way (frame = blockIdx.z) and reads the raw guide and float32 or uint16 depth while it stages its tile.
+// same way (frame = blockIdx.z) and reads the raw guide and the DT depth while it stages its tile.
 #pragma once
 #include <type_traits>
 #include "common.cuh"
@@ -35,8 +35,7 @@ namespace kdme {
 template <int WS_CT>
 struct GuidedParams {
     int width, height;
-    const float* depth;
-    const uint16_t* depth16;  // the depth as uint16 millimetres, read instead of `depth` by the U16 kernels
+    const void* depth;      // DT samples: width x height per frame, or wl x hl for the upsampling
     const int32_t* labels;  // nullable
     const uint8_t* bgr;     // RAW guide, packed C-channel pixels (kernel template parameter C = 1, 3 or 4)
     long long bgr_step;
@@ -44,10 +43,8 @@ struct GuidedParams {
     float sigma_c;
     int radius;
     double kc, kd;   // 1/(2 sigma_c^2), 1/(2 sigma_d^2) in double; 0 where that sigma is 0 (factor skipped)
-    // upsampling form (SURVEY.md 8(d) config 3, label-guided variant): when depth_lo or depth_lo16 is non-null the
-    // depth plane is the sparse scatter of a wl x hl low-res map (see upsample_site) and `depth` is ignored
-    const float* depth_lo;
-    const uint16_t* depth_lo16;   // read instead of depth_lo by the U16 kernels
+    // upsampling form (SURVEY.md 8(d) config 3, label-guided variant): when wl > 0 the depth plane is the sparse
+    // scatter of the wl x hl low-res map `depth` (see upsample_site); the fill has wl = hl = 0
     int wl, hl;
     // per-frame strides (frame = blockIdx.z): depth samples (width*height, or wl*hl for the upsampling), guide bytes
     // (height*bgr_step), labels (width*height; 0 without labels), output floats (width*height)
@@ -58,14 +55,6 @@ struct GuidedParams {
     std::conditional_t<(WS_CT > 0), double, float> sfac[WS_CT > 0 ? WS_CT * WS_CT : 31 * 31];
 };
 
-// low-res sample index landing on high-res coordinate x, or -1: x_hi(xl) = floor((2 xl + 1) * W / (2 wl))
-__device__ __forceinline__ int guided_upsample_site(int x, int W, int wl) {
-    long long num = 2LL * wl * x - W;
-    int xl = (num <= 0) ? 0 : (int)((num + 2LL * W - 1) / (2LL * W));
-    if (xl >= wl) return -1;
-    return ((int)(((2LL * xl + 1) * W) / (2LL * wl)) == x) ? xl : -1;
-}
-
 // Pixel gx of a raw guide row of C = 1, 3 or 4 bytes per pixel as the word the colour distance reads: GRAY g is
 // {g,0,0,0}, BGR and BGRX (b,g,r,x) are {b,g,r,0}.
 template <int C>
@@ -73,21 +62,6 @@ __device__ __forceinline__ uint32_t guide_word(const uint8_t* row, int gx) {
     const uint8_t* q = row + C * gx;
     if constexpr (C == 1) return (uint32_t)__ldg(q);
     else return (uint32_t)__ldg(q) | ((uint32_t)__ldg(q + 1) << 8) | ((uint32_t)__ldg(q + 2) << 16);
-}
-
-// Depth at image pixel (gx, gy) of `frame`: every depth read of both guided kernels goes through here.  The
-// upsampling reads the low-res sample landing on the pixel (0 where none does).  A uint16 sample s reads as the
-// float (float)s, exactly (s <= 50 is a hole, as for the float input).
-template <bool U16, class P>
-__device__ __forceinline__ float guided_depth(const P& p, long long frame, int gx, int gy) {
-    if (p.depth_lo || p.depth_lo16) {
-        const int xl = guided_upsample_site(gx, p.width, p.wl), yl = guided_upsample_site(gy, p.height, p.hl);
-        if ((xl < 0) | (yl < 0)) return 0.f;
-        const long long i = (long long)frame * p.depth_stride + (long long)yl * p.wl + xl;
-        if constexpr (U16) return (float)__ldg(p.depth_lo16 + i); else return __ldg(p.depth_lo + i);
-    }
-    const long long i = (long long)frame * p.depth_stride + (long long)gy * p.width + gx;
-    if constexpr (U16) return (float)__ldg(p.depth16 + i); else return __ldg(p.depth + i);
 }
 
 // The three sweeps of the pixel whose window starts at staged index `base`, in double (DESIGN.md section 2): the
@@ -185,7 +159,7 @@ __device__ __forceinline__ float guided_sweeps(const float* sD, const uint32_t* 
 // once.  A compile-time window (WS_CT > 0: windows 3..7) keeps the tile in static shared arrays and the fully
 // unrolled sweeps read the spatial factors straight from the constant bank; the run-time window (WS_CT = 0) sizes
 // the tile at launch (dynamic shared memory) and stages the factors into shared doubles.
-template <int WS_CT, int TW, int TH, int C, bool U16>
+template <int WS_CT, int TW, int TH, int C, class DT>
 __global__ void __launch_bounds__(TW * TH) guided_fill_kernel(const __grid_constant__ GuidedParams<WS_CT> p) {
     constexpr int NT = TW * TH;
     const int R = (WS_CT > 0) ? WS_CT / 2 : p.radius, WS = 2 * R + 1, SP = TW + 2 * R, SH = TH + 2 * R;
@@ -222,7 +196,12 @@ __global__ void __launch_bounds__(TW * TH) guided_fill_kernel(const __grid_const
         uint32_t g = 0u;
         int32_t l = 0;
         if (in) {
-            d = guided_depth<U16>(p, frame, gx, gy);
+            if (p.wl > 0) {   // upsampling: the low-res sample landing on the pixel, 0 where none does
+                const int xl = upsample_site(gx, p.width, p.wl), yl = upsample_site(gy, p.height, p.hl);
+                if ((xl >= 0) & (yl >= 0)) d = load_depth<DT>(p.depth, frame * p.depth_stride + (long long)yl * p.wl + xl);
+            } else {
+                d = load_depth<DT>(p.depth, frame * p.depth_stride + (long long)gy * p.width + gx);
+            }
             g = guide_word<C>(bgr + (long long)gy * p.bgr_step, gx);
             if (labels) l = __ldg(labels + (long long)gy * p.width + gx);
         }
@@ -250,8 +229,7 @@ __device__ __forceinline__ double ex2_weight(float a, float m = 1.0f) {
 // The parameters of mrf_kernel: n frames stored back to back, the raw guide in the kernel's format C.
 struct MrfParams {
     int width, height, radius;
-    const float* depth;       // float32 millimetres, or
-    const uint16_t* depth16;  // uint16 millimetres (the U16 kernels)
+    const void* depth;        // DT millimetres
     const uint8_t* bgr;       // RAW guide, C bytes per pixel
     long long bgr_step;
     float* out;
@@ -265,7 +243,7 @@ struct MrfParams {
 // centre seeds num even when it is a hole; out of bounds is 0) and the raw guide as guide_word, so the colour
 // distances are those of the internal u8x4 guide and no conversion pass is needed.
 // R_CT >= 0 is a compile-time radius (the window fully unrolled); -1 takes the radius at run time.
-template <int R_CT, int TW, int TH, int C, bool U16>
+template <int R_CT, int TW, int TH, int C, class DT>
 __global__ void __launch_bounds__(TW * TH) mrf_kernel(const __grid_constant__ MrfParams p) {
     constexpr int NT = TW * TH;
     const int R = (R_CT >= 0) ? R_CT : p.radius, WS = 2 * R + 1, SP = TW + 2 * R, SH = TH + 2 * R;
@@ -283,8 +261,7 @@ __global__ void __launch_bounds__(TW * TH) mrf_kernel(const __grid_constant__ Mr
         float d = 0.f;
         uint32_t g = 0u;
         if (in) {
-            const long long i = f0 + (long long)gy * p.width + gx;
-            if constexpr (U16) d = (float)__ldg(p.depth16 + i); else d = __ldg(p.depth + i);
+            d = load_depth<DT>(p.depth, f0 + (long long)gy * p.width + gx);
             g = guide_word<C>(bgr + (long long)gy * p.bgr_step, gx);
         }
         sD[idx] = d;

@@ -48,10 +48,7 @@ enum StageMode : int { kStagePlain = 0, kStageTma = 1, kStageUpsample = 2 };
 
 struct JbfParams {
     int width, height, n_frames;
-    union {
-        const float* depth;      // [n][H][W]                      (plain / TMA)
-        const uint16_t* depth16; // the same as uint16 millimetres when depth_u16
-    };
+    const void* depth;           // [n][H][W] float32, or uint16 millimetres when depth_u16 (plain / TMA)
     const uint32_t* guide4;      // [n][H][guide_pitch] u8x4 BGR0  (smoothed guide)
     float* out;                  // [n][H][W]
     long long depth_frame_stride;   // elements
@@ -67,8 +64,11 @@ struct JbfParams {
     float flag_scale;            // a pixel is refined in fp64 when den < wsum * flag_scale (ill-conditioned)
     double kc, kd;               // 1/(2 sigma_c^2), 1/(2 sigma_d^2) (fp64 refinement path)
     int mode;                    // StageMode
-    const float* depth_lo;       // upsample: low-res depth [n][hl][wl] ...
-    const uint16_t* depth_lo16;  // ... or, when non-null, the same as uint16 millimetres (read through upsample_sample)
+    // upsample: the low-res depth [n][hl][wl], float32 (depth_lo) or uint16 millimetres (depth_lo16, when non-null),
+    // read through upsample_sample.  A pointer pair rather than `depth` and depth_u16: with the block's layout and this
+    // null test as they are, jbf_upsample_gather_kernel keeps its code (any other form re-scheduled it, 0.5 % slower)
+    const float* depth_lo;
+    const uint16_t* depth_lo16;
     long long lo_frame_stride;   // samples per low-res frame (wl * hl)
     int wl, hl;
     const int* ups_inv_x;        // upsample, optional: low-res column landing on high-res column x, or -1 ([width]); null = compute
@@ -105,21 +105,11 @@ struct JbfParams {
     unsigned int* q_count_prev;  // the previous launch's counter (two alternate): re-armed by this launch's filter kernel
     unsigned int* q_items;
     unsigned int q_capacity;
-    // 1: the plain / TMA depth is depth16, read by the DT = uint16_t instantiations (same layout and frame stride;
-    // whole frames only: no row bands, no peer halos).  Kept in q_capacity's padding: the layout of the block, and so
-    // the code of every kernel that takes it, stays as it was.
+    // 1: the plain / TMA depth is uint16 millimetres, read by the DT = uint16_t instantiations (whole frames only: no
+    // row bands, no peer halos).  Kept in q_capacity's padding, so the layout of the block stays as it was.
     int depth_u16;
     unsigned long long* stats;   // [0] += pixels refined in fp64, [1] += pixels dropped (queue full)
 };
-
-// First sample of `frame` in the plain / TMA depth of a DT instantiation.  Its samples are read as (float)__ldg(..): a
-// uint16 sample s reads as the float (float)s, exactly, so a uint16 frame filters bit for bit like its float32 image
-// (s <= 50 is a hole).
-template <class DT>
-__device__ __forceinline__ const DT* jbf_depth_frame(const JbfParams& p, int frame) {
-    if constexpr (std::is_same<DT, uint16_t>::value) return p.depth16 + (long long)frame * p.depth_frame_stride;
-    else return p.depth + (long long)frame * p.depth_frame_stride;
-}
 
 template <int R, int TW, int TH>
 struct JbfTile {
@@ -141,20 +131,11 @@ struct JbfTile {
     static_assert((SP16 * 2) % 16 == 0 && SP16 * SH * 2 <= PLANE, "uint16 TMA box: 16-byte rows inside one plane");
 };
 
-// low-res sample index landing on high-res coordinate x, or -1 (SURVEY.md 8(d) config 3):
-// x_hi(xl) = floor((2 xl + 1) * W / (2 wl)); at most one xl per x when W >= wl.
-__device__ __forceinline__ int upsample_site(int x, int W, int wl) {
-    long long num = 2LL * wl * x - W;
-    int xl = (num <= 0) ? 0 : (int)((num + 2LL * W - 1) / (2LL * W));
-    if (xl >= wl) return -1;
-    return ((int)(((2LL * xl + 1) * W) / (2LL * wl)) == x) ? xl : -1;
-}
-
-// low-res sample (xl, yl) of `frame`: every upsampling kernel reads the low-res depth through here.  A uint16
-// sample s reads as the float (float)s, exactly (s <= 50 is a hole, as for the float input).
+// low-res sample (xl, yl) of `frame`: every upsampling kernel reads the low-res depth through here.  Its type is a
+// run-time branch, so the upsampling kernels have one instantiation for both types.
 __device__ __forceinline__ float upsample_sample(const JbfParams& p, int frame, int xl, int yl) {
     const long long i = (long long)frame * p.lo_frame_stride + (long long)yl * p.wl + xl;
-    return p.depth_lo16 ? (float)__ldg(p.depth_lo16 + i) : __ldg(p.depth_lo + i);
+    return p.depth_lo16 ? load_depth<uint16_t>(p.depth_lo16, i) : load_depth<float>(p.depth_lo, i);
 }
 
 // pass-1 row sums are first added plainly in groups of this many window rows, the group sums are then
@@ -176,7 +157,7 @@ __device__ __forceinline__ void two_sum2(f32x2& a, const f32x2 b, f32x2& lo) {
 // a warp instruction costs the same pipe time however few lanes are active (tools/mufu_lanes.cu), so work can only
 // be cut finer than a warp by dropping instructions.  Same arithmetic per pixel (the accumulation origin is still
 // that of the 4-pixel group): results are bit-identical whichever way a pixel is computed.
-// DT: the plain / TMA depth is float32 or uint16 millimetres (JbfParams::depth16); every step from stage B on is the
+// DT: the plain / TMA depth is float32 or uint16 millimetres (JbfParams::depth_u16); every step from stage B on is the
 // same for both.
 template <int R, int TW, int TH, int PSEL, class DT>
 __device__ __forceinline__ void jbf_fast_body(const CUtensorMap& tm_depth, const CUtensorMap& tm_guide, const JbfParams& p) {
@@ -242,7 +223,7 @@ __device__ __forceinline__ void jbf_fast_body(const CUtensorMap& tm_depth, const
         }
     } else {
         const uint32_t* gsrc = p.guide4 + (long long)frame * p.guide_frame_stride;
-        const DT* dsrc = jbf_depth_frame<DT>(p, frame);
+        const DT* dsrc = static_cast<const DT*>(p.depth) + (long long)frame * p.depth_frame_stride;
         // upsample: the low-res sample (if any) of every staged column and row, computed once per tile
         // (sM is free until stage B: its first SP + SH words hold the two maps)
         int* colmap = reinterpret_cast<int*>(sM);
@@ -269,12 +250,12 @@ __device__ __forceinline__ void jbf_fast_body(const CUtensorMap& tm_depth, const
                 g = __ldg(gsrc + (long long)gy * p.guide_pitch + gx);
                 if (mode == kStagePlain) {
                     if constexpr (std::is_same<DT, uint16_t>::value) {
-                        d = (float)__ldg(dsrc + (long long)gy * p.width + gx);
+                        d = load_depth<DT>(dsrc, (long long)gy * p.width + gx);
                     } else {
                         const float* row = dsrc + (long long)gy * p.width;
                         if (p.depth_up != nullptr && gy < p.band0) row = p.depth_up + (long long)gy * p.width;
                         else if (p.depth_dn != nullptr && gy >= p.band1) row = p.depth_dn + (long long)(gy - p.band1) * p.width;
-                        d = __ldg(row + gx);
+                        d = load_depth<float>(row, gx);
                     }
                 } else {  // scatter the low-res sample onto its high-res site
                     const int xl = colmap[sx], yl = rowmap[sy];
@@ -1039,10 +1020,10 @@ __device__ __forceinline__ float jbf_sample_depth(const JbfParams& p, int frame,
         const int yl = p.ups_inv_y ? __ldg(p.ups_inv_y + gy) : upsample_site(gy, p.height, p.hl);
         return ((xl >= 0) & (yl >= 0)) ? upsample_sample(p, frame, xl, yl) : 0.f;
     }
-    const float* row = p.depth + (long long)frame * p.depth_frame_stride + (long long)gy * p.width;
+    const float* row = static_cast<const float*>(p.depth) + (long long)frame * p.depth_frame_stride + (long long)gy * p.width;
     if (p.depth_up != nullptr && gy < p.band0) row = p.depth_up + (long long)gy * p.width;
     else if (p.depth_dn != nullptr && gy >= p.band1) row = p.depth_dn + (long long)(gy - p.band1) * p.width;
-    return __ldg(row + gx);
+    return load_depth<float>(row, gx);
 }
 
 // exp(-x) for x >= 0 in fp64 without the library's special-case handling: 2^(-x log2e) by Cody-Waite
@@ -1116,7 +1097,7 @@ __global__ void __launch_bounds__(128) jbf_refine_kernel(const JbfParams p, cons
         const int oy = (int)(rem / (unsigned)p.width), x = (int)(rem - (unsigned)oy * (unsigned)p.width);
         const int y = oy + p.y_off;
         const uint32_t* gsrc = p.guide4 + (long long)frame * p.guide_frame_stride;
-        const DT* dsrc = jbf_depth_frame<DT>(p, frame);
+        const DT* dsrc = static_cast<const DT*>(p.depth) + (long long)frame * p.depth_frame_stride;
         // all of the lane's loads are issued before the first use (the taps are independent: one round trip
         // to L2 per pixel instead of two per tap); out-of-window taps read the centre and are masked
         float dfl[KMAX];
@@ -1127,7 +1108,7 @@ __global__ void __launch_bounds__(128) jbf_refine_kernel(const JbfParams p, cons
             const int ty = y + tdy[u], tx = x + tdx[u];
             const bool in = tx >= 0 && tx < p.width && ty >= 0 && ty < p.height;
             const int cy_ = in ? ty : y, cx_ = in ? tx : x;
-            const float df = PLAIN ? (float)__ldg(dsrc + (long long)cy_ * p.width + cx_) : jbf_sample_depth(p, frame, cx_, cy_);
+            const float df = PLAIN ? load_depth<DT>(dsrc, (long long)cy_ * p.width + cx_) : jbf_sample_depth(p, frame, cx_, cy_);
             gql[u] = __ldg(gsrc + (long long)cy_ * p.guide_pitch + cx_);
             dfl[u] = in ? df : 0.f;
         }
@@ -1209,7 +1190,7 @@ jbf_generic_kernel(const JbfGenericParams gp_) {
     const int tid = threadIdx.x;
     const int x0 = blockIdx.x * TW, y0 = p.y_off + blockIdx.y * TH, frame = blockIdx.z;
     const uint32_t* gsrc = p.guide4 + (long long)frame * p.guide_frame_stride;
-    const DT* dsrc = jbf_depth_frame<DT>(p, frame);
+    const DT* dsrc = static_cast<const DT*>(p.depth) + (long long)frame * p.depth_frame_stride;
     for (int idx = tid; idx < SP * SH; idx += NT) {
         int sy = idx / SP, sx = idx - sy * SP;
         int gx = x0 - R + sx, gy = y0 - R + sy;
@@ -1223,7 +1204,7 @@ jbf_generic_kernel(const JbfGenericParams gp_) {
                 int yl = upsample_site(gy, p.height, p.hl);
                 if ((xl >= 0) & (yl >= 0)) d = upsample_sample(p, frame, xl, yl);
             } else {
-                d = (float)__ldg(dsrc + (long long)gy * p.width + gx);
+                d = load_depth<DT>(dsrc, (long long)gy * p.width + gx);
             }
         }
         sD[idx] = d;

@@ -50,6 +50,16 @@ static bool ranges_overlap(const void* in, unsigned long long in_bytes, const fl
     return i0 < o1 && o0 < i1;
 }
 
+// A depth input of frames stored back to back: float32 millimetres, or uint16 millimetres (the sensors' format) when
+// u16.  The kernels take the sample type as their template parameter DT (with_depth_type).
+struct DepthIn {
+    const void* ptr;
+    bool u16;
+    size_t sample_bytes() const { return u16 ? sizeof(uint16_t) : sizeof(float); }
+    // the same input from sample n on (the first sample of a later frame)
+    DepthIn advance(long long n) const { return {static_cast<const char*>(ptr) + n * (long long)sample_bytes(), u16}; }
+};
+
 struct DeviceGuard {
     int prev = -1;
     bool ok = true;
@@ -173,8 +183,7 @@ struct jbf_handle {
     // host pipeline (jbf_process_host)
     cudaStream_t s_h2d = nullptr, s_d2h = nullptr;
     cudaEvent_t ev_in[kPipeDepth] = {}, ev_done[kPipeDepth] = {}, ev_free[kPipeDepth] = {};
-    float* pipe_depth[kPipeDepth] = {};
-    uint16_t* pipe_depth16[kPipeDepth] = {};   // u16 sensor depth staging (jbf_process_host_u16), lazy
+    float* pipe_depth[kPipeDepth] = {};   // a uint16 chunk (jbf_process_host_u16) uses the first half
     uint8_t* pipe_bgr[kPipeDepth] = {};
     float* pipe_out[kPipeDepth] = {};
     size_t pipe_bgr_step = 0;
@@ -417,7 +426,7 @@ extern "C" void jbf_destroy(jbf_handle* h) {
     cudaFree(h->ps_space_dev);
     cudaFree(h->ps_color_dev);
     for (int b = 0; b < kPipeDepth; b++) {
-        cudaFree(h->pipe_depth[b]); cudaFree(h->pipe_bgr[b]); cudaFree(h->pipe_out[b]); cudaFree(h->pipe_depth16[b]);
+        cudaFree(h->pipe_depth[b]); cudaFree(h->pipe_bgr[b]); cudaFree(h->pipe_out[b]);
         if (h->ev_in[b]) cudaEventDestroy(h->ev_in[b]);
         if (h->ev_done[b]) cudaEventDestroy(h->ev_done[b]);
         if (h->ev_free[b]) cudaEventDestroy(h->ev_free[b]);
@@ -478,6 +487,12 @@ static auto with_channels(int c, Fn&& fn) {
         case 4: return fn(std::integral_constant<int, 4>{});
         default: return fn(std::integral_constant<int, 3>{});
     }
+}
+
+// fn(DT{}) for depth samples of type DT: uint16_t when u16, float otherwise.
+template <class Fn>
+static auto with_depth_type(bool u16, Fn&& fn) {
+    return u16 ? fn(uint16_t{}) : fn(float{});
 }
 
 // cudaLaunchKernelEx, with programmatic stream serialisation when `pdl`: the kernel may launch before the previous
@@ -582,7 +597,7 @@ static int launch_fast_rt(jbf_handle* h, Lane& lane, JbfParams p, bool want_tma,
         constexpr bool u16 = std::is_same<DT, uint16_t>::value;
         constexpr CUtensorMapDataType dt = u16 ? CU_TENSOR_MAP_DATA_TYPE_UINT16 : CU_TENSOR_MAP_DATA_TYPE_FLOAT32;
         constexpr int bx = u16 ? T::SP16 : T::SP;   // depth box columns (see JbfTile::RP16)
-        const void* depth = p.depth;                 // depth16 shares the slot
+        const void* depth = p.depth;
         jbf_handle::MapKey& k = lane.map_key;
         if (k.depth != depth || k.guide != p.guide4 || k.rows != rows || k.n != p.n_frames || k.gp != p.guide_pitch ||
             k.bx != bx || k.by != T::SH || k.dt != (int)dt) {
@@ -705,11 +720,11 @@ static int ensure_ups_table(jbf_handle* h, int wl, int hl, int rows) {
 
 // The request of a filter launch over n whole frames: rows = out_rows = height, no halos, no low-res input, no
 // back-projection, plain mode.  Callers set what their call differs in; launch_filter fills the rest.
-static JbfParams filter_request(const jbf_handle* h, const float* depth, const uint32_t* guide4, int guide_pitch,
+static JbfParams filter_request(const jbf_handle* h, DepthIn depth, const uint32_t* guide4, int guide_pitch,
                                 float* out, int n) {
     JbfParams p = {};
     p.width = h->width; p.height = h->height; p.out_rows = h->height; p.n_frames = n;
-    p.depth = depth; p.guide4 = guide4; p.guide_pitch = guide_pitch; p.out = out;
+    p.depth = depth.ptr; p.depth_u16 = depth.u16; p.guide4 = guide4; p.guide_pitch = guide_pitch; p.out = out;
     p.mode = kStagePlain;
     return p;
 }
@@ -733,7 +748,7 @@ static int launch_generic_dt(jbf_handle* h, Lane& lane, const JbfParams& p) {
 }
 
 static int launch_generic(jbf_handle* h, Lane& lane, const JbfParams& p) {
-    return p.depth_u16 ? launch_generic_dt<uint16_t>(h, lane, p) : launch_generic_dt<float>(h, lane, p);
+    return with_depth_type(p.depth_u16, [&](auto dt) { return launch_generic_dt<decltype(dt)>(h, lane, p); });
 }
 
 template <int R, class DT>
@@ -765,13 +780,14 @@ static int launch_fast(jbf_handle* h, Lane& lane, const JbfParams& p, bool pdl) 
         if (cost < best_cost * 0.97) { best_cost = cost; best_th = th; }
     }
     if (h->force_tile_h == 16 || h->force_tile_h == 8 || h->force_tile_h == 4) best_th = h->force_tile_h;
-    switch (h->radius) {
-#define X(R) case R: return p.depth_u16 ? launch_fast_th<R, uint16_t>(h, lane, p, best_th, want_tma, pdl)          \
-                                      : launch_fast_th<R, float>(h, lane, p, best_th, want_tma, pdl);
-        KDME_FAST_RADII(X)
+    return with_depth_type(p.depth_u16, [&](auto dt) {
+        switch (h->radius) {
+#define X(R) case R: return launch_fast_th<R, decltype(dt)>(h, lane, p, best_th, want_tma, pdl);
+            KDME_FAST_RADII(X)
 #undef X
-        default: return fail(KDME_ENOTSUP, "no fast kernel for this radius");
-    }
+            default: return fail(KDME_ENOTSUP, "no fast kernel for this radius");
+        }
+    });
 }
 
 template <int MAXC>
@@ -807,18 +823,20 @@ static int launch_gather(jbf_handle* h, Lane& lane, JbfParams& p, UpsampleGeom g
 
 // fp64 re-evaluation of the queued pixels; launched with programmatic stream serialisation so its launch latency
 // hides behind the filter (it waits for the filter's completion on the device).
-// uint16 depth is always plain (whole frames).
+template <int KMAX, class DT>
+static int launch_refine_k(const jbf_handle* h, Lane& lane, const JbfParams& p) {
+    constexpr bool u16 = std::is_same<DT, uint16_t>::value;   // uint16 depth is always plain (whole frames)
+    const bool plain = u16 || (p.mode != kStageUpsample && !p.depth_up && !p.depth_dn);
+    return launch_ex(plain ? jbf_refine_kernel<KMAX, true, DT> : jbf_refine_kernel<KMAX, u16, DT>, dim3(148 * 5),
+                     dim3(128), 0, lane.stream, true, p, h->radius);
+}
+
 static int launch_refine(const jbf_handle* h, Lane& lane, const JbfParams& p) {
-    const bool plain = p.mode != kStageUpsample && !p.depth_up && !p.depth_dn;
-    auto launch = [&](auto kern) { return launch_ex(kern, dim3(148 * 5), dim3(128), 0, lane.stream, true, p, h->radius); };
-    if (h->radius <= 7)
-        return p.depth_u16 ? launch(jbf_refine_kernel<8, true, uint16_t>)
-             : plain ? launch(jbf_refine_kernel<8, true, float>) : launch(jbf_refine_kernel<8, false, float>);
-    if (h->radius <= 10)
-        return p.depth_u16 ? launch(jbf_refine_kernel<16, true, uint16_t>)
-             : plain ? launch(jbf_refine_kernel<16, true, float>) : launch(jbf_refine_kernel<16, false, float>);
-    return p.depth_u16 ? launch(jbf_refine_kernel<31, true, uint16_t>)
-         : plain ? launch(jbf_refine_kernel<31, true, float>) : launch(jbf_refine_kernel<31, false, float>);
+    return with_depth_type(p.depth_u16, [&](auto dt) {
+        using DT = decltype(dt);
+        return h->radius <= 7 ? launch_refine_k<8, DT>(h, lane, p)
+             : h->radius <= 10 ? launch_refine_k<16, DT>(h, lane, p) : launch_refine_k<31, DT>(h, lane, p);
+    });
 }
 
 // Launches request p on `lane`: its stream, refinement queue and TMA descriptors.
@@ -878,7 +896,7 @@ extern "C" int jbf_filter_guide4(jbf_handle* h, const float* depth_dev, const ui
     { int rc = guide4_step(h, &guide_step, &pitch, "jbf_filter_guide4"); if (rc != KDME_OK) return rc; }
     DeviceGuard g(h->device);
     return launch_filter(h, h->lanes[0],
-                         filter_request(h, depth_dev, reinterpret_cast<const uint32_t*>(guide4_dev), pitch, out_dev, n_frames),
+                         filter_request(h, {depth_dev, false}, reinterpret_cast<const uint32_t*>(guide4_dev), pitch, out_dev, n_frames),
                          /*pdl=*/false);
 }
 
@@ -900,7 +918,7 @@ extern "C" int jbf_filter_rows(jbf_handle* h, const float* depth_dev, const uint
     int pitch = 0;
     { int rc = guide4_step(h, &guide_step, &pitch, "jbf_filter_rows"); if (rc != KDME_OK) return rc; }
     DeviceGuard g(h->device);
-    JbfParams p = filter_request(h, depth_dev, reinterpret_cast<const uint32_t*>(guide4_dev), pitch, out_dev, 1);
+    JbfParams p = filter_request(h, {depth_dev, false}, reinterpret_cast<const uint32_t*>(guide4_dev), pitch, out_dev, 1);
     p.height = rows; p.y_off = y_off; p.out_rows = out_rows;
     return launch_filter(h, h->lanes[0], p, /*pdl=*/false);
 }
@@ -930,7 +948,7 @@ extern "C" int jbf_filter_rows_p2p(jbf_handle* h, const float* depth_dev, const 
     int pitch = 0;
     { int rc = guide4_step(h, &guide_step, &pitch, "jbf_filter_rows_p2p"); if (rc != KDME_OK) return rc; }
     DeviceGuard g(h->device);
-    JbfParams p = filter_request(h, depth_dev, reinterpret_cast<const uint32_t*>(guide4_dev), pitch, out_dev, 1);
+    JbfParams p = filter_request(h, {depth_dev, false}, reinterpret_cast<const uint32_t*>(guide4_dev), pitch, out_dev, 1);
     p.height = rows; p.y_off = y_off; p.out_rows = out_rows;
     p.depth_up = depth_up; p.depth_dn = depth_dn; p.band0 = band0; p.band1 = band1;
     return launch_filter(h, h->lanes[0], p, /*pdl=*/false);
@@ -971,20 +989,19 @@ static int launch_projective(const float* depth, float* xyz, int width, int heig
     return KDME_OK;
 }
 
-// Every jbf_process_batch* entry point: n_frames frames of float32 (depth) or uint16 (depth16) depth filtered into out
-// and, for the xyz forms (want_xyz), back-projected into xyz.  jbf_process_batch (float32, no cloud) keeps the checks
-// it always had; the newer forms also reject zero focal lengths and outputs that overlap the input or each other.
-static int process_batch(jbf_handle* h, const float* depth, const uint16_t* depth16, const uint8_t* bgr, size_t bgr_step,
-                         float* out, bool want_xyz, float* xyz, int n_frames, float fx, float fy, int cx, int cy,
-                         const char* who) {
-    const void* in = depth ? (const void*)depth : (const void*)depth16;
+// Every jbf_process_batch* entry point: n_frames depth frames filtered into out and, for the xyz forms (want_xyz),
+// back-projected into xyz.  jbf_process_batch (float32, no cloud) keeps the checks it always had; the newer forms also
+// reject zero focal lengths and outputs that overlap the input or each other.
+static int process_batch(jbf_handle* h, DepthIn depth, const uint8_t* bgr, size_t bgr_step, float* out, bool want_xyz,
+                         float* xyz, int n_frames, float fx, float fy, int cx, int cy, const char* who) {
+    const void* in = depth.ptr;
     if (!h || !in || !bgr || !out || (want_xyz && !xyz)) return fail(KDME_EINVAL, std::string(who) + ": NULL argument");
     if (n_frames < 1) return fail(KDME_EINVAL, std::string(who) + ": n_frames must be >= 1");
     if (want_xyz && (!(fx != 0.f) || !(fy != 0.f)))
         return fail(KDME_EINVAL, std::string(who) + ": focal lengths must be non-zero");
     const size_t plane = (size_t)h->width * h->height;
-    if (depth16 || want_xyz) {
-        const unsigned long long px = (unsigned long long)plane * n_frames, in_bytes = px * (depth16 ? 2 : 4);
+    if (depth.u16 || want_xyz) {
+        const unsigned long long px = (unsigned long long)plane * n_frames, in_bytes = px * depth.sample_bytes();
         if (ranges_overlap(in, in_bytes, out, px) ||
             (want_xyz && (ranges_overlap(in, in_bytes, xyz, 3 * px) || ranges_overlap(out, 4 * px, xyz, 3 * px))))
             return fail(KDME_EINVAL, std::string(who) + ": an output overlaps the depth input or the other output "
@@ -997,8 +1014,7 @@ static int process_batch(jbf_handle* h, const float* depth, const uint16_t* dept
                                   h->guide_pitch, n);
         if (rc != KDME_OK) return rc;
         float* o = out + (size_t)f0 * plane;
-        JbfParams p = filter_request(h, depth ? depth + (size_t)f0 * plane : nullptr, lane.guide4, h->guide_pitch, o, n);
-        if (depth16) { p.depth16 = depth16 + (size_t)f0 * plane; p.depth_u16 = 1; }
+        JbfParams p = filter_request(h, depth.advance((long long)f0 * plane), lane.guide4, h->guide_pitch, o, n);
         float* x = want_xyz ? xyz + 3 * (size_t)f0 * plane : nullptr;
         if (x && h->fast) { p.xyz = x; p.fx = fx; p.fy = fy; p.cx = cx; p.cy = cy; }   // the fused epilogue
         rc = launch_filter(h, lane, p, /*pdl=*/true);
@@ -1010,26 +1026,26 @@ static int process_batch(jbf_handle* h, const float* depth, const uint16_t* dept
 
 extern "C" int jbf_process_batch(jbf_handle* h, const float* depth_dev, const uint8_t* bgr_dev, size_t bgr_step,
                                  float* out_dev, int n_frames) {
-    return process_batch(h, depth_dev, nullptr, bgr_dev, bgr_step, out_dev, false, nullptr, n_frames, 0.f, 0.f, 0, 0,
+    return process_batch(h, {depth_dev, false}, bgr_dev, bgr_step, out_dev, false, nullptr, n_frames, 0.f, 0.f, 0, 0,
                          "jbf_process_batch");
 }
 
 extern "C" int jbf_process_batch_u16(jbf_handle* h, const uint16_t* depth_dev, const uint8_t* bgr_dev, size_t bgr_step,
                                      float* out_dev, int n_frames) {
-    return process_batch(h, nullptr, depth_dev, bgr_dev, bgr_step, out_dev, false, nullptr, n_frames, 0.f, 0.f, 0, 0,
+    return process_batch(h, {depth_dev, true}, bgr_dev, bgr_step, out_dev, false, nullptr, n_frames, 0.f, 0.f, 0, 0,
                          "jbf_process_batch_u16");
 }
 
 extern "C" int jbf_process_batch_xyz(jbf_handle* h, const float* depth_dev, const uint8_t* bgr_dev, size_t bgr_step,
                                      float* out_dev, float* xyz_dev, int n_frames, float fx, float fy, int cx, int cy) {
-    return process_batch(h, depth_dev, nullptr, bgr_dev, bgr_step, out_dev, true, xyz_dev, n_frames, fx, fy, cx, cy,
+    return process_batch(h, {depth_dev, false}, bgr_dev, bgr_step, out_dev, true, xyz_dev, n_frames, fx, fy, cx, cy,
                          "jbf_process_batch_xyz");
 }
 
 extern "C" int jbf_process_batch_xyz_u16(jbf_handle* h, const uint16_t* depth_dev, const uint8_t* bgr_dev,
                                          size_t bgr_step, float* out_dev, float* xyz_dev, int n_frames, float fx,
                                          float fy, int cx, int cy) {
-    return process_batch(h, nullptr, depth_dev, bgr_dev, bgr_step, out_dev, true, xyz_dev, n_frames, fx, fy, cx, cy,
+    return process_batch(h, {depth_dev, true}, bgr_dev, bgr_step, out_dev, true, xyz_dev, n_frames, fx, fy, cx, cy,
                          "jbf_process_batch_xyz_u16");
 }
 
@@ -1055,7 +1071,7 @@ extern "C" int jbf_process_xyz(jbf_handle* h, const float* depth_dev, const uint
     Lane& lane = h->lanes[0];   // one frame: one chunk, on the caller's stream
     int rc = launch_presmooth(h, lane, bgr_dev, bgr_step, lane.guide4, h->guide_pitch, 1);
     if (rc != KDME_OK) return rc;
-    JbfParams p = filter_request(h, depth_dev, lane.guide4, h->guide_pitch, h->filtered_dev, 1);
+    JbfParams p = filter_request(h, {depth_dev, false}, lane.guide4, h->guide_pitch, h->filtered_dev, 1);
     p.xyz = xyz_dev; p.fx = fx; p.fy = fy; p.cx = cx; p.cy = cy;
     return launch_filter(h, lane, p, /*pdl=*/true);
 }
@@ -1074,10 +1090,10 @@ extern "C" int jbf_refine_stats(jbf_handle* h, unsigned long long* refined, unsi
     return KDME_OK;
 }
 
-// n_frames Upsampling calls; the low-res depth is float (depth_lo) or uint16 (depth_lo16), the other one is NULL
-static int upsample_batch(jbf_handle* h, const float* depth_lo, const uint16_t* depth_lo16, int wl, int hl,
-                          const uint8_t* bgr_dev, size_t bgr_step, float* out_dev, int n_frames, const char* who) {
-    if (!h || !(depth_lo || depth_lo16) || !bgr_dev || !out_dev) return fail(KDME_EINVAL, std::string(who) + ": NULL argument");
+// n_frames Upsampling calls of the low-res depth depth_lo (wl x hl samples per frame)
+static int upsample_batch(jbf_handle* h, DepthIn depth_lo, int wl, int hl, const uint8_t* bgr_dev, size_t bgr_step,
+                          float* out_dev, int n_frames, const char* who) {
+    if (!h || !depth_lo.ptr || !bgr_dev || !out_dev) return fail(KDME_EINVAL, std::string(who) + ": NULL argument");
     if (n_frames < 1) return fail(KDME_EINVAL, std::string(who) + ": n_frames must be >= 1");
     if (wl <= 0 || hl <= 0 || wl > h->width || hl > h->height)
         return fail(KDME_EINVAL, std::string(who) + ": low-res size must be positive and <= the handle's size");
@@ -1094,23 +1110,24 @@ static int upsample_batch(jbf_handle* h, const float* depth_lo, const uint16_t* 
         int rc = launch_presmooth(h, lane, bgr_dev + (size_t)f0 * bgr_step * h->height, bgr_step, lane.guide4,
                                   h->guide_pitch, n);
         if (rc != KDME_OK) return rc;
-        JbfParams p = filter_request(h, nullptr, lane.guide4, h->guide_pitch, out_dev + (size_t)f0 * plane, n);
+        JbfParams p = filter_request(h, {nullptr, false}, lane.guide4, h->guide_pitch, out_dev + (size_t)f0 * plane, n);
         p.mode = kStageUpsample; p.wl = wl; p.hl = hl;
-        p.depth_lo = depth_lo ? depth_lo + (size_t)f0 * lo_plane : nullptr;
-        p.depth_lo16 = depth_lo16 ? depth_lo16 + (size_t)f0 * lo_plane : nullptr;
+        const DepthIn lo = depth_lo.advance((long long)f0 * lo_plane);
+        if (lo.u16) p.depth_lo16 = static_cast<const uint16_t*>(lo.ptr);
+        else p.depth_lo = static_cast<const float*>(lo.ptr);
         return launch_filter(h, lane, p, /*pdl=*/true);
     });
 }
 
 extern "C" int jbf_upsample_batch(jbf_handle* h, const float* depth_lo_dev, int wl, int hl, const uint8_t* bgr_hi_dev,
                                   size_t bgr_step, float* out_hi_dev, int n_frames) {
-    return upsample_batch(h, depth_lo_dev, nullptr, wl, hl, bgr_hi_dev, bgr_step, out_hi_dev, n_frames,
+    return upsample_batch(h, {depth_lo_dev, false}, wl, hl, bgr_hi_dev, bgr_step, out_hi_dev, n_frames,
                           "jbf_upsample_batch");
 }
 
 extern "C" int jbf_upsample_batch_u16(jbf_handle* h, const uint16_t* depth_lo_dev, int wl, int hl,
                                       const uint8_t* bgr_hi_dev, size_t bgr_step, float* out_hi_dev, int n_frames) {
-    return upsample_batch(h, nullptr, depth_lo_dev, wl, hl, bgr_hi_dev, bgr_step, out_hi_dev, n_frames,
+    return upsample_batch(h, {depth_lo_dev, true}, wl, hl, bgr_hi_dev, bgr_step, out_hi_dev, n_frames,
                           "jbf_upsample_batch_u16");
 }
 
@@ -1148,26 +1165,19 @@ static int ensure_pipe(jbf_handle* h, size_t bgr_step) {
     return KDME_OK;
 }
 
-static int process_host_impl(jbf_handle* h, const float* depth_host, const uint16_t* depth16_host,
-                             const uint8_t* bgr_host, size_t bgr_step, float* out_host, int n_frames) {
+static int process_host_impl(jbf_handle* h, DepthIn depth_host, const uint8_t* bgr_host, size_t bgr_step,
+                             float* out_host, int n_frames) {
     { int rc = guide_step(h, &bgr_step, "jbf_process_host"); if (rc != KDME_OK) return rc; }
     DeviceGuard g(h->device);
     int rc = ensure_pipe(h, bgr_step);   // re-sizes the guide slots when the guide's row bytes change
     if (rc != KDME_OK) return rc;
     const size_t plane = (size_t)h->width * h->height;
     const size_t bgr_frame = bgr_step * h->height;
-    if (depth16_host)
-        for (int b = 0; b < kPipeDepth; b++)
-            if (!h->pipe_depth16[b]) CK(cudaMalloc(&h->pipe_depth16[b], plane * h->pipe_chunk * sizeof(uint16_t)));
     rc = run_chunks(h, n_frames, h->pipe_chunk, [&](Lane& lane, int c, int f0, int n) {
         const int b = c % kPipeDepth;
         if (c >= kPipeDepth) CK(cudaStreamWaitEvent(h->s_h2d, h->ev_done[b], 0));  // slot inputs consumed
-        if (depth16_host)
-            CK(cudaMemcpyAsync(h->pipe_depth16[b], depth16_host + (size_t)f0 * plane, plane * n * sizeof(uint16_t),
-                               cudaMemcpyHostToDevice, h->s_h2d));
-        else
-            CK(cudaMemcpyAsync(h->pipe_depth[b], depth_host + (size_t)f0 * plane, plane * n * sizeof(float),
-                               cudaMemcpyHostToDevice, h->s_h2d));
+        CK(cudaMemcpyAsync(h->pipe_depth[b], depth_host.advance((long long)f0 * plane).ptr,
+                           plane * n * depth_host.sample_bytes(), cudaMemcpyHostToDevice, h->s_h2d));
         CK(cudaMemcpyAsync(h->pipe_bgr[b], bgr_host + (size_t)f0 * bgr_frame, bgr_frame * n, cudaMemcpyHostToDevice,
                            h->s_h2d));
         CK(cudaEventRecord(h->ev_in[b], h->s_h2d));
@@ -1176,8 +1186,7 @@ static int process_host_impl(jbf_handle* h, const float* depth_host, const uint1
         int rc = launch_presmooth(h, lane, h->pipe_bgr[b], bgr_step, lane.guide4, h->guide_pitch, n);
         if (rc != KDME_OK) return rc;
         // the filter reads the sensor's uint16 millimetres straight from the slot
-        JbfParams p = filter_request(h, h->pipe_depth[b], lane.guide4, h->guide_pitch, h->pipe_out[b], n);
-        if (depth16_host) { p.depth16 = h->pipe_depth16[b]; p.depth_u16 = 1; }
+        JbfParams p = filter_request(h, {h->pipe_depth[b], depth_host.u16}, lane.guide4, h->guide_pitch, h->pipe_out[b], n);
         rc = launch_filter(h, lane, p, /*pdl=*/true);
         if (rc != KDME_OK) return rc;
         CK(cudaEventRecord(h->ev_done[b], lane.stream));
@@ -1197,14 +1206,14 @@ extern "C" int jbf_process_host(jbf_handle* h, const float* depth_host, const ui
                                 float* out_host, int n_frames) {
     if (!h || !depth_host || !bgr_host || !out_host) return fail(KDME_EINVAL, "jbf_process_host: NULL argument");
     if (n_frames < 1) return fail(KDME_EINVAL, "jbf_process_host: n_frames must be >= 1");
-    return process_host_impl(h, depth_host, nullptr, bgr_host, bgr_step, out_host, n_frames);
+    return process_host_impl(h, {depth_host, false}, bgr_host, bgr_step, out_host, n_frames);
 }
 
 extern "C" int jbf_process_host_u16(jbf_handle* h, const uint16_t* depth_host, const uint8_t* bgr_host, size_t bgr_step,
                                     float* out_host, int n_frames) {
     if (!h || !depth_host || !bgr_host || !out_host) return fail(KDME_EINVAL, "jbf_process_host_u16: NULL argument");
     if (n_frames < 1) return fail(KDME_EINVAL, "jbf_process_host_u16: n_frames must be >= 1");
-    return process_host_impl(h, nullptr, depth_host, bgr_host, bgr_step, out_host, n_frames);
+    return process_host_impl(h, {depth_host, true}, bgr_host, bgr_step, out_host, n_frames);
 }
 
 // Page-locked host memory for the buffers of jbf_process_host*: write-combined memory is read by the copy
@@ -1282,16 +1291,15 @@ template <class T>
 static T* advance(T* ptr, long long n) { return ptr ? ptr + n : ptr; }
 
 // n_frames MRF filters of the handle's size and guide format on its stream, in slices of at most kMaxGridZ frames.
-// Exactly one of depth / depth16 is set.  Nothing is staged in HBM and the handle's buffers are not touched.
-static int mrf_batch(jbf_handle* h, const float* depth, const uint16_t* depth16, const uint8_t* bgr, size_t bgr_step,
-                     float* out, int n_frames, int radius, float color_sigma, float smooth_sigma, const char* who) {
+// Nothing is staged in HBM and the handle's buffers are not touched.
+static int mrf_batch(jbf_handle* h, DepthIn depth, const uint8_t* bgr, size_t bgr_step, float* out, int n_frames,
+                     int radius, float color_sigma, float smooth_sigma, const char* who) {
     const std::string w(who);
     if (n_frames < 1) return fail(KDME_EINVAL, w + ": n_frames must be >= 1");
     if (radius < 0 || radius > KDME_MAX_RADIUS) return fail(KDME_EINVAL, w + ": bad radius");
-    if (!h || !(depth || depth16) || !bgr || !out) return fail(KDME_EINVAL, w + ": NULL argument");
+    if (!h || !depth.ptr || !bgr || !out) return fail(KDME_EINVAL, w + ": NULL argument");
     const unsigned long long px = (unsigned long long)h->width * h->height * n_frames;
-    const void* in = depth ? (const void*)depth : (const void*)depth16;
-    if (ranges_overlap(in, px * (depth ? sizeof(float) : sizeof(uint16_t)), out, px))
+    if (ranges_overlap(depth.ptr, px * depth.sample_bytes(), out, px))
         return fail(KDME_EINVAL, w + ": the output overlaps the depth input (in-place operation is not supported)");
     { int rc = guide_step(h, &bgr_step, who); if (rc != KDME_OK) return rc; }
     DeviceGuard g(h->device);
@@ -1304,48 +1312,44 @@ static int mrf_batch(jbf_handle* h, const float* depth, const uint16_t* depth16,
     const size_t smem = (size_t)(kMrfTW + 2 * radius) * (kMrfTH + 2 * radius) * 8;
     const cudaStream_t st = h->lanes[0].stream;
     return with_channels(h->guide_channels, [&](auto c) {
-        constexpr int C = decltype(c)::value;
-        for (int f0 = 0; f0 < n_frames; f0 += kMaxGridZ) {
-            const long long f = f0;
-            p.depth = advance(depth, f * p.plane);
-            p.depth16 = advance(depth16, f * p.plane);
-            p.bgr = bgr + f * p.bgr_stride;
-            p.out = out + f * p.plane;
-            const dim3 grd((h->width + kMrfTW - 1) / kMrfTW, (h->height + kMrfTH - 1) / kMrfTH,
-                           std::min(kMaxGridZ, n_frames - f0));
-            // the reference's window 5 (r = 2) has a compile-time-window instantiation: 5.1 against 7.2 us per
-            // 640x480 frame batched (DESIGN.md section 4.4)
-            if (radius == 2) {
-                if (depth16) mrf_kernel<2, kMrfTW, kMrfTH, C, true><<<grd, kMrfTW * kMrfTH, smem, st>>>(p);
-                else mrf_kernel<2, kMrfTW, kMrfTH, C, false><<<grd, kMrfTW * kMrfTH, smem, st>>>(p);
-            } else if (depth16) {
-                mrf_kernel<-1, kMrfTW, kMrfTH, C, true><<<grd, kMrfTW * kMrfTH, smem, st>>>(p);
-            } else {
-                mrf_kernel<-1, kMrfTW, kMrfTH, C, false><<<grd, kMrfTW * kMrfTH, smem, st>>>(p);
+        return with_depth_type(depth.u16, [&](auto dt) {
+            constexpr int C = decltype(c)::value;
+            using DT = decltype(dt);
+            for (int f0 = 0; f0 < n_frames; f0 += kMaxGridZ) {
+                const long long f = f0;
+                p.depth = depth.advance(f * p.plane).ptr;
+                p.bgr = bgr + f * p.bgr_stride;
+                p.out = out + f * p.plane;
+                const dim3 grd((h->width + kMrfTW - 1) / kMrfTW, (h->height + kMrfTH - 1) / kMrfTH,
+                               std::min(kMaxGridZ, n_frames - f0));
+                // the reference's window 5 (r = 2) has a compile-time-window instantiation: 5.1 against 7.2 us per
+                // 640x480 frame batched (DESIGN.md section 4.4)
+                if (radius == 2) mrf_kernel<2, kMrfTW, kMrfTH, C, DT><<<grd, kMrfTW * kMrfTH, smem, st>>>(p);
+                else mrf_kernel<-1, kMrfTW, kMrfTH, C, DT><<<grd, kMrfTW * kMrfTH, smem, st>>>(p);
+                CK(cudaGetLastError());
             }
-            CK(cudaGetLastError());
-        }
-        return KDME_OK;
+            return KDME_OK;
+        });
     });
 }
 
 extern "C" int jbf_mrf_batch(jbf_handle* h, const float* depth_dev, const uint8_t* bgr_dev, size_t bgr_step,
                              float* out_dev, int n_frames, int window_radius, float color_sigma, float smooth_sigma) {
-    return mrf_batch(h, depth_dev, nullptr, bgr_dev, bgr_step, out_dev, n_frames, window_radius, color_sigma,
+    return mrf_batch(h, {depth_dev, false}, bgr_dev, bgr_step, out_dev, n_frames, window_radius, color_sigma,
                      smooth_sigma, "jbf_mrf_batch");
 }
 
 extern "C" int jbf_mrf_batch_u16(jbf_handle* h, const uint16_t* depth_dev, const uint8_t* bgr_dev, size_t bgr_step,
                                  float* out_dev, int n_frames, int window_radius, float color_sigma,
                                  float smooth_sigma) {
-    return mrf_batch(h, nullptr, depth_dev, bgr_dev, bgr_step, out_dev, n_frames, window_radius, color_sigma,
+    return mrf_batch(h, {depth_dev, true}, bgr_dev, bgr_step, out_dev, n_frames, window_radius, color_sigma,
                      smooth_sigma, "jbf_mrf_batch_u16");
 }
 
 // The batch of one.
 extern "C" int jbf_mrf(jbf_handle* h, const float* depth_dev, const uint8_t* bgr_dev, size_t bgr_step, float* out_dev,
                        int window_radius, float color_sigma, float smooth_sigma) {
-    return mrf_batch(h, depth_dev, nullptr, bgr_dev, bgr_step, out_dev, 1, window_radius, color_sigma, smooth_sigma,
+    return mrf_batch(h, {depth_dev, false}, bgr_dev, bgr_step, out_dev, 1, window_radius, color_sigma, smooth_sigma,
                      "jbf_mrf");
 }
 
@@ -1438,11 +1442,10 @@ extern "C" int kdme_mean_3d_error(const float* points_dev, const float* truth_de
 }
 
 // ------------------------------------------------------------------ guided fill
-// One guided call over n_frames frames stored back to back.  The depth is exactly one of depth / depth16 (the fill:
-// width x height samples per frame) or depth_lo / depth_lo16 (the upsampling: wl x hl samples per frame).
+// One guided call over n_frames frames stored back to back: a fill (wl = hl = 0, width x height depth samples per
+// frame) or an upsampling (wl x hl samples per frame).
 struct GuidedCall {
-    const float* depth; const uint16_t* depth16;
-    const float* depth_lo; const uint16_t* depth_lo16; int wl, hl;
+    DepthIn depth; int wl, hl;
     const int32_t* labels; const uint8_t* bgr; size_t bgr_step;
     float* out; int width, height, n_frames, radius;
     float sigma_s, sigma_c, sigma_d;
@@ -1460,10 +1463,10 @@ static GuidedParams<WS_CT> guided_params(const GuidedCall& c) {
     GuidedParams<WS_CT> p;
     const long long plane = (long long)c.width * c.height;
     p.width = c.width; p.height = c.height;
-    p.depth = c.depth; p.depth16 = c.depth16; p.depth_lo = c.depth_lo; p.depth_lo16 = c.depth_lo16;
+    p.depth = c.depth.ptr;
     p.wl = c.wl; p.hl = c.hl;
     p.labels = c.labels; p.bgr = c.bgr; p.bgr_step = (long long)c.bgr_step; p.out = c.out;
-    p.depth_stride = (c.depth_lo || c.depth_lo16) ? (long long)c.wl * c.hl : plane;
+    p.depth_stride = (c.wl > 0) ? (long long)c.wl * c.hl : plane;
     p.bgr_stride = (long long)c.height * (long long)c.bgr_step;
     p.labels_stride = c.labels ? plane : 0;
     p.out_stride = plane;
@@ -1480,14 +1483,12 @@ static GuidedParams<WS_CT> guided_params(const GuidedCall& c) {
 // Launches `kernel` over the call's frames in slices of at most kMaxGridZ frames (blockIdx.z), in order on one
 // stream; each slice's pointers start at its first frame.
 template <class P>
-static int guided_slices(const P& p0, int n_frames, void (*kernel)(const P), size_t smem, cudaStream_t st) {
+static int guided_slices(const P& p0, DepthIn depth, int n_frames, void (*kernel)(const P), size_t smem,
+                         cudaStream_t st) {
     P p = p0;
     for (int f0 = 0; f0 < n_frames; f0 += kMaxGridZ) {
         const long long f = f0;
-        p.depth = advance(p0.depth, f * p0.depth_stride);
-        p.depth16 = advance(p0.depth16, f * p0.depth_stride);
-        p.depth_lo = advance(p0.depth_lo, f * p0.depth_stride);
-        p.depth_lo16 = advance(p0.depth_lo16, f * p0.depth_stride);
+        p.depth = depth.advance(f * p0.depth_stride).ptr;
         p.labels = advance(p0.labels, f * p0.labels_stride);
         p.bgr = p0.bgr + f * p0.bgr_stride;
         p.out = p0.out + f * p0.out_stride;
@@ -1504,9 +1505,10 @@ template <int WS_CT, int C>
 static int guided_launch(const GuidedCall& c, cudaStream_t stream) {
     const GuidedParams<WS_CT> p = guided_params<WS_CT>(c);
     const size_t smem = (WS_CT > 0) ? 0 : (size_t)(kGuidedTW + 2 * c.radius) * (kGuidedTH + 2 * c.radius) * 12;
-    if (c.depth16 || c.depth_lo16)
-        return guided_slices(p, c.n_frames, guided_fill_kernel<WS_CT, kGuidedTW, kGuidedTH, C, true>, smem, stream);
-    return guided_slices(p, c.n_frames, guided_fill_kernel<WS_CT, kGuidedTW, kGuidedTH, C, false>, smem, stream);
+    return with_depth_type(c.depth.u16, [&](auto dt) {
+        return guided_slices(p, c.depth, c.n_frames, guided_fill_kernel<WS_CT, kGuidedTW, kGuidedTH, C, decltype(dt)>,
+                             smem, stream);
+    });
 }
 
 // Windows 3..7 run the compile-time-window form, every other window the run-time one; both at any sigmas.
@@ -1520,11 +1522,10 @@ static int guided_launch_c(const GuidedCall& c, cudaStream_t stream) {
     }
 }
 
-// Every guided entry point: the checks in order, then the launch.  The call is a fill when its depth is depth or
-// depth16, an upsampling when it is depth_lo or depth_lo16; the other three are NULL.
-static int guided_batch(GuidedCall c, int channels, void* stream, const char* who) {
-    const void* lo = c.depth_lo ? (const void*)c.depth_lo : (const void*)c.depth_lo16;
-    const void* in = lo ? lo : c.depth ? (const void*)c.depth : (const void*)c.depth16;
+// Every guided entry point: the checks in order, then the launch.  `lo`: the call is an upsampling (else a fill, whose
+// wl = hl = 0).
+static int guided_batch(GuidedCall c, bool lo, int channels, void* stream, const char* who) {
+    const void* in = c.depth.ptr;
     if (!in || !c.bgr || !c.out) return fail(KDME_EINVAL, std::string(who) + ": NULL argument");
     if (c.n_frames < 1) return fail(KDME_EINVAL, std::string(who) + ": n_frames must be >= 1");
     if (!lo && (c.width <= 0 || c.height <= 0)) return fail(KDME_EINVAL, std::string(who) + ": bad size");
@@ -1532,8 +1533,7 @@ static int guided_batch(GuidedCall c, int channels, void* stream, const char* wh
         return fail(KDME_EINVAL, std::string(who) + ": low-res size must be positive and <= the high-res size");
     const unsigned long long plane = (unsigned long long)c.width * c.height;
     const unsigned long long in_samples = lo ? (unsigned long long)c.wl * c.hl : plane;
-    const size_t sample_bytes = (c.depth16 || c.depth_lo16) ? sizeof(uint16_t) : sizeof(float);
-    if (ranges_overlap(in, in_samples * c.n_frames * sample_bytes, c.out, plane * c.n_frames))
+    if (ranges_overlap(in, in_samples * c.n_frames * c.depth.sample_bytes(), c.out, plane * c.n_frames))
         return fail(KDME_EINVAL, std::string(who) + ": the output overlaps the depth input (in-place operation is not supported)");
     if (c.radius < 0 || c.radius > KDME_MAX_RADIUS) return fail(KDME_EINVAL, std::string(who) + ": bad radius");
     if (channels != KDME_GUIDE_GRAY && channels != KDME_GUIDE_BGR && channels != KDME_GUIDE_BGRX)
@@ -1547,27 +1547,27 @@ extern "C" int kdme_guided_fill_batch(const float* depth_dev, const int32_t* lab
                                       size_t bgr_step, int guide_channels, float* out_dev, int width, int height,
                                       int n_frames, int window_radius, float sigma_spatial, float sigma_color,
                                       float sigma_depth, void* stream) {
-    return guided_batch({depth_dev, nullptr, nullptr, nullptr, 0, 0, labels_dev, bgr_dev, bgr_step, out_dev, width,
+    return guided_batch({{depth_dev, false}, 0, 0, labels_dev, bgr_dev, bgr_step, out_dev, width,
                          height, n_frames, window_radius, sigma_spatial, sigma_color, sigma_depth},
-                        guide_channels, stream, "kdme_guided_fill_batch");
+                        /*lo=*/false, guide_channels, stream, "kdme_guided_fill_batch");
 }
 
 extern "C" int kdme_guided_fill_batch_u16(const uint16_t* depth_dev, const int32_t* labels_dev, const uint8_t* bgr_dev,
                                           size_t bgr_step, int guide_channels, float* out_dev, int width, int height,
                                           int n_frames, int window_radius, float sigma_spatial, float sigma_color,
                                           float sigma_depth, void* stream) {
-    return guided_batch({nullptr, depth_dev, nullptr, nullptr, 0, 0, labels_dev, bgr_dev, bgr_step, out_dev, width,
+    return guided_batch({{depth_dev, true}, 0, 0, labels_dev, bgr_dev, bgr_step, out_dev, width,
                          height, n_frames, window_radius, sigma_spatial, sigma_color, sigma_depth},
-                        guide_channels, stream, "kdme_guided_fill_batch_u16");
+                        /*lo=*/false, guide_channels, stream, "kdme_guided_fill_batch_u16");
 }
 
 extern "C" int kdme_guided_fill_ex(const float* depth_dev, const int32_t* labels_dev, const uint8_t* bgr_dev,
                                    size_t bgr_step, int guide_channels, float* out_dev, int width, int height,
                                    int window_radius, float sigma_spatial, float sigma_color, float sigma_depth,
                                    void* stream) {
-    return guided_batch({depth_dev, nullptr, nullptr, nullptr, 0, 0, labels_dev, bgr_dev, bgr_step, out_dev, width,
+    return guided_batch({{depth_dev, false}, 0, 0, labels_dev, bgr_dev, bgr_step, out_dev, width,
                          height, 1, window_radius, sigma_spatial, sigma_color, sigma_depth},
-                        guide_channels, stream, "kdme_guided_fill");
+                        /*lo=*/false, guide_channels, stream, "kdme_guided_fill");
 }
 
 extern "C" int kdme_guided_fill(const float* depth_dev, const int32_t* labels_dev, const uint8_t* bgr_dev,
@@ -1581,9 +1581,9 @@ extern "C" int kdme_guided_upsample_batch(const float* depth_lo_dev, int wl, int
                                           const uint8_t* bgr_hi_dev, size_t bgr_step, int guide_channels,
                                           float* out_hi_dev, int width, int height, int n_frames, int window_radius,
                                           float sigma_spatial, float sigma_color, float sigma_depth, void* stream) {
-    return guided_batch({nullptr, nullptr, depth_lo_dev, nullptr, wl, hl, labels_hi_dev, bgr_hi_dev, bgr_step, out_hi_dev,
+    return guided_batch({{depth_lo_dev, false}, wl, hl, labels_hi_dev, bgr_hi_dev, bgr_step, out_hi_dev,
                          width, height, n_frames, window_radius, sigma_spatial, sigma_color, sigma_depth},
-                        guide_channels, stream, "kdme_guided_upsample_batch");
+                        /*lo=*/true, guide_channels, stream, "kdme_guided_upsample_batch");
 }
 
 extern "C" int kdme_guided_upsample_batch_u16(const uint16_t* depth_lo_dev, int wl, int hl,
@@ -1591,18 +1591,18 @@ extern "C" int kdme_guided_upsample_batch_u16(const uint16_t* depth_lo_dev, int 
                                               int guide_channels, float* out_hi_dev, int width, int height,
                                               int n_frames, int window_radius, float sigma_spatial, float sigma_color,
                                               float sigma_depth, void* stream) {
-    return guided_batch({nullptr, nullptr, nullptr, depth_lo_dev, wl, hl, labels_hi_dev, bgr_hi_dev, bgr_step, out_hi_dev,
+    return guided_batch({{depth_lo_dev, true}, wl, hl, labels_hi_dev, bgr_hi_dev, bgr_step, out_hi_dev,
                          width, height, n_frames, window_radius, sigma_spatial, sigma_color, sigma_depth},
-                        guide_channels, stream, "kdme_guided_upsample_batch_u16");
+                        /*lo=*/true, guide_channels, stream, "kdme_guided_upsample_batch_u16");
 }
 
 extern "C" int kdme_guided_upsample_ex(const float* depth_lo_dev, int wl, int hl, const int32_t* labels_hi_dev,
                                        const uint8_t* bgr_hi_dev, size_t bgr_step, int guide_channels, float* out_hi_dev,
                                        int width, int height, int window_radius, float sigma_spatial, float sigma_color,
                                        float sigma_depth, void* stream) {
-    return guided_batch({nullptr, nullptr, depth_lo_dev, nullptr, wl, hl, labels_hi_dev, bgr_hi_dev, bgr_step, out_hi_dev,
+    return guided_batch({{depth_lo_dev, false}, wl, hl, labels_hi_dev, bgr_hi_dev, bgr_step, out_hi_dev,
                          width, height, 1, window_radius, sigma_spatial, sigma_color, sigma_depth},
-                        guide_channels, stream, "kdme_guided_upsample");
+                        /*lo=*/true, guide_channels, stream, "kdme_guided_upsample");
 }
 
 extern "C" int kdme_guided_upsample(const float* depth_lo_dev, int wl, int hl, const int32_t* labels_hi_dev,

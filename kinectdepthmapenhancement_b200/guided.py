@@ -5,12 +5,10 @@ from __future__ import annotations
 import torch
 
 from . import _lib
-from .jbf import _check_cuda, _ptr, guide_channels
+from .jbf import _check_cuda, _depth_entry, _ptr, guide_channels
 
 # EdgeRefinedSuperpixel.cpp:4-7
 WindowSize, SpatialSigma, ColorSigma, DepthSigma = 7, 30.0, 50.0, 70.0
-
-_DEPTH_DTYPES = (torch.float32, torch.uint16, torch.int16)
 
 
 def _one(t):
@@ -18,14 +16,14 @@ def _one(t):
     return None if t is None else t[None]
 
 
-def _batch_depth(depth: torch.Tensor, name: str) -> tuple:
-    """Checks a [N, rows, cols] float32 or uint16 depth batch (torch.uint16 or an int16 view of the same bits)."""
-    if depth.dtype not in _DEPTH_DTYPES:
-        raise TypeError(f"{name} must be a float32 or uint16 tensor, got {depth.dtype}")
+def _batch_depth(depth: torch.Tensor, name: str, entry: str) -> tuple:
+    """Checks a [N, rows, cols] float32 or uint16 depth batch (torch.uint16 or an int16 view of the same bits):
+    (`entry` for its dtype, its shape)."""
+    entry = _depth_entry(depth, name, entry)
     _check_cuda(depth, depth.dtype, name, depth.device)
     if depth.shape[0] < 1:
         raise ValueError(f"{name} must be [N, ...] with N >= 1, got {list(depth.shape)}")
-    return tuple(int(v) for v in depth.shape)
+    return entry, tuple(int(v) for v in depth.shape)
 
 
 def _batch_labels(labels: torch.Tensor | None, lead: tuple, dev, name: str):
@@ -64,13 +62,13 @@ def guided_fill(depth: torch.Tensor, color: torch.Tensor, labels: torch.Tensor |
 
 
 def _guided_fill_batch(depth, color, labels, window_radius, spatial_sigma, color_sigma, depth_sigma, out):
-    n, h, w = _batch_depth(depth, "depth")
+    entry, (n, h, w) = _batch_depth(depth, "depth", "kdme_guided_fill_batch")
     dev = depth.device
     _check_cuda(color, torch.uint8, "color", dev)
     c = guide_channels(color, (n, h, w))
     lab = _batch_labels(labels, (n, h, w), dev, "labels")
     out = _batch_out(out, (n, h, w), dev)
-    fn = _lib.lib().kdme_guided_fill_batch if depth.dtype == torch.float32 else _lib.lib().kdme_guided_fill_batch_u16
+    fn = getattr(_lib.lib(), entry)
     with torch.cuda.device(dev):
         _lib.check(fn(_ptr(depth), lab, _ptr(color), c * w, c, _ptr(out), w, h, n, window_radius, spatial_sigma,
                       color_sigma, depth_sigma, torch.cuda.current_stream().cuda_stream))
@@ -97,7 +95,7 @@ def guided_upsample(depth_lo: torch.Tensor, color_hi: torch.Tensor, labels_hi: t
 
 def _guided_upsample_batch(depth_lo, color_hi, labels_hi, window_radius, spatial_sigma, color_sigma, depth_sigma,
                            out):
-    n, hl, wl = _batch_depth(depth_lo, "depth_lo")
+    entry, (n, hl, wl) = _batch_depth(depth_lo, "depth_lo", "kdme_guided_upsample_batch")
     dev = depth_lo.device
     _check_cuda(color_hi, torch.uint8, "color_hi", dev)
     if color_hi.dim() not in (3, 4):
@@ -108,8 +106,7 @@ def _guided_upsample_batch(depth_lo, color_hi, labels_hi, window_radius, spatial
         raise ValueError(f"low-res size {wl}x{hl} must be positive and at most the high-res {w}x{h}")
     lab = _batch_labels(labels_hi, (n, h, w), dev, "labels_hi")
     out = _batch_out(out, (n, h, w), dev)
-    fn = (_lib.lib().kdme_guided_upsample_batch if depth_lo.dtype == torch.float32
-          else _lib.lib().kdme_guided_upsample_batch_u16)
+    fn = getattr(_lib.lib(), entry)
     with torch.cuda.device(dev):
         _lib.check(fn(_ptr(depth_lo), wl, hl, lab, _ptr(color_hi), c * w, c, _ptr(out), w, h, n, window_radius,
                       spatial_sigma, color_sigma, depth_sigma, torch.cuda.current_stream().cuda_stream))

@@ -17,6 +17,14 @@ def _ptr(t: torch.Tensor) -> int:
     return t.data_ptr()
 
 
+def _depth_entry(depth, name: str, entry: str) -> str:
+    """The library entry point for the depth tensor `name`: `entry` for float32 millimetres, `entry + "_u16"` for
+    uint16 millimetres (torch.uint16 or an int16 view of the same bits).  Any other dtype is a TypeError."""
+    if not isinstance(depth, torch.Tensor) or depth.dtype not in (torch.float32, torch.uint16, torch.int16):
+        raise TypeError(f"{name} must be a float32 or uint16 tensor, got {getattr(depth, 'dtype', type(depth))}")
+    return entry if depth.dtype == torch.float32 else entry + "_u16"
+
+
 def _check_cuda(t: torch.Tensor, dtype, name: str, device: torch.device):
     if not isinstance(t, torch.Tensor) or not t.is_cuda:
         raise TypeError(f"{name} must be a CUDA tensor (there is no CPU path)")
@@ -188,8 +196,7 @@ class JointBilateralFilter:
         sensor's format, read directly; torch.uint16 or a torch.int16 view of the same bits), color_hi
         [N, H, W, 3] u8 (or [N, H, W] / [N, H, W, 1] GRAY, [N, H, W, 4] BGRX) -> out [N, H, W] float32.  Frame k
         equals Upsampling of frame k alone, bit for bit."""
-        if not isinstance(depth_lo, torch.Tensor) or depth_lo.dtype not in (torch.float32, torch.uint16, torch.int16):
-            raise TypeError("depth_lo must be a float32 or uint16 tensor")
+        entry = _depth_entry(depth_lo, "depth_lo", "jbf_upsample_batch")
         _check_cuda(depth_lo, depth_lo.dtype, "depth_lo", self.device)
         _check_cuda(color_hi, torch.uint8, "color_hi", self.device)
         if depth_lo.dim() != 3 or depth_lo.shape[0] < 1:
@@ -203,15 +210,13 @@ class JointBilateralFilter:
         _check_cuda(out, torch.float32, "out", self.device)
         if tuple(out.shape) != (n, self.height, self.width):
             raise ValueError(f"out must be [{n}, {self.height}, {self.width}]")
-        fn = _lib.lib().jbf_upsample_batch if depth_lo.dtype == torch.float32 else _lib.lib().jbf_upsample_batch_u16
-        _lib.check(fn(self._h, _ptr(depth_lo), wl, hl, _ptr(color_hi), step, _ptr(out), n))
+        _lib.check(getattr(_lib.lib(), entry)(self._h, _ptr(depth_lo), wl, hl, _ptr(color_hi), step, _ptr(out), n))
         return out
 
     # -- batched / staged forms (B200-native additions) ----------------------
-    def _batch_args(self, depth: torch.Tensor, color: torch.Tensor, out: torch.Tensor | None):
-        """Checks of the process_batch forms: (N, guide step, u16?, out)."""
-        if not isinstance(depth, torch.Tensor) or depth.dtype not in (torch.float32, torch.uint16, torch.int16):
-            raise TypeError("depth must be a float32 or uint16 tensor")
+    def _batch_args(self, depth: torch.Tensor, color: torch.Tensor, out: torch.Tensor | None, entry: str):
+        """Checks of the process_batch forms: (N, guide step, the library's `entry` for depth's dtype, out)."""
+        entry = _depth_entry(depth, "depth", entry)
         _check_cuda(depth, depth.dtype, "depth", self.device)
         _check_cuda(color, torch.uint8, "color", self.device)
         if depth.dim() != 3 or tuple(depth.shape[1:]) != (self.height, self.width):
@@ -223,14 +228,13 @@ class JointBilateralFilter:
         _check_cuda(out, torch.float32, "out", self.device)
         if tuple(out.shape) != tuple(depth.shape):
             raise ValueError(f"out must be [{n}, {self.height}, {self.width}]")
-        return n, step, depth.dtype != torch.float32, out
+        return n, step, getattr(_lib.lib(), entry), out
 
     def process_batch(self, depth: torch.Tensor, color: torch.Tensor, out: torch.Tensor | None = None):
         """N independent frames: depth [N,H,W] float32 millimetres or uint16 millimetres (the sensor's format, read
         directly; torch.uint16 or a torch.int16 view of the same bits), color [N,H,W,3] u8 (or [N,H,W] / [N,H,W,1]
         GRAY, [N,H,W,4] BGRX) -> out [N,H,W] f32.  A uint16 frame filters bit for bit like its float32 image."""
-        n, step, u16, out = self._batch_args(depth, color, out)
-        fn = _lib.lib().jbf_process_batch_u16 if u16 else _lib.lib().jbf_process_batch
+        n, step, fn, out = self._batch_args(depth, color, out, "jbf_process_batch")
         _lib.check(fn(self._h, _ptr(depth), _ptr(color), step, _ptr(out), n))
         return out
 
@@ -239,14 +243,13 @@ class JointBilateralFilter:
         """process_batch + DimensionConvertor::projectiveToReal of every frame (main.cpp:179 + :182 over a stream):
         depth [N,H,W] float32 or uint16 millimetres -> (out [N,H,W] f32, xyz [N,H,W,3] f32).  Frame k of both equals
         process_xyz on frame k alone (the depth plane and the cloud), bit for bit."""
-        n, step, u16, out = self._batch_args(depth, color, out)
+        n, step, fn, out = self._batch_args(depth, color, out, "jbf_process_batch_xyz")
         if xyz is None:
             xyz = torch.empty((n, self.height, self.width, 3), dtype=torch.float32, device=self.device)
         _check_cuda(xyz, torch.float32, "xyz", self.device)
         if tuple(xyz.shape) != (n, self.height, self.width, 3):
             raise ValueError(f"xyz must be [{n}, {self.height}, {self.width}, 3]")
         self._keep = (depth, color)
-        fn = _lib.lib().jbf_process_batch_xyz_u16 if u16 else _lib.lib().jbf_process_batch_xyz
         _lib.check(fn(self._h, _ptr(depth), _ptr(color), step, _ptr(out), _ptr(xyz), n, float(fx), float(fy), int(cx),
                       int(cy)))
         return out, xyz
@@ -294,8 +297,7 @@ class JointBilateralFilter:
         """End-to-end with HOST tensors (ideally pinned, see host_buffer()): upload, Process, download;
         synchronous.  depth_host may be float32 millimetres or uint16 millimetres (the sensor's format,
         converted on the device)."""
-        if depth_host.dtype not in (torch.float32, torch.uint16, torch.int16):
-            raise TypeError("depth_host must be float32 or uint16")
+        entry = _depth_entry(depth_host, "depth_host", "jbf_process_host")
         for t, dt, nm in ((depth_host, depth_host.dtype, "depth_host"), (color_host, torch.uint8, "color_host"),
                           (out_host, torch.float32, "out_host")):
             if t.is_cuda or t.dtype != dt or not t.is_contiguous():
@@ -306,8 +308,7 @@ class JointBilateralFilter:
         if tuple(out_host.shape) != (n, self.height, self.width):
             raise ValueError(f"out_host must be [{n}, {self.height}, {self.width}]")
         step = self._use_guide(color_host, (n, self.height, self.width), "color_host")
-        fn = _lib.lib().jbf_process_host if depth_host.dtype == torch.float32 else _lib.lib().jbf_process_host_u16
-        _lib.check(fn(self._h, _ptr(depth_host), _ptr(color_host), step, _ptr(out_host), n))
+        _lib.check(getattr(_lib.lib(), entry)(self._h, _ptr(depth_host), _ptr(color_host), step, _ptr(out_host), n))
         return out_host
 
     def mrf(self, depth: torch.Tensor, color: torch.Tensor, window_radius=2, color_sigma=50.0, smooth_sigma=150.0,
@@ -320,12 +321,10 @@ class JointBilateralFilter:
             _check_cuda(depth, torch.float32, "depth", self.device)
             if out is not None and out.dim() == 2:
                 out = out[None]
-            _, step, _, out = self._batch_args(depth[None], color[None], out)
-            _lib.check(_lib.lib().jbf_mrf(self._h, _ptr(depth), _ptr(color), step, _ptr(out), window_radius,
-                                          color_sigma, smooth_sigma))
+            _, step, fn, out = self._batch_args(depth[None], color[None], out, "jbf_mrf")   # float32: jbf_mrf
+            _lib.check(fn(self._h, _ptr(depth), _ptr(color), step, _ptr(out), window_radius, color_sigma, smooth_sigma))
             return out[0]
-        n, step, u16, out = self._batch_args(depth, color, out)
-        fn = _lib.lib().jbf_mrf_batch_u16 if u16 else _lib.lib().jbf_mrf_batch
+        n, step, fn, out = self._batch_args(depth, color, out, "jbf_mrf_batch")
         _lib.check(fn(self._h, _ptr(depth), _ptr(color), step, _ptr(out), n, window_radius, color_sigma, smooth_sigma))
         return out
 
